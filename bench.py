@@ -2,6 +2,7 @@
 """Headline benchmark: Newton-solved sweep states per second (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--instances I] [--impl reference] [--single-process]
+                    [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[2], the configuration the metric's target is quoted on):
 mirrored double-wishbone axle with pushrod-rocker coilovers and U-bar ARB (reference
@@ -281,22 +282,23 @@ def run_reference(args) -> None:
     worker = cpu_worker()
     kind, what = cpu_kind()
     # warm-up (imports, process pool start) then K timed steps of `per_step` instances each
+    warmup = min(args.warmup, 1)              # one warm-up step is enough for a CPU pool
     times, solved, solve_s = [], 0, 0.0
     import multiprocessing as mp
     with mp.get_context("spawn").Pool(cores) as pool:
-        for step in range(args.warmup + args.steps):
+        for step in range(warmup + args.steps):
             seeds = [(5000 + step * per_step + i,) for i in range(per_step)]
             t0 = time.perf_counter()
             recs = pool.map(worker, seeds, chunksize=1)
             dt = time.perf_counter() - t0
-            if step >= min(args.warmup, 1):   # one warm-up step is enough for a CPU pool
+            if step >= warmup:
                 times.append(dt)
                 solved += sum(r[0] for r in recs)
                 solve_s += sum(r[2] for r in recs)
     value = solved / sum(times)
     line = {
         "impl": "reference", "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": args.gpus,
-        "steps": args.steps, "warmup": args.warmup, "ms_per_step": 1e3 * float(np.mean(times)),
+        "steps": args.steps, "warmup": warmup, "ms_per_step": 1e3 * float(np.mean(times)),
         "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f64", "data": "synthetic",
         "config": {"workload": WORKLOAD, "instances_per_step": per_step, "sweep_steps": N_STEPS_SWEEP,
                    "sigma_mm": SIGMA_MM},
@@ -334,6 +336,28 @@ def parity_check(solver) -> dict:
                 np.array_equal(res.status, arr["status"]) and np.array_equal(res.failed_step, arr["failed_step"])),
             "parity_source": "tests/golden/batch256_c3 (reference tight run), steps "
                              + str([int(v) for v in arr["steps"]])}
+
+
+DUMP_BYTES = 60_000_000     # --dump-outputs stays below 64 MB in all
+
+
+def dump_outputs(out_dir: str, t: dict) -> None:
+    """Write the outputs of the device-resident path's last launch as float64 ``.npy`` files: all
+    instances if they fit in DUMP_BYTES, else a fixed seeded sample of instances (sorted; their
+    indices in ``instance_index.npy``).  The inputs are seeded, so two builds run with the same
+    arguments can be compared file for file."""
+    import torch
+    names = {"positions": "pos", "status": "status", "failed_step": "failed", "iters": "iters",
+             "max_residual": "maxres"}
+    n_inst = t["pos"].shape[0]
+    per_inst = 8 * (1 + sum(t[key][0].numel() for key in names.values()))
+    k = min(n_inst, DUMP_BYTES // per_inst)
+    index = np.sort(np.random.default_rng(0).choice(n_inst, k, replace=False)) if k < n_inst else np.arange(n_inst)
+    rows = torch.from_numpy(index).to(t["pos"].device)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "instance_index.npy"), index.astype(np.float64))
+    for name, key in names.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t[key][rows].double().cpu().numpy())
 
 
 def moving_point_keys(solver) -> list:
@@ -437,6 +461,8 @@ def run_cuda(args) -> None:
     clocks = sampler.stop() if rank == 0 else None
 
     first = sets[devices[0]]
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, first)
     status_np, failed_np = first["status"].cpu().numpy(), first["failed"].cpu().numpy()
     ok_frac = float((status_np == 0).mean())
     solved_frac = accepted_states(status_np, failed_np, S) / float(n_inst * S)
@@ -456,7 +482,7 @@ def run_cuda(args) -> None:
     for k, index in enumerate(devices):
         lo, hi = k * per, min((k + 1) * per, e2e_inst)
         host_hp[lo:hi] = sets[index]["hp"][: hi - lo].cpu().numpy()
-    e2e_steps = max(2, min(args.steps, 5))
+    e2e_steps = args.steps
 
     def time_e2e(label, slv, rows, **want):
         """K calls of BatchSolver.solve on the same page-locked buffers (allocated by the first call)."""
@@ -593,7 +619,14 @@ def main() -> None:
     ap.add_argument("--single-process", action="store_true",
                     help="with --gpus N > 1 and no torchrun: one process drives all N devices")
     ap.add_argument("--e2e-all-points-only", action="store_true", help="skip the packed / metrics-only e2e variants")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the outputs of the last device-resident launch "
+                         "(rank 0, first device) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl cuda)")
     if args.impl == "reference":
         run_reference(args)
     else:
