@@ -1765,48 +1765,137 @@ OKIN_FN double okin_scale_norm2(const OkinProgram& pr, double* sm, double* v, do
   return okin_red_sum(red);
 }
 
+// a . b (warp-uniform).
+template <typename Dummy = void>
+OKIN_FN double okin_dot(const OkinProgram& pr, double* sm, const double* a, const double* b) {
+  sm = OKIN_SHARED(sm);
+  const int n = 3 * pr.hdr[OKIN_H_NF];
+  double* red = sm + pr.hdr[OKIN_H_OFF_RED];
+  OKIN_PHASE_BEGIN
+  double acc = 0.0;
+  OKIN_LANE_LOOP
+  for (int u = lane; u < n; u += 32) acc += a[u] * b[u];
+  red[lane] = acc;
+  OKIN_PHASE_END
+  return okin_red_sum(red);
+}
+
+template <typename Dummy = void>
+OKIN_FN void okin_copy(const OkinProgram& pr, double* dst, const double* src) {
+  const int n = 3 * pr.hdr[OKIN_H_NF];
+  OKIN_PHASE_BEGIN
+  OKIN_LANE_LOOP
+  for (int u = lane; u < n; u += 32) dst[u] = src[u];
+  OKIN_PHASE_END
+}
+
+struct OkinGram2 { double aa, ab, bb; };
+
+// Gram-Schmidt on the pair {a, b} in place; returns their Gram matrix from before.
+template <typename Dummy = void>
+OKIN_FN OkinGram2 okin_orthonormalise2(const OkinProgram& pr, double* sm, double* a, double* b) {
+  sm = OKIN_SHARED(sm);
+  const int n = 3 * pr.hdr[OKIN_H_NF];
+  double* red = sm + pr.hdr[OKIN_H_OFF_RED];
+  OkinGram2 g;
+  g.aa = okin_dot(pr, sm, a, a);
+  g.ab = okin_dot(pr, sm, a, b);
+  const double p = g.ab / g.aa, s = 1.0 / sqrt(g.aa);
+  OKIN_PHASE_BEGIN
+  double acc = 0.0;
+  OKIN_LANE_LOOP
+  for (int u = lane; u < n; u += 32) {
+    const double w = b[u] - p * a[u];
+    b[u] = w;
+    a[u] *= s;
+    acc += w * w;
+  }
+  red[lane] = acc;
+  OKIN_PHASE_END
+  const double bb = okin_red_sum(red);
+  g.bb = bb + p * g.ab;
+  okin_scale_norm2(pr, sm, b, 1.0 / sqrt(bb));
+  return g;
+}
+
+// Largest eigenvalue of the symmetric [[a, b], [b, d]] and its unit eigenvector (c0, c1).
+OKIN_HD double okin_sym2_top(double a, double b, double d, double* c0, double* c1) {
+  const double h = 0.5 * (a - d), r = sqrt(h * h + b * b);
+  const double u = h >= 0.0 ? h + r : b, v = h >= 0.0 ? b : r - h;   // (t - d, b) or (b, t - a)
+  const double nrm = sqrt(u * u + v * v);
+  *c0 = nrm > 0.0 ? u / nrm : 1.0;
+  *c1 = nrm > 0.0 ? v / nrm : 0.0;
+  return 0.5 * (a + d) + r;
+}
+
 // Numerical health of the tangent system at the current factorisation (TangentSolveInfo,
 // sensitivity.py:42-55, :97-113): the extreme singular values of the pinned Jacobian are the
-// square roots of the extreme eigenvalues of A = L L^T.  sigma_max by power iteration with the
-// factor, sigma_min by inverse iteration with the triangular solves; both are read off as
-// Rayleigh quotients x^T A x = |L^T x|^2, so they are estimates from inside (sigma_max from
-// below, sigma_min from above) whose error is quadratic in the eigenvector error.
+// square roots of the extreme eigenvalues of A = L L^T.  sigma_max by subspace iteration with
+// A (the factor), sigma_min by subspace iteration with A^{-1} (the triangular solves), each on
+// two vectors with a Rayleigh-Ritz step: the extreme eigenvalues of the shipped mechanisms come
+// in near-degenerate pairs (left / right of an axle: 2e-5 .. 2e-2 apart), which a single vector
+// separates only over thousands of steps, while two vectors span the pair and converge at the
+// ratio to the third eigenvalue.  The Ritz values are estimates from inside (sigma_max from
+// below, sigma_min from above).  Each iteration stops once the residual of its top Ritz pair
+// (theta, u), |B u - theta u|^2 = |B u|^2 - theta^2 (B = A or A^{-1}), is below
+// OKIN_HEALTH_TOL * theta: an eigenvalue of B then lies within that distance of theta, so the
+// eigenvalue error is at most OKIN_HEALTH_TOL relative however close its neighbours are.
 // out2 = {sigma_min, sigma_max / sigma_min}.  Scratch: the row-gradient storage (dead until the
-// next row evaluation) and vec[0].
-#define OKIN_HEALTH_ITERS 24
+// next row evaluation; two vectors) and vec[0] (staging of one vector).
+#define OKIN_HEALTH_TOL 1e-5
+#define OKIN_HEALTH_MAX_ITERS 200
 template <typename Dummy = void>
 OKIN_FN void okin_tangent_health(const OkinProgram& pr, double* sm, bool notpd, double* out2) {
   sm = OKIN_SHARED(sm);
   const int32_t* hdr = OKIN_SHARED(pr.hdr);
   const int n = 3 * hdr[OKIN_H_NF];
-  double* x = sm + hdr[OKIN_H_OFF_RG];
-  double* z = x + n;
+  double* x1 = sm + hdr[OKIN_H_OFF_RG];
+  double* x2 = x1 + n;
   double* v0 = sm + hdr[OKIN_H_OFF_VEC];
-  OKIN_PHASE_BEGIN
-  OKIN_LANE_LOOP
-  for (int u = lane; u < n; u += 32) {
-    // deterministic start vectors: positive for the dominant direction, signed for the weakest
-    const uint32_t hsh = ((uint32_t)u + 1u) * 2654435761u;
-    x[u] = 1.0 + 0.37 * (double)((hsh >> 16) & 0xffu) / 256.0;
-    v0[u] = (double)((hsh >> 12) & 0xffffu) / 65536.0 - 0.5;
+  const double tol2 = OKIN_HEALTH_TOL * OKIN_HEALTH_TOL;
+  double theta[2] = {0.0, 0.0};     // top Ritz values of A and of A^{-1}
+  for (int inverse = 0; inverse < 2 && !notpd; ++inverse) {
+    OKIN_PHASE_BEGIN
+    OKIN_LANE_LOOP
+    for (int u = lane; u < n; u += 32) {
+      // deterministic start vectors: one positive, one signed
+      const uint32_t hsh = ((uint32_t)u + 1u) * 2654435761u;
+      x1[u] = 1.0 + 0.37 * (double)((hsh >> 16) & 0xffu) / 256.0;
+      x2[u] = (double)((hsh >> 12) & 0xffffu) / 65536.0 - 0.5;
+    }
+    OKIN_PHASE_END
+    double th = 0.0, c0 = 1.0, c1 = 0.0;
+    for (int it = 0; it < OKIN_HEALTH_MAX_ITERS; ++it) {
+      // {x1, x2} = B X of the previous iteration: its Gram matrix gives |B u|^2 = c^T G c
+      const OkinGram2 g = okin_orthonormalise2(pr, sm, x1, x2);
+      if (it > 0) {
+        const double r2 = c0 * c0 * g.aa + 2.0 * c0 * c1 * g.ab + c1 * c1 * g.bb - th * th;
+        if (!(r2 > tol2 * th * th)) break;   // (NaN stops too)
+      }
+      double h11, h12, h22;     // X^T B X, with X <- B X in place
+      if (!inverse) {
+        h11 = okin_factor_multiply(pr, sm, x1, v0, true);     // |L^T x1|^2
+        okin_factor_multiply(pr, sm, v0, x1, false);          // x1 <- A x1
+        h12 = okin_dot(pr, sm, x1, x2);
+        h22 = okin_factor_multiply(pr, sm, x2, v0, true);
+        okin_factor_multiply(pr, sm, v0, x2, false);
+      } else {
+        okin_copy(pr, v0, x1);
+        okin_solve(pr, sm, 0, 1, false);                      // v0 <- A^{-1} x1
+        h11 = okin_dot(pr, sm, x1, v0);
+        h12 = okin_dot(pr, sm, x2, v0);
+        okin_copy(pr, x1, v0);
+        okin_copy(pr, v0, x2);
+        okin_solve(pr, sm, 0, 1, false);
+        h22 = okin_dot(pr, sm, x2, v0);
+        okin_copy(pr, x2, v0);
+      }
+      th = okin_sym2_top(h11, h12, h22, &c0, &c1);
+    }
+    theta[inverse] = th;
   }
-  OKIN_PHASE_END
-  double smax2 = 0.0;
-  double nx = okin_scale_norm2(pr, sm, x, 1.0);
-  for (int it = 0; it < OKIN_HEALTH_ITERS; ++it) {
-    okin_scale_norm2(pr, sm, x, 1.0 / sqrt(nx));
-    smax2 = okin_factor_multiply(pr, sm, x, z, true);    // Rayleigh quotient of A at x
-    nx = okin_factor_multiply(pr, sm, z, x, false);      // x <- A x
-  }
-  double nv = okin_scale_norm2(pr, sm, v0, 1.0);
-  for (int it = 0; it < OKIN_HEALTH_ITERS; ++it) {
-    okin_scale_norm2(pr, sm, v0, 1.0 / sqrt(nv));
-    okin_solve(pr, sm, 0, 1, false);                      // v0 <- A^{-1} v0
-    nv = okin_scale_norm2(pr, sm, v0, 1.0);
-  }
-  okin_scale_norm2(pr, sm, v0, 1.0 / sqrt(nv));
-  const double smin2 = okin_factor_multiply(pr, sm, v0, z, true);
-  const bool good = !notpd && smin2 == smin2 && smin2 > 0.0 && smax2 == smax2;
+  const double smax2 = theta[0], smin2 = 1.0 / theta[1];
+  const bool good = !notpd && smin2 == smin2 && smin2 > 0.0 && smin2 < INFINITY && smax2 == smax2;
   OKIN_PHASE_BEGIN
   if (lane == 0) {
     out2[0] = good ? sqrt(smin2) : 0.0;

@@ -76,11 +76,11 @@ def test_point_velocities_and_tangent_health_match_reference(case):
     order = [prog.out_keys.index(key_from_name(n)) for n in meta["point_keys"]]
     vel = out["velocities"][0][:, :, order]
     assert np.abs(vel - arr["velocities"]).max() <= 1e-7 * max(1.0, np.abs(arr["velocities"]).max())
-    # Power / inverse iteration approach the extreme singular values from inside (the 1e-5 slack:
-    # the reference keeps the zero-gradient point-on-line rows next to their pins).
+    # Within 1e-5 relative: the bound okin_tangent_health's stopping rule guarantees (the states
+    # themselves differ from the reference's by up to 1e-6 mm).
     smin, cond = out["tangent_health"][0, :, 0], out["tangent_health"][0, :, 1]
-    assert (smin >= arr["tangent_sigma_min"] * (1 - 1e-5)).all() and (smin <= arr["tangent_sigma_min"] * 1.05).all()
-    assert (cond <= arr["tangent_cond"] * (1 + 1e-5)).all() and (cond >= arr["tangent_cond"] * 0.9).all()
+    assert np.abs(smin / arr["tangent_sigma_min"] - 1).max() <= 1e-5
+    assert np.abs(cond / arr["tangent_cond"] - 1).max() <= 1e-5
 
 
 def test_predictor_does_not_change_the_answer():
