@@ -66,6 +66,14 @@
  *   instance_targets [n_instances][n_targets][n_steps] per-instance sweep tables (Monte Carlo over the sweep
  *                                                    itself; SURVEY.md section 8b); when given it replaces the
  *                                                    shared target_values
+ *   hardpoint_sensitivity [n_instances][n_steps][n_sens][n_out_points*3]  d position / d hardpoint
+ *                                                    coordinate: row k is the coordinate the topology lists
+ *                                                    k-th among its sensitivity inputs (3 * input slot + axis),
+ *                                                    params held fixed.  Free points: the Gauss-Newton
+ *                                                    sensitivity -A^-1 J^T dR/dp_k with the factor the tangents
+ *                                                    use; fixed points: e_k; derived points: through their op.
+ *                                                    NaN after a failed step.  Not available on a topology
+ *                                                    with camber-shim records (OKIN_ERR_USAGE)
  *   status_out      [n_instances]                    OKIN_STATUS_*
  *   failed_step_out [n_instances]                    -1 or the first failed step
  *   worst_row_out   [n_instances]                    device row owning max|r| at the failed step, -1 when the
@@ -150,6 +158,7 @@ typedef struct okin_batch_io {
   double* jumps;
   const double* instance_targets; /* optional [n_instances][n_targets][n_steps]; replaces target_values */
   int32_t* worst_row;             /* optional [n_instances] */
+  double* hardpoint_sensitivity;  /* optional [n_instances][n_steps][n_sens][n_out_points*3] */
 } okin_batch_io;
 
 int okin_device_count(int* out);

@@ -43,12 +43,12 @@ class BatchIO(ctypes.Structure):
 
     INPUTS = ("hardpoints", "params", "target_values", "instance_targets")
     OUTPUTS = ("status", "failed_step", "positions", "iters", "max_residual", "tangents", "velocities",
-               "tangent_health", "metrics", "design", "diagnostics", "jumps", "worst_row")
+               "tangent_health", "metrics", "design", "diagnostics", "jumps", "worst_row", "hardpoint_sensitivity")
     # field order of the C struct (include/okin.h)
     _fields_ = [(n, ctypes.c_void_p) for n in (
         "hardpoints", "params", "target_values", "status", "failed_step", "positions", "iters", "max_residual",
         "tangents", "velocities", "tangent_health", "metrics", "design", "diagnostics", "jumps",
-        "instance_targets", "worst_row")]
+        "instance_targets", "worst_row", "hardpoint_sensitivity")]
 
     @classmethod
     def of(cls, **buffers) -> "BatchIO":
@@ -238,12 +238,15 @@ class DeviceTopology:
                     devices=None, want_positions=True, want_tangents=False, want_metrics=False,
                     want_design=False, params: np.ndarray | None = None, want_velocities=False,
                     want_health=False, want_diagnostics=False, instance_targets: np.ndarray | None = None,
-                    want_worst_row=False, out: dict | None = None, pinned: bool = False) -> dict:
+                    want_worst_row=False, out: dict | None = None, pinned: bool = False,
+                    want_hardpoint_sensitivity=False) -> dict:
         """hardpoints [n_inst, n_in*3]; target_values [n_targets, n_steps];
         instance_targets optional [n_inst, n_targets, n_steps] (replaces target_values).
         ``out``: a dict returned by an earlier call; arrays of matching shape are overwritten instead
         of allocated (the way to reuse page-locked buffers).  ``pinned``: allocate what is missing in
-        page-locked memory next to the first device."""
+        page-locked memory next to the first device.  ``want_hardpoint_sensitivity``: d position /
+        d hardpoint coordinate ``[n_inst, n_steps, n_sens, n_out, 3]``, rows in the order of
+        ``program.sensitivity_inputs`` (not on a topology with camber-shim records)."""
         require_device()
         prog = self.program
         hp = np.ascontiguousarray(hardpoints, dtype=np.float64)
@@ -293,6 +296,8 @@ class DeviceTopology:
             "diagnostics": buf("diagnostics", want_diagnostics, (n_inst, n_steps, len(prog.diagnostic_names))),
             "jumps": buf("jumps", want_diagnostics, (n_inst, n_steps, prog.n_unknowns // 3)),
             "worst_row": buf("worst_row", want_worst_row, (n_inst,), np.int32),
+            "hardpoint_sensitivity": buf("hardpoint_sensitivity", want_hardpoint_sensitivity,
+                                         (n_inst, n_steps, len(prog.sensitivity_inputs), prog.n_out, 3)),
         }
         if want_diagnostics and not prog.diagnostic_names:
             raise ValueError("This topology was compiled without a diagnostic program")

@@ -118,3 +118,14 @@ def compute_state_tangents(state: SuspensionState, constraints: list, derived_ma
     fields = fields_from_velocities(out["velocities"][0, 0], list(step_targets), program.out_keys)
     info = solve_info_from_health(out["tangent_health"][0, 0], program.n_unknowns, program.stats["n_rows"])
     return fields, info
+
+
+def linearised_std(hardpoint_sensitivity: np.ndarray, sigma) -> np.ndarray:
+    """First-order standard deviation of every output coordinate, ``[n, n_steps, n_out, 3]``, for
+    independent hardpoint coordinates with standard deviations ``sigma`` (a scalar or one value per
+    sensitivity row): ``sqrt(sum_k S_k^2 sigma_k^2)`` over the rows ``S_k`` of
+    ``BatchSweepResult.hardpoint_sensitivity`` ``[n, n_steps, n_sens, n_out, 3]``.  Valid while the
+    tolerances are small against the curvature of the response (no second-order terms)."""
+    s = np.asarray(hardpoint_sensitivity, dtype=np.float64)
+    sig = np.broadcast_to(np.asarray(sigma, dtype=np.float64), (s.shape[2],))
+    return np.sqrt(np.einsum("nsk...,k->ns...", s * s, sig * sig))

@@ -58,11 +58,16 @@ class BatchSweepResult:
     jumps: np.ndarray | None = None            # [n_instances, n_steps, n_free]; row 0 = thresholds
     worst_row: np.ndarray | None = None        # [n_instances] device row owning max|r| at the failed step, or -1
     design: np.ndarray | None = None           # [n_instances, n_out_points, 3] design (setup) pose
+    # [n_instances, n_steps, n_sens, n_out_points, 3] d position / d hardpoint coordinate; row k is
+    # ``sensitivity_inputs[k]`` = (input point key, axis)
+    hardpoint_sensitivity: np.ndarray | None = None
+    sensitivity_inputs: list | None = None
 
     _BUFFERS = (("positions", "positions"), ("status", "status"), ("failed_step", "failed_step"), ("nfev", "iters"),
                 ("max_residual", "max_residual"), ("tangents", "tangents"), ("metrics", "metrics"),
                 ("velocities", "velocities"), ("tangent_health", "tangent_health"), ("diagnostics", "diagnostics"),
-                ("jumps", "jumps"), ("worst_row", "worst_row"), ("design", "design"))
+                ("jumps", "jumps"), ("worst_row", "worst_row"), ("design", "design"),
+                ("hardpoint_sensitivity", "hardpoint_sensitivity"))
 
     def buffers(self) -> dict:
         """The arrays keyed like ``DeviceTopology.solve_batch``'s result (for ``solve(out=...)`` reuse)."""
@@ -100,10 +105,12 @@ class BatchSolver:
     the device from that instance's hardpoints (reference recomputes them in
     ``Suspension.constraints()``, core/sweep.py:58-63)."""
 
-    def __init__(self, suspension, sweep_config: SweepConfig, output_points=None, tune_layout: bool = False):
+    def __init__(self, suspension, sweep_config: SweepConfig, output_points=None, tune_layout: bool = False,
+                 sensitivity_inputs=None):
         """``tune_layout``: spend a few seconds at compile time placing the factor blocks so that the
         kernel's shared-memory accesses hit fewer bank conflicts (core/layout_tuning.py); worth it for
-        large batches, results are unchanged."""
+        large batches, results are unchanged.  ``sensitivity_inputs``: the ``(input point key, axis)``
+        hardpoint coordinates ``solve(want_hardpoint_sensitivity=True)`` differentiates by (default all)."""
         validate_sweep_controls(sweep_config, suspension.actuator_dofs())
         self.suspension = suspension
         self.heads, self.values = sweep_target_values(sweep_config)
@@ -111,16 +118,28 @@ class BatchSolver:
         from .metrics_program import build_metric_program
         from .shim_program import shim_records
         state, constraints = suspension.structure()
-        self.program = compile_topology(
-            state, constraints, suspension.derived_spec(), self.heads,
-            output_points=output_points, design_rules=True,
-            metrics=(lambda pidx: build_metric_program(suspension, self.heads, pidx))
-            if suspension.config is not None else None,
-            shims=shim_records(suspension),
-            diagnostics=lambda pidx, design_pts: build_diagnostic_program(suspension, pidx, design_pts),
-            tune_layout=tune_layout,
-        )
+
+        def compile_with(shims):
+            return compile_topology(
+                state, constraints, suspension.derived_spec(), self.heads,
+                output_points=output_points, design_rules=True,
+                metrics=(lambda pidx: build_metric_program(suspension, self.heads, pidx))
+                if suspension.config is not None else None,
+                shims=shims,
+                diagnostics=lambda pidx, design_pts: build_diagnostic_program(suspension, pidx, design_pts),
+                tune_layout=tune_layout, sensitivity_inputs=sensitivity_inputs,
+            )
+
+        shims = shim_records(suspension)
+        self.program = compile_with(shims)
         self.topology = _lib.DeviceTopology(self.program)
+        # Hardpoint sensitivities do not differentiate the camber-shim pre-solve.  A shim at its design
+        # thickness leaves the design pose as authored (okin_shim_presolve skips a thickness change below
+        # OKIN_GEOM_EPS = 1e-6 mm), so such a model is solved for sensitivities by the same topology without
+        # its shim records.
+        self._sens_shims_inactive = all(abs(sh["params"][9] - sh["params"][10]) < 1e-6 for sh in shims)
+        self._compile_without_shims = lambda: compile_with(None)
+        self._sens_topology = None
 
     def nominal_hardpoints(self) -> np.ndarray:
         """Authored positions of the input points, shape ``[n_in*3]`` (input slot order)."""
@@ -147,7 +166,8 @@ class BatchSolver:
               want_metrics: bool = False, params: np.ndarray | None = None, want_velocities: bool = False,
               want_health: bool = False, want_diagnostics: bool = False, want_design: bool = False,
               want_worst_row: bool = False, instance_targets: np.ndarray | None = None,
-              out: BatchSweepResult | None = None, pinned: bool = False) -> BatchSweepResult:
+              out: BatchSweepResult | None = None, pinned: bool = False,
+              want_hardpoint_sensitivity: bool = False) -> BatchSweepResult:
         """``params``: optional ``[n_instances, n_params]`` per-instance scalars in the order of
         ``program.param_names`` (camber-shim datums and thicknesses); default = the model's.
         ``instance_targets``: optional ``[n_instances, n_targets, n_steps]`` per-instance sweep tables
@@ -155,21 +175,34 @@ class BatchSolver:
         ``devices``: CUDA device ids; the instance range is split evenly over them.
         ``out``: an earlier result of the same shape whose arrays are overwritten (no allocation);
         ``pinned``: allocate result arrays in page-locked host memory (slow to allocate, fast to fill:
-        keep the result and pass it back as ``out``)."""
+        keep the result and pass it back as ``out``).
+        ``want_hardpoint_sensitivity``: d position / d hardpoint coordinate of every output point at every
+        state (``hardpoint_sensitivity``, rows named by ``sensitivity_inputs``), params held fixed; see
+        DESIGN.md.  Not available with active camber shims (ValueError)."""
         cfg = _lib.default_cfg(residual_tol=float(solver_config.residual_tolerance))
         hp = np.asarray(hardpoints, dtype=np.float64)
         hp = hp.reshape(hp.shape[0], -1)
-        res = self.topology.solve_batch(hp, self.values, cfg, devices=devices,
+        topology = self.topology
+        if want_hardpoint_sensitivity and self.program.param_names:
+            if params is not None or not self._sens_shims_inactive:
+                raise ValueError("Hardpoint sensitivities are not available with camber shims away from their "
+                                 "design thickness (the shim pre-solve is not differentiated)")
+            if self._sens_topology is None:
+                self._sens_topology = _lib.DeviceTopology(self._compile_without_shims())
+            topology = self._sens_topology
+        res = topology.solve_batch(hp, self.values, cfg, devices=devices,
                                         want_positions=want_positions, want_tangents=want_tangents,
                                         want_metrics=want_metrics, params=params,
                                         want_velocities=want_velocities, want_health=want_health,
                                         want_diagnostics=want_diagnostics, want_design=want_design,
                                         want_worst_row=want_worst_row, instance_targets=instance_targets,
-                                        out=out.buffers() if out is not None else None, pinned=pinned)
+                                        out=out.buffers() if out is not None else None, pinned=pinned,
+                                        **({"want_hardpoint_sensitivity": True} if want_hardpoint_sensitivity else {}))
         return BatchSweepResult(self.program, res["positions"], res["status"], res["failed_step"],
                                 res["iters"], res["max_residual"], res["tangents"], res["metrics"],
                                 res["velocities"], res["tangent_health"], res["diagnostics"], res["jumps"],
-                                res.get("worst_row"), res.get("design"))
+                                res.get("worst_row"), res.get("design"), res.get("hardpoint_sensitivity"),
+                                list(self.program.sensitivity_inputs) if want_hardpoint_sensitivity else None)
 
     def pinned_hardpoints(self, n_instances: int, device: int = 0) -> np.ndarray:
         """Page-locked ``[n_instances, n_in*3]`` input array (fill it, pass it to ``solve``)."""
@@ -177,6 +210,8 @@ class BatchSolver:
 
     def close(self) -> None:
         self.topology.close()
+        if self._sens_topology is not None:
+            self._sens_topology.close()
 
 
 def solve_sweep_batch(suspension, sweep_config: SweepConfig, hardpoints: np.ndarray, **kwargs) -> BatchSweepResult:

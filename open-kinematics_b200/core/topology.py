@@ -129,6 +129,7 @@ class TopologyProgram:
     diagnostic_checks: list = field(default_factory=list)
     param_names: list = field(default_factory=list)
     param_default: np.ndarray = field(default_factory=lambda: np.zeros(0))
+    sensitivity_inputs: list = field(default_factory=list)   # (input point key, axis) per sensitivity row
 
     @property
     def n_unknowns(self) -> int:
@@ -291,6 +292,7 @@ def compile_topology(
     shims=None,
     diagnostics=None,
     tune_layout: bool = False,
+    sensitivity_inputs=None,
 ) -> TopologyProgram:
     """Compile one topology.
 
@@ -299,6 +301,8 @@ def compile_topology(
     recompute every design constant from each instance's own hardpoints (batch
     use); ``False`` bakes the explicit constants of the given constraint objects
     (the single-instance ``solve_suspension_sweep`` boundary).
+    ``sensitivity_inputs``: the ``(input point key, axis)`` hardpoint coordinates whose sensitivities
+    the device reports, in row order (default: every coordinate of every input point, slot order).
     """
     positions = initial_state.positions
     manager = DerivedPointsManager(derived_spec)
@@ -815,6 +819,12 @@ def compile_topology(
     design_pts = list(design_pts)
     dprog = diagnostics(pidx, design_pts) if diagnostics is not None else None
     free_out = [out_keys.index(k) if k in out_keys else -1 for k in free_order]
+    if sensitivity_inputs is None:
+        sensitivity_inputs = [(k, axis) for k in in_keys for axis in range(3)]
+    sensitivity_inputs = [(k, int(axis)) for k, axis in sensitivity_inputs]
+    for k, axis in sensitivity_inputs:
+        if k not in in_slot or axis not in (0, 1, 2):
+            raise ValueError(f"Sensitivity input {(k, axis)!r} is not a hardpoint coordinate of this topology")
     ndsn = len(design_pts)
     layout["OKIN_H_OFF_DSN"] = take(max(3 * ndsn, 1))
     layout["OKIN_H_OFF_MCTX"] = take(4 * max(len(mcorners), 2))
@@ -839,6 +849,7 @@ def compile_topology(
         "OKIN_S_SHIM": shim_recs, "OKIN_S_SHIM_PTS": shim_pts,
         "OKIN_S_FREE_OUT": free_out, "OKIN_S_DGOP": dprog.ops if dprog else [],
         "OKIN_S_ELIM_OUT": [free_out[c] for c in elim_col],
+        "OKIN_S_SENS_IN": [3 * in_slot[k] + axis for k, axis in sensitivity_inputs],
     }
     isecs["OKIN_S_ROW_HOT"] = row_hot
     # Cold sections (setup, outputs requested per state, metrics, diagnostics) go last: the kernel
@@ -883,7 +894,7 @@ def compile_topology(
         "OKIN_H_NSHIM": len(shim_recs), "OKIN_H_NPARAM": len(param_default),
         "OKIN_H_NDROW": len(fast_rows), "OKIN_H_NGROW": len(row_order),
         "OKIN_H_FREE_ALL_OUT": int(all(v >= 0 for v in free_out)),
-        "OKIN_H_NHOT": n_hot, "OKIN_H_NDIAG": len(dprog.names) if dprog else 0, "OKIN_H_NDGOP": len(dprog.ops) if dprog else 0,
+        "OKIN_H_NHOT": n_hot, "OKIN_H_NSENS": len(sensitivity_inputs), "OKIN_H_NDIAG": len(dprog.names) if dprog else 0, "OKIN_H_NDGOP": len(dprog.ops) if dprog else 0,
         **layout,
     }
     for name, value in counts.items():
@@ -906,6 +917,7 @@ def compile_topology(
         diagnostic_names=list(dprog.names) if dprog else [],
         diagnostic_checks=list(dprog.checks) if dprog else [],
         param_names=param_names, param_default=np.asarray(param_default, dtype=np.float64),
+        sensitivity_inputs=sensitivity_inputs,
     )
 
 
@@ -917,8 +929,11 @@ def structure_point_index(suspension) -> dict:
 
 
 def compile_suspension(suspension, sweep_config, output_points=None, design_rules: bool = True,
-                       with_metrics: bool = True, tune_layout: bool = False) -> TopologyProgram:
-    """Compile a built suspension + sweep (first-step targets define the target rows)."""
+                       with_metrics: bool = True, tune_layout: bool = False, sensitivity_inputs=None,
+                       with_shims: bool = True) -> TopologyProgram:
+    """Compile a built suspension + sweep (first-step targets define the target rows).
+    ``with_shims=False`` leaves the camber-shim pre-solve out (hardpoint sensitivities need that; the
+    caller must make sure every shim is at its design thickness)."""
     from .diagnostics_program import build_diagnostic_program
     from .metrics_program import build_metric_program
     from .shim_program import shim_records
@@ -930,7 +945,7 @@ def compile_suspension(suspension, sweep_config, output_points=None, design_rule
     return compile_topology(
         state, constraints, suspension.derived_spec(), targets,
         output_points=output_points, design_rules=design_rules, metrics=metrics,
-        shims=shim_records(suspension) if design_rules else None,
+        shims=shim_records(suspension) if (design_rules and with_shims) else None,
         diagnostics=lambda pidx, design_pts: build_diagnostic_program(suspension, pidx, design_pts),
-        tune_layout=tune_layout,
+        tune_layout=tune_layout, sensitivity_inputs=sensitivity_inputs,
     )

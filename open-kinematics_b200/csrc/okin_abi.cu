@@ -7,15 +7,17 @@
 // systems of tens of unknowns (SURVEY.md section 8d; measured: the shared-memory data pipe is the
 // binding unit, profiles/r02_d_*), so tensor cores and TMA have nothing to act on; the only global
 // traffic is the coalesced instance-major hardpoint read and state write.
-// okin_sweep_kernel<FULL, SHIM, MAX_THREADS> has six instantiations: full outputs (128 registers) and
-// two lean families (128 / 168 registers), each with / without the camber-shim pre-solve; the
-// continuity pass of the diagnostics is a second kernel on the same stream.
+// okin_sweep_kernel<FULL, SHIM, MAX_THREADS, SENS> has seven instantiations: full outputs (128 registers)
+// and two lean families (128 / 168 registers), each with / without the camber-shim pre-solve, plus the
+// full outputs with hardpoint sensitivities (no pre-solve); the continuity pass of the diagnostics is a
+// second kernel on the same stream.
 #include <cuda_runtime.h>
 
 #include <pthread.h>
 #include <sched.h>
 
 #include <algorithm>
+#include <cstddef>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -38,7 +40,7 @@
 // 101-step T-bar axle 128), so the first large launch of a topology on a device times both.
 #define OKIN_MAX_THREADS 512
 #define OKIN_LEAN_WIDE_THREADS 384
-enum { OKIN_FAM_LEAN_WIDE = 0, OKIN_FAM_FULL = 1, OKIN_FAM_LEAN = 2, OKIN_FAM_COUNT = 3 };
+enum { OKIN_FAM_LEAN_WIDE = 0, OKIN_FAM_FULL = 1, OKIN_FAM_LEAN = 2, OKIN_FAM_SENS = 3, OKIN_FAM_COUNT = 4 };
 #ifndef OKIN_DRIFT
 #define OKIN_DRIFT 1             // how many instances a warp may run ahead of the slowest warp of its CTA
 #endif
@@ -85,6 +87,30 @@ struct DeviceCopy {
   cudaStream_t streams[OKIN_PIPE_SLOTS] = {};
 };
 
+// okin_batch_io without its last field: the kernels take the sensitivity output as a trailing
+// parameter instead, so that the parameter layout (and the code) of the instantiations that never
+// write it stays what it was before that output existed.
+struct OkinKernelIO {
+  const double* hardpoints;
+  const double* params;
+  const double* target_values;
+  int32_t* status;
+  int32_t* failed_step;
+  double* positions;
+  int32_t* iters;
+  double* max_residual;
+  double* tangents;
+  double* velocities;
+  double* tangent_health;
+  double* metrics;
+  double* design;
+  double* diagnostics;
+  double* jumps;
+  const double* instance_targets;
+  int32_t* worst_row;
+};
+static_assert(sizeof(OkinKernelIO) == offsetof(okin_batch_io, hardpoint_sensitivity), "OkinKernelIO layout");
+
 }  // namespace
 
 struct okin_topology {
@@ -97,11 +123,12 @@ struct okin_topology {
 // Shared memory of a CTA = [topology tables (int32 blob)] [one state slice per warp].  The tables are
 // copied once per (persistent) CTA so that every index lookup of the interpreter is a shared-memory
 // load instead of a global one (ncu round 1: long-scoreboard stalls on __ldg were the top stall).
-template <bool FULL, bool SHIM, int MAX_THREADS>
+// SENS: sens_out = [n_instances][n_steps][NSENS][NOUT*3], sens_ws = okin_sens_ws_doubles per resident warp.
+template <bool FULL, bool SHIM, int MAX_THREADS, bool SENS = false>
 __global__ void __launch_bounds__(MAX_THREADS, 1)
 okin_sweep_kernel(const int32_t* __restrict__ hdr, const int32_t* __restrict__ ib, const double* __restrict__ fb,
-                  long long n_instances, int n_steps, OkinSolverCfg cfg, okin_batch_io io, int n_iblob,
-                  int table_doubles, unsigned long long* __restrict__ counter) {
+                  long long n_instances, int n_steps, OkinSolverCfg cfg, OkinKernelIO io, int n_iblob,
+                  int table_doubles, unsigned long long* __restrict__ counter, double* sens_out, double* sens_ws) {
   // [section pointers][header][hot tables][one state slice per warp]
   const int32_t** sec = reinterpret_cast<const int32_t**>(okin_smem);
   int32_t* shdr = reinterpret_cast<int32_t*>(okin_smem + OKIN_S_COUNT);
@@ -157,7 +184,11 @@ okin_sweep_kernel(const int32_t* __restrict__ hdr, const int32_t* __restrict__ i
       out.status = io.status + i;
       out.failed_step = io.failed_step + i;
       out.worst_row = io.worst_row ? io.worst_row + i : nullptr;
-      okin_sweep<FULL, SHIM>(pr, sm, io.hardpoints + (size_t)i * 3 * nin,
+      if (SENS) {
+        out.sensitivity = sens_out ? sens_out + (size_t)i * n_steps * hdr[OKIN_H_NSENS] * 3 * nout : nullptr;
+        out.sens_ws = sens_ws + ((size_t)blockIdx.x * warps_per_cta + warp) * okin_sens_ws_doubles(hdr);
+      }
+      okin_sweep<FULL, SHIM, SENS>(pr, sm, io.hardpoints + (size_t)i * 3 * nin,
                  io.params ? io.params + (size_t)i * hdr[OKIN_H_NPARAM] : nullptr,
                  io.instance_targets ? io.instance_targets + (size_t)i * nt * n_steps : io.target_values, n_steps,
                  cfg, out);
@@ -207,6 +238,8 @@ namespace {
 
 const void* kernel_of(int fam, bool shim) {
   switch (fam) {
+    case OKIN_FAM_SENS:
+      return (const void*)okin_sweep_kernel<true, false, OKIN_MAX_THREADS, true>;
     case OKIN_FAM_FULL:
       return shim ? (const void*)okin_sweep_kernel<true, true, OKIN_MAX_THREADS>
                   : (const void*)okin_sweep_kernel<true, false, OKIN_MAX_THREADS>;
@@ -244,7 +277,7 @@ int ensure_device(okin_topology* t, int device, DeviceCopy** out) {
     const size_t table_bytes = (size_t)d.table_doubles * 8;
     const size_t sm_budget = prop.sharedMemPerMultiprocessor;
     for (int fam = 0; fam < OKIN_FAM_COUNT; ++fam) {
-      const bool full = fam == OKIN_FAM_FULL;
+      const bool full = fam == OKIN_FAM_FULL || fam == OKIN_FAM_SENS;
       const size_t slice_bytes =
           (size_t)t->hdr[full ? OKIN_H_SMEM_DOUBLES : OKIN_H_SMEM_DOUBLES_LEAN] * sizeof(double);
       const int max_threads = fam == OKIN_FAM_LEAN_WIDE ? OKIN_LEAN_WIDE_THREADS : OKIN_MAX_THREADS;
@@ -272,7 +305,7 @@ int ensure_device(okin_topology* t, int device, DeviceCopy** out) {
       sh.warps_per_cta = best_w;
       sh.smem_bytes = (int)(table_bytes + best_w * slice_bytes);
       sh.ctas_per_sm = 1 << 30;
-      for (int shim = 0; shim < 2; ++shim) {
+      for (int shim = 0; shim < (fam == OKIN_FAM_SENS ? 1 : 2); ++shim) {
         const void* kernel = kernel_of(fam, shim != 0);
         OKIN_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, sh.smem_bytes));
         int ctas = 0;
@@ -312,10 +345,19 @@ int launch_family(okin_topology* t, DeviceCopy* d, int fam, const OkinSolverCfg&
   long long n = (long long)n_instances;
   int n_iblob = (int)t->ib.size();
   OkinSolverCfg cfg = c;
-  okin_batch_io bio = io;
-  void* args[] = {&d->hdr, &d->ib, &d->fb, &n, &n_steps, &cfg, &bio, &n_iblob, &d->table_doubles, &counter};
+  OkinKernelIO kio;
+  std::memcpy(&kio, &io, sizeof(kio));
+  // per-resident-warp scratch of the sensitivity phase (stream-ordered, like the counter)
+  double* sens_out = io.hardpoint_sensitivity;
+  double* sens_ws = nullptr;
+  if (fam == OKIN_FAM_SENS)
+    OKIN_CUDA(cudaMallocAsync(&sens_ws, (size_t)grid * w * okin_sens_ws_doubles(t->hdr.data()) * sizeof(double) + 8,
+                              stream));
+  void* args[] = {&d->hdr, &d->ib, &d->fb, &n, &n_steps, &cfg, &kio, &n_iblob, &d->table_doubles, &counter,
+                  &sens_out, &sens_ws};
   const cudaError_t launch_err = cudaLaunchKernel(kernel, dim3(grid), dim3(w * 32), args, sh.smem_bytes, stream);
   OKIN_CUDA(cudaFreeAsync(counter, stream));
+  if (sens_ws) OKIN_CUDA(cudaFreeAsync(sens_ws, stream));
   OKIN_CUDA(launch_err);
   return OKIN_OK;
 }
@@ -327,8 +369,8 @@ int launch(okin_topology* t, DeviceCopy* d, const okin_solver_cfg* cfg, cudaStre
                   cfg->use_predictor};
   // lean instantiation when no per-state tangent / metric / diagnostic output is wanted
   const bool full = io.tangents || io.velocities || io.tangent_health || io.metrics || io.diagnostics;
-  int fam = OKIN_FAM_FULL;
-  if (!full) {
+  int fam = io.hardpoint_sensitivity ? OKIN_FAM_SENS : OKIN_FAM_FULL;
+  if (!full && !io.hardpoint_sensitivity) {
     fam = d->lean_family;
     const int64_t sample = 4 * (int64_t)d->num_sms * std::max(d->shape[OKIN_FAM_LEAN].ctas_per_sm * d->shape[OKIN_FAM_LEAN].warps_per_cta,
                                                               d->shape[OKIN_FAM_LEAN_WIDE].ctas_per_sm * d->shape[OKIN_FAM_LEAN_WIDE].warps_per_cta);
@@ -390,6 +432,9 @@ int check_common(const okin_topology* t, const okin_solver_cfg* cfg, int64_t n_i
   if ((io->diagnostics || io->jumps) && !t->hdr[OKIN_H_NDIAG])
     return fail(OKIN_ERR_USAGE, "topology was compiled without a diagnostic program");
   if (io->jumps && !io->diagnostics) return fail(OKIN_ERR_USAGE, "jumps output needs the diagnostics output");
+  if (io->hardpoint_sensitivity && t->hdr[OKIN_H_NSHIM] > 0)
+    return fail(OKIN_ERR_USAGE, "hardpoint sensitivities are not available on a topology with camber-shim records "
+                                "(the shim pre-solve is not differentiated)");
   if (cfg->max_iter < 1 || !(cfg->step_tol > 0.0) || !(cfg->coarse_tol >= cfg->step_tol)) return fail(OKIN_ERR_USAGE, "invalid solver config");
   return OKIN_OK;
 }
@@ -398,7 +443,7 @@ int check_common(const okin_topology* t, const okin_solver_cfg* cfg, int64_t n_i
 // Every per-instance array of a call is one "lane" of a pipeline slot: (host pointer, bytes per
 // instance).  scratch: device buffer needed although the caller does not want the array back.
 struct Lane { const void* host; size_t per_inst; bool input; bool scratch; size_t bytes; };
-constexpr int kLanes = 16;
+constexpr int kLanes = 17;
 
 struct HostBatch {
   Lane lanes[kLanes];
@@ -428,6 +473,7 @@ struct HostBatch {
         {io->jumps, S * (n / 3) * 8, false, false, 0},
         {(io->instance_targets && nt * S) ? io->instance_targets : nullptr, nt * S * 8, true, false, 0},
         {io->worst_row, 4, false, false, 0},
+        {io->hardpoint_sensitivity, S * (size_t)h[OKIN_H_NSENS] * nout3 * 8, false, false, 0},
     };
     std::memcpy(lanes, init, sizeof(init));
     chunk = (size_t)std::min<int64_t>(std::max<int64_t>(n_instances, 1), OKIN_PIPE_CHUNK);
@@ -556,6 +602,7 @@ void run_shard(okin_topology* t, const okin_solver_cfg* cfg, const HostBatch& hb
     dio.jumps = (double*)dev[13];
     dio.instance_targets = (const double*)dev[14];
     dio.worst_row = (int32_t*)dev[15];
+    dio.hardpoint_sensitivity = (double*)dev[16];
     const int rc = launch(t, d, cfg, st, (int64_t)c, hb.n_steps, dio);
     if (rc) {
       drain();
@@ -611,9 +658,15 @@ int okin_topology_create(const okin_topology_desc* desc, okin_topology** out) {
   if (desc->hdr[OKIN_H_MAGIC] != OKIN_MAGIC) return fail(OKIN_ERR_USAGE, "bad topology magic");
   if (desc->n_iblob < 0 || desc->n_fblob < 0) return fail(OKIN_ERR_USAGE, "negative blob size");
   // every section must lie inside its blob
-  for (int s = 0; s < OKIN_S_COUNT; ++s) {
+  for (int s = 0; s < OKIN_S_COUNT_ALL; ++s) {
     const int64_t off = desc->hdr[OKIN_H_SEC0 + 2 * s], len = desc->hdr[OKIN_H_SEC0 + 2 * s + 1];
     if (off < 0 || len < 0 || off + len > desc->n_iblob) return fail(OKIN_ERR_USAGE, "int section out of range");
+  }
+  if (desc->hdr[OKIN_H_NSENS] != desc->hdr[OKIN_H_SEC0 + 2 * OKIN_S_SENS_IN + 1])
+    return fail(OKIN_ERR_USAGE, "sensitivity input count does not match its section");
+  for (int k = 0; k < desc->hdr[OKIN_H_NSENS]; ++k) {
+    const int32_t coord = desc->iblob[desc->hdr[OKIN_H_SEC0 + 2 * OKIN_S_SENS_IN] + k];
+    if (coord < 0 || coord >= 3 * desc->hdr[OKIN_H_NIN]) return fail(OKIN_ERR_USAGE, "sensitivity input out of range");
   }
   for (int s = 0; s < OKIN_F_COUNT; ++s) {
     const int64_t off = desc->hdr[OKIN_H_FSEC0 + 2 * s], len = desc->hdr[OKIN_H_FSEC0 + 2 * s + 1];
@@ -623,7 +676,7 @@ int okin_topology_create(const okin_topology_desc* desc, okin_topology** out) {
     return fail(OKIN_ERR_USAGE, "hot prefix out of range");
   // The device code addresses sections below OKIN_S_COLD0 as shared memory: they must lie in the
   // hot prefix, the others behind it.
-  for (int s = 0; s < OKIN_S_COUNT; ++s) {
+  for (int s = 0; s < OKIN_S_COUNT_ALL; ++s) {
     const int64_t off = desc->hdr[OKIN_H_SEC0 + 2 * s], len = desc->hdr[OKIN_H_SEC0 + 2 * s + 1];
     const bool in_hot = off + len <= desc->hdr[OKIN_H_NHOT];
     if (s < OKIN_S_COLD0 ? !in_hot : (len > 0 && off < desc->hdr[OKIN_H_NHOT]))

@@ -1904,6 +1904,275 @@ OKIN_FN void okin_tangent_health(const OkinProgram& pr, double* sm, bool notpd, 
   OKIN_PHASE_END
 }
 
+// ---------------------------------------------------------------------------------------
+// Hardpoint sensitivities: d pos_o / d p_k for the hardpoint coordinates p_k listed in OKIN_S_SENS_IN
+// (k = 3 * input slot + axis), params held fixed.  At an accepted state x*(p),
+//   dx*/dp_k = -A^{-1} J_x^T dR/dp_k,   A = J_x^T J_x the factor the tangents use (Gauss-Newton: the
+//   sum r_i Hess(r_i) is dropped, as for the tangents),
+//   dR/dp_k = (dR/dpos) (dpos/dp_k)|_x + (dR/dc) (dc/dp_k),
+// where c are the per-instance design constants (okin_setup rules) and derived-op parameters depend on
+// p through the design pose.  The part that depends on p alone (dc/dp, dpar/dp) is evaluated once per
+// instance at the design pose; the rest per accepted state, after every other output of the state.
+// Per-warp scratch in global memory (okin_sens_ws_doubles):
+//   dcst [NSENS][NCST]   dc/dp_k of every per-instance constant (0 for explicit ones)
+//   dpar [NSENS][NPAR]   d(derived-op parameter)/dp_k
+//   grad [NROW][13]      dR/d(row point s), s = 0..3, and R of every least-squares row at the state
+//   tan  [3P]            tangent of every point for the column being processed
+// ---------------------------------------------------------------------------------------
+OKIN_HD const int32_t* okin_sec_cold(const OkinProgram& pr, int s) { return pr.ibc + pr.hdr[OKIN_H_SEC0 + 2 * s]; }
+OKIN_HD size_t okin_sens_ws_doubles(const int32_t* hdr) {
+  return (size_t)hdr[OKIN_H_NSENS] * (hdr[OKIN_H_NCST] + hdr[OKIN_H_NPAR]) + 13 * (size_t)hdr[OKIN_H_NROW] +
+         3 * (size_t)hdr[OKIN_H_P];
+}
+
+// d out / d par of a derived op: the unit direction its parameter scales (okin_dop_eval).
+OKIN_HD void okin_dop_par_dir(int op, const double* a, const double* b, const double* c, double dir[3]) {
+  dir[0] = dir[1] = dir[2] = 0.0;
+  if (op == OKIN_DOP_MIDPOINT) return;
+  const double z[3] = {0.0, 0.0, 0.0};
+  double v[3], u[3], du[3], il;
+  if (op == OKIN_DOP_ALONG_LINE) {
+    for (int k = 0; k < 3; ++k) v[k] = b[k] - a[k];
+    okin_unit_jvp(v, z, dir, du, &il);
+    return;
+  }
+  for (int k = 0; k < 3; ++k) v[k] = c[k] - b[k];
+  okin_unit_jvp(v, z, u, du, &il);
+  const double s = -u[2];
+  double w[3] = {-s * u[0], -s * u[1], -s * u[2] - 1.0};
+  okin_unit_jvp(w, z, dir, du, &il);
+}
+
+// Tangent of every point along hardpoint coordinate `coord` into tan[3P], one derived level per
+// phase.  Fixed points move with their hardpoint (e_k); free points take free[] (elimination order)
+// when given, their hardpoint when `design` (the design pose is the authored one), else stay;
+// derived points push their inputs' tangents and dpar[] through the op at the current pos[].  An input
+// slot holding a derived point's authored position acts only through dpar.
+template <typename Dummy = void>
+OKIN_FN void okin_sens_points(const OkinProgram& pr, double* sm, int coord, const double* dpar, const double* free,
+                              bool design, double* tan) {
+  sm = OKIN_SHARED(sm);
+  const int32_t* hdr = OKIN_SHARED(pr.hdr);
+  const int np = hdr[OKIN_H_P];
+  const int32_t* kind = okin_sec(pr, OKIN_S_POINT_KIND);
+  const int32_t* pelim = OKIN_SHARED(okin_sec(pr, OKIN_S_POINT_ELIM));
+  const int moved = OKIN_LDG(okin_sec(pr, OKIN_S_IN_POINT) + coord / 3), axis = coord % 3;
+  OKIN_PHASE_BEGIN
+  OKIN_LANE_LOOP
+  for (int t = lane; t < 3 * np; t += 32) {
+    const int q = t / 3, kq = OKIN_LDG(kind + q);
+    double v = 0.0;
+    if (kq == OKIN_PT_FIXED || (kq == OKIN_PT_FREE && design)) v = (q == moved && t % 3 == axis) ? 1.0 : 0.0;
+    else if (kq == OKIN_PT_FREE && free) v = free[3 * OKIN_LDG(pelim + q) + t % 3];
+    tan[t] = v;
+  }
+  OKIN_PHASE_END
+  const int32_t* dop = OKIN_SHARED(okin_sec(pr, OKIN_S_DOP));
+  const int32_t* lev = OKIN_SHARED(okin_sec(pr, OKIN_S_DOP_LEV));
+  const int nlev = okin_sec_len(pr, OKIN_S_DOP_LEV) - 1;
+  const double* pos = sm + hdr[OKIN_H_OFF_POS];
+  const double* par = sm + hdr[OKIN_H_OFF_PAR];
+  for (int lv = 0; lv < nlev; ++lv) {
+    const int b = OKIN_LDG(lev + lv), e = OKIN_LDG(lev + lv + 1);
+    OKIN_PHASE_BEGIN
+    OKIN_LANE_LOOP
+    for (int d = b + lane; d < e; d += 32) {
+      const int32_t* rec = dop + d * OKIN_DOP_STRIDE;
+      const int op = OKIN_LDG(rec + 0), pi = OKIN_LDG(rec + 5);
+      const int ia = OKIN_LDG(rec + 2), ib = OKIN_LDG(rec + 3) < 0 ? ia : OKIN_LDG(rec + 3);
+      const int ic = OKIN_LDG(rec + 4) < 0 ? ia : OKIN_LDG(rec + 4);
+      double out[3], dout[3], dir[3];
+      okin_dop_eval(op, par[pi], pos + 3 * ia, pos + 3 * ib, pos + 3 * ic, tan + 3 * ia, tan + 3 * ib, tan + 3 * ic,
+                    out, dout);
+      okin_dop_par_dir(op, pos + 3 * ia, pos + 3 * ib, pos + 3 * ic, dir);
+      const double dp = dpar[pi];
+      double* o = tan + 3 * OKIN_LDG(rec + 1);
+      o[0] = dout[0] + dp * dir[0]; o[1] = dout[1] + dp * dir[1]; o[2] = dout[2] + dp * dir[2];
+    }
+    OKIN_PHASE_END
+  }
+}
+
+// Once per instance, at the design pose okin_setup left in pos[]: dpar/dp_k and dc/dp_k of every
+// sensitivity column (forward mode through the okin_setup rules).
+template <typename Dummy = void>
+OKIN_FN void okin_sens_setup(const OkinProgram& pr, double* sm, const double* __restrict__ hardpoints, double* ws) {
+  sm = OKIN_SHARED(sm);
+  const int32_t* hdr = OKIN_SHARED(pr.hdr);
+  const int nsens = hdr[OKIN_H_NSENS], ncst = hdr[OKIN_H_NCST], npar = hdr[OKIN_H_NPAR];
+  const int ndop = hdr[OKIN_H_NDOP], nls = hdr[OKIN_H_NROW];
+  const int32_t* sens_in = okin_sec_cold(pr, OKIN_S_SENS_IN);
+  const int32_t* in_point = okin_sec(pr, OKIN_S_IN_POINT);
+  const int32_t* dop = OKIN_SHARED(okin_sec(pr, OKIN_S_DOP));
+  const int32_t* par_mode = okin_sec(pr, OKIN_S_PAR_MODE);
+  const int32_t* rows = okin_sec(pr, OKIN_S_ROW);
+  const double* pos = sm + hdr[OKIN_H_OFF_POS];
+  const double* cst = sm + hdr[OKIN_H_OFF_CST];
+  double* tan = ws + (size_t)nsens * (ncst + npar) + 13 * (size_t)nls;
+  for (int k = 0; k < nsens; ++k) {
+    const int coord = OKIN_LDG(sens_in + k), moved = OKIN_LDG(in_point + coord / 3), axis = coord % 3;
+    double* dpar = ws + (size_t)nsens * ncst + (size_t)k * npar;
+    double* dc_all = ws + (size_t)k * ncst;
+    OKIN_PHASE_BEGIN
+    OKIN_LANE_LOOP
+    for (int d = lane; d < ndop; d += 32) {  // design projection (okin_setup): (o - a) . unit(b - a)
+      const int32_t* rec = dop + d * OKIN_DOP_STRIDE;
+      const int p = OKIN_LDG(rec + 5);
+      double value = 0.0;
+      if (OKIN_LDG(par_mode + p) == OKIN_PAR_DESIGN_PROJECTION) {
+        const int ia = OKIN_LDG(rec + 2), ib = OKIN_LDG(rec + 3), io = OKIN_LDG(rec + 6);
+        const double* a = pos + 3 * ia;
+        const double* b = pos + 3 * ib;
+        const double* o = hardpoints + 3 * io;
+        double v[3], u[3], du[3], dv[3], il, dd[3];
+        for (int c = 0; c < 3; ++c) {
+          const double da = (ia == moved && c == axis) ? 1.0 : 0.0, db = (ib == moved && c == axis) ? 1.0 : 0.0;
+          v[c] = b[c] - a[c];
+          dv[c] = db - da;
+          dd[c] = ((coord / 3 == io && c == axis) ? 1.0 : 0.0) - da;
+        }
+        okin_unit_jvp(v, dv, u, du, &il);
+        for (int c = 0; c < 3; ++c) value += dd[c] * u[c] + (o[c] - a[c]) * du[c];
+      }
+      dpar[p] = value;
+    }
+    OKIN_LANE_LOOP
+    for (int t = lane; t < ncst; t += 32) dc_all[t] = 0.0;
+    OKIN_PHASE_END
+    okin_sens_points(pr, sm, coord, dpar, nullptr, true, tan);
+    OKIN_PHASE_BEGIN
+    OKIN_LANE_LOOP
+    for (int t = lane; t < nls; t += 32) {
+      const int32_t* rec = rows + t * OKIN_ROW_STRIDE;
+      const int rule = OKIN_LDG(rec + OKIN_R_RULE);
+      if (rule == OKIN_RULE_EXPLICIT) continue;
+      const int fam = OKIN_LDG(rec + OKIN_R_FAM);
+      const double* c = cst + OKIN_LDG(rec + OKIN_R_CST);
+      double* dc = dc_all + OKIN_LDG(rec + OKIN_R_CST);
+      OkinDual q[4][3];
+      for (int s = 0; s < 4; ++s) {
+        const int pi = OKIN_LDG(rec + OKIN_R_P0 + s);
+        for (int m = 0; m < 3; ++m) q[s][m] = pi < 0 ? OkinDual{0.0, 0.0} : OkinDual{pos[3 * pi + m], tan[3 * pi + m]};
+      }
+      if (rule == OKIN_RULE_DESIGN_POINT) {
+        dc[0] = q[0][0].d; dc[1] = q[0][1].d; dc[2] = q[0][2].d;
+      } else if (rule == OKIN_RULE_TARGET_BASE) {
+        dc[3] = c[0] * q[0][0].d + c[1] * q[0][1].d + c[2] * q[0][2].d;
+      } else if (fam == OKIN_FAM_DISTANCE) {
+        OkinDual s2 = {0.0, 0.0};
+        for (int m = 0; m < 3; ++m) s2 = s2 + (q[1][m] - q[0][m]) * (q[1][m] - q[0][m]);
+        dc[0] = okin_sqrt(s2).d;
+      } else if (fam == OKIN_FAM_ANGLE) {
+        OkinDual a[3], b[3], na = {0.0, 0.0}, nb = {0.0, 0.0};
+        for (int m = 0; m < 3; ++m) { a[m] = q[1][m] - q[0][m]; b[m] = q[3][m] - q[2][m]; na = na + a[m] * a[m]; nb = nb + b[m] * b[m]; }
+        na = okin_sqrt(na); nb = okin_sqrt(nb);
+        for (int m = 0; m < 3; ++m) { a[m] = a[m] / na; b[m] = b[m] / nb; }
+        const OkinDual cx = a[1] * b[2] - a[2] * b[1], cy = a[2] * b[0] - a[0] * b[2], cz = a[0] * b[1] - a[1] * b[0];
+        dc[0] = okin_atan2(okin_sqrt(cx * cx + cy * cy + cz * cz), a[0] * b[0] + a[1] * b[1] + a[2] * b[2]).d;
+      } else if (fam == OKIN_FAM_SCALAR_TRIPLE) {
+        OkinDual a[3], b[3], e[3];
+        for (int m = 0; m < 3; ++m) { a[m] = q[1][m] - q[0][m]; b[m] = q[2][m] - q[0][m]; e[m] = q[3][m] - q[0][m]; }
+        const OkinDual v = a[0] * (b[1] * e[2] - b[2] * e[1]) + a[1] * (b[2] * e[0] - b[0] * e[2]) +
+                           a[2] * (b[0] * e[1] - b[1] * e[0]);
+        dc[0] = v.d;
+        dc[1] = -(v.v > 0.0 ? 1.0 : -1.0) * v.d / (v.v * v.v);   // c[1] = 1/|V|
+      }
+    }
+    OKIN_PHASE_END
+  }
+}
+
+// One accepted state: d pos_o / d p_k of every output point for every sensitivity column into
+// dst[NSENS][NOUT*3].  Needs the factor of A at the state (okin_factor) and pos[] at the state; the
+// right-hand sides use vec[0 .. NT] (the tangents have been exported by then).
+template <typename Dummy = void>
+OKIN_FN void okin_sens_state(const OkinProgram& pr, double* sm, const double* tval, double* ws, double* dst) {
+  sm = OKIN_SHARED(sm);
+  const int32_t* hdr = OKIN_SHARED(pr.hdr);
+  const int nsens = hdr[OKIN_H_NSENS], ncst = hdr[OKIN_H_NCST], npar = hdr[OKIN_H_NPAR];
+  const int nls = hdr[OKIN_H_NROW], nout = hdr[OKIN_H_NOUT], n = 3 * hdr[OKIN_H_NF];
+  const int group = 1 + hdr[OKIN_H_NT];
+  const int32_t* sens_in = okin_sec_cold(pr, OKIN_S_SENS_IN);
+  const int32_t* rows = okin_sec(pr, OKIN_S_ROW);
+  const int32_t* out_point = OKIN_SHARED(okin_sec(pr, OKIN_S_OUT_POINT));
+  const double* pos = sm + hdr[OKIN_H_OFF_POS];
+  const double* cst = sm + hdr[OKIN_H_OFF_CST];
+  double* r = sm + hdr[OKIN_H_OFF_R];
+  double* vec = sm + hdr[OKIN_H_OFF_VEC];
+  double* grad = ws + (size_t)nsens * (ncst + npar);
+  double* tan = grad + 13 * (size_t)nls;
+  // Row gradients J_x at the state (the tangent health uses their storage as scratch), and the
+  // per-point gradients of every least-squares row.
+  OkinState scratch_state;
+  okin_eval_rows(pr, sm, tval, true, scratch_state);
+  OKIN_PHASE_BEGIN
+  OKIN_LANE_LOOP
+  for (int t = lane; t < nls; t += 32) {
+    const int32_t* rec = rows + t * OKIN_ROW_STRIDE;
+    const int fam = OKIN_LDG(rec + OKIN_R_FAM);
+    const double* c = cst + OKIN_LDG(rec + OKIN_R_CST);
+    double p[12], g[12];
+    for (int m = 0; m < 12; ++m) { p[m] = 0.0; g[m] = 0.0; }
+    for (int s = 0; s < 4; ++s) {
+      const int pi = OKIN_LDG(rec + OKIN_R_P0 + s);
+      if (pi < 0) break;
+      p[3 * s] = pos[3 * pi]; p[3 * s + 1] = pos[3 * pi + 1]; p[3 * s + 2] = pos[3 * pi + 2];
+    }
+    if (fam == OKIN_FAM_TARGET) { g[0] = c[0]; g[1] = c[1]; g[2] = c[2]; }
+    else okin_family_resgrad(fam, p, c, g);
+    double* o = grad + 13 * (size_t)t;
+    for (int m = 0; m < 12; ++m) o[m] = g[m];
+    o[12] = r[t];
+  }
+  OKIN_PHASE_END
+  for (int k0 = 0; k0 < nsens; k0 += group) {
+    const int m = nsens - k0 < group ? nsens - k0 : group;
+    for (int j = m - 1; j >= 0; --j) {  // vec[0] last: the gather below writes it
+      const int k = k0 + j, coord = OKIN_LDG(sens_in + k);
+      const double* dc_all = ws + (size_t)k * ncst;
+      okin_sens_points(pr, sm, coord, ws + (size_t)nsens * ncst + (size_t)k * npar, nullptr, false, tan);
+      OKIN_PHASE_BEGIN
+      OKIN_LANE_LOOP
+      for (int t = lane; t < nls; t += 32) {  // r[t] <- dR_t/dp_k
+        const int32_t* rec = rows + t * OKIN_ROW_STRIDE;
+        const double* g = grad + 13 * (size_t)t;
+        double acc = 0.0;
+        for (int s = 0; s < 4; ++s) {
+          const int pi = OKIN_LDG(rec + OKIN_R_P0 + s);
+          if (pi < 0) break;
+          acc += g[3 * s] * tan[3 * pi] + g[3 * s + 1] * tan[3 * pi + 1] + g[3 * s + 2] * tan[3 * pi + 2];
+        }
+        const int rule = OKIN_LDG(rec + OKIN_R_RULE);
+        const double* c = cst + OKIN_LDG(rec + OKIN_R_CST);
+        const double* dc = dc_all + OKIN_LDG(rec + OKIN_R_CST);
+        if (rule == OKIN_RULE_DESIGN_POINT) {          // linear pin n.(p - anchor)
+          acc -= g[0] * dc[0] + g[1] * dc[1] + g[2] * dc[2];
+        } else if (rule == OKIN_RULE_TARGET_BASE) {    // dir.p - (base + value)
+          acc -= dc[3];
+        } else if (rule == OKIN_RULE_DESIGN_VALUE) {
+          if (OKIN_LDG(rec + OKIN_R_FAM) == OKIN_FAM_SCALAR_TRIPLE) acc += -c[1] * dc[0] + g[12] / c[1] * dc[1];
+          else acc -= dc[0];                            // quantity - design value
+        }
+        r[t] = acc;
+      }
+      OKIN_PHASE_END
+      okin_assemble(pr, sm, 0.0, true);  // vec[0] = -J_x^T dR/dp_k
+      if (j > 0) okin_copy(pr, vec + j * n, vec);
+    }
+    okin_solve(pr, sm, 0, m, false);
+    for (int j = 0; j < m; ++j) {
+      const int k = k0 + j;
+      okin_sens_points(pr, sm, OKIN_LDG(sens_in + k), ws + (size_t)nsens * ncst + (size_t)k * npar, vec + j * n,
+                       false, tan);
+      double* o = dst + (size_t)k * 3 * nout;
+      OKIN_PHASE_BEGIN
+      OKIN_LANE_LOOP
+      for (int t = lane; t < 3 * nout; t += 32) o[t] = tan[3 * OKIN_LDG(out_point + t / 3) + t % 3];
+      OKIN_PHASE_END
+    }
+  }
+}
+
 struct OkinOutputs {
   double* positions;      // [n_steps][NOUT*3] or null
   int32_t* iters;         // [n_steps] or null
@@ -1917,6 +2186,8 @@ struct OkinOutputs {
   int32_t* status;        // [1]
   int32_t* failed_step;   // [1]
   int32_t* worst_row;     // [1] or null: row owning max|r| at the failed step (solver.py:640-651), else -1
+  double* sensitivity;    // [n_steps][NSENS][NOUT*3] hardpoint sensitivities or null (SENS instantiation only)
+  double* sens_ws;        // okin_sens_ws_doubles scratch of the warp (SENS instantiation only)
 };
 
 // Index of the row with the largest |r| in r[0 .. nrows) (first one on ties, like np.argmax;
@@ -1963,8 +2234,9 @@ OKIN_FN int okin_worst_row(const OkinProgram& pr, double* sm) {
 // FULL: tangents / velocities / health / metrics / diagnostics outputs are compiled in (the lean
 // instantiation only writes positions, solver statistics and the design pose: the throughput
 // path, whose code footprint matters -- see profiles/r01_g_*).  SHIM: the topology has camber-shim
-// records (the pre-solve is a large, once-per-instance piece of code).
-template <bool FULL, bool SHIM>
+// records (the pre-solve is a large, once-per-instance piece of code).  SENS (with FULL, without SHIM):
+// the hardpoint-sensitivity output is compiled in.
+template <bool FULL, bool SHIM, bool SENS = false>
 OKIN_HD void okin_sweep(const OkinProgram& pr, double* sm, const double* __restrict__ hardpoints,
                         const double* __restrict__ params, const double* __restrict__ tvals, int n_steps,
                         const OkinSolverCfg& cfg, const OkinOutputs& out) {
@@ -1985,8 +2257,10 @@ OKIN_HD void okin_sweep(const OkinProgram& pr, double* sm, const double* __restr
   double* const o_health = FULL ? out.health : nullptr;
   double* const o_metrics = FULL ? out.metrics : nullptr;
   double* const o_diagnostics = FULL ? out.diagnostics : nullptr;
+  double* const o_sens = SENS ? out.sensitivity : nullptr;
   int invalid = 0;
   okin_setup<SHIM>(pr, sm, hardpoints, params, &invalid, FULL);
+  if (SENS && o_sens && !invalid) okin_sens_setup(pr, sm, hardpoints, out.sens_ws);
   if (out.design) {  // design (setup) pose of every output point
     OKIN_PHASE_BEGIN
     OKIN_LANE_LOOP
@@ -2036,7 +2310,7 @@ OKIN_HD void okin_sweep(const OkinProgram& pr, double* sm, const double* __restr
       okin_extrapolate(pr, sm, order);
       const bool predicted = order > 0;
       bool conv = false;
-      const bool relinearise = o_tangents || o_velocities || o_health || o_metrics;
+      const bool relinearise = o_tangents || o_velocities || o_health || o_metrics || o_sens;
       bool at_solution = false;
       int nfev = 0;
       bool valid = true;
@@ -2144,6 +2418,18 @@ OKIN_HD void okin_sweep(const OkinProgram& pr, double* sm, const double* __restr
       } else {
         OKIN_PHASE_BEGIN
         if (lane == 0) { o_health[2 * s] = NAN; o_health[2 * s + 1] = NAN; }
+        OKIN_PHASE_END
+      }
+    }
+    if (SENS && o_sens) {
+      const int nsens = hdr[OKIN_H_NSENS];
+      double* dst = o_sens + (size_t)s * nsens * 3 * nout;
+      if (ok) {
+        okin_sens_state(pr, sm, tcur, out.sens_ws, dst);
+      } else {
+        OKIN_PHASE_BEGIN
+        OKIN_LANE_LOOP
+        for (int t = lane; t < nsens * 3 * nout; t += 32) dst[t] = NAN;
         OKIN_PHASE_END
       }
     }

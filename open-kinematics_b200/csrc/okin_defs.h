@@ -131,6 +131,7 @@ enum okin_hdr_slot {
   OKIN_H_OFF_XPREV,  // previous accepted solution (3*NF doubles, elimination order)
   OKIN_H_OFF_DHIST,  // three older solution increments as float32 vectors (extrapolation predictor)
   OKIN_H_SMEM_DOUBLES_LEAN,  // slice size of an instance solved without tangents / metrics / diagnostics
+  OKIN_H_NSENS,    // hardpoint-sensitivity rows (entries of OKIN_S_SENS_IN)
   OKIN_H_SEC0 = 64,                      // room for 64 scalar slots,
   OKIN_H_FSEC0 = 64 + 2 * 64,            // 64 int32 sections
   OKIN_HDR_SIZE = 64 + 2 * 64 + 2 * 8    // and 8 double sections
@@ -198,7 +199,11 @@ enum okin_isec {
   OKIN_S_DGOP,           // [NDGOP][OKIN_DGOP_STRIDE] topology diagnostic ops
   OKIN_S_ELIM_COL,       // [NF] elimination position -> reference column block (sorted free-point order)
   OKIN_S_ELIM_OUT,       // [NF] elimination position -> output slot of that free point, -1 = not exported
-  OKIN_S_COUNT
+  OKIN_S_COUNT,
+  // Sections from here on are not in the per-CTA section table (okin_resolve_section), so the kernels
+  // that never read them keep their shared-memory layout; device code reaches them with okin_sec_cold.
+  OKIN_S_SENS_IN = OKIN_S_COUNT,  // [NSENS] hardpoint coordinate 3 * input slot + axis of each sensitivity row
+  OKIN_S_COUNT_ALL
 };
 #define OKIN_ASM_DIAG 0x40000000
 // Contribution words carry a negate flag: the product enters with a minus sign (a fast distance
