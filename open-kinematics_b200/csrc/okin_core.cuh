@@ -1120,6 +1120,7 @@ OKIN_HD int okin_solve_step(const OkinProgram& pr, double* sm, const double* tva
   int nfev = 0;
   st.mu = 0.0;
   double nu = 2.0;
+  bool gn_rejected = false;  // an undamped step of this solve has been rejected
   okin_eval_rows(pr, sm, tval, true, st);
   ++nfev;
   *converged = false;
@@ -1175,32 +1176,50 @@ OKIN_HD int okin_solve_step(const OkinProgram& pr, double* sm, const double* tva
       ++nfev;
       continue;
     }
+    // Damped step: ||r + J h||^2, the linear model's prediction (r[] and rg[] still hold the old point),
+    // for the gain ratio below.
+    double f2_model = 0.0;
+    if (st.mu > 0.0) {
+      okin_linear_residuals(pr, sm, st);
+      f2_model = st.f2;
+    }
     okin_eval_rows(pr, sm, tval, true, st);
     ++nfev;
-    if (hmax <= cfg.step_tol) {
-      // Tiny step under damping: drop the damping and let undamped steps confirm.
+    if (hmax <= cfg.step_tol && !gn_rejected) {
+      // Tiny step under damping: drop the damping and let undamped steps confirm.  (Not after a rejected
+      // undamped step: that would cycle rejected -> mu_init -> tiny -> 0 -> rejected until max_iter;
+      // such a step goes through the acceptance test below, where it ends the iteration as stagnation.)
       st.mu = 0.0;
       nu = 2.0;
     } else if (st.f2 <= f2_old * (1.0 + 1e-12) + 1e-300) {
       // Accepted.  A damped step that no longer reduces ||r||^2 means the iteration sits at a
-      // least-squares compromise of an unreachable target (MINPACK's ftol exit, reference
-      // SolverConfig.ftol); report it converged so that the residual test rejects the state
-      // exactly like solver.py:735-747.
+      // least-squares compromise of an unreachable target, or at a root the undamped steps overshoot
+      // (MINPACK's ftol exit, reference SolverConfig.ftol); report it converged so that the residual
+      // test decides exactly like solver.py:735-747.
       if (st.mu > 0.0 && f2_old - st.f2 <= 1e-7 * f2_old) { *converged = true; break; }
-      // Relax the damping towards pure Gauss-Newton.
       if (st.mu > 0.0) {
-        st.mu *= (1.0 / 3.0);
-        if (st.mu < 1e-10) st.mu = 0.0;
+        // Gain-ratio update (Nielsen): rho = actual / predicted reduction; mu / 3 for a step the model
+        // predicted well, up to mu * 2 for one it did not.  Towards pure Gauss-Newton, but not back to it
+        // once an undamped step of this solve has been rejected.
+        const double rho = (f2_old - st.f2) / fmax(f2_old - f2_model, 1e-300);
+        const double t = 2.0 * rho - 1.0;
+        st.mu *= fmax(1.0 / 3.0, 1.0 - t * t * t);
+        if (st.mu < 1e-10 && !gn_rejected) st.mu = 0.0;
       }
       nu = 2.0;
     } else {
       okin_restore(pr, sm);
       okin_eval_rows(pr, sm, tval, true, st);
       ++nfev;
+      gn_rejected = gn_rejected || st.mu == 0.0;
       st.mu = st.mu > 0.0 ? st.mu * nu : cfg.mu_init;
       nu *= 2.0;
       if (st.mu > 1e12) break;
     }
+    // A damped iteration (after a rejected undamped step) that used up its budget has stagnated: it
+    // creeps along a weak direction towards a root or a least-squares compromise.  Report it converged,
+    // like the compromise exit above, so that the residual test decides on the current point.
+    if (gn_rejected && it == cfg.max_iter - 1) *converged = true;
   }
   return nfev;
 }

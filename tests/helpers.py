@@ -85,6 +85,13 @@ def oracle_problem(suspension, sweep_config, from_design: bool = True, structure
         state, constraints = suspension.structure()
     else:
         state, constraints = suspension.initial_state(), suspension.constraints()
+    heads, values = sweep_target_values(sweep_config)
+    return oracle_problem_of(state, constraints, suspension.derived_spec(), heads, from_design), values
+
+
+def oracle_problem_of(state, constraints, spec, heads, from_design: bool = True) -> OracleProblem:
+    """``(state, constraint declarations, derived spec, one PointTarget per sweep dimension)`` ->
+    ``OracleProblem``: the mapping of ``oracle_problem`` for a linkage built without a suspension."""
     cons = []
     for c in constraints:
         fam = _FAMILY[type(c)]
@@ -106,17 +113,15 @@ def oracle_problem(suspension, sweep_config, from_design: bool = True, structure
             consts = []
         design = from_design and fam in ("distance", "angle", "scalar_triple", "point_on_line")
         cons.append(OracleConstraint(fam, c.point_keys, list(map(float, consts)), design))
-    spec = suspension.derived_spec()
     from open_kinematics_b200.core.points.derived.manager import DerivedPointsManager
     derived = []
     for key in DerivedPointsManager(spec).update_order:
         fn = spec.functions[key]
         derived.append(OracleDerived(fn.OP, key, tuple(fn.inputs), float(fn.param),
                                      fn.design_projection if from_design else None))
-    heads, values = sweep_target_values(sweep_config)
     targets = [OracleTarget(h.point_id, resolve_target(h.direction).data.copy(),
                             TargetPositionMode(h.mode) == TargetPositionMode.RELATIVE) for h in heads]
-    return OracleProblem(sorted(state.positions), list(state.free_points_order), cons, derived, targets), values
+    return OracleProblem(sorted(state.positions), list(state.free_points_order), cons, derived, targets)
 
 
 def build_case(meta: dict):
