@@ -202,6 +202,84 @@ int okin_lean_calibration(okin_topology* topo, int32_t device, int32_t* register
  * (the roofline denominator; MEASURED_PEAKS.json carries no fp64 figure). */
 int okin_fp64_peak(int32_t device, double* tflops_out);
 
+/* ---- Tolerance studies ---------------------------------------------------------------------
+ * okin_study solves n_instances instances whose inputs are generated on the device from
+ * (seed, instance id) and reduces every wanted (step, quantity) over the instances on the device;
+ * nothing per instance crosses to the host.  Sampling contract (stable: changing it changes every
+ * study's draws).  Instance i (global, 0-based) draws n_variates variates z_v:
+ *   normal / uniform: one Philox4x32-10 call per variate, key = (lo32(seed), hi32(seed)),
+ *     counter = (lo32(i), hi32(i), v, 0) -> words x0..x3; u = ((x1 << 32 | x0) >> 11) * 2^-53,
+ *     u' = ((x3 << 32 | x2) >> 11) * 2^-53;
+ *     normal: z = sqrt(-2 log(1 - u)) * cospi(2 u');  uniform: z = 2u - 1 in [-1, 1)
+ *   grid (full factorial): node = i mod prod(L_g) over the grid variates, the first grid variate
+ *     varying fastest; d_g = mixed-radix digit g of node; z = d_g / (L_g - 1) * 2.0 - 1.0
+ * Coordinate c (3 * input slot + axis, then the params, n_coords = 3 * n_in_points + n_params) takes
+ *   value_c = nominal_c + scale_c * z_{source_c}   (nominal_c when source_c = -1).
+ * Reduction: a quantity's value at (instance, step) counts iff the step was accepted (status OK or
+ * step < failed_step) and the value is finite; accepted non-finite values (NaN = the reference's None,
+ * +inf tie markers) are counted in nonfinite.  Instances are cut into chunks of OKIN_STUDY_CHUNK,
+ * dealt round-robin over device_ids; within a chunk the moments are reduced in an order fixed by the
+ * instance indices alone and the chunk partials are folded on the host in global chunk order, so a
+ * result is bit-identical for any device list and any scheduling.  min / max carry the global id of
+ * the instance that produced them (smallest id on a tie).  Histograms: n_bins uniform bins on
+ * [hist_lo, hist_hi) plus an underflow (bin 0) and an overflow bin (bin n_bins + 1). */
+#define OKIN_STUDY_CHUNK 65536
+
+#define OKIN_VARIATE_NORMAL 0
+#define OKIN_VARIATE_UNIFORM 1
+#define OKIN_VARIATE_GRID 2
+
+#define OKIN_QUANTITY_POSITION 0      /* index = 3 * output slot + axis (positions_out column) */
+#define OKIN_QUANTITY_METRIC 1        /* index = metric column */
+#define OKIN_QUANTITY_MAX_RESIDUAL 2  /* index ignored */
+#define OKIN_QUANTITY_NFEV 3          /* index ignored */
+
+typedef struct okin_study_desc {
+  uint64_t seed;
+  int32_t n_variates;
+  const int32_t* variate_kind;    /* [n_variates] OKIN_VARIATE_* */
+  const int32_t* grid_levels;     /* [n_variates] L >= 2 for grid variates; ignored for the others */
+  int32_t n_coords;               /* 3 * n_in_points + n_params */
+  const double* nominal;          /* [n_coords] */
+  const int32_t* source;          /* [n_coords] variate index, or -1 = held at nominal */
+  const double* scale;            /* [n_coords] */
+  int32_t n_quantities;
+  const int32_t* quantity_kind;   /* [n_quantities] OKIN_QUANTITY_* */
+  const int32_t* quantity_index;  /* [n_quantities] */
+  int32_t n_bins;                 /* 0 (no histograms) .. 4096 */
+  const double* hist_lo;          /* [n_quantities] when n_bins > 0 */
+  const double* hist_hi;          /* [n_quantities] when n_bins > 0, > hist_lo */
+} okin_study_desc;
+
+/* Results of okin_study, host buffers, [S][Q] = [n_steps][n_quantities].  m2 = sum of squared
+ * deviations from the mean; mean / m2 / min / max are NaN and argmin / argmax -1 where count is 0. */
+typedef struct okin_study_out {
+  int64_t* count;           /* [S][Q] required */
+  int64_t* nonfinite;       /* [S][Q] required */
+  double* mean;             /* [S][Q] required */
+  double* m2;               /* [S][Q] required */
+  double* min;              /* [S][Q] required */
+  double* max;              /* [S][Q] required */
+  int64_t* argmin;          /* [S][Q] required, global instance id */
+  int64_t* argmax;          /* [S][Q] required, global instance id */
+  int64_t* histogram;       /* [S][Q][n_bins + 2], required when n_bins > 0 */
+  int64_t* status_counts;   /* [4] instances per OKIN_STATUS_*, required */
+  int64_t* failed_at_step;  /* [S] instances whose first failed step is s, required */
+} okin_study_out;
+
+/* Generate, solve and reduce n_instances instances (positions-only quantities use the lean kernel
+ * family, a metric quantity the full one).  Device memory is bounded by the chunk size, host memory
+ * by the number of devices; neither grows with n_instances. */
+int okin_study(okin_topology* topo, const okin_solver_cfg* cfg, int64_t n_instances, int32_t n_steps,
+               const double* target_values, const okin_study_desc* desc, okin_study_out* out,
+               const int32_t* device_ids, int32_t n_devices);
+
+/* The inputs okin_study generates for the instances instance_ids[0..n_ids), generated on `device`:
+ * hardpoints_out [n_ids][n_in_points*3], params_out [n_ids][n_params] (may be NULL when n_params = 0).
+ * The quantity fields of desc are not read. */
+int okin_study_sample(okin_topology* topo, const okin_study_desc* desc, int64_t n_ids, const int64_t* instance_ids,
+                      double* hardpoints_out, double* params_out, int32_t device);
+
 int okin_last_error(char* buf, int32_t len);
 
 #ifdef __cplusplus

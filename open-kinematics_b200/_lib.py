@@ -69,6 +69,38 @@ class TopologyInfo(ctypes.Structure):
         "smem_bytes_per_instance", "n_levels", "n_metrics", "n_params", "n_diagnostics")]
 
 
+class StudyDesc(ctypes.Structure):
+    """``okin_study_desc``: sampling tables and quantity list of a tolerance study (host addresses)."""
+    _fields_ = [("seed", ctypes.c_uint64), ("n_variates", ctypes.c_int32), ("variate_kind", ctypes.c_void_p),
+                ("grid_levels", ctypes.c_void_p), ("n_coords", ctypes.c_int32), ("nominal", ctypes.c_void_p),
+                ("source", ctypes.c_void_p), ("scale", ctypes.c_void_p), ("n_quantities", ctypes.c_int32),
+                ("quantity_kind", ctypes.c_void_p), ("quantity_index", ctypes.c_void_p), ("n_bins", ctypes.c_int32),
+                ("hist_lo", ctypes.c_void_p), ("hist_hi", ctypes.c_void_p)]
+
+    @classmethod
+    def of(cls, arrays: dict, seed: int = 0, n_bins: int = 0) -> "StudyDesc":
+        """From the int32 / float64 arrays ``variate_kind``, ``grid_levels``, ``nominal``, ``source``,
+        ``scale``, ``quantity_kind``, ``quantity_index``, ``hist_lo``, ``hist_hi`` (kept alive by the
+        caller; missing ones are NULL)."""
+        d = cls()
+        d.seed = int(seed) & 0xFFFFFFFFFFFFFFFF
+        d.n_bins = int(n_bins)
+        for name, arr in arrays.items():
+            if arr is not None:
+                setattr(d, name, arr.ctypes.data)
+        d.n_variates = len(arrays["variate_kind"])
+        d.n_coords = len(arrays["nominal"])
+        d.n_quantities = len(arrays["quantity_kind"]) if arrays.get("quantity_kind") is not None else 0
+        return d
+
+
+class StudyOut(ctypes.Structure):
+    """``okin_study_out``: host result buffers of ``okin_study``."""
+    FIELDS = ("count", "nonfinite", "mean", "m2", "min", "max", "argmin", "argmax", "histogram", "status_counts",
+              "failed_at_step")
+    _fields_ = [(n, ctypes.c_void_p) for n in FIELDS]
+
+
 # name -> (restype, argtypes); also the list the "exports every declared symbol" test checks.
 SIGNATURES = {
     "okin_device_count": (ctypes.c_int, [ctypes.POINTER(ctypes.c_int)]),
@@ -90,6 +122,12 @@ SIGNATURES = {
     "okin_lean_calibration": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int32, c_i32p, c_f64p, c_f64p]),
     "okin_host_alloc": (ctypes.c_int, [ctypes.c_int64, ctypes.c_int32, ctypes.POINTER(ctypes.c_void_p)]),
     "okin_host_free": (ctypes.c_int, [ctypes.c_void_p]),
+    "okin_study": (ctypes.c_int, [
+        ctypes.c_void_p, ctypes.POINTER(SolverCfg), ctypes.c_int64, ctypes.c_int32, ctypes.c_void_p,
+        ctypes.POINTER(StudyDesc), ctypes.POINTER(StudyOut), ctypes.c_void_p, ctypes.c_int32]),
+    "okin_study_sample": (ctypes.c_int, [
+        ctypes.c_void_p, ctypes.POINTER(StudyDesc), ctypes.c_int64, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_void_p,
+        ctypes.c_int32]),
     "okin_last_error": (ctypes.c_int, [ctypes.c_char_p, ctypes.c_int32]),
 }
 
@@ -232,6 +270,41 @@ class DeviceTopology:
             self.close()
         except Exception:  # noqa: BLE001 - interpreter shutdown
             pass
+
+    # -- tolerance studies ------------------------------------------------------------
+    def study(self, target_values: np.ndarray, n_instances: int, desc: StudyDesc, cfg: SolverCfg | None = None,
+              devices=None) -> dict:
+        """``okin_study``: generate, solve and reduce ``n_instances`` instances on the device(s).
+        Returns the ``okin_study_out`` arrays, ``[n_steps, n_quantities]`` each (``histogram``
+        ``[n_steps, n_quantities, n_bins + 2]`` or None, ``status_counts`` [4], ``failed_at_step``
+        [n_steps])."""
+        require_device()
+        tv = np.ascontiguousarray(target_values, dtype=np.float64)
+        nt = len(self.program.target_points)
+        if tv.ndim != 2 or tv.shape[0] != nt:
+            raise ValueError(f"target_values must have shape ({nt}, n_steps), got {tv.shape}")
+        S, Q, nb = tv.shape[1], desc.n_quantities, desc.n_bins
+        out = {name: np.zeros((S, Q), np.int64 if name in ("count", "nonfinite", "argmin", "argmax") else np.float64)
+               for name in StudyOut.FIELDS[:8]}
+        out["histogram"] = np.zeros((S, Q, nb + 2), np.int64) if nb > 0 else None
+        out["status_counts"] = np.zeros(4, np.int64)
+        out["failed_at_step"] = np.zeros(S, np.int64)
+        o = StudyOut(**{k: (v.ctypes.data if v is not None else None) for k, v in out.items()})
+        dev = np.ascontiguousarray(devices if devices is not None else [0], dtype=np.int32)
+        check(load().okin_study(self.handle, ctypes.byref(cfg or default_cfg()), int(n_instances), S, tv.ctypes.data,
+                                ctypes.byref(desc), ctypes.byref(o), dev.ctypes.data, dev.size), "okin_study")
+        return out
+
+    def study_sample(self, desc: StudyDesc, ids, device: int = 0) -> tuple:
+        """``okin_study_sample``: the generated ``(hardpoints [n, n_in*3], params [n, n_params])`` of
+        the instances ``ids``."""
+        require_device()
+        ids = np.ascontiguousarray(ids, dtype=np.int64).reshape(-1)
+        hp = np.zeros((ids.size, 3 * self.program.n_in))
+        par = np.zeros((ids.size, len(self.program.param_names)))
+        check(load().okin_study_sample(self.handle, ctypes.byref(desc), ids.size, ids.ctypes.data, hp.ctypes.data,
+                                       par.ctypes.data if par.size else None, device), "okin_study_sample")
+        return hp, par
 
     # -- host buffers ------------------------------------------------------------------
     def solve_batch(self, hardpoints: np.ndarray, target_values: np.ndarray, cfg: SolverCfg | None = None,

@@ -204,6 +204,25 @@ class BatchSolver:
                                 res.get("worst_row"), res.get("design"), res.get("hardpoint_sensitivity"),
                                 list(self.program.sensitivity_inputs) if want_hardpoint_sensitivity else None)
 
+    def study(self, sampling, n_instances: int, seed: int = 0, points=None, metrics=None, solver_quantities=(),
+              histograms=None, bins: int = 64, solver_config: SolverConfig = SolverConfig(), devices=None):
+        """Tolerance study (core/study.py): ``n_instances`` instances drawn by ``sampling``
+        (a ``Sampling`` of this solver) from ``(seed, instance id)``, generated, solved and reduced on
+        the device(s) ``devices`` (default ``[0]``).  Quantities: ``points`` (output point keys or
+        names, or ``"all"``: ``<point>_{x,y,z}``), ``metrics`` (metric names or ``"all"``) and
+        ``solver_quantities`` (``"solver_max_residual"``, ``"solver_nfev"``).  ``histograms``:
+        optional ``{quantity: (lo, hi)}`` for every quantity, ``bins`` bins each.  Returns a
+        ``StudyResult``; the result does not depend on ``devices``."""
+        from .study import run_study
+        return run_study(self, sampling, n_instances, seed, points, metrics, solver_quantities, histograms, bins,
+                         solver_config, devices)
+
+    def study_inputs(self, sampling, seed: int, ids, device: int = 0) -> tuple:
+        """``(hardpoints [n, n_in*3], params [n, n_params])`` a study with ``sampling`` and ``seed``
+        gives the instances ``ids``, ready for ``solve(hardpoints, params=params)``."""
+        from .study import study_inputs
+        return study_inputs(self, sampling, seed, ids, device)
+
     def pinned_hardpoints(self, n_instances: int, device: int = 0) -> np.ndarray:
         """Page-locked ``[n_instances, n_in*3]`` input array (fill it, pass it to ``solve``)."""
         return _lib.pinned_empty((n_instances, 3 * self.program.n_in), np.float64, device)

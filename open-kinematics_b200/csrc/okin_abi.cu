@@ -17,6 +17,7 @@
 #include <sched.h>
 
 #include <algorithm>
+#include <condition_variable>
 #include <cstddef>
 #include <cstdio>
 #include <cstdlib>
@@ -29,6 +30,7 @@
 
 #include "../../include/okin.h"
 #include "okin_core.cuh"
+#include "okin_study.cuh"
 
 // Kernel families.  The register cap follows from the CTA size limit (65536 / threads):
 //   full outputs        512 threads -> 128 registers, up to 16 warps per SM
@@ -232,6 +234,88 @@ __global__ void okin_dfma_kernel(double* out, int iters, double a, double b) {
     x4 = fma(x4, a, b); x5 = fma(x5, a, b); x6 = fma(x6, a, b); x7 = fma(x7, a, b);
   }
   out[(size_t)blockIdx.x * blockDim.x + threadIdx.x] = x0 + x1 + x2 + x3 + x4 + x5 + x6 + x7;
+}
+
+// ---- tolerance studies (okin_study.cuh) ------------------------------------------------------
+// Inputs of instances base + r (ids == NULL) or ids[r], r < count: one thread per coordinate.
+__global__ void okin_study_generate(OkinStudyTables t, long long base, const long long* __restrict__ ids,
+                                    long long count, int nin3, int npar, double* __restrict__ hp,
+                                    double* __restrict__ par) {
+  const long long total = count * t.n_coords;
+  for (long long k = (long long)blockIdx.x * blockDim.x + threadIdx.x; k < total;
+       k += (long long)gridDim.x * blockDim.x) {
+    const long long r = k / t.n_coords;
+    const int c = (int)(k - r * t.n_coords);
+    const double v = okin_study_coord(t, (uint64_t)(ids ? ids[r] : base + r), c);
+    if (c < nin3) hp[r * nin3 + c] = v;
+    else par[r * npar + (c - nin3)] = v;
+  }
+}
+
+// Grid (ceil(S*Q / 32), OKIN_STUDY_GROUPS), block (32, OKIN_STUDY_GROUP): lane x owns column
+// j = s * Q + q of the block's 32, row y of the block partition blockIdx.y * GROUP + y, which it
+// reduces over the chunk rows p, p + PARTS, ...; the block then merges its GROUP partitions in order
+// into groups[blockIdx.y][j].  Histogram counts go to `hist` through a per-block shared copy when
+// `hist_shared` (n_bins small enough), else directly; status counts are taken by column block 0.
+__global__ void __launch_bounds__(32 * OKIN_STUDY_GROUP)
+okin_study_reduce(OkinStudyChunk ch, long long rows, long long base, int Q, const int32_t* __restrict__ qkind,
+                  const int32_t* __restrict__ qindex, int n_bins, const double* __restrict__ lo,
+                  const double* __restrict__ hi, int hist_shared, OkinMoments* __restrict__ groups,
+                  unsigned long long* hist, unsigned long long* status_counts, unsigned long long* failed_at_step) {
+  __shared__ OkinMoments part[OKIN_STUDY_GROUP][32];
+  unsigned long long* sh = reinterpret_cast<unsigned long long*>(okin_smem);
+  const int SQ = ch.n_steps * Q, tx = threadIdx.x, ty = threadIdx.y, nb2 = n_bins + 2;
+  const int j = blockIdx.x * 32 + tx, p = blockIdx.y * OKIN_STUDY_GROUP + ty;
+  if (hist_shared)
+    for (int k = ty * 32 + tx; k < 32 * nb2; k += 32 * OKIN_STUDY_GROUP) sh[k] = 0ull;
+  __syncthreads();
+  OkinMoments m;
+  okin_moments_clear(m);
+  if (j < SQ) {
+    const int s = j / Q, q = j - s * Q, kind = qkind[q], index = qindex[q];
+    const double l = n_bins ? lo[q] : 0.0, h = n_bins ? hi[q] : 0.0;
+    for (long long r = p; r < rows; r += OKIN_STUDY_PARTS) {
+      double x;
+      if (!okin_study_fetch(ch, kind, index, r, s, &x)) continue;
+      okin_moments_push(m, x, base + r);
+      if (n_bins && isfinite(x)) {
+        const int b = okin_study_bin(x, l, h, n_bins);
+        if (hist_shared) atomicAdd(&sh[tx * nb2 + b], 1ull);
+        else atomicAdd(&hist[(size_t)j * nb2 + b], 1ull);
+      }
+    }
+  }
+  part[ty][tx] = m;
+  if (blockIdx.x == 0 && tx == 0) {
+    unsigned long long sc[4] = {0ull, 0ull, 0ull, 0ull};
+    for (long long r = p; r < rows; r += OKIN_STUDY_PARTS) {
+      const int st = ch.status[r], f = ch.failed_step[r];
+      if (st >= 0 && st < 4) ++sc[st];
+      if (f >= 0 && f < ch.n_steps) atomicAdd(&failed_at_step[f], 1ull);
+    }
+    for (int k = 0; k < 4; ++k)
+      if (sc[k]) atomicAdd(&status_counts[k], sc[k]);
+  }
+  __syncthreads();
+  if (ty == 0 && j < SQ) {
+    OkinMoments g = part[0][tx];
+    for (int k = 1; k < OKIN_STUDY_GROUP; ++k) okin_moments_merge(g, part[k][tx]);
+    groups[(size_t)blockIdx.y * SQ + j] = g;
+  }
+  if (hist_shared)
+    for (int k = ty * 32 + tx; k < 32 * nb2; k += 32 * OKIN_STUDY_GROUP) {
+      const int col = blockIdx.x * 32 + k / nb2;
+      if (sh[k] && col < SQ) atomicAdd(&hist[(size_t)col * nb2 + k % nb2], sh[k]);
+    }
+}
+
+// chunk[j] = groups[0][j] (+) groups[1][j] (+) ... in group order.
+__global__ void okin_study_merge(const OkinMoments* __restrict__ groups, int SQ, OkinMoments* __restrict__ chunk) {
+  const int j = blockIdx.x * blockDim.x + threadIdx.x;
+  if (j >= SQ) return;
+  OkinMoments g = groups[j];
+  for (int k = 1; k < OKIN_STUDY_GROUPS; ++k) okin_moments_merge(g, groups[(size_t)k * SQ + j]);
+  chunk[j] = g;
 }
 
 namespace {
@@ -619,6 +703,295 @@ void run_shard(okin_topology* t, const okin_solver_cfg* cfg, const HostBatch& hb
 #undef OKIN_SHARD_CUDA
 }
 
+// ---- tolerance studies ------------------------------------------------------------------------
+// Generator part of a study descriptor; fills the mixed-radix place values of the grid variates.
+int study_check_generator(const okin_topology* t, const okin_study_desc* desc, std::vector<uint64_t>* stride,
+                          uint64_t* period) {
+  if (!t || !desc) return fail(OKIN_ERR_USAGE, "null topology or study descriptor");
+  const int32_t* h = t->hdr.data();
+  const int nc = 3 * h[OKIN_H_NIN] + h[OKIN_H_NPARAM], nv = desc->n_variates;
+  if (desc->n_coords != nc) return fail(OKIN_ERR_USAGE, "study n_coords must be 3 * n_in_points + n_params");
+  if (nv < 0) return fail(OKIN_ERR_USAGE, "negative n_variates");
+  if (!desc->nominal || !desc->source || !desc->scale || (nv > 0 && (!desc->variate_kind || !desc->grid_levels)))
+    return fail(OKIN_ERR_USAGE, "null study generator table");
+  for (int v = 0; v < nv; ++v) {
+    const int kind = desc->variate_kind[v];
+    if (kind < OKIN_VARIATE_NORMAL || kind > OKIN_VARIATE_GRID) return fail(OKIN_ERR_USAGE, "unknown variate kind");
+    if (kind == OKIN_VARIATE_GRID && desc->grid_levels[v] < 2)
+      return fail(OKIN_ERR_USAGE, "a grid variate needs at least 2 levels");
+  }
+  stride->assign(nv + 1, 0);
+  okin_study_grid_places(nv, desc->variate_kind, desc->grid_levels, stride->data(), period);
+  for (int c = 0; c < nc; ++c) {
+    if (desc->source[c] < -1 || desc->source[c] >= nv) return fail(OKIN_ERR_USAGE, "study source out of range");
+    if (!std::isfinite(desc->nominal[c]) || !std::isfinite(desc->scale[c]))
+      return fail(OKIN_ERR_USAGE, "non-finite study nominal or scale");
+  }
+  return OKIN_OK;
+}
+
+int study_check_quantities(const okin_topology* t, int32_t n_steps, const okin_study_desc* desc,
+                           const okin_study_out* out) {
+  const int32_t* h = t->hdr.data();
+  const int Q = desc->n_quantities;
+  if (Q < 1) return fail(OKIN_ERR_USAGE, "a study needs at least one quantity");
+  if (!desc->quantity_kind || !desc->quantity_index) return fail(OKIN_ERR_USAGE, "null study quantity table");
+  for (int q = 0; q < Q; ++q) {
+    const int kind = desc->quantity_kind[q], index = desc->quantity_index[q];
+    if (kind == OKIN_QUANTITY_POSITION) {
+      if (index < 0 || index >= 3 * h[OKIN_H_NOUT]) return fail(OKIN_ERR_USAGE, "study position quantity out of range");
+    } else if (kind == OKIN_QUANTITY_METRIC) {
+      if (!h[OKIN_H_NM]) return fail(OKIN_ERR_USAGE, "metric quantity on a topology compiled without a metric program");
+      if (index < 0 || index >= h[OKIN_H_NM]) return fail(OKIN_ERR_USAGE, "study metric quantity out of range");
+    } else if (kind != OKIN_QUANTITY_MAX_RESIDUAL && kind != OKIN_QUANTITY_NFEV) {
+      return fail(OKIN_ERR_USAGE, "unknown study quantity kind");
+    }
+  }
+  if (desc->n_bins < 0 || desc->n_bins > 4096) return fail(OKIN_ERR_USAGE, "n_bins must lie in 0..4096");
+  if (desc->n_bins > 0) {
+    if (!desc->hist_lo || !desc->hist_hi) return fail(OKIN_ERR_USAGE, "null histogram range");
+    for (int q = 0; q < Q; ++q)
+      if (!std::isfinite(desc->hist_lo[q]) || !std::isfinite(desc->hist_hi[q]) || !(desc->hist_lo[q] < desc->hist_hi[q]))
+        return fail(OKIN_ERR_USAGE, "histogram range needs finite lo < hi");
+  }
+  if (!out || !out->count || !out->nonfinite || !out->mean || !out->m2 || !out->min || !out->max || !out->argmin ||
+      !out->argmax || !out->status_counts || !out->failed_at_step || (desc->n_bins > 0 && !out->histogram))
+    return fail(OKIN_ERR_USAGE, "null study output");
+  (void)n_steps;
+  return OKIN_OK;
+}
+
+// Device allocations of one study call on one device, released together.
+struct DeviceAllocs {
+  std::vector<void*> dev, host;
+  ~DeviceAllocs() {
+    for (void* p : dev) cudaFree(p);
+    for (void* p : host) cudaFreeHost(p);
+  }
+  template <class T>
+  cudaError_t alloc(T** p, size_t n) {
+    *p = nullptr;
+    const cudaError_t e = cudaMalloc((void**)p, std::max<size_t>(n, 1) * sizeof(T));
+    if (e == cudaSuccess) dev.push_back(*p);
+    return e;
+  }
+  template <class T>
+  cudaError_t alloc_host(T** p, size_t n) {
+    *p = nullptr;
+    const cudaError_t e = cudaHostAlloc((void**)p, std::max<size_t>(n, 1) * sizeof(T), cudaHostAllocPortable);
+    if (e == cudaSuccess) host.push_back(*p);
+    return e;
+  }
+};
+
+// The generator tables of `desc` on the current device.
+int upload_study_tables(const okin_study_desc* desc, const std::vector<uint64_t>& stride, uint64_t period,
+                        DeviceAllocs& a, OkinStudyTables* t) {
+  const int nc = desc->n_coords, nv = desc->n_variates;
+  double *nominal, *scale;
+  int32_t *source, *kind, *levels;
+  uint64_t* st;
+  OKIN_CUDA(a.alloc(&nominal, nc));
+  OKIN_CUDA(a.alloc(&scale, nc));
+  OKIN_CUDA(a.alloc(&source, nc));
+  OKIN_CUDA(a.alloc(&kind, nv));
+  OKIN_CUDA(a.alloc(&levels, nv));
+  OKIN_CUDA(a.alloc(&st, nv));
+  OKIN_CUDA(cudaMemcpy(nominal, desc->nominal, nc * sizeof(double), cudaMemcpyHostToDevice));
+  OKIN_CUDA(cudaMemcpy(scale, desc->scale, nc * sizeof(double), cudaMemcpyHostToDevice));
+  OKIN_CUDA(cudaMemcpy(source, desc->source, nc * sizeof(int32_t), cudaMemcpyHostToDevice));
+  if (nv > 0) {
+    OKIN_CUDA(cudaMemcpy(kind, desc->variate_kind, nv * sizeof(int32_t), cudaMemcpyHostToDevice));
+    OKIN_CUDA(cudaMemcpy(levels, desc->grid_levels, nv * sizeof(int32_t), cudaMemcpyHostToDevice));
+    OKIN_CUDA(cudaMemcpy(st, stride.data(), nv * sizeof(uint64_t), cudaMemcpyHostToDevice));
+  }
+  *t = OkinStudyTables{desc->seed, period, nc, nominal, scale, source, kind, levels, st};
+  return OKIN_OK;
+}
+
+int launch_study_generate(const OkinStudyTables& t, long long base, const long long* ids, long long count, int nin3,
+                          int npar, double* hp, double* par, int num_sms, cudaStream_t stream) {
+  if (count == 0) return OKIN_OK;
+  const long long total = count * t.n_coords;
+  const int grid = (int)std::min<long long>((total + 255) / 256, (long long)num_sms * 16);
+  okin_study_generate<<<grid, 256, 0, stream>>>(t, base, ids, count, nin3, npar, hp, par);
+  OKIN_CUDA(cudaGetLastError());
+  return OKIN_OK;
+}
+
+// State shared by the device threads of one okin_study call.  Chunk k goes to device k % G; a device
+// starts chunk k only when k < next + window, so the reorder ring (window = G x slots chunk partials)
+// never overflows and host memory does not grow with the number of instances.
+struct StudyRun {
+  okin_topology* t;
+  const okin_solver_cfg* cfg;
+  int64_t n;
+  int32_t S;
+  const double* target_values;
+  const okin_study_desc* desc;
+  std::vector<uint64_t> stride;
+  uint64_t period = 0;
+  int Q = 0, SQ = 0, nb = 0, n_devices = 0, slots = 0;
+  bool want_pos = false, want_met = false;
+  int64_t n_chunks = 0, window = 0;
+  std::mutex mu;
+  std::condition_variable cv;
+  int64_t next = 0;
+  bool abort = false;
+  std::vector<std::vector<OkinMoments>> ring;
+  std::vector<char> have;
+  std::vector<OkinMoments> acc;
+
+  void deliver(int64_t k, const OkinMoments* part) {
+    std::lock_guard<std::mutex> lock(mu);
+    const size_t r = (size_t)(k % window);
+    ring[r].assign(part, part + SQ);
+    have[r] = 1;
+    while (next < n_chunks && have[(size_t)(next % window)]) {
+      const size_t rr = (size_t)(next % window);
+      for (int j = 0; j < SQ; ++j) okin_moments_merge(acc[j], ring[rr][j]);
+      have[rr] = 0;
+      ++next;
+    }
+    cv.notify_all();
+  }
+  bool wait_window(int64_t k) {
+    std::unique_lock<std::mutex> lock(mu);
+    cv.wait(lock, [&] { return abort || k < next + window; });
+    return !abort;
+  }
+  void stop() {
+    std::lock_guard<std::mutex> lock(mu);
+    abort = true;
+    cv.notify_all();
+  }
+};
+
+// Integer results of one device (exact in any order, summed over devices at the end).
+struct StudyShard {
+  int index = 0, device = 0;
+  DeviceCopy* d = nullptr;
+  std::vector<unsigned long long> hist, status, failed_at;
+  int rc = OKIN_OK;
+  std::string err;
+};
+
+int run_study_shard_body(StudyRun& run, StudyShard& sh, DeviceAllocs& a) {
+  DeviceCopy* d = sh.d;
+  OKIN_CUDA(cudaSetDevice(sh.device));
+  const int32_t* h = run.t->hdr.data();
+  const int nin3 = 3 * h[OKIN_H_NIN], npar = h[OKIN_H_NPARAM], nout3 = 3 * h[OKIN_H_NOUT], nm = h[OKIN_H_NM];
+  const int nt = h[OKIN_H_NT], S = run.S, Q = run.Q, SQ = run.SQ, nb = run.nb;
+  const size_t CH = OKIN_STUDY_CHUNK;
+  const int64_t G = run.n_devices;
+  const int64_t n_mine = run.n_chunks > sh.index ? (run.n_chunks - sh.index + G - 1) / G : 0;
+  const int slots = (int)std::min<int64_t>(run.slots, n_mine);
+  OkinStudyTables tab;
+  int rc = upload_study_tables(run.desc, run.stride, run.period, a, &tab);
+  if (rc) return rc;
+  int32_t *qkind, *qindex;
+  double *lo = nullptr, *hi = nullptr, *tv = nullptr;
+  OKIN_CUDA(a.alloc(&qkind, Q));
+  OKIN_CUDA(a.alloc(&qindex, Q));
+  OKIN_CUDA(cudaMemcpy(qkind, run.desc->quantity_kind, Q * sizeof(int32_t), cudaMemcpyHostToDevice));
+  OKIN_CUDA(cudaMemcpy(qindex, run.desc->quantity_index, Q * sizeof(int32_t), cudaMemcpyHostToDevice));
+  if (nb) {
+    OKIN_CUDA(a.alloc(&lo, Q));
+    OKIN_CUDA(a.alloc(&hi, Q));
+    OKIN_CUDA(cudaMemcpy(lo, run.desc->hist_lo, Q * sizeof(double), cudaMemcpyHostToDevice));
+    OKIN_CUDA(cudaMemcpy(hi, run.desc->hist_hi, Q * sizeof(double), cudaMemcpyHostToDevice));
+  }
+  if ((size_t)nt * S) {
+    OKIN_CUDA(a.alloc(&tv, (size_t)nt * S));
+    OKIN_CUDA(cudaMemcpy(tv, run.target_values, (size_t)nt * S * sizeof(double), cudaMemcpyHostToDevice));
+  }
+  const size_t nb2 = (size_t)nb + 2, n_hist = nb ? (size_t)SQ * nb2 : 0;
+  unsigned long long *hist = nullptr, *status_counts, *failed_at;
+  if (n_hist) OKIN_CUDA(a.alloc(&hist, n_hist));
+  OKIN_CUDA(a.alloc(&status_counts, 4));
+  OKIN_CUDA(a.alloc(&failed_at, S));
+  if (n_hist) OKIN_CUDA(cudaMemset(hist, 0, n_hist * sizeof(unsigned long long)));
+  OKIN_CUDA(cudaMemset(status_counts, 0, 4 * sizeof(unsigned long long)));
+  OKIN_CUDA(cudaMemset(failed_at, 0, std::max(S, 1) * sizeof(unsigned long long)));
+  struct Slot {
+    double *hp = nullptr, *par = nullptr, *pos = nullptr, *met = nullptr, *res = nullptr;
+    int32_t *iters = nullptr, *status = nullptr, *failed = nullptr;
+    OkinMoments *groups = nullptr, *chunk = nullptr, *host = nullptr;
+  } slot[OKIN_PIPE_SLOTS];
+  for (int k = 0; k < slots; ++k) {
+    Slot& s = slot[k];
+    OKIN_CUDA(a.alloc(&s.hp, CH * nin3));
+    if (npar) OKIN_CUDA(a.alloc(&s.par, CH * npar));
+    if (run.want_pos) OKIN_CUDA(a.alloc(&s.pos, CH * S * nout3));
+    if (run.want_met) OKIN_CUDA(a.alloc(&s.met, CH * S * nm));
+    OKIN_CUDA(a.alloc(&s.res, CH * S));
+    OKIN_CUDA(a.alloc(&s.iters, CH * S));
+    OKIN_CUDA(a.alloc(&s.status, CH));
+    OKIN_CUDA(a.alloc(&s.failed, CH));
+    OKIN_CUDA(a.alloc(&s.groups, (size_t)OKIN_STUDY_GROUPS * SQ));
+    OKIN_CUDA(a.alloc(&s.chunk, SQ));
+    OKIN_CUDA(a.alloc_host(&s.host, SQ));
+  }
+  const int hist_shared = nb && 32 * nb2 * sizeof(unsigned long long) <= 32 * 1024;
+  const size_t hist_smem = hist_shared ? 32 * nb2 * sizeof(unsigned long long) : 0;
+  auto finish = [&](int64_t l) -> int {   // deliver the partial of this device's l-th chunk
+    OKIN_CUDA(cudaStreamSynchronize(d->streams[l % slots]));
+    run.deliver(sh.index + l * G, slot[l % slots].host);
+    return OKIN_OK;
+  };
+  for (int64_t l = 0; l < n_mine; ++l) {
+    const int64_t k = sh.index + l * G;
+    Slot& s = slot[l % slots];
+    cudaStream_t st = d->streams[l % slots];
+    if (l >= slots && (rc = finish(l - slots))) return rc;
+    if (!run.wait_window(k)) return fail(OKIN_ERR_CUDA, "study stopped by another device's error");
+    const long long base = k * (long long)CH, c = std::min<long long>((long long)CH, run.n - base);
+    rc = launch_study_generate(tab, base, nullptr, c, nin3, npar, s.hp, s.par, d->num_sms, st);
+    if (rc) return rc;
+    okin_batch_io io{};
+    io.hardpoints = s.hp;
+    io.params = s.par;
+    io.target_values = tv;
+    io.status = s.status;
+    io.failed_step = s.failed;
+    io.positions = s.pos;
+    io.iters = s.iters;
+    io.max_residual = s.res;
+    io.metrics = s.met;
+    rc = launch(run.t, d, run.cfg, st, c, S, io);
+    if (rc) return rc;
+    const OkinStudyChunk ch{s.pos, s.met, s.iters, s.res, s.status, s.failed, S, nout3, nm};
+    okin_study_reduce<<<dim3((SQ + 31) / 32, OKIN_STUDY_GROUPS), dim3(32, OKIN_STUDY_GROUP), hist_smem, st>>>(
+        ch, c, base, Q, qkind, qindex, nb, lo, hi, hist_shared, s.groups, hist, status_counts, failed_at);
+    OKIN_CUDA(cudaGetLastError());
+    okin_study_merge<<<(SQ + 127) / 128, 128, 0, st>>>(s.groups, SQ, s.chunk);
+    OKIN_CUDA(cudaGetLastError());
+    OKIN_CUDA(cudaMemcpyAsync(s.host, s.chunk, SQ * sizeof(OkinMoments), cudaMemcpyDeviceToHost, st));
+  }
+  for (int64_t l = std::max<int64_t>(0, n_mine - slots); l < n_mine; ++l)
+    if ((rc = finish(l))) return rc;
+  sh.hist.assign(n_hist, 0);
+  sh.status.assign(4, 0);
+  sh.failed_at.assign(S, 0);
+  if (n_hist) OKIN_CUDA(cudaMemcpy(sh.hist.data(), hist, n_hist * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
+  OKIN_CUDA(cudaMemcpy(sh.status.data(), status_counts, 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
+  if (S) OKIN_CUDA(cudaMemcpy(sh.failed_at.data(), failed_at, S * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
+  return OKIN_OK;
+}
+
+void run_study_shard(StudyRun& run, StudyShard& sh) {
+  {
+    DeviceAllocs a;
+    sh.rc = run_study_shard_body(run, sh, a);
+    if (sh.rc) {
+      sh.err = g_last_error;
+      run.stop();
+    }
+    // nothing may still run on the buffers `a` releases
+    for (int k = 0; k < OKIN_PIPE_SLOTS; ++k) cudaStreamSynchronize(sh.d->streams[k]);
+  }
+}
+
 }  // namespace
 
 extern "C" {
@@ -810,6 +1183,122 @@ int okin_solve_batch(okin_topology* t, const okin_solver_cfg* cfg, int64_t n_ins
   }
   for (const Shard& sh : shards)
     if (sh.rc) return fail(sh.rc, sh.err);
+  return OKIN_OK;
+}
+
+int okin_study(okin_topology* t, const okin_solver_cfg* cfg, int64_t n_instances, int32_t n_steps,
+               const double* target_values, const okin_study_desc* desc, okin_study_out* out,
+               const int32_t* device_ids, int32_t n_devices) {
+  StudyRun run;
+  int rc = study_check_generator(t, desc, &run.stride, &run.period);
+  if (rc) return rc;
+  if (!cfg) return fail(OKIN_ERR_USAGE, "null solver config");
+  if (n_instances < 0 || n_steps < 0) return fail(OKIN_ERR_USAGE, "negative size");
+  if (n_steps == 0) return fail(OKIN_ERR_USAGE, "a study needs at least one sweep step");
+  if (t->hdr[OKIN_H_NT] > 0 && !target_values) return fail(OKIN_ERR_USAGE, "null target_values");
+  if (cfg->max_iter < 1 || !(cfg->step_tol > 0.0) || !(cfg->coarse_tol >= cfg->step_tol))
+    return fail(OKIN_ERR_USAGE, "invalid solver config");
+  if ((rc = study_check_quantities(t, n_steps, desc, out))) return rc;
+  const int32_t default_dev = 0;
+  if (!device_ids || n_devices <= 0) {
+    device_ids = &default_dev;
+    n_devices = 1;
+  }
+  if (n_devices > OKIN_MAX_DEVICES) return fail(OKIN_ERR_USAGE, "too many devices");
+  for (int a = 0; a < n_devices; ++a)
+    for (int b = a + 1; b < n_devices; ++b)
+      if (device_ids[a] == device_ids[b]) return fail(OKIN_ERR_USAGE, "device listed twice");
+  run.t = t;
+  run.cfg = cfg;
+  run.n = n_instances;
+  run.S = n_steps;
+  run.target_values = target_values;
+  run.desc = desc;
+  run.Q = desc->n_quantities;
+  run.SQ = n_steps * run.Q;
+  run.nb = desc->n_bins;
+  run.n_devices = n_devices;
+  run.slots = OKIN_PIPE_SLOTS;
+  for (int q = 0; q < run.Q; ++q) {
+    run.want_pos |= desc->quantity_kind[q] == OKIN_QUANTITY_POSITION;
+    run.want_met |= desc->quantity_kind[q] == OKIN_QUANTITY_METRIC;
+  }
+  run.n_chunks = (n_instances + OKIN_STUDY_CHUNK - 1) / OKIN_STUDY_CHUNK;
+  run.window = (int64_t)n_devices * run.slots;
+  run.ring.resize(run.window);
+  run.have.assign(run.window, 0);
+  run.acc.resize(run.SQ);
+  for (OkinMoments& m : run.acc) okin_moments_clear(m);
+  std::vector<StudyShard> shards(n_devices);
+  for (int k = 0; k < n_devices; ++k) {
+    shards[k].index = k;
+    shards[k].device = device_ids[k];
+    if ((rc = ensure_device(t, device_ids[k], &shards[k].d))) return rc;
+  }
+  if (n_devices == 1) {
+    run_study_shard(run, shards[0]);
+  } else {
+    std::vector<std::thread> workers;
+    for (StudyShard& sh : shards) workers.emplace_back([&, psh = &sh] { run_study_shard(run, *psh); });
+    for (std::thread& w : workers) w.join();
+  }
+  const StudyShard* failed = nullptr;
+  for (const StudyShard& sh : shards)
+    if (sh.rc && (!failed || failed->err.rfind("study stopped", 0) == 0)) failed = &sh;
+  if (failed) return fail(failed->rc, failed->err);
+  const size_t SQ = run.SQ, nb2 = (size_t)run.nb + 2;
+  for (size_t j = 0; j < SQ; ++j) {
+    const OkinMoments& m = run.acc[j];
+    const bool empty = m.count == 0;
+    out->count[j] = m.count;
+    out->nonfinite[j] = m.nonfinite;
+    out->mean[j] = empty ? NAN : m.mean;
+    out->m2[j] = empty ? NAN : m.m2;
+    out->min[j] = empty ? NAN : m.min;
+    out->max[j] = empty ? NAN : m.max;
+    out->argmin[j] = empty ? -1 : m.argmin;
+    out->argmax[j] = empty ? -1 : m.argmax;
+  }
+  if (run.nb) std::fill(out->histogram, out->histogram + SQ * nb2, (int64_t)0);
+  std::fill(out->status_counts, out->status_counts + 4, (int64_t)0);
+  std::fill(out->failed_at_step, out->failed_at_step + n_steps, (int64_t)0);
+  for (const StudyShard& sh : shards) {
+    for (size_t k = 0; k < sh.hist.size(); ++k) out->histogram[k] += (int64_t)sh.hist[k];
+    for (int k = 0; k < 4 && k < (int)sh.status.size(); ++k) out->status_counts[k] += (int64_t)sh.status[k];
+    for (size_t k = 0; k < sh.failed_at.size(); ++k) out->failed_at_step[k] += (int64_t)sh.failed_at[k];
+  }
+  return OKIN_OK;
+}
+
+int okin_study_sample(okin_topology* t, const okin_study_desc* desc, int64_t n_ids, const int64_t* instance_ids,
+                      double* hardpoints_out, double* params_out, int32_t device) {
+  std::vector<uint64_t> stride;
+  uint64_t period = 0;
+  int rc = study_check_generator(t, desc, &stride, &period);
+  if (rc) return rc;
+  const int nin3 = 3 * t->hdr[OKIN_H_NIN], npar = t->hdr[OKIN_H_NPARAM];
+  if (n_ids < 0) return fail(OKIN_ERR_USAGE, "negative n_ids");
+  if (n_ids > 0 && (!instance_ids || !hardpoints_out || (npar > 0 && !params_out)))
+    return fail(OKIN_ERR_USAGE, "null study sample buffer");
+  for (int64_t r = 0; r < n_ids; ++r)
+    if (instance_ids[r] < 0) return fail(OKIN_ERR_USAGE, "negative instance id");
+  if (n_ids == 0) return OKIN_OK;
+  DeviceCopy* d = nullptr;
+  if ((rc = ensure_device(t, device, &d))) return rc;
+  OKIN_CUDA(cudaSetDevice(device));
+  DeviceAllocs a;
+  OkinStudyTables tab;
+  if ((rc = upload_study_tables(desc, stride, period, a, &tab))) return rc;
+  long long* ids;
+  double *hp, *par = nullptr;
+  OKIN_CUDA(a.alloc(&ids, n_ids));
+  OKIN_CUDA(a.alloc(&hp, (size_t)n_ids * nin3));
+  if (npar) OKIN_CUDA(a.alloc(&par, (size_t)n_ids * npar));
+  OKIN_CUDA(cudaMemcpy(ids, instance_ids, n_ids * sizeof(long long), cudaMemcpyHostToDevice));
+  if ((rc = launch_study_generate(tab, 0, ids, n_ids, nin3, npar, hp, par, d->num_sms, d->streams[0]))) return rc;
+  OKIN_CUDA(cudaStreamSynchronize(d->streams[0]));
+  OKIN_CUDA(cudaMemcpy(hardpoints_out, hp, (size_t)n_ids * nin3 * sizeof(double), cudaMemcpyDeviceToHost));
+  if (npar) OKIN_CUDA(cudaMemcpy(params_out, par, (size_t)n_ids * npar * sizeof(double), cudaMemcpyDeviceToHost));
   return OKIN_OK;
 }
 

@@ -1,23 +1,28 @@
 #!/usr/bin/env python3
-"""BASELINE.json configs[3] and configs[4] at their stated sizes, on 1..8 GPUs.
+"""BASELINE.json configs[3] and configs[4] at their stated sizes, as tolerance studies
+(``BatchSolver.study``: inputs generated and statistics reduced on the device).
 
-    python tools/config_scale.py --config c4 [--instances 10000000] [--steps 101]
-    python -m torch.distributed.run --nnodes=1 --nproc-per-node 8 --master-addr 127.0.0.1 \
-        --master-port 29511 tools/config_scale.py --config c5
+    python tools/config_scale.py --config c4 [--instances 10000000] [--steps 101] [--devices 0,1,...]
+    python tools/config_scale.py --config c5 --arm both --repeats 2
 
 c4: double-wishbone axle with torsion bars, T-bar ARB, rocker-to-rocker heave link and camber shims,
-    101-step bump and 101-step roll sweeps, 1e7 Monte-Carlo tolerance instances (hardpoints sigma
-    0.25 mm, shim set-up thickness drawn per instance) in total over the ranks.
+    101-step bump (or roll) sweep, 1e7 Monte-Carlo tolerance instances: every left / centre hardpoint
+    coordinate normal with sigma 0.25 mm (right points mirror their left twins, centre-line y held),
+    every shim set-up thickness uniform on +-0.5 mm.
 c5: DoE sensitivity sweep over a hardpoint grid: 1e8 instance-steps (4 761 905 instances x 21 steps of
-    the flagship axle, each instance one grid node of a 6-factor design) with every metric column
-    (motion ratios, roll-centre metrics, ...) evaluated on the device.
+    the flagship axle, each instance one node of a 13-level, 6-factor full factorial on +-2 mm) with
+    every metric column evaluated on the device.
 
-The instance range of a rank is processed in chunks whose outputs stay on the device (1e7 x 101
-states of all-point positions would be 1.1 TB): per chunk the positions / metrics are reduced on the
-device to what a tolerance study keeps (status counts, min / max / mean of selected metric columns),
-and the chunk buffers are reused.  One JSON line per run (rank 0): whole-job states/s, timed with
-CUDA events on the launch stream, max over ranks.  No data-path collective: ranks only reduce the
-timing and the summary statistics at the end.
+Arms, run alternately in one call (``--arm both``):
+  study   ``BatchSolver.study`` end to end (generation, sweep kernel, reduction, host fold), timed on
+          the host clock around the call; the result has arrived on the host when it returns.
+  kernel  the device-resident sweep kernel alone (``okin_solve_batch_device``) on the same chunks of
+          the same inputs, timed with CUDA events around each launch (inputs are regenerated per chunk
+          outside the timed window; needs torch and a single device).
+One JSON line per arm and repeat.  ``--memory`` samples free device memory while the study runs.
+``--profile`` runs the study arm once more under torch.profiler and reports the device time of the
+sweep kernel, the generator (``okin_study_generate``) and the reduction (``okin_study_reduce`` +
+``okin_study_merge``).
 """
 
 from __future__ import annotations
@@ -27,10 +32,10 @@ import ctypes
 import json
 import os
 import sys
+import threading
+import time
 
 import numpy as np
-import torch
-import torch.distributed as dist
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
@@ -38,80 +43,114 @@ sys.path.insert(0, os.path.join(ROOT, "tests"))
 import bench  # noqa: E402
 from helpers import build_case, load_golden  # noqa: E402
 from open_kinematics_b200 import _lib  # noqa: E402
-from open_kinematics_b200.core.input import build_sweep  # noqa: E402
+from open_kinematics_b200.core.study import Sampling  # noqa: E402
 from open_kinematics_b200.core.sweep import BatchSolver  # noqa: E402
 
-sys.path.insert(0, os.path.join(ROOT, "tools"))
-from config_throughput import axle_sweep  # noqa: E402
+# the metric columns whose ranges the c5 line reports
+C5_RANGE_COLUMNS = ("roll_center_z", "camber_left", "deriv_damper_length_wrt_hub_z_left",
+                    "deriv_arb_twist_wrt_hub_z_left")
 
 
-def doe_levels(rank_begin: int, count: int, n_factors: int, levels: int, device) -> torch.Tensor:
-    """Grid coordinates in [-1, 1] of DoE nodes [rank_begin, rank_begin + count): node index written
-    in base ``levels`` (a full factorial design walked in order, wrapped when exhausted)."""
-    idx = torch.arange(rank_begin, rank_begin + count, device=device, dtype=torch.int64)
-    cols = []
-    for _ in range(n_factors):
-        cols.append((idx % levels).double() / (levels - 1) * 2.0 - 1.0)
-        idx = idx // levels
-    return torch.stack(cols, dim=1)
+def c4_sampling(solver) -> Sampling:
+    smp = Sampling(solver, mirror_right=True).normal("all", 0.25)
+    return smp.uniform([n for n in solver.program.param_names if n.endswith("setup_thickness")], 0.5)
 
 
-def main() -> None:
-    ap = argparse.ArgumentParser()
-    ap.add_argument("--config", choices=["c4", "c5"], required=True)
-    ap.add_argument("--instances", type=int, default=None, help="total over all ranks")
-    ap.add_argument("--steps", type=int, default=None)
-    ap.add_argument("--chunk", type=int, default=65536)
-    ap.add_argument("--mode", default="bump", choices=["bump", "roll"], help="c4 sweep kind")
-    args = ap.parse_args()
-    rank = int(os.environ.get("RANK", "0"))
-    world = int(os.environ.get("WORLD_SIZE", "1"))
-    local = int(os.environ.get("LOCAL_RANK", "0"))
-    if world > 1:
-        os.environ.setdefault("MASTER_ADDR", "127.0.0.1")
-        dist.init_process_group("nccl", device_id=torch.device("cuda", local))
-    torch.cuda.set_device(local)
-    dev = torch.device("cuda", local)
-    _lib.require_device()
+def c5_sampling(solver) -> tuple:
+    """(sampling, factor coordinates): six left / centre hardpoint coordinates on a 13-level grid of
+    +-2 mm, the first factor varying fastest; right points mirror their left twins."""
+    own, _ = bench.perturbation_mask(solver.program)
+    coords = [3 * int(own[k % own.size]) + k % 3 for k in range(0, 6 * 5, 5)]
+    smp = Sampling(solver, mirror_right=True)
+    for c in coords:
+        smp.grid((solver.program.in_keys[c // 3], c % 3), 2.0, 13)
+    return smp, coords
 
+
+def case(args):
     if args.config == "c4":
+        from open_kinematics_b200.core.input import build_sweep
+        sys.path.insert(0, os.path.join(ROOT, "tools"))
+        from config_throughput import axle_sweep
         meta, _ = load_golden("c4_tbar_heave_shim_bump")
         sus, _ = build_case(meta)
         steps = args.steps or 101
         sweep = build_sweep(axle_sweep(steps, 50.0, args.mode == "roll"), sus)
-        total = args.instances or 10_000_000
-        want_metrics, sigma = False, 0.25
-        label = f"c4_tbar_heave_shim_{args.mode}{steps}_montecarlo"
-    else:
-        meta, _ = load_golden("c3_rocker_ubar_coilover_roll")
-        sus, sweep = build_case(meta)
-        steps = sweep.n_steps
-        total = args.instances or -(-100_000_000 // steps)      # 1e8 instance-steps
-        want_metrics, sigma = True, 0.0
-        label = "c5_doe_grid_c3_axle_roll21_all_metrics"
+        solver = BatchSolver(sus, sweep, tune_layout=True)
+        return (solver, c4_sampling(solver), args.instances or 10_000_000,
+                f"c4_tbar_heave_shim_{args.mode}{steps}_montecarlo", dict(points="all", solver_quantities=(
+                    "solver_nfev",)))
+    meta, _ = load_golden("c3_rocker_ubar_coilover_roll")
+    sus, sweep = build_case(meta)
     solver = BatchSolver(sus, sweep, tune_layout=True)
+    total = args.instances or -(-100_000_000 // sweep.n_steps)      # 1e8 instance-steps
+    return (solver, c5_sampling(solver)[0], total, "c5_doe_grid_c3_axle_roll21_all_metrics",
+            dict(metrics="all", solver_quantities=("solver_nfev",)))
+
+
+class MemorySampler:
+    """Smallest free device memory seen while running (cudaMemGetInfo through torch)."""
+
+    def __init__(self, device: int):
+        import torch
+        self.torch, self.device = torch, device
+        self.min_free = self.free()
+        self._stop = threading.Event()
+        self._thread = threading.Thread(target=self._run, daemon=True)
+
+    def free(self) -> int:
+        return int(self.torch.cuda.mem_get_info(self.device)[0])
+
+    def _run(self):
+        while not self._stop.wait(0.05):
+            self.min_free = min(self.min_free, self.free())
+
+    def __enter__(self):
+        self._thread.start()
+        return self
+
+    def __exit__(self, *exc):
+        self._stop.set()
+        self._thread.join()
+
+
+def study_arm(solver, smp, total, kw, devices, seed, memory) -> dict:
+    sampler = MemorySampler(devices[0]) if memory else None
+    before = sampler.free() if sampler else None
+    t0 = time.perf_counter()
+    if sampler:
+        with sampler:
+            res = solver.study(smp, total, seed=seed, devices=devices, **kw)
+    else:
+        res = solver.study(smp, total, seed=seed, devices=devices, **kw)
+    seconds = time.perf_counter() - t0
+    nfev = res.quantities.index("solver_nfev")
+    accepted = float(res.count[:, nfev].sum())
+    line = {"arm": "study", "seconds": seconds, "accepted_states": accepted, "states_per_s": accepted / seconds,
+            "ok_fraction": float(res.status_counts[0]) / total, "status_counts": res.status_counts.tolist(),
+            "mean_nfev_per_state": float((res.mean[:, nfev] * res.count[:, nfev]).sum()) / max(accepted, 1.0)}
+    if kw.get("metrics"):
+        line["metric_ranges"] = {c: [float(np.nanmin(res.min[:, res.quantities.index(c)])),
+                                     float(np.nanmax(res.max[:, res.quantities.index(c)]))]
+                                 for c in C5_RANGE_COLUMNS if c in res.quantities}
+    if sampler:
+        line["device_free_bytes_before"] = before
+        line["device_used_bytes_during_peak"] = before - sampler.min_free
+    return line
+
+
+def kernel_arm(solver, smp, total, want_metrics, seed, device) -> dict:
+    """The sweep kernel alone on the study's chunks: inputs regenerated per chunk (okin_study_sample)
+    and uploaded outside the timed window."""
+    import torch
     prog, topo = solver.program, solver.topology
-    begin, count = _lib.shard_range(total, rank, world)
-    nominal = torch.tensor(solver.nominal_hardpoints(), device=dev, dtype=torch.float64)
-    own, pairs = bench.perturbation_mask(prog)
-    own_t = torch.tensor(own, device=dev)
-    p_left, p_right = torch.tensor(pairs[:, 0], device=dev), torch.tensor(pairs[:, 1], device=dev)
-    flip = torch.tensor([1.0, -1.0, 1.0], device=dev, dtype=torch.float64)
-    # centre-line points keep y = 0 (T-bar pivot: the reference's build validation, axle/mechanisms.py:626-643)
-    from open_kinematics_b200.core.primitives.point_ref import Side
-    centre = [i for i, k in enumerate(prog.in_keys) if getattr(k, "side", None) is Side.CENTER
-              and abs(float(solver.nominal_hardpoints()[3 * i + 1])) < 1e-9]
-    centre_t = torch.tensor(centre, device=dev, dtype=torch.int64)
-    S, nin, nout, nm = steps, prog.n_in, prog.n_out, len(prog.metric_names)
-    chunk = min(args.chunk, max(count, 1))
-    # chunk buffers, reused
-    hp = torch.empty((chunk, nin, 3), device=dev, dtype=torch.float64)
-    par = None
-    if prog.param_names:
-        par = torch.tensor(prog.param_default, device=dev, dtype=torch.float64).repeat(chunk, 1)
-        shim_cols = torch.tensor([i for i, nme in enumerate(prog.param_names) if nme.endswith("setup_thickness")], device=dev)
+    S, nout3, nm = solver.values.shape[1], 3 * prog.n_out, len(prog.metric_names)
+    chunk = 65536
+    dev = torch.device("cuda", device)
+    hp = torch.empty((chunk, 3 * prog.n_in), device=dev, dtype=torch.float64)
+    par = torch.empty((chunk, len(prog.param_names)), device=dev, dtype=torch.float64) if prog.param_names else None
     tv = torch.tensor(solver.values, device=dev, dtype=torch.float64).contiguous()
-    pos = torch.empty((chunk, S, 3 * nout), device=dev, dtype=torch.float64) if not want_metrics else None
+    pos = None if want_metrics else torch.empty((chunk, S, nout3), device=dev, dtype=torch.float64)
     met = torch.empty((chunk, S, nm), device=dev, dtype=torch.float64) if want_metrics else None
     status = torch.empty(chunk, device=dev, dtype=torch.int32)
     failed = torch.empty(chunk, device=dev, dtype=torch.int32)
@@ -122,107 +161,84 @@ def main() -> None:
                          metrics=met.data_ptr() if met is not None else None, status=status.data_ptr(),
                          failed_step=failed.data_ptr(), iters=iters.data_ptr(), max_residual=maxres.data_ptr())
     lib, cfg = _lib.load(), _lib.default_cfg()
-    gen = torch.Generator(device=dev)
-    gen.manual_seed(1234 + rank)
-    # DoE factors: six left-side hardpoint coordinates moved +-2 mm (c5); Monte Carlo: all of them (c4)
-    n_factors, levels = 6, 13                                  # 13^6 = 4.83e6 grid nodes >= 4.76e6 instances
-    factor_slots = [(int(own[k % own.size]), k % 3) for k in range(0, 6 * 5, 5)]
-
-    def fill(lo: int, c: int) -> None:
-        hp[:c] = nominal.reshape(1, nin, 3)
-        if args.config == "c4":
-            hp[:c, own_t, :] += sigma * torch.randn((c, own.size, 3), device=dev, dtype=torch.float64, generator=gen)
-            par[:c, shim_cols] = 29.5 + torch.rand((c, shim_cols.numel()), device=dev, dtype=torch.float64, generator=gen)
-        else:
-            grid = doe_levels(begin + lo, c, n_factors, levels, dev)
-            for f, (slot, axis) in enumerate(factor_slots):
-                hp[:c, slot, axis] += 2.0 * grid[:, f]
-        if centre:
-            hp[:c, centre_t, 1] = 0.0
-        hp[:c, p_right, :] = hp[:c, p_left, :] * flip
-
-    def launch(c: int) -> None:
-        _lib.check(lib.okin_solve_batch_device(topo.handle, ctypes.byref(cfg), local, ctypes.c_void_p(
-            torch.cuda.current_stream().cuda_stream), c, S, ctypes.byref(io)), label)
-
-    n_ok = torch.zeros((), device=dev, dtype=torch.int64)
-    accepted = torch.zeros((), device=dev, dtype=torch.int64)
-    nfev = torch.zeros((), device=dev, dtype=torch.int64)
-    stat_cols = [prog.metric_names.index(k) for k in prog.metric_names
-                 if k in ("roll_center_z", "camber_left", "deriv_damper_length_wrt_hub_z_left",
-                          "deriv_arb_twist_wrt_hub_z_left")] if want_metrics else []
-    col_min = torch.full((len(stat_cols),), float("inf"), device=dev, dtype=torch.float64)
-    col_max = torch.full((len(stat_cols),), float("-inf"), device=dev, dtype=torch.float64)
-    col_idx = torch.tensor(stat_cols, device=dev, dtype=torch.int64)
-
-    def process(lo: int, c: int, events) -> None:
-        """One chunk: inputs on the device, solve, reduce what a tolerance study keeps."""
-        nonlocal n_ok, accepted, nfev, col_min, col_max
-        fill(lo, c)
-        events[0].record()
-        launch(c)
-        events[1].record()
+    from open_kinematics_b200.core.study import study_request
+    _, _, _, desc = study_request(solver, smp, seed, None, None, ("solver_nfev",), None, 0)
+    stream = torch.cuda.current_stream(dev)
+    kernel_ms, accepted, n_ok = 0.0, 0, 0
+    for lo in range(0, total, chunk):
+        c = min(chunk, total - lo)
+        h, p = topo.study_sample(desc, np.arange(lo, lo + c), device)
+        hp[:c].copy_(torch.from_numpy(h))
+        if par is not None:
+            par[:c].copy_(torch.from_numpy(p))
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record(stream)
+        _lib.check(lib.okin_solve_batch_device(topo.handle, ctypes.byref(cfg), device,
+                                               ctypes.c_void_p(stream.cuda_stream), c, S, ctypes.byref(io)), "kernel arm")
+        e1.record(stream)
+        e1.synchronize()
+        kernel_ms += e0.elapsed_time(e1)
         ok = status[:c] == 0
-        n_ok += ok.sum()
-        accepted += torch.where(ok, torch.full_like(failed[:c], S), failed[:c].clamp(min=0)).sum()
-        nfev += iters[:c].sum()
-        if stat_cols:
-            sel = met[:c].index_select(2, col_idx)                                   # [c, S, k]
-            good = ok[:, None, None] & ~torch.isnan(sel)
-            col_min = torch.minimum(col_min, torch.where(good, sel, float("inf")).amin(dim=(0, 1)))
-            col_max = torch.maximum(col_max, torch.where(good, sel, float("-inf")).amax(dim=(0, 1)))
+        n_ok += int(ok.sum())
+        accepted += int(torch.where(ok, torch.full_like(failed[:c], S), failed[:c].clamp(min=0)).sum())
+    return {"arm": "kernel", "kernel_seconds": kernel_ms * 1e-3, "accepted_states": float(accepted),
+            "states_per_s": accepted / (kernel_ms * 1e-3), "ok_fraction": n_ok / total}
 
-    # warm-up on one chunk (untimed: kernel-family calibration, torch kernel loading), counters reset after
-    warm = [torch.cuda.Event(enable_timing=True) for _ in range(2)]
-    for _ in range(2):
-        process(0, chunk, warm)
-    torch.cuda.synchronize()
-    n_ok.zero_(), accepted.zero_(), nfev.zero_()
-    col_min.fill_(float("inf")), col_max.fill_(float("-inf"))
-    if world > 1:
-        dist.barrier()
-    n_chunks = (count + chunk - 1) // chunk
-    ev = [[torch.cuda.Event(enable_timing=True) for _ in range(2)] for _ in range(n_chunks)]
-    wall0, wall1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    wall0.record()
-    for k, lo in enumerate(range(0, count, chunk)):
-        process(lo, min(chunk, count - lo), ev[k])           # no host synchronisation inside the loop
-    wall1.record()
-    torch.cuda.synchronize()
-    kernel_ms = sum(a.elapsed_time(b) for a, b in ev)
-    launches = n_chunks
-    wall_ms = wall0.elapsed_time(wall1)
-    t = torch.tensor([kernel_ms, wall_ms], device=dev, dtype=torch.float64)
-    sums = torch.stack([n_ok, accepted, nfev]).double()
-    if world > 1:
-        dist.all_reduce(t, op=dist.ReduceOp.MAX)
-        dist.all_reduce(sums, op=dist.ReduceOp.SUM)
-        if stat_cols:
-            dist.all_reduce(col_min, op=dist.ReduceOp.MIN)
-            dist.all_reduce(col_max, op=dist.ReduceOp.MAX)
-    if rank == 0:
-        k_ms, w_ms = float(t[0]), float(t[1])
-        n_ok_all, accepted_all, nfev_all = (float(v) for v in sums)
-        line = {
-            "config": label, "n_gpus": world, "instances_total": total, "sweep_steps": S,
-            "instance_steps_total": total * S, "chunk_instances": chunk, "metrics_on_device": bool(want_metrics),
-            "n_metric_columns": nm if want_metrics else 0, "n_unknowns": prog.n_unknowns,
-            "states_per_s": accepted_all / (k_ms * 1e-3),
-            "states_per_s_incl_input_generation_and_reductions": accepted_all / (w_ms * 1e-3),
-            "kernel_seconds_max_over_ranks": k_ms * 1e-3, "wall_seconds_max_over_ranks": w_ms * 1e-3,
-            "ok_fraction": n_ok_all / total, "accepted_states": accepted_all,
-            "mean_nfev_per_state": nfev_all / max(accepted_all, 1.0), "launches_per_rank": launches,
-            "outputs": "metrics (all columns) + nfev + max_residual + status, reduced on the device per chunk"
-                       if want_metrics else "positions (all points) + nfev + max_residual + status, kept on the device per chunk",
-            "launch": topo.launch_geometry(chunk, local), "scaling": "strong (total work fixed)",
-        }
-        if stat_cols:
-            line["metric_ranges"] = {prog.metric_names[c]: [float(col_min[i]), float(col_max[i])]
-                                     for i, c in enumerate(stat_cols)}
-        print(json.dumps(line), flush=True)
+
+def main() -> None:
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--config", choices=["c4", "c5"], required=True)
+    ap.add_argument("--instances", type=int, default=None)
+    ap.add_argument("--steps", type=int, default=None)
+    ap.add_argument("--mode", default="bump", choices=["bump", "roll"], help="c4 sweep kind")
+    ap.add_argument("--arm", default="study", choices=["study", "kernel", "both"])
+    ap.add_argument("--repeats", type=int, default=1)
+    ap.add_argument("--devices", default="0", help="comma-separated device ids of the study arm")
+    ap.add_argument("--seed", type=int, default=1234)
+    ap.add_argument("--memory", action="store_true", help="sample device memory during the study arm")
+    ap.add_argument("--profile", action="store_true", help="kernel-time split of one study run")
+    args = ap.parse_args()
+    _lib.require_device()
+    devices = [int(d) for d in args.devices.split(",")]
+    solver, smp, total, label, kw = case(args)
+    arms = ["kernel", "study"] if args.arm == "both" else [args.arm]
+    if "kernel" in arms and len(devices) != 1:
+        raise SystemExit("the kernel arm runs on a single device")
+    # warm-up of both arms on one chunk (module load, lean-family calibration)
+    solver.study(smp, 65536, seed=args.seed, devices=devices, **kw)
+    base = {"config": label, "instances_total": total, "sweep_steps": int(solver.values.shape[1]),
+            "instance_steps_total": total * int(solver.values.shape[1]), "devices": devices,
+            "n_metric_columns": len(solver.program.metric_names) if kw.get("metrics") else 0,
+            "n_unknowns": solver.program.n_unknowns}
+    for rep in range(args.repeats):
+        for arm in arms:
+            if arm == "study":
+                line = study_arm(solver, smp, total, kw, devices, args.seed, args.memory)
+            else:
+                line = kernel_arm(solver, smp, total, bool(kw.get("metrics")), args.seed, devices[0])
+            print(json.dumps(dict(base, repeat=rep, **line)), flush=True)
+    if args.profile:
+        print(json.dumps(dict(base, **profile_study(solver, smp, total, kw, devices, args.seed))), flush=True)
     solver.close()
-    if world > 1:
-        dist.destroy_process_group()
+
+
+def profile_study(solver, smp, total, kw, devices, seed) -> dict:
+    from torch.profiler import ProfilerActivity, profile
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        solver.study(smp, total, seed=seed, devices=devices, **kw)
+    us = {"sweep_kernel": 0.0, "generate": 0.0, "reduce": 0.0, "other": 0.0}
+    for ev in prof.key_averages():
+        t = float(getattr(ev, "device_time_total", 0.0) or getattr(ev, "cuda_time_total", 0.0))
+        if "okin_sweep_kernel" in ev.key:
+            us["sweep_kernel"] += t
+        elif "okin_study_generate" in ev.key:
+            us["generate"] += t
+        elif "okin_study_reduce" in ev.key or "okin_study_merge" in ev.key:
+            us["reduce"] += t
+        else:
+            us["other"] += t
+    return {"arm": "profile", "device_us": us,
+            "generate_plus_reduce_over_sweep_kernel": (us["generate"] + us["reduce"]) / max(us["sweep_kernel"], 1e-9)}
 
 
 if __name__ == "__main__":
