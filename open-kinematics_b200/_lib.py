@@ -100,6 +100,40 @@ class StudyOut(ctypes.Structure):
               "failed_at_step")
     _fields_ = [(n, ctypes.c_void_p) for n in FIELDS]
 
+    @classmethod
+    def allocate(cls, n_steps: int, n_quantities: int, n_bins: int) -> tuple:
+        """``(arrays, struct)``: zeroed result arrays by field name, ``[n_steps, n_quantities]`` each
+        (``histogram`` ``[n_steps, n_quantities, n_bins + 2]`` or None, ``status_counts`` [4],
+        ``failed_at_step`` [n_steps]), and the ``okin_study_out`` pointing at them."""
+        S, Q = n_steps, n_quantities
+        out = {n: np.zeros((S, Q), np.int64 if n in ("count", "nonfinite", "argmin", "argmax") else np.float64)
+               for n in cls.FIELDS[:8]}
+        out["histogram"] = np.zeros((S, Q, n_bins + 2), np.int64) if n_bins > 0 else None
+        out["status_counts"] = np.zeros(4, np.int64)
+        out["failed_at_step"] = np.zeros(S, np.int64)
+        return out, cls(**{k: (v.ctypes.data if v is not None else None) for k, v in out.items()})
+
+
+def batch_shapes(program, n_instances: int, n_steps: int) -> dict:
+    """Shape and dtype of every ``okin_batch_io`` output of a batch of ``program`` (include/okin.h)."""
+    n, nt, nout, nu = n_instances, len(program.target_points), program.n_out, program.n_unknowns
+    return {
+        "positions": ((n, n_steps, nout, 3), np.float64),
+        "status": ((n,), np.int32),
+        "failed_step": ((n,), np.int32),
+        "iters": ((n, n_steps), np.int32),
+        "max_residual": ((n, n_steps), np.float64),
+        "tangents": ((n, n_steps, nt, nu), np.float64),
+        "velocities": ((n, n_steps, nt, nout, 3), np.float64),
+        "tangent_health": ((n, n_steps, 2), np.float64),
+        "metrics": ((n, n_steps, len(program.metric_names)), np.float64),
+        "design": ((n, nout, 3), np.float64),
+        "diagnostics": ((n, n_steps, len(program.diagnostic_names)), np.float64),
+        "jumps": ((n, n_steps, nu // 3), np.float64),
+        "worst_row": ((n,), np.int32),
+        "hardpoint_sensitivity": ((n, n_steps, len(program.sensitivity_inputs), nout, 3), np.float64),
+    }
+
 
 # name -> (restype, argtypes); also the list the "exports every declared symbol" test checks.
 SIGNATURES = {
@@ -283,13 +317,8 @@ class DeviceTopology:
         nt = len(self.program.target_points)
         if tv.ndim != 2 or tv.shape[0] != nt:
             raise ValueError(f"target_values must have shape ({nt}, n_steps), got {tv.shape}")
-        S, Q, nb = tv.shape[1], desc.n_quantities, desc.n_bins
-        out = {name: np.zeros((S, Q), np.int64 if name in ("count", "nonfinite", "argmin", "argmax") else np.float64)
-               for name in StudyOut.FIELDS[:8]}
-        out["histogram"] = np.zeros((S, Q, nb + 2), np.int64) if nb > 0 else None
-        out["status_counts"] = np.zeros(4, np.int64)
-        out["failed_at_step"] = np.zeros(S, np.int64)
-        o = StudyOut(**{k: (v.ctypes.data if v is not None else None) for k, v in out.items()})
+        S = tv.shape[1]
+        out, o = StudyOut.allocate(S, desc.n_quantities, desc.n_bins)
         dev = np.ascontiguousarray(devices if devices is not None else [0], dtype=np.int32)
         check(load().okin_study(self.handle, ctypes.byref(cfg or default_cfg()), int(n_instances), S, tv.ctypes.data,
                                 ctypes.byref(desc), ctypes.byref(o), dev.ctypes.data, dev.size), "okin_study")
@@ -346,7 +375,7 @@ class DeviceTopology:
         dev = np.ascontiguousarray(devices if devices is not None else [0], dtype=np.int32)
         prev = out or {}
 
-        def buf(name, want, shape, dtype=np.float64):
+        def buf(name, want, shape, dtype):
             if not want:
                 return None
             old = prev.get(name)
@@ -355,23 +384,13 @@ class DeviceTopology:
                 return old
             return pinned_empty(shape, dtype, int(dev[0])) if pinned else np.empty(shape, dtype)
 
-        out = {
-            "positions": buf("positions", want_positions, (n_inst, n_steps, prog.n_out, 3)),
-            "status": buf("status", True, (n_inst,), np.int32),
-            "failed_step": buf("failed_step", True, (n_inst,), np.int32),
-            "iters": buf("iters", True, (n_inst, n_steps), np.int32),
-            "max_residual": buf("max_residual", True, (n_inst, n_steps)),
-            "tangents": buf("tangents", want_tangents, (n_inst, n_steps, nt, prog.n_unknowns)),
-            "velocities": buf("velocities", want_velocities, (n_inst, n_steps, nt, prog.n_out, 3)),
-            "tangent_health": buf("tangent_health", want_health, (n_inst, n_steps, 2)),
-            "metrics": buf("metrics", want_metrics, (n_inst, n_steps, len(prog.metric_names))),
-            "design": buf("design", want_design, (n_inst, prog.n_out, 3)),
-            "diagnostics": buf("diagnostics", want_diagnostics, (n_inst, n_steps, len(prog.diagnostic_names))),
-            "jumps": buf("jumps", want_diagnostics, (n_inst, n_steps, prog.n_unknowns // 3)),
-            "worst_row": buf("worst_row", want_worst_row, (n_inst,), np.int32),
-            "hardpoint_sensitivity": buf("hardpoint_sensitivity", want_hardpoint_sensitivity,
-                                         (n_inst, n_steps, len(prog.sensitivity_inputs), prog.n_out, 3)),
-        }
+        want = {"positions": want_positions, "status": True, "failed_step": True, "iters": True, "max_residual": True,
+                "tangents": want_tangents, "velocities": want_velocities, "tangent_health": want_health,
+                "metrics": want_metrics, "design": want_design, "diagnostics": want_diagnostics,
+                "jumps": want_diagnostics, "worst_row": want_worst_row,
+                "hardpoint_sensitivity": want_hardpoint_sensitivity}
+        out = {name: buf(name, want[name], shape, dtype)
+               for name, (shape, dtype) in batch_shapes(prog, n_inst, n_steps).items()}
         if want_diagnostics and not prog.diagnostic_names:
             raise ValueError("This topology was compiled without a diagnostic program")
         if want_metrics and not prog.metric_names:

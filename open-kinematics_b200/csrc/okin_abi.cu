@@ -89,30 +89,6 @@ struct DeviceCopy {
   cudaStream_t streams[OKIN_PIPE_SLOTS] = {};
 };
 
-// okin_batch_io without its last field: the kernels take the sensitivity output as a trailing
-// parameter instead, so that the parameter layout (and the code) of the instantiations that never
-// write it stays what it was before that output existed.
-struct OkinKernelIO {
-  const double* hardpoints;
-  const double* params;
-  const double* target_values;
-  int32_t* status;
-  int32_t* failed_step;
-  double* positions;
-  int32_t* iters;
-  double* max_residual;
-  double* tangents;
-  double* velocities;
-  double* tangent_health;
-  double* metrics;
-  double* design;
-  double* diagnostics;
-  double* jumps;
-  const double* instance_targets;
-  int32_t* worst_row;
-};
-static_assert(sizeof(OkinKernelIO) == offsetof(okin_batch_io, hardpoint_sensitivity), "OkinKernelIO layout");
-
 }  // namespace
 
 struct okin_topology {
@@ -145,7 +121,7 @@ okin_sweep_kernel(const int32_t* __restrict__ hdr, const int32_t* __restrict__ i
   const int warp = threadIdx.x >> 5;
   const int warps_per_cta = blockDim.x >> 5;
   double* sm = okin_smem + table_doubles + (size_t)warp * hdr[FULL ? OKIN_H_SMEM_DOUBLES : OKIN_H_SMEM_DOUBLES_LEAN];
-  const int nin = hdr[OKIN_H_NIN], nout = hdr[OKIN_H_NOUT], nt = hdr[OKIN_H_NT], n = 3 * hdr[OKIN_H_NF];
+  const OkinIOShape shape = okin_io_shape(hdr);
   // Instances are claimed one at a time from a global counter (no static partition: a warp whose
   // instance is slow -- a failing sweep costs a few normal ones -- simply claims fewer).  The warps of
   // a CTA are kept loosely in step instead of meeting at a barrier: before claiming, a warp compares its
@@ -174,26 +150,10 @@ okin_sweep_kernel(const int32_t* __restrict__ hdr, const int32_t* __restrict__ i
     if (i >= n_instances) break;
     {
       OkinOutputs out;
-      out.positions = io.positions ? io.positions + (size_t)i * n_steps * 3 * nout : nullptr;
-      out.iters = io.iters ? io.iters + (size_t)i * n_steps : nullptr;
-      out.max_residual = io.max_residual ? io.max_residual + (size_t)i * n_steps : nullptr;
-      out.tangents = io.tangents ? io.tangents + (size_t)i * n_steps * nt * n : nullptr;
-      out.velocities = io.velocities ? io.velocities + (size_t)i * n_steps * nt * 3 * nout : nullptr;
-      out.health = io.tangent_health ? io.tangent_health + (size_t)i * n_steps * 2 : nullptr;
-      out.metrics = io.metrics ? io.metrics + (size_t)i * n_steps * hdr[OKIN_H_NM] : nullptr;
-      out.design = io.design ? io.design + (size_t)i * 3 * nout : nullptr;
-      out.diagnostics = io.diagnostics ? io.diagnostics + (size_t)i * n_steps * hdr[OKIN_H_NDIAG] : nullptr;
-      out.status = io.status + i;
-      out.failed_step = io.failed_step + i;
-      out.worst_row = io.worst_row ? io.worst_row + i : nullptr;
-      if (SENS) {
-        out.sensitivity = sens_out ? sens_out + (size_t)i * n_steps * hdr[OKIN_H_NSENS] * 3 * nout : nullptr;
-        out.sens_ws = sens_ws + ((size_t)blockIdx.x * warps_per_cta + warp) * okin_sens_ws_doubles(hdr);
-      }
-      okin_sweep<FULL, SHIM, SENS>(pr, sm, io.hardpoints + (size_t)i * 3 * nin,
-                 io.params ? io.params + (size_t)i * hdr[OKIN_H_NPARAM] : nullptr,
-                 io.instance_targets ? io.instance_targets + (size_t)i * nt * n_steps : io.target_values, n_steps,
-                 cfg, out);
+      const double *hp, *par, *tv;
+      if (SENS) out.sens_ws = sens_ws + ((size_t)blockIdx.x * warps_per_cta + warp) * okin_sens_ws_doubles(hdr);
+      okin_instance_io(io, SENS ? sens_out : nullptr, shape, n_steps, i, out, hp, par, tv);
+      okin_sweep<FULL, SHIM, SENS>(pr, sm, hp, par, tv, n_steps, cfg, out);
       __syncwarp();
     }
     ++mine;
@@ -274,16 +234,10 @@ okin_study_reduce(OkinStudyChunk ch, long long rows, long long base, int Q, cons
   if (j < SQ) {
     const int s = j / Q, q = j - s * Q, kind = qkind[q], index = qindex[q];
     const double l = n_bins ? lo[q] : 0.0, h = n_bins ? hi[q] : 0.0;
-    for (long long r = p; r < rows; r += OKIN_STUDY_PARTS) {
-      double x;
-      if (!okin_study_fetch(ch, kind, index, r, s, &x)) continue;
-      okin_moments_push(m, x, base + r);
-      if (n_bins && isfinite(x)) {
-        const int b = okin_study_bin(x, l, h, n_bins);
-        if (hist_shared) atomicAdd(&sh[tx * nb2 + b], 1ull);
-        else atomicAdd(&hist[(size_t)j * nb2 + b], 1ull);
-      }
-    }
+    okin_study_partition(ch, kind, index, s, p, rows, base, n_bins, l, h, m, [&](int b) {
+      if (hist_shared) atomicAdd(&sh[tx * nb2 + b], 1ull);
+      else atomicAdd(&hist[(size_t)j * nb2 + b], 1ull);
+    });
   }
   part[ty][tx] = m;
   if (blockIdx.x == 0 && tx == 0) {
@@ -451,10 +405,8 @@ int launch(okin_topology* t, DeviceCopy* d, const okin_solver_cfg* cfg, cudaStre
   if (n_instances == 0) return OKIN_OK;
   OkinSolverCfg c{cfg->step_tol, cfg->coarse_tol, cfg->fine_tol, cfg->residual_tol, cfg->mu_init, cfg->max_iter,
                   cfg->use_predictor};
-  // lean instantiation when no per-state tangent / metric / diagnostic output is wanted
-  const bool full = io.tangents || io.velocities || io.tangent_health || io.metrics || io.diagnostics;
   int fam = io.hardpoint_sensitivity ? OKIN_FAM_SENS : OKIN_FAM_FULL;
-  if (!full && !io.hardpoint_sensitivity) {
+  if (!okin_wants_full(io) && !io.hardpoint_sensitivity) {
     fam = d->lean_family;
     const int64_t sample = 4 * (int64_t)d->num_sms * std::max(d->shape[OKIN_FAM_LEAN].ctas_per_sm * d->shape[OKIN_FAM_LEAN].warps_per_cta,
                                                               d->shape[OKIN_FAM_LEAN_WIDE].ctas_per_sm * d->shape[OKIN_FAM_LEAN_WIDE].warps_per_cta);
@@ -505,6 +457,39 @@ int launch(okin_topology* t, DeviceCopy* d, const okin_solver_cfg* cfg, cudaStre
   return OKIN_OK;
 }
 
+int check_cfg(const okin_solver_cfg* cfg) {
+  if (cfg->max_iter < 1 || !(cfg->step_tol > 0.0) || !(cfg->coarse_tol >= cfg->step_tol))
+    return fail(OKIN_ERR_USAGE, "invalid solver config");
+  return OKIN_OK;
+}
+
+// The devices of a call: {0} when device_ids is NULL or n_devices <= 0, else the list, each at most once.
+int device_list(const int32_t* device_ids, int32_t n_devices, std::vector<int32_t>* out) {
+  if (!device_ids || n_devices <= 0) {
+    out->assign(1, 0);
+    return OKIN_OK;
+  }
+  if (n_devices > OKIN_MAX_DEVICES) return fail(OKIN_ERR_USAGE, "too many devices");
+  for (int a = 0; a < n_devices; ++a)
+    for (int b = a + 1; b < n_devices; ++b)
+      if (device_ids[a] == device_ids[b]) return fail(OKIN_ERR_USAGE, "device listed twice");
+  out->assign(device_ids, device_ids + n_devices);
+  return OKIN_OK;
+}
+
+// work(k) for k < n: on the calling thread when n == 1, else on one host thread each (copies from / to
+// pageable caller buffers block the issuing thread; with a thread per device the devices run concurrently).
+template <class Work>
+void run_per_device(size_t n, Work work) {
+  if (n == 1) {
+    work(0);
+    return;
+  }
+  std::vector<std::thread> workers;
+  for (size_t k = 0; k < n; ++k) workers.emplace_back(work, k);
+  for (std::thread& w : workers) w.join();
+}
+
 int check_common(const okin_topology* t, const okin_solver_cfg* cfg, int64_t n_instances, int32_t n_steps,
                  const okin_batch_io* io) {
   if (!t || !cfg || !io) return fail(OKIN_ERR_USAGE, "null topology, config or io");
@@ -519,52 +504,43 @@ int check_common(const okin_topology* t, const okin_solver_cfg* cfg, int64_t n_i
   if (io->hardpoint_sensitivity && t->hdr[OKIN_H_NSHIM] > 0)
     return fail(OKIN_ERR_USAGE, "hardpoint sensitivities are not available on a topology with camber-shim records "
                                 "(the shim pre-solve is not differentiated)");
-  if (cfg->max_iter < 1 || !(cfg->step_tol > 0.0) || !(cfg->coarse_tol >= cfg->step_tol)) return fail(OKIN_ERR_USAGE, "invalid solver config");
-  return OKIN_OK;
+  return check_cfg(cfg);
 }
 
 // ---- host-buffer path ------------------------------------------------------------------------
-// Every per-instance array of a call is one "lane" of a pipeline slot: (host pointer, bytes per
+// okin_batch_io is handled as an array of its pointer fields (okin_io_field order, copied with memcpy).
+static_assert(sizeof(okin_batch_io) == OKIN_IO_COUNT * sizeof(void*), "okin_batch_io is a list of pointers");
+
+// Every per-instance field of a call is one "lane" of a pipeline slot: (host pointer, bytes per
 // instance).  scratch: device buffer needed although the caller does not want the array back.
+// target_values is shared by the instances: it has its own region at the start of a slot.
 struct Lane { const void* host; size_t per_inst; bool input; bool scratch; size_t bytes; };
-constexpr int kLanes = 17;
 
 struct HostBatch {
-  Lane lanes[kLanes];
+  Lane lanes[OKIN_IO_COUNT];
   size_t chunk, b_tv, slot_bytes, tv_count;
   const okin_batch_io* io;
   int32_t n_steps;
   HostBatch(const okin_topology* t, int64_t n_instances, int32_t n_steps_, const okin_batch_io* io_) : io(io_), n_steps(n_steps_) {
     const int32_t* h = t->hdr.data();
-    const size_t nin3 = 3 * (size_t)h[OKIN_H_NIN], nout3 = 3 * (size_t)h[OKIN_H_NOUT];
-    const size_t nt = h[OKIN_H_NT], n = 3 * (size_t)h[OKIN_H_NF];
-    const size_t nm = (size_t)h[OKIN_H_NM], npar = (size_t)h[OKIN_H_NPARAM], nd = (size_t)h[OKIN_H_NDIAG];
-    const size_t S = (size_t)n_steps;
-    const Lane init[kLanes] = {
-        {io->hardpoints, nin3 * 8, true, false, 0},
-        {(io->params && npar) ? io->params : nullptr, npar * 8, true, false, 0},
-        {io->status, 4, false, false, 0},
-        {io->failed_step, 4, false, false, 0},
-        {io->positions, S * nout3 * 8, false, io->diagnostics && !io->positions, 0},
-        {io->iters, S * 4, false, false, 0},
-        {io->max_residual, S * 8, false, false, 0},
-        {io->tangents, S * nt * n * 8, false, false, 0},
-        {io->velocities, S * nt * nout3 * 8, false, false, 0},
-        {io->tangent_health, S * 2 * 8, false, false, 0},
-        {(io->metrics && nm) ? io->metrics : nullptr, S * nm * 8, false, false, 0},
-        {io->design, nout3 * 8, false, false, 0},
-        {io->diagnostics, S * nd * 8, false, false, 0},
-        {io->jumps, S * (n / 3) * 8, false, false, 0},
-        {(io->instance_targets && nt * S) ? io->instance_targets : nullptr, nt * S * 8, true, false, 0},
-        {io->worst_row, 4, false, false, 0},
-        {io->hardpoint_sensitivity, S * (size_t)h[OKIN_H_NSENS] * nout3 * 8, false, false, 0},
-    };
-    std::memcpy(lanes, init, sizeof(init));
     chunk = (size_t)std::min<int64_t>(std::max<int64_t>(n_instances, 1), OKIN_PIPE_CHUNK);
-    tv_count = nt * S;
+    tv_count = (size_t)h[OKIN_H_NT] * n_steps;
     b_tv = align(std::max<size_t>(tv_count, 1) * 8);
     slot_bytes = b_tv;
-    for (Lane& l : lanes) {
+    const OkinIOShape shape = okin_io_shape(h);
+    const void* host[OKIN_IO_COUNT];
+    std::memcpy(host, io, sizeof(host));
+    for (int f = 0; f < OKIN_IO_COUNT; ++f) {
+      const bool i32 = f == OKIN_IO_STATUS || f == OKIN_IO_FAILED_STEP || f == OKIN_IO_ITERS || f == OKIN_IO_WORST_ROW;
+      const size_t per_inst = okin_io_count(f, shape, n_steps) * (i32 ? 4 : 8);
+      const bool input = f == OKIN_IO_HARDPOINTS || f == OKIN_IO_PARAMS || f == OKIN_IO_INSTANCE_TARGETS;
+      Lane& l = lanes[f];
+      // empty params, metrics and instance targets stay null; positions are scratch for the
+      // continuity pass when diagnostics are wanted without them
+      l = {f == OKIN_IO_TARGET_VALUES ? nullptr : host[f], per_inst, input,
+           f == OKIN_IO_POSITIONS && io->diagnostics && !io->positions, 0};
+      if ((f == OKIN_IO_PARAMS || f == OKIN_IO_METRICS || f == OKIN_IO_INSTANCE_TARGETS) && per_inst == 0)
+        l.host = nullptr;
       l.bytes = (l.host || l.scratch) ? align(chunk * std::max<size_t>(l.per_inst, 1)) : 0;
       slot_bytes += l.bytes;
     }
@@ -655,38 +631,23 @@ void run_shard(okin_topology* t, const okin_solver_cfg* cfg, const HostBatch& hb
     const size_t b0 = (size_t)(sh.begin + done);
     cudaStream_t st = d->streams[slot];
     char* p = (char*)d->ws + hb.slot_bytes * slot;
-    void* dev[kLanes];
-    double* w_tv = (double*)p;
+    // this chunk's device buffers: target_values (copied once per slot), then one region per lane
+    void* dev[OKIN_IO_COUNT] = {};
+    if (hb.io->target_values) dev[OKIN_IO_TARGET_VALUES] = p;
     p += hb.b_tv;
-    for (int l = 0; l < kLanes; ++l) {
-      dev[l] = hb.lanes[l].bytes ? p : nullptr;
+    for (int l = 0; l < OKIN_IO_COUNT; ++l) {
+      if (hb.lanes[l].bytes) dev[l] = p;
       p += hb.lanes[l].bytes;
     }
-    for (int l = 0; l < kLanes; ++l)
+    for (int l = 0; l < OKIN_IO_COUNT; ++l)
       if (dev[l] && hb.lanes[l].input)
         OKIN_SHARD_CUDA(cudaMemcpyAsync(dev[l], (const char*)hb.lanes[l].host + b0 * hb.lanes[l].per_inst,
                                         c * hb.lanes[l].per_inst, cudaMemcpyHostToDevice, st));
     if (hb.tv_count && hb.io->target_values && ck < slots)
-      OKIN_SHARD_CUDA(cudaMemcpyAsync(w_tv, hb.io->target_values, hb.tv_count * 8, cudaMemcpyHostToDevice, st));
-    okin_batch_io dio{};
-    dio.hardpoints = (const double*)dev[0];
-    dio.params = (const double*)dev[1];
-    dio.target_values = hb.io->target_values ? w_tv : nullptr;
-    dio.status = (int32_t*)dev[2];
-    dio.failed_step = (int32_t*)dev[3];
-    dio.positions = (double*)dev[4];
-    dio.iters = (int32_t*)dev[5];
-    dio.max_residual = (double*)dev[6];
-    dio.tangents = (double*)dev[7];
-    dio.velocities = (double*)dev[8];
-    dio.tangent_health = (double*)dev[9];
-    dio.metrics = (double*)dev[10];
-    dio.design = (double*)dev[11];
-    dio.diagnostics = (double*)dev[12];
-    dio.jumps = (double*)dev[13];
-    dio.instance_targets = (const double*)dev[14];
-    dio.worst_row = (int32_t*)dev[15];
-    dio.hardpoint_sensitivity = (double*)dev[16];
+      OKIN_SHARD_CUDA(cudaMemcpyAsync(dev[OKIN_IO_TARGET_VALUES], hb.io->target_values, hb.tv_count * 8,
+                                      cudaMemcpyHostToDevice, st));
+    okin_batch_io dio;
+    std::memcpy(&dio, dev, sizeof(dio));
     const int rc = launch(t, d, cfg, st, (int64_t)c, hb.n_steps, dio);
     if (rc) {
       drain();
@@ -694,7 +655,7 @@ void run_shard(okin_topology* t, const okin_solver_cfg* cfg, const HostBatch& hb
       sh.err = g_last_error;
       return;
     }
-    for (int l = 0; l < kLanes; ++l)
+    for (int l = 0; l < OKIN_IO_COUNT; ++l)
       if (dev[l] && hb.lanes[l].host && !hb.lanes[l].input && hb.lanes[l].per_inst)
         OKIN_SHARD_CUDA(cudaMemcpyAsync((char*)const_cast<void*>(hb.lanes[l].host) + b0 * hb.lanes[l].per_inst, dev[l],
                                         c * hb.lanes[l].per_inst, cudaMemcpyDeviceToHost, st));
@@ -918,16 +879,18 @@ int run_study_shard_body(StudyRun& run, StudyShard& sh, DeviceAllocs& a) {
     int32_t *iters = nullptr, *status = nullptr, *failed = nullptr;
     OkinMoments *groups = nullptr, *chunk = nullptr, *host = nullptr;
   } slot[OKIN_PIPE_SLOTS];
+  const OkinIOShape shape = okin_io_shape(h);
+  auto chunk_count = [&](int f) { return CH * okin_io_count(f, shape, S); };
   for (int k = 0; k < slots; ++k) {
     Slot& s = slot[k];
-    OKIN_CUDA(a.alloc(&s.hp, CH * nin3));
-    if (npar) OKIN_CUDA(a.alloc(&s.par, CH * npar));
-    if (run.want_pos) OKIN_CUDA(a.alloc(&s.pos, CH * S * nout3));
-    if (run.want_met) OKIN_CUDA(a.alloc(&s.met, CH * S * nm));
-    OKIN_CUDA(a.alloc(&s.res, CH * S));
-    OKIN_CUDA(a.alloc(&s.iters, CH * S));
-    OKIN_CUDA(a.alloc(&s.status, CH));
-    OKIN_CUDA(a.alloc(&s.failed, CH));
+    OKIN_CUDA(a.alloc(&s.hp, chunk_count(OKIN_IO_HARDPOINTS)));
+    if (npar) OKIN_CUDA(a.alloc(&s.par, chunk_count(OKIN_IO_PARAMS)));
+    if (run.want_pos) OKIN_CUDA(a.alloc(&s.pos, chunk_count(OKIN_IO_POSITIONS)));
+    if (run.want_met) OKIN_CUDA(a.alloc(&s.met, chunk_count(OKIN_IO_METRICS)));
+    OKIN_CUDA(a.alloc(&s.res, chunk_count(OKIN_IO_MAX_RESIDUAL)));
+    OKIN_CUDA(a.alloc(&s.iters, chunk_count(OKIN_IO_ITERS)));
+    OKIN_CUDA(a.alloc(&s.status, chunk_count(OKIN_IO_STATUS)));
+    OKIN_CUDA(a.alloc(&s.failed, chunk_count(OKIN_IO_FAILED_STEP)));
     OKIN_CUDA(a.alloc(&s.groups, (size_t)OKIN_STUDY_GROUPS * SQ));
     OKIN_CUDA(a.alloc(&s.chunk, SQ));
     OKIN_CUDA(a.alloc_host(&s.host, SQ));
@@ -1150,37 +1113,24 @@ int okin_solve_batch(okin_topology* t, const okin_solver_cfg* cfg, int64_t n_ins
                      const okin_batch_io* io, const int32_t* device_ids, int32_t n_devices) {
   int rc = check_common(t, cfg, n_instances, n_steps, io);
   if (rc) return rc;
-  const int32_t default_dev = 0;
-  if (!device_ids || n_devices <= 0) {
-    device_ids = &default_dev;
-    n_devices = 1;
-  }
-  if (n_devices > OKIN_MAX_DEVICES) return fail(OKIN_ERR_USAGE, "too many devices");
-  for (int a = 0; a < n_devices; ++a)
-    for (int b = a + 1; b < n_devices; ++b)
-      if (device_ids[a] == device_ids[b]) return fail(OKIN_ERR_USAGE, "device listed twice");
+  std::vector<int32_t> devices;
+  if ((rc = device_list(device_ids, n_devices, &devices))) return rc;
+  const int G = (int)devices.size();
   HostBatch hb(t, n_instances, n_steps, io);
 
   // Contiguous instance ranges [k*N/G, (k+1)*N/G) per device: the host-side "gather" is the D2H
-  // copies.  One host thread per device (copies from / to pageable caller buffers block the
-  // issuing thread; with a thread per device the devices still run concurrently).
+  // copies.
   std::vector<Shard> shards;
-  for (int k = 0; k < n_devices; ++k) {
+  for (int k = 0; k < G; ++k) {
     Shard sh;
-    okin_shard_range(n_instances, k, n_devices, &sh.begin, &sh.count);
+    okin_shard_range(n_instances, k, G, &sh.begin, &sh.count);
     if (sh.count == 0) continue;
-    sh.device = device_ids[k];
+    sh.device = devices[k];
     rc = ensure_device(t, sh.device, &sh.d);
     if (rc) return rc;
     shards.push_back(sh);
   }
-  if (shards.size() == 1) {
-    run_shard(t, cfg, hb, shards[0]);
-  } else {
-    std::vector<std::thread> workers;
-    for (Shard& sh : shards) workers.emplace_back([&, psh = &sh] { run_shard(t, cfg, hb, *psh); });
-    for (std::thread& w : workers) w.join();
-  }
+  run_per_device(shards.size(), [&](size_t k) { run_shard(t, cfg, hb, shards[k]); });
   for (const Shard& sh : shards)
     if (sh.rc) return fail(sh.rc, sh.err);
   return OKIN_OK;
@@ -1196,18 +1146,11 @@ int okin_study(okin_topology* t, const okin_solver_cfg* cfg, int64_t n_instances
   if (n_instances < 0 || n_steps < 0) return fail(OKIN_ERR_USAGE, "negative size");
   if (n_steps == 0) return fail(OKIN_ERR_USAGE, "a study needs at least one sweep step");
   if (t->hdr[OKIN_H_NT] > 0 && !target_values) return fail(OKIN_ERR_USAGE, "null target_values");
-  if (cfg->max_iter < 1 || !(cfg->step_tol > 0.0) || !(cfg->coarse_tol >= cfg->step_tol))
-    return fail(OKIN_ERR_USAGE, "invalid solver config");
+  if ((rc = check_cfg(cfg))) return rc;
   if ((rc = study_check_quantities(t, n_steps, desc, out))) return rc;
-  const int32_t default_dev = 0;
-  if (!device_ids || n_devices <= 0) {
-    device_ids = &default_dev;
-    n_devices = 1;
-  }
-  if (n_devices > OKIN_MAX_DEVICES) return fail(OKIN_ERR_USAGE, "too many devices");
-  for (int a = 0; a < n_devices; ++a)
-    for (int b = a + 1; b < n_devices; ++b)
-      if (device_ids[a] == device_ids[b]) return fail(OKIN_ERR_USAGE, "device listed twice");
+  std::vector<int32_t> devices;
+  if ((rc = device_list(device_ids, n_devices, &devices))) return rc;
+  n_devices = (int32_t)devices.size();
   run.t = t;
   run.cfg = cfg;
   run.n = n_instances;
@@ -1232,41 +1175,17 @@ int okin_study(okin_topology* t, const okin_solver_cfg* cfg, int64_t n_instances
   std::vector<StudyShard> shards(n_devices);
   for (int k = 0; k < n_devices; ++k) {
     shards[k].index = k;
-    shards[k].device = device_ids[k];
-    if ((rc = ensure_device(t, device_ids[k], &shards[k].d))) return rc;
+    shards[k].device = devices[k];
+    if ((rc = ensure_device(t, devices[k], &shards[k].d))) return rc;
   }
-  if (n_devices == 1) {
-    run_study_shard(run, shards[0]);
-  } else {
-    std::vector<std::thread> workers;
-    for (StudyShard& sh : shards) workers.emplace_back([&, psh = &sh] { run_study_shard(run, *psh); });
-    for (std::thread& w : workers) w.join();
-  }
+  run_per_device(shards.size(), [&](size_t k) { run_study_shard(run, shards[k]); });
   const StudyShard* failed = nullptr;
   for (const StudyShard& sh : shards)
     if (sh.rc && (!failed || failed->err.rfind("study stopped", 0) == 0)) failed = &sh;
   if (failed) return fail(failed->rc, failed->err);
-  const size_t SQ = run.SQ, nb2 = (size_t)run.nb + 2;
-  for (size_t j = 0; j < SQ; ++j) {
-    const OkinMoments& m = run.acc[j];
-    const bool empty = m.count == 0;
-    out->count[j] = m.count;
-    out->nonfinite[j] = m.nonfinite;
-    out->mean[j] = empty ? NAN : m.mean;
-    out->m2[j] = empty ? NAN : m.m2;
-    out->min[j] = empty ? NAN : m.min;
-    out->max[j] = empty ? NAN : m.max;
-    out->argmin[j] = empty ? -1 : m.argmin;
-    out->argmax[j] = empty ? -1 : m.argmax;
-  }
-  if (run.nb) std::fill(out->histogram, out->histogram + SQ * nb2, (int64_t)0);
-  std::fill(out->status_counts, out->status_counts + 4, (int64_t)0);
-  std::fill(out->failed_at_step, out->failed_at_step + n_steps, (int64_t)0);
-  for (const StudyShard& sh : shards) {
-    for (size_t k = 0; k < sh.hist.size(); ++k) out->histogram[k] += (int64_t)sh.hist[k];
-    for (int k = 0; k < 4 && k < (int)sh.status.size(); ++k) out->status_counts[k] += (int64_t)sh.status[k];
-    for (size_t k = 0; k < sh.failed_at.size(); ++k) out->failed_at_step[k] += (int64_t)sh.failed_at[k];
-  }
+  std::vector<OkinStudyCounts> counts;
+  for (const StudyShard& sh : shards) counts.push_back({sh.hist.data(), sh.status.data(), sh.failed_at.data()});
+  okin_study_fold(run.acc.data(), n_steps, run.SQ, run.nb, counts.data(), n_devices, out);
   return OKIN_OK;
 }
 

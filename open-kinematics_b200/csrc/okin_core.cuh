@@ -42,6 +42,9 @@
 #ifndef OKIN_COMPACT_LOOPS
 #define OKIN_COMPACT_LOOPS 2
 #endif
+#include <stddef.h>
+
+#include "../../include/okin.h"
 #include "okin_defs.h"
 #include "okin_gen_constraints.cuh"
 #include "okin_metrics.cuh"
@@ -2460,4 +2463,103 @@ OKIN_HD void okin_sweep(const OkinProgram& pr, double* sm, const double* __restr
     if (out.worst_row) out.worst_row[0] = worst;
   }
   OKIN_PHASE_END
+}
+
+// ---- per-instance slices of the batch buffers (okin_batch_io, include/okin.h) -------------------
+// okin_batch_io without its last field: the kernels take the sensitivity output as a trailing
+// parameter instead, so that the parameter layout (and the code) of the instantiations that never
+// write it stays what it was before that output existed.
+struct OkinKernelIO {
+  const double* hardpoints;
+  const double* params;
+  const double* target_values;
+  int32_t* status;
+  int32_t* failed_step;
+  double* positions;
+  int32_t* iters;
+  double* max_residual;
+  double* tangents;
+  double* velocities;
+  double* tangent_health;
+  double* metrics;
+  double* design;
+  double* diagnostics;
+  double* jumps;
+  const double* instance_targets;
+  int32_t* worst_row;
+};
+static_assert(sizeof(OkinKernelIO) == offsetof(okin_batch_io, hardpoint_sensitivity), "OkinKernelIO layout");
+
+// The fields of okin_batch_io in struct order.
+enum okin_io_field {
+  OKIN_IO_HARDPOINTS = 0, OKIN_IO_PARAMS, OKIN_IO_TARGET_VALUES, OKIN_IO_STATUS, OKIN_IO_FAILED_STEP,
+  OKIN_IO_POSITIONS, OKIN_IO_ITERS, OKIN_IO_MAX_RESIDUAL, OKIN_IO_TANGENTS, OKIN_IO_VELOCITIES,
+  OKIN_IO_TANGENT_HEALTH, OKIN_IO_METRICS, OKIN_IO_DESIGN, OKIN_IO_DIAGNOSTICS, OKIN_IO_JUMPS,
+  OKIN_IO_INSTANCE_TARGETS, OKIN_IO_WORST_ROW, OKIN_IO_HARDPOINT_SENSITIVITY, OKIN_IO_COUNT
+};
+
+// The counts of the header every instance's slices depend on, read once (the sweep kernel keeps
+// them in registers across its instance loop); the counts of optional fields are read from hdr when
+// the field is wanted.
+struct OkinIOShape {
+  int32_t nin, nout, nt, n;   // input points, output points, targets, unknowns (3 * NF)
+  const int32_t* hdr;
+};
+OKIN_HD OkinIOShape okin_io_shape(const int32_t* hdr) {
+  return {hdr[OKIN_H_NIN], hdr[OKIN_H_NOUT], hdr[OKIN_H_NT], 3 * hdr[OKIN_H_NF], hdr};
+}
+
+// Elements of field f that belong to one instance (int32 for status, failed_step, iters and
+// worst_row, double otherwise); 0 for target_values, which all instances share.
+OKIN_HD size_t okin_io_count(int f, const OkinIOShape& h, int n_steps) {
+  const size_t S = (size_t)n_steps;
+  switch (f) {
+    case OKIN_IO_HARDPOINTS: return 3 * (size_t)h.nin;
+    case OKIN_IO_PARAMS: return (size_t)h.hdr[OKIN_H_NPARAM];
+    case OKIN_IO_POSITIONS: return S * 3 * h.nout;
+    case OKIN_IO_ITERS:
+    case OKIN_IO_MAX_RESIDUAL: return S;
+    case OKIN_IO_TANGENTS: return S * h.nt * h.n;
+    case OKIN_IO_VELOCITIES: return S * h.nt * 3 * h.nout;
+    case OKIN_IO_TANGENT_HEALTH: return S * 2;
+    case OKIN_IO_METRICS: return S * h.hdr[OKIN_H_NM];
+    case OKIN_IO_DESIGN: return 3 * (size_t)h.nout;
+    case OKIN_IO_DIAGNOSTICS: return S * h.hdr[OKIN_H_NDIAG];
+    case OKIN_IO_JUMPS: return S * (h.n / 3);
+    case OKIN_IO_INSTANCE_TARGETS: return (size_t)h.nt * S;
+    case OKIN_IO_HARDPOINT_SENSITIVITY: return S * h.hdr[OKIN_H_NSENS] * 3 * h.nout;
+    case OKIN_IO_TARGET_VALUES: return 0;
+    default: return 1;   // status, failed_step, worst_row
+  }
+}
+
+// Full instantiation when a per-state tangent / metric / diagnostic output is wanted, else lean.
+OKIN_HD bool okin_wants_full(const okin_batch_io& io) {
+  return io.tangents || io.velocities || io.tangent_health || io.metrics || io.diagnostics;
+}
+
+// Instance i's outputs in the batch buffers (null where the batch does not want a field; sens_out:
+// the hardpoint_sensitivity buffer or null) and its inputs: hardpoints, params (null = defaults) and
+// sweep targets (its own row of instance_targets when given, else the shared target_values).
+OKIN_HD void okin_instance_io(const OkinKernelIO& io, double* sens_out, const OkinIOShape& shape, int n_steps,
+                              long long i, OkinOutputs& out, const double*& hardpoints, const double*& params,
+                              const double*& targets) {
+#define OKIN_SLICE(p, f) ((p) ? (p) + (size_t)i * okin_io_count(f, shape, n_steps) : nullptr)
+  out.positions = OKIN_SLICE(io.positions, OKIN_IO_POSITIONS);
+  out.iters = OKIN_SLICE(io.iters, OKIN_IO_ITERS);
+  out.max_residual = OKIN_SLICE(io.max_residual, OKIN_IO_MAX_RESIDUAL);
+  out.tangents = OKIN_SLICE(io.tangents, OKIN_IO_TANGENTS);
+  out.velocities = OKIN_SLICE(io.velocities, OKIN_IO_VELOCITIES);
+  out.health = OKIN_SLICE(io.tangent_health, OKIN_IO_TANGENT_HEALTH);
+  out.metrics = OKIN_SLICE(io.metrics, OKIN_IO_METRICS);
+  out.design = OKIN_SLICE(io.design, OKIN_IO_DESIGN);
+  out.diagnostics = OKIN_SLICE(io.diagnostics, OKIN_IO_DIAGNOSTICS);
+  out.status = io.status + i;
+  out.failed_step = io.failed_step + i;
+  out.worst_row = OKIN_SLICE(io.worst_row, OKIN_IO_WORST_ROW);
+  out.sensitivity = OKIN_SLICE(sens_out, OKIN_IO_HARDPOINT_SENSITIVITY);
+  hardpoints = io.hardpoints + (size_t)i * okin_io_count(OKIN_IO_HARDPOINTS, shape, n_steps);
+  params = OKIN_SLICE(io.params, OKIN_IO_PARAMS);
+  targets = io.instance_targets ? OKIN_SLICE(io.instance_targets, OKIN_IO_INSTANCE_TARGETS) : io.target_values;
+#undef OKIN_SLICE
 }

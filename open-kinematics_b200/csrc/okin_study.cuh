@@ -188,3 +188,53 @@ OKIN_STUDY_HD inline int okin_study_bin(double x, double lo, double hi, int n_bi
   const int b = (int)((x - lo) / (hi - lo) * (double)n_bins);
   return 1 + (b < n_bins - 1 ? b : n_bins - 1);
 }
+
+// Rows p, p + OKIN_STUDY_PARTS, ... < rows of one column (step s, quantity (kind, index)) of a chunk
+// whose first row is instance `base`: pushed in row order into m; count_bin(b) records a finite
+// value in histogram bin b (n_bins > 0; lo, hi: the quantity's range).
+template <class CountBin>
+OKIN_STUDY_HD inline void okin_study_partition(const OkinStudyChunk& ch, int kind, int index, int s, long long p,
+                                               long long rows, long long base, int n_bins, double lo, double hi,
+                                               OkinMoments& m, CountBin count_bin) {
+  for (long long r = p; r < rows; r += OKIN_STUDY_PARTS) {
+    double x;
+    if (!okin_study_fetch(ch, kind, index, r, s, &x)) continue;
+    okin_moments_push(m, x, base + r);
+    if (n_bins && isfinite(x)) count_bin(okin_study_bin(x, lo, hi, n_bins));
+  }
+}
+
+// Integer results of one device: hist [SQ][n_bins + 2] (unused when n_bins == 0), status [4],
+// failed_at [n_steps].  Exact in any order, summed over the devices.
+struct OkinStudyCounts {
+  const unsigned long long* hist;
+  const unsigned long long* status;
+  const unsigned long long* failed_at;
+};
+
+// Host: the study result of the accumulated moments acc[SQ] (NaN moments and extremes and -1
+// arguments in an empty column) and of the counts of n_devices devices.
+inline void okin_study_fold(const OkinMoments* acc, int n_steps, int SQ, int n_bins, const OkinStudyCounts* devices,
+                            int n_devices, okin_study_out* out) {
+  for (int j = 0; j < SQ; ++j) {
+    const OkinMoments& m = acc[j];
+    const bool empty = m.count == 0;
+    out->count[j] = m.count;
+    out->nonfinite[j] = m.nonfinite;
+    out->mean[j] = empty ? NAN : m.mean;
+    out->m2[j] = empty ? NAN : m.m2;
+    out->min[j] = empty ? NAN : m.min;
+    out->max[j] = empty ? NAN : m.max;
+    out->argmin[j] = empty ? -1 : m.argmin;
+    out->argmax[j] = empty ? -1 : m.argmax;
+  }
+  const size_t n_hist = n_bins ? (size_t)SQ * (n_bins + 2) : 0;
+  for (size_t k = 0; k < n_hist; ++k) out->histogram[k] = 0;
+  for (int k = 0; k < 4; ++k) out->status_counts[k] = 0;
+  for (int s = 0; s < n_steps; ++s) out->failed_at_step[s] = 0;
+  for (int d = 0; d < n_devices; ++d) {
+    for (size_t k = 0; k < n_hist; ++k) out->histogram[k] += (int64_t)devices[d].hist[k];
+    for (int k = 0; k < 4; ++k) out->status_counts[k] += (int64_t)devices[d].status[k];
+    for (int s = 0; s < n_steps; ++s) out->failed_at_step[s] += (int64_t)devices[d].failed_at[s];
+  }
+}

@@ -134,6 +134,9 @@ def build_case(meta: dict):
 # Lane-emulation build of csrc/okin_core.cuh (tests only; the product never loads it).
 # ---------------------------------------------------------------------------
 _EMU = None
+# okin_default_cfg
+DEFAULT_CFG = dict(step_tol=1e-6, coarse_tol=1e-3, fine_tol=1e-4, residual_tol=1e-3, mu_init=1e-3, max_iter=50,
+                   use_predictor=4)
 
 
 def emu_lib():
@@ -151,8 +154,21 @@ def emu_lib():
         lib.okin_emu_sweep.argtypes = [ctypes.c_void_p] * 3 + [ctypes.c_long, ctypes.c_int] + [ctypes.c_void_p] * 2
         lib.okin_emu_family.restype = ctypes.c_int
         lib.okin_emu_family.argtypes = [ctypes.c_int] + [ctypes.c_void_p] * 5
+        lib.okin_emu_study.restype = ctypes.c_int
+        lib.okin_emu_study.argtypes = [ctypes.c_void_p] * 3 + [ctypes.c_longlong, ctypes.c_int] + \
+            [ctypes.c_void_p] * 4 + [ctypes.c_longlong, ctypes.c_int]
+        lib.okin_emu_study_sample.restype = ctypes.c_int
+        lib.okin_emu_study_sample.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_longlong] + [ctypes.c_void_p] * 3
+        lib.okin_emu_philox.restype = None
+        lib.okin_emu_philox.argtypes = [ctypes.c_void_p, ctypes.c_void_p]
         _EMU = lib
     return _EMU
+
+
+def emu_cfg(**overrides):
+    """``okin_solver_cfg`` of the default settings with ``overrides``."""
+    from open_kinematics_b200._lib import SolverCfg
+    return SolverCfg(**{**DEFAULT_CFG, **overrides})
 
 
 def emu_family(fam_code: int, points: np.ndarray, consts) -> tuple:
@@ -208,44 +224,40 @@ def generic_mechanism():
     return state, cons, sweep, manager, spec, arrays
 
 
+class UsageError(RuntimeError):
+    """The library would return OKIN_ERR_USAGE (hardpoint sensitivities on a topology with camber-shim records)."""
+
+
 def emu_solve(program, hardpoints: np.ndarray, values: np.ndarray, params=None, want_health=False,
-              instance_targets=None, lean=False, **cfg) -> dict:
+              instance_targets=None, lean=False, want_hardpoint_sensitivity=False, **cfg) -> dict:
     """Run the lane-emulation build of the device core; ``cfg`` overrides ``okin_solver_cfg`` fields.
     ``lean``: no tangent / metric / diagnostic outputs, i.e. the lean kernel instantiation (its own
-    predictor and the short slice)."""
-    from open_kinematics_b200._lib import BatchIO, SolverCfg
+    predictor and the short slice).  ``want_hardpoint_sensitivity``: the sensitivity instantiation and
+    its ``hardpoint_sensitivity`` output ``[n, n_steps, n_sens, n_out, 3]``."""
+    from open_kinematics_b200._lib import BatchIO, batch_shapes
     hp = np.ascontiguousarray(hardpoints, dtype=np.float64).reshape(-1, 3 * program.n_in)
     tv = np.ascontiguousarray(values, dtype=np.float64)
-    n_inst, n_steps, nt, n = hp.shape[0], tv.shape[1], tv.shape[0], program.n_unknowns
-    out = {
-        "positions": np.zeros((n_inst, n_steps, program.n_out, 3)), "iters": np.zeros((n_inst, n_steps), np.int32),
-        "max_residual": np.zeros((n_inst, n_steps)), "tangents": np.zeros((n_inst, n_steps, nt, n)),
-        "velocities": np.zeros((n_inst, n_steps, nt, program.n_out, 3)),
-        "tangent_health": np.zeros((n_inst, n_steps, 2)) if want_health else None,
-        "status": np.zeros(n_inst, np.int32), "failed_step": np.zeros(n_inst, np.int32),
-        "metrics": np.zeros((n_inst, n_steps, len(program.metric_names))) if program.metric_names else None,
-        "design": np.zeros((n_inst, program.n_out, 3)),
-        "diagnostics": np.zeros((n_inst, n_steps, len(program.diagnostic_names))) if program.diagnostic_names else None,
-        "jumps": np.zeros((n_inst, n_steps, n // 3)) if program.diagnostic_names else None,
-        "worst_row": np.zeros(n_inst, np.int32),
-    }
+    n_inst, n_steps = hp.shape[0], tv.shape[1]
+    full = not lean
+    want = {"tangents": full, "velocities": full, "tangent_health": full and want_health,
+            "metrics": full and bool(program.metric_names), "diagnostics": full and bool(program.diagnostic_names),
+            "jumps": full and bool(program.diagnostic_names), "hardpoint_sensitivity": want_hardpoint_sensitivity}
+    out = {name: np.zeros(shape, dtype) if want.get(name, True) else None
+           for name, (shape, dtype) in batch_shapes(program, n_inst, n_steps).items()}
     itv = None if instance_targets is None else np.ascontiguousarray(instance_targets, dtype=np.float64)
-    if lean:
-        for name in ("tangents", "velocities", "tangent_health", "metrics", "diagnostics", "jumps"):
-            out[name] = None
     par = None if params is None else np.ascontiguousarray(params, dtype=np.float64)
-    settings = dict(step_tol=1e-6, coarse_tol=1e-3, fine_tol=1e-4, residual_tol=1e-3, mu_init=1e-3, max_iter=50,
-                    use_predictor=4)
-    settings.update(cfg)
-    c = SolverCfg(**settings)
     hdr = np.ascontiguousarray(program.hdr)
     io = BatchIO.of(hardpoints=hp, params=par, target_values=tv, instance_targets=itv, **out)
     rc = emu_lib().okin_emu_sweep(
         hdr.ctypes.data, program.iblob.ctypes.data, program.fblob.ctypes.data, n_inst, n_steps,
-        ctypes.byref(c), ctypes.byref(io))
+        ctypes.byref(emu_cfg(**cfg)), ctypes.byref(io))
+    if rc == -3:
+        raise UsageError("hardpoint sensitivities are not available on a topology with camber-shim records")
     assert rc == 0, rc
     if out["metrics"] is None:
         out["metrics"] = np.zeros((n_inst, n_steps, 1))
+    if not want_hardpoint_sensitivity:
+        del out["hardpoint_sensitivity"]
     return out
 
 

@@ -17,8 +17,7 @@ from __future__ import annotations
 import numpy as np
 import pytest
 
-from helpers import SWEEP_CASES, authored_positions, build_case, emu_solve, generic_mechanism, load_golden
-from sens_emu import UsageError, emu_solve_sens
+from helpers import SWEEP_CASES, UsageError, authored_positions, build_case, emu_solve, generic_mechanism, load_golden
 from test_batches import batch_inputs, compile_batch
 
 # Shim-free sweeps plus the C1 corners, whose camber shim sits at its design thickness (solved without
@@ -80,7 +79,7 @@ FD_FLOOR = 2e-9
 
 
 def check_fd(prog, hp, values, n_coords=8):
-    out = emu_solve_sens(prog, hp, values)
+    out = emu_solve(prog, hp, values, want_hardpoint_sensitivity=True)
     assert (out["status"] == 0).all()
     sens = out["hardpoint_sensitivity"][0]
     k_all = len(prog.sensitivity_inputs)
@@ -120,7 +119,7 @@ QUALIFY = set(CASES) - {"c4_tbar_roll", "c4_tbar_bump"}
 @pytest.mark.parametrize("name", CASES)
 def test_invariants_emu(name):
     prog, hp, values = compile_case(name)
-    out = emu_solve_sens(prog, hp, values)
+    out = emu_solve(prog, hp, values, want_hardpoint_sensitivity=True)
     sens = out["hardpoint_sensitivity"][0]          # [S, K, n_out, 3]
     from open_kinematics_b200.core.topology import D
     kind = prog.section("OKIN_S_POINT_KIND")
@@ -149,7 +148,7 @@ def test_failed_steps_are_nan_emu():
     sus, sweep, prog = compile_batch(meta)
     hp, par = batch_inputs(meta, arr, prog, range(48))
     _, values = sweep_target_values(sweep)
-    out = emu_solve_sens(prog, hp, values)
+    out = emu_solve(prog, hp, values, want_hardpoint_sensitivity=True)
     failed = np.flatnonzero(out["status"] != 0)
     assert failed.size > 0
     sens = out["hardpoint_sensitivity"]
@@ -167,7 +166,7 @@ def test_other_outputs_unchanged_emu(name):
     rng = np.random.default_rng(3)
     hp = hp + rng.normal(0.0, 0.3, (4, hp.shape[1]))
     base = emu_solve(prog, hp, values, want_health=True)
-    with_sens = emu_solve_sens(prog, hp, values, want_health=True)
+    with_sens = emu_solve(prog, hp, values, want_health=True, want_hardpoint_sensitivity=True)
     for key in FULL_OUTPUTS:
         a, b = base[key], with_sens[key]
         if a is None:
@@ -181,8 +180,8 @@ def test_sensitivity_input_subset_emu():
     pick = [prog.sensitivity_inputs[k] for k in (5, 0, 40, 77, 13, 2)]
     sub, _, _ = compile_case("c3_rocker_ubar_coilover_roll", sensitivity_inputs=pick)
     assert sub.sensitivity_inputs == pick
-    full = emu_solve_sens(prog, hp, values)["hardpoint_sensitivity"]
-    part = emu_solve_sens(sub, hp, values)["hardpoint_sensitivity"]
+    full = emu_solve(prog, hp, values, want_hardpoint_sensitivity=True)["hardpoint_sensitivity"]
+    part = emu_solve(sub, hp, values, want_hardpoint_sensitivity=True)["hardpoint_sensitivity"]
     assert np.array_equal(part, full[:, :, [5, 0, 40, 77, 13, 2]])
     with pytest.raises(ValueError):
         compile_case("c3_rocker_ubar_coilover_roll", sensitivity_inputs=[(prog.in_keys[0], 3)])
@@ -198,7 +197,7 @@ def test_shim_topology_is_refused_emu():
     hp = np.concatenate([authored_positions(sus)[k] for k in prog.in_keys])[None]
     _, values = sweep_target_values(sweep)
     with pytest.raises(UsageError):
-        emu_solve_sens(prog, hp, values)
+        emu_solve(prog, hp, values, want_hardpoint_sensitivity=True)
 
 
 def test_linearised_std():

@@ -7,8 +7,7 @@ from __future__ import annotations
 import numpy as np
 import pytest
 
-from helpers import authored_positions, build_case, load_golden
-from sens_emu import emu_solve_sens
+from helpers import authored_positions, build_case, emu_solve, load_golden
 from test_batches import batch_inputs
 from test_hardpoint_sensitivity import FULL_OUTPUTS
 
@@ -47,7 +46,7 @@ def test_device_matches_emulation(name):
     for key in FULL_OUTPUTS:      # requesting sensitivities changes no other output
         if base.get(key) is not None:
             assert np.array_equal(base[key], dev[key], equal_nan=True), (name, key)
-    emu = emu_solve_sens(prog, hp, values)
+    emu = emu_solve(prog, hp, values, want_hardpoint_sensitivity=True)
     assert (dev["status"] == 0).all() and (emu["status"] == 0).all()
     s_dev, s_emu = dev["hardpoint_sensitivity"], emu["hardpoint_sensitivity"]
     # same algorithm, different contraction / rounding of the fp64 arithmetic; the states themselves agree

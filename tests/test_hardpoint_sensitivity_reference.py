@@ -13,8 +13,7 @@ from __future__ import annotations
 import numpy as np
 import pytest
 
-from helpers import authored_positions, build_case, load_golden, oracle_problem
-from sens_emu import emu_solve_sens
+from helpers import authored_positions, build_case, emu_solve, load_golden, oracle_problem
 from oracle.solve import ResidualComputer, design_setup, pin_rows, target_bases
 
 CASES = ["c1_dw_corner_bump", "c1_dw_corner_bump_steer", "c2_macpherson_bump_steer", "c3_rocker_ubar_coilover_roll",
@@ -118,7 +117,7 @@ def test_golden_sweep_against_restatement_emu(name):
     auth = authored_positions(sus)
     hp = np.concatenate([auth[k] for k in prog.in_keys])[None]
     _, values = sweep_target_values(sweep)
-    out = emu_solve_sens(prog, hp, np.asarray(values, dtype=np.float64))
+    out = emu_solve(prog, hp, np.asarray(values, dtype=np.float64), want_hardpoint_sensitivity=True)
     assert (out["status"] == 0).all()
     S = out["positions"].shape[1]
     K = len(prog.sensitivity_inputs)
@@ -137,7 +136,7 @@ def test_perturbed_batch_against_restatement_emu(name):
     prog = compile_suspension(sus, sweep, with_shims=False)
     hp, _ = batch_inputs(meta, arr, prog, range(32))
     _, values = sweep_target_values(sweep)
-    out = emu_solve_sens(prog, hp, np.asarray(values, dtype=np.float64))
+    out = emu_solve(prog, hp, np.asarray(values, dtype=np.float64), want_hardpoint_sensitivity=True)
     assert (out["status"] == 0).all()
     S, K = out["positions"].shape[1], len(prog.sensitivity_inputs)
     compare(prog, sus, sweep, hp, out, [S - 1], list(range(0, K, max(1, K // 4))))

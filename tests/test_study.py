@@ -1,5 +1,5 @@
 """Tolerance studies on the CPU: the sampling contract against its numpy restatement
-(tests/study_reference.py), the lane-emulated study pipeline (tests/emu/okin_emu_study.cpp: the
+(tests/study_reference.py), the lane-emulated study pipeline (tests/emu/okin_emu.cpp: the
 library's generator and reduction order with a small chunk size) against numpy statistics of the
 emulation's own per-instance outputs, shard-split invariance, the linearised spread of the hardpoint
 sensitivities, and every usage error of the C ABI."""
@@ -15,7 +15,6 @@ import pytest
 
 import study_reference as ref
 from helpers import ROOT, build_case, emu_solve, load_golden
-from sens_emu import emu_solve_sens
 from study_emu import emu_philox, emu_study, emu_study_inputs
 
 PHILOX_KAT = [
@@ -244,7 +243,7 @@ def test_linearised_spread_c1(c1):
     res = emu_study(c1, smp, 512, seed=5, points="all", chunk=128)
     prog, hp, values = compile_case("c1_dw_corner_bump")
     assert prog.in_keys == c1.program.in_keys and prog.out_keys == c1.program.out_keys
-    sens = emu_solve_sens(prog, hp, values)["hardpoint_sensitivity"]
+    sens = emu_solve(prog, hp, values, want_hardpoint_sensitivity=True)["hardpoint_sensitivity"]
     sig = np.array([0.01 if smp.source[3 * prog.in_keys.index(k) + a] >= 0 else 0.0 for k, a in prog.sensitivity_inputs])
     lin = linearised_std(sens, sig)[0].reshape(values.shape[1], -1)
     mask = lin > 1e-4
