@@ -33,6 +33,7 @@ from .constraints import (
 )
 from .enums import TargetPositionMode
 from .points.derived.manager import DerivedPointsManager, DerivedPointsSpec
+from .schedule import Dest, schedule
 from .targeting import resolve_target
 
 _CSRC = os.path.join(os.path.dirname(os.path.abspath(__file__)), "..", "csrc")
@@ -598,20 +599,36 @@ def compile_topology(
         rep_pins += [pin_row[(row.source[1], 0)], pin_row[(row.source[1], 1)]]
 
     # ---- left-looking update lists, scale tasks -------------------------------
-    # One task per block *row* (3 entries): acc[c] -= a . B[c][:] for every earlier column K,
+    # One task per block *row* (3 entries): acc[c] -= a . B[c][:] for earlier columns K,
     # a = row r of L_iK, B = L_jK.  The right-hand side of the step equation is carried as one
     # extra block-row of the factor (a = y_K), which makes the forward substitution part of the
     # factorisation; the tangent right-hand sides ride along the same way.  Offsets are relative
-    # to the instance's shared-memory base.
+    # to the instance's shared-memory base.  The contribution of column K runs in the update phase
+    # of some level in [level(K) + 1, level(j)] (core/schedule.py), so a destination may be visited
+    # by one task in each of several levels.
     cols_with = [[] for _ in range(NF)]        # cols_with[j] = K < j with L_jK != 0
     for k in range(NF):
         for i in struct[k]:
             cols_with[i].append(k)
     lev_cols = [[j for j in range(NF) if level[j] == lv] for lv in range(NLEV)]
+    LB, VEC = "LB", "VEC"      # symbolic bases, resolved once the layout is known
+
+    # destinations: (block row i of column j, or i = None for the carried right-hand sides, its sources)
+    upd_dests = []
+    for lv in range(NLEV):
+        for j in lev_cols[lv]:
+            for i in [j] + struct[j]:
+                ks = [k for k in cols_with[j] if i == j or i in struct[k]]
+                if ks:
+                    upd_dests.append((i, j, ks))
+            if cols_with[j]:
+                upd_dests.append((None, j, cols_with[j]))
+    upd_phase, upd_before, upd_after = schedule(
+        [Dest(1 if i is None else 3, level[j], [level[k] + 1 for k in ks]) for i, j, ks in upd_dests], NLEV)
+
     lev_upd, upd_dst, upd_ptr, upd_con = [0], [], [0], []
     lev_scl, scl = [0], []
     lev_upd_mid, lev_scl_mid = [], []   # end of the tasks a solve without tangents needs, per level
-    LB, VEC = "LB", "VEC"      # symbolic bases, resolved once the layout is known
 
     def add_update(dst, cons):
         upd_dst.append(dst)
@@ -619,23 +636,23 @@ def compile_topology(
         upd_ptr.append(len(upd_con))
 
     for lv in range(NLEV):
-        # block rows and the step right-hand side first, the tangent right-hand sides last: a solve that
-        # does not carry tangents (lean kernel) stops at the "mid" pointer of the level
+        # heaviest first; block rows and the step right-hand side before the tangent right-hand sides: a
+        # solve that does not carry tangents (lean kernel) stops at the "mid" pointer of the level
+        here = [(d, [k for k, p in zip(ks, upd_phase[d]) if p == lv]) for d, (_, _, ks) in enumerate(upd_dests)]
+        here = sorted((t for t in here if t[1]), key=lambda t: -len(t[1]))
         for tangent_pass in (False, True):
-            for j in lev_cols[lv]:
-                if not tangent_pass:
-                    for i in [j] + struct[j]:
-                        ks = [k for k in cols_with[j] if i == j or i in struct[k]]
-                        if not ks:
-                            continue
-                        for r in range(3):
-                            add_update((LB, boff(i, j) + 3 * r),
-                                       [((LB, boff(i, k) + 3 * r), (LB, boff(j, k))) for k in ks])
-                if cols_with[j]:
+            for d, ks in here:
+                i, j, _ = upd_dests[d]
+                if i is not None and not tangent_pass:
+                    for r in range(3):
+                        add_update((LB, boff(i, j) + 3 * r),
+                                   [((LB, boff(i, k) + 3 * r), (LB, boff(j, k))) for k in ks])
+                elif i is None:
                     for rhs in (range(1, 1 + len(targets)) if tangent_pass else (0,)):
                         # carried right-hand sides: step (0) and tangents (1..NT)
                         add_update((VEC, rhs * 3 * NF + 3 * j),
-                                   [((VEC, rhs * 3 * NF + 3 * k), (LB, boff(j, k))) for k in cols_with[j]])
+                                   [((VEC, rhs * 3 * NF + 3 * k), (LB, boff(j, k))) for k in ks])
+            for j in lev_cols[lv]:
                 if not tangent_pass:
                     for i in struct[j]:
                         for r in range(3):
@@ -648,6 +665,7 @@ def compile_topology(
         lev_upd.append(len(upd_dst))
         lev_scl.append(len(scl))
 
+    # per-column lists of the factor products L z / L^T z (okin_factor_multiply)
     fw_ptr, fw_con, bw_ptr, bw_con = [0], [], [0], []
     for j in range(NF):
         for k in cols_with[j]:
@@ -660,6 +678,29 @@ def compile_topology(
     for lv in range(NLEV):
         lev_col.extend(lev_cols[lv])
         lev_col_ptr.append(len(lev_col))
+
+    # triangular solves: per phase, tasks {destination column j, finalise flag, its contributions}.  The
+    # forward phases run the levels upwards (y_K is final after level(K)), the backward ones from the
+    # root down (x_I is final after level(I)); a column is finalised (3x3 diagonal solve) in its own level.
+    fw_phase, fw_before, fw_after = schedule(
+        [Dest(1, level[j], [level[k] + 1 for k in cols_with[j]], True) for j in range(NF)], NLEV)
+    bw_phase, bw_before, bw_after = schedule(
+        [Dest(1, NLEV - 1 - level[j], [NLEV - level[i] for i in struct[j]], True) for j in range(NF)], NLEV)
+    sol_lev, sol_task = [], []        # task = (column, finalise, [(block ref, 3 * source column)])
+    for srcs, phase, of in ((cols_with, fw_phase, lambda j, k: boff(j, k)), (struct, bw_phase, lambda j, i: boff(i, j))):
+        for ph in range(NLEV):
+            sol_lev.append(len(sol_task))
+            here = []
+            for j in range(NF):
+                cons = [((LB, of(j, s)), 3 * s) for s, p in zip(srcs[j], phase[j]) if p == ph]
+                fin = ph == (level[j] if srcs is cols_with else NLEV - 1 - level[j])
+                if cons or fin:
+                    here.append((j, fin, cons))
+            sol_task += sorted(here, key=lambda t: -len(t[2]))
+        sol_lev.append(len(sol_task))
+    sched_stats = {"factor_update": {"before": upd_before, "after": upd_after},
+                   "forward_solve": {"before": fw_before, "after": fw_after},
+                   "backward_solve": {"before": bw_before, "after": bw_after}}
 
     elim_point = [pidx[free_order[order[j]]] for j in range(NF)]
     elim_col = [order[j] for j in range(NF)]
@@ -742,14 +783,15 @@ def compile_topology(
                 trace.access(lanes, [ref(scl[t][0]) for t in ts], (1, 3, 4, 6, 7, 8))
                 trace.access(lanes, [ref(scl[t][1]) for t in ts], (0, 1, 2, 0, 1, 2))   # load + store
         nrhs = 1 + len(targets)
-        for lv in range(NLEV):                                        # backward solve, all right-hand sides
-            tasks = [(j, r) for j in lev_cols[lv] for r in range(nrhs)]
+        for ph in range(NLEV):                                        # backward solve, all right-hand sides
+            tasks = [t for t in sol_task[sol_lev[NLEV + 1 + ph]:sol_lev[NLEV + 2 + ph]] for _ in range(nrhs)]
             for r0 in range(0, len(tasks), 32):
                 ts = tasks[r0:r0 + 32]
-                for q in range(max((bw_ptr[j + 1] - bw_ptr[j] for j, _ in ts), default=0)):
-                    act = [(n, j) for n, (j, _) in enumerate(ts) if bw_ptr[j + 1] - bw_ptr[j] > q]
-                    trace.access([n for n, _ in act], [ref(bw_con[bw_ptr[j] + q][0]) for _, j in act], range(9))
-                trace.access(list(range(len(ts))), [("LB", boff(j, j)) for j, _ in ts], (1, 3, 4, 6, 7, 8))
+                for q in range(max(len(t[2]) for t in ts)):
+                    act = [(n, t) for n, t in enumerate(ts) if len(t[2]) > q]
+                    trace.access([n for n, _ in act], [ref(t[2][q][0]) for _, t in act], range(9))
+                fin = [(n, t[0]) for n, t in enumerate(ts) if t[1]]
+                trace.access([n for n, _ in fin], [("LB", boff(j, j)) for _, j in fin], (1, 3, 4, 6, 7, 8))
         for r0 in range(0, NAT, 32):                                  # assembly: block stores
             ts = range(r0, min(r0 + 32, NAT))
             trace.access([t - r0 for t in ts], [("LB", 9 * (asm_task[t] & 0xFFFF)) for t in ts], range(9))
@@ -770,6 +812,13 @@ def compile_topology(
     scl = [sm(d) | (sm(r) << 16) for d, r in scl]
     fw_con = [(sm(b) << 16) | v for b, v in fw_con]
     bw_con = [(sm(b) << 16) | v for b, v in bw_con]
+    sol_con, sol_words = [], []
+    for j, fin, cons in sol_task:
+        sol_words.append((len(sol_con) << 16) | (D["OKIN_SOLVE_FIN"] if fin else 0) | j)
+        sol_con += [(sm(b) << 16) | v for b, v in cons]
+    sol_words.append(len(sol_con) << 16)          # end of the last task's contributions
+    if len(sol_con) >= 65536:
+        raise ValueError("Triangular-solve lists exceed the 16-bit index range")
 
     # ---- blobs ------------------------------------------------------------------
     row_tab = []
@@ -840,6 +889,7 @@ def compile_topology(
         "OKIN_S_LEV_UPD": lev_upd, "OKIN_S_UPD_DST": upd_dst, "OKIN_S_UPD_PTR": upd_ptr, "OKIN_S_UPD_CON": upd_con,
         "OKIN_S_LEV_SCL": lev_scl, "OKIN_S_SCL": scl,
         "OKIN_S_LEV_COL_PTR": lev_col_ptr, "OKIN_S_LEV_COL": lev_col,
+        "OKIN_S_SOLVE_LEV": sol_lev, "OKIN_S_SOLVE_TASK": sol_words, "OKIN_S_SOLVE_CON": sol_con,
         "OKIN_S_FW_PTR": fw_ptr, "OKIN_S_FW_CON": fw_con, "OKIN_S_BW_PTR": bw_ptr, "OKIN_S_BW_CON": bw_con,
         "OKIN_S_ELIM_POINT": elim_point, "OKIN_S_ELIM_COL": elim_col,
         "OKIN_S_TGT_SC_PTR": tgt_sc_ptr, "OKIN_S_TGT_SC": tgt_sc,
@@ -907,7 +957,7 @@ def compile_topology(
         "asm_fma": 9 * len(asm_con), "g_fma": 3 * len(g_con), "update_fma": 9 * len(upd_con),
         "scale_tasks": len(scl) + NF, "solve_fma": 9 * (len(fw_con) + len(bw_con)) + 12 * NF,
         "smem_doubles": off, "iblob_words": int(iblob.size), "dense_lu_flops": dense_flops,
-        "layout_tuning": tuning,
+        "layout_tuning": tuning, "schedule_wavefronts": sched_stats,
     }
     return TopologyProgram(
         hdr=hdr, iblob=iblob, fblob=fblob, point_keys=point_keys, free_order=free_order, in_keys=in_keys,

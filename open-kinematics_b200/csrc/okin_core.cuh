@@ -839,33 +839,34 @@ OKIN_FN_HOT void okin_factor(const OkinProgram& pr, double* sm, OkinState& st, b
 
 // Solve A X = B for nrhs right-hand sides stored at vec[first .. first+nrhs) (elimination order),
 // in place.  skip_forward: vec[first] already holds L^{-1} b (the factorisation carries vec[0]
-// as an extra row).
+// as an extra row).  Each phase runs tasks {column j, contributions, finalise}: a task subtracts its
+// contributions from v_j and, on the column's last visit, applies the 3x3 diagonal solve.
 template <typename Dummy = void>
 OKIN_FN_HOT void okin_solve(const OkinProgram& pr, double* sm, int first, int nrhs, bool skip_forward) {
   sm = OKIN_SHARED(sm);
   const int32_t* hdr = OKIN_SHARED(pr.hdr);
   const int nlev = hdr[OKIN_H_NLEV];
   const int n = 3 * hdr[OKIN_H_NF];
-  const int32_t* lcp = OKIN_SHARED(okin_sec(pr, OKIN_S_LEV_COL_PTR));
-  const int32_t* lcol = OKIN_SHARED(okin_sec(pr, OKIN_S_LEV_COL));
-  const int32_t* fptr = OKIN_SHARED(okin_sec(pr, OKIN_S_FW_PTR));
-  const int32_t* fcon = OKIN_SHARED(okin_sec(pr, OKIN_S_FW_CON));
-  const int32_t* bptr = OKIN_SHARED(okin_sec(pr, OKIN_S_BW_PTR));
-  const int32_t* bcon = OKIN_SHARED(okin_sec(pr, OKIN_S_BW_CON));
+  const int32_t* slev = OKIN_SHARED(okin_sec(pr, OKIN_S_SOLVE_LEV));
+  const int32_t* stask = OKIN_SHARED(okin_sec(pr, OKIN_S_SOLVE_TASK));
+  const int32_t* scon = OKIN_SHARED(okin_sec(pr, OKIN_S_SOLVE_CON));
   const double* Lb = sm;
   const int32_t* doffs = OKIN_SHARED(okin_sec(pr, OKIN_S_DIAG_OFF));
   double* vec = sm + hdr[OKIN_H_OFF_VEC] + first * n;
   for (int lv = 0; lv < (skip_forward ? 0 : nlev); ++lv) {  // L y = b
-    const int cb = OKIN_LDG(lcp + lv), ce = OKIN_LDG(lcp + lv + 1);
+    const int tb = OKIN_LDG(slev + lv), te = OKIN_LDG(slev + lv + 1);
     OKIN_PHASE_BEGIN
     OKIN_LANE_LOOP
-    for (int t = lane; t < (ce - cb) * nrhs; t += 32) {
-      const int j = OKIN_LDG(lcol + cb + t / nrhs);
+    for (int t = lane; t < (te - tb) * nrhs; t += 32) {
+      const int k = tb + t / nrhs;
+      const uint32_t task = (uint32_t)OKIN_LDG(stask + k);
+      const int j = task & 0x7fffu;
+      const int qe = (int)((uint32_t)OKIN_LDG(stask + k + 1) >> 16);
       double* v = vec + (t % nrhs) * n;
       double t0 = v[3 * j], t1 = v[3 * j + 1], t2 = v[3 * j + 2];
       OKIN_UNROLL_INNER
-      for (int q = OKIN_LDG(fptr + j); q < OKIN_LDG(fptr + j + 1); ++q) {
-        const uint32_t w = (uint32_t)OKIN_LDG(fcon + q);
+      for (int q = (int)(task >> 16); q < qe; ++q) {
+        const uint32_t w = (uint32_t)OKIN_LDG(scon + q);
         const double* B = Lb + (w >> 16);
         const double* y = v + (w & 0xffffu);
         const double y0 = y[0], y1 = y[1], y2 = y[2];
@@ -874,25 +875,30 @@ OKIN_FN_HOT void okin_solve(const OkinProgram& pr, double* sm, int first, int nr
         t0 = fma(-b1, y1, t0); t1 = fma(-b4, y1, t1); t2 = fma(-b7, y1, t2);
         t0 = fma(-b2, y2, t0); t1 = fma(-b5, y2, t1); t2 = fma(-b8, y2, t2);
       }
-      const double* f = sm + OKIN_LDG(doffs + j);
-      const double y0 = t0 * f[6];
-      const double y1 = (t1 - f[1] * y0) * f[7];
-      const double y2 = (t2 - f[3] * y0 - f[4] * y1) * f[8];
-      v[3 * j] = y0; v[3 * j + 1] = y1; v[3 * j + 2] = y2;
+      if (task & OKIN_SOLVE_FIN) {
+        const double* f = sm + OKIN_LDG(doffs + j);
+        t0 = t0 * f[6];
+        t1 = (t1 - f[1] * t0) * f[7];
+        t2 = (t2 - f[3] * t0 - f[4] * t1) * f[8];
+      }
+      v[3 * j] = t0; v[3 * j + 1] = t1; v[3 * j + 2] = t2;
     }
     OKIN_PHASE_END
   }
-  for (int lv = nlev - 1; lv >= 0; --lv) {  // L^T x = y
-    const int cb = OKIN_LDG(lcp + lv), ce = OKIN_LDG(lcp + lv + 1);
+  for (int ph = 0; ph < nlev; ++ph) {  // L^T x = y
+    const int tb = OKIN_LDG(slev + nlev + 1 + ph), te = OKIN_LDG(slev + nlev + 2 + ph);
     OKIN_PHASE_BEGIN
     OKIN_LANE_LOOP
-    for (int t = lane; t < (ce - cb) * nrhs; t += 32) {
-      const int j = OKIN_LDG(lcol + cb + t / nrhs);
+    for (int t = lane; t < (te - tb) * nrhs; t += 32) {
+      const int k = tb + t / nrhs;
+      const uint32_t task = (uint32_t)OKIN_LDG(stask + k);
+      const int j = task & 0x7fffu;
+      const int qe = (int)((uint32_t)OKIN_LDG(stask + k + 1) >> 16);
       double* v = vec + (t % nrhs) * n;
       double t0 = v[3 * j], t1 = v[3 * j + 1], t2 = v[3 * j + 2];
       OKIN_UNROLL_INNER
-      for (int q = OKIN_LDG(bptr + j); q < OKIN_LDG(bptr + j + 1); ++q) {
-        const uint32_t w = (uint32_t)OKIN_LDG(bcon + q);
+      for (int q = (int)(task >> 16); q < qe; ++q) {
+        const uint32_t w = (uint32_t)OKIN_LDG(scon + q);
         const double* B = Lb + (w >> 16);
         const double* x = v + (w & 0xffffu);
         const double x0 = x[0], x1 = x[1], x2 = x[2];
@@ -901,11 +907,13 @@ OKIN_FN_HOT void okin_solve(const OkinProgram& pr, double* sm, int first, int nr
         t0 = fma(-b3, x1, t0); t1 = fma(-b4, x1, t1); t2 = fma(-b5, x1, t2);
         t0 = fma(-b6, x2, t0); t1 = fma(-b7, x2, t1); t2 = fma(-b8, x2, t2);
       }
-      const double* f = sm + OKIN_LDG(doffs + j);
-      const double x2 = t2 * f[8];
-      const double x1 = (t1 - f[4] * x2) * f[7];
-      const double x0 = (t0 - f[1] * x1 - f[3] * x2) * f[6];
-      v[3 * j] = x0; v[3 * j + 1] = x1; v[3 * j + 2] = x2;
+      if (task & OKIN_SOLVE_FIN) {
+        const double* f = sm + OKIN_LDG(doffs + j);
+        t2 = t2 * f[8];
+        t1 = (t1 - f[4] * t2) * f[7];
+        t0 = (t0 - f[1] * t1 - f[3] * t2) * f[6];
+      }
+      v[3 * j] = t0; v[3 * j + 1] = t1; v[3 * j + 2] = t2;
     }
     OKIN_PHASE_END
   }

@@ -164,10 +164,11 @@ enum okin_isec {
   OKIN_S_SCL,            // [..] = diag block offset | row offset << 16 (shared-memory offsets)
   OKIN_S_LEV_COL_PTR,    // [NLEV+1]
   OKIN_S_LEV_COL,        // elimination columns of each level
-  OKIN_S_FW_PTR,         // [NF+1]
-  OKIN_S_FW_CON,         // (block offset << 16) | (3*K)
-  OKIN_S_BW_PTR,         // [NF+1]
-  OKIN_S_BW_CON,         // (block offset << 16) | (3*I)
+  OKIN_S_SOLVE_LEV,      // [2][NLEV+1] task ranges of the forward phases (levels upwards), then of the
+                         // backward phases (levels from the root down)
+  OKIN_S_SOLVE_TASK,     // (first contribution << 16) | OKIN_SOLVE_FIN | column; the next word's first
+                         // contribution ends the range (one extra word after the last task)
+  OKIN_S_SOLVE_CON,      // (block offset << 16) | (3 * source column)
   OKIN_S_ELIM_POINT,     // [NF] elimination position -> point index
   OKIN_S_TGT_SC_PTR,     // [NT+1]
   OKIN_S_TGT_SC,         // (rg index << 16) | unknown index (elimination order)
@@ -199,6 +200,10 @@ enum okin_isec {
   OKIN_S_DGOP,           // [NDGOP][OKIN_DGOP_STRIDE] topology diagnostic ops
   OKIN_S_ELIM_COL,       // [NF] elimination position -> reference column block (sorted free-point order)
   OKIN_S_ELIM_OUT,       // [NF] elimination position -> output slot of that free point, -1 = not exported
+  OKIN_S_FW_PTR,         // [NF+1] per-column lists of L z (okin_factor_multiply)
+  OKIN_S_FW_CON,         // (block offset << 16) | (3*K)
+  OKIN_S_BW_PTR,         // [NF+1] per-column lists of L^T z
+  OKIN_S_BW_CON,         // (block offset << 16) | (3*I)
   OKIN_S_COUNT,
   // Sections from here on are not in the per-CTA section table (okin_resolve_section), so the kernels
   // that never read them keep their shared-memory layout; device code reaches them with okin_sec_cold.
@@ -206,6 +211,8 @@ enum okin_isec {
   OKIN_S_COUNT_ALL
 };
 #define OKIN_ASM_DIAG 0x40000000
+// Solve task flag: the visit finalises its column (3x3 diagonal solve after the contributions).
+#define OKIN_SOLVE_FIN 0x8000
 // Contribution words carry a negate flag: the product enters with a minus sign (a fast distance
 // row stores u = dR/dp2 once, dR/dp1 = -u).
 #define OKIN_CON_NEG 0x80000000
