@@ -86,7 +86,9 @@
 #ifndef OKIN_H
 #define OKIN_H
 
+#ifndef __CUDACC_RTC__
 #include <stdint.h>
+#endif
 
 #ifdef __cplusplus
 extern "C" {
@@ -193,10 +195,28 @@ int okin_shard_range(int64_t n_instances, int32_t shard, int32_t n_shards, int64
 int okin_launch_geometry(okin_topology* topo, int32_t device, int64_t n_instances, int32_t* grid, int32_t* block,
                          int32_t* smem_bytes, int32_t* ctas_per_sm);
 
-/* Which lean kernel family (positions + solver statistics only) this topology uses on `device`:
- * registers = 128 or 168 once the first large batch has timed both on that device, 0 before;
- * the two calibration times in ms (0 when fixed by OKIN_LEAN_REGS or not yet run). */
-int okin_lean_calibration(okin_topology* topo, int32_t device, int32_t* registers, double* ms_wide, double* ms_128);
+/* Which lean kernel family (positions + solver statistics only) this topology uses on `device`.  The
+ * first large batch on a device times the generic 168- and 128-register families and, when the
+ * topology has a spec (okin_topology_set_spec) that NVRTC compiles, the same two families specialised
+ * to the topology, and keeps the fastest; OKIN_LEAN_REGS = 128 | 168 | spec128 | spec168 pins one. */
+typedef struct okin_lean_family {
+  int32_t registers;     /* 128 or 168 once chosen on that device, 0 before */
+  int32_t specialised;   /* 1: the topology-specialised kernel of that register cap */
+  double ms[4];          /* calibration times in ms: generic 168, generic 128, specialised 168, specialised 128
+                            (0 when not timed: pinned, not yet run, or the specialised kernels unavailable) */
+  double spec_compile_s; /* NVRTC compile time of the specialised kernels (s), 0 when not compiled */
+  char spec_error[256];  /* why the specialised kernels are not in use ("" when they compiled and loaded) */
+} okin_lean_family;
+int okin_lean_calibration(okin_topology* topo, int32_t device, okin_lean_family* out);
+
+/* Source of the topology's generated spec (okin_spec.h, TopologyProgram.spec_source); set before the
+ * first lean launch.  Without one only the generic lean kernels run. */
+int okin_topology_set_spec(okin_topology* topo, const char* source);
+
+/* Compile the lean kernels of a spec with NVRTC for sm_100a and --ptxas-options=-v, without a device:
+ * the log (registers, spills) and the cubin (copied when cubin_capacity suffices). */
+int okin_spec_compile(const char* source, int32_t shim, char* log, int32_t log_len, int64_t* cubin_bytes,
+                      void* cubin, int64_t cubin_capacity);
 
 /* Dependent-DFMA-chain microbenchmark: measured fp64 FMA peak of `device` in TFLOP/s
  * (the roofline denominator; MEASURED_PEAKS.json carries no fp64 figure). */

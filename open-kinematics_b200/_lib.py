@@ -69,6 +69,12 @@ class TopologyInfo(ctypes.Structure):
         "smem_bytes_per_instance", "n_levels", "n_metrics", "n_params", "n_diagnostics")]
 
 
+class LeanFamily(ctypes.Structure):
+    """``okin_lean_family``: the lean kernel family a topology uses on a device."""
+    _fields_ = [("registers", ctypes.c_int32), ("specialised", ctypes.c_int32), ("ms", ctypes.c_double * 4),
+                ("spec_compile_s", ctypes.c_double), ("spec_error", ctypes.c_char * 256)]
+
+
 class StudyDesc(ctypes.Structure):
     """``okin_study_desc``: sampling tables and quantity list of a tolerance study (host addresses)."""
     _fields_ = [("seed", ctypes.c_uint64), ("n_variates", ctypes.c_int32), ("variate_kind", ctypes.c_void_p),
@@ -153,7 +159,10 @@ SIGNATURES = {
     "okin_launch_geometry": (ctypes.c_int, [
         ctypes.c_void_p, ctypes.c_int32, ctypes.c_int64, c_i32p, c_i32p, c_i32p, c_i32p]),
     "okin_fp64_peak": (ctypes.c_int, [ctypes.c_int32, c_f64p]),
-    "okin_lean_calibration": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int32, c_i32p, c_f64p, c_f64p]),
+    "okin_lean_calibration": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int32, ctypes.POINTER(LeanFamily)]),
+    "okin_topology_set_spec": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_char_p]),
+    "okin_spec_compile": (ctypes.c_int, [ctypes.c_char_p, ctypes.c_int32, ctypes.c_char_p, ctypes.c_int32,
+                                         ctypes.POINTER(ctypes.c_int64), ctypes.c_void_p, ctypes.c_int64]),
     "okin_host_alloc": (ctypes.c_int, [ctypes.c_int64, ctypes.c_int32, ctypes.POINTER(ctypes.c_void_p)]),
     "okin_host_free": (ctypes.c_int, [ctypes.c_void_p]),
     "okin_study": (ctypes.c_int, [
@@ -176,7 +185,7 @@ def build(force: bool = False, verbose: bool = False) -> str:
     if not force and os.path.exists(LIB_PATH):
         if os.path.getmtime(LIB_PATH) >= max(os.path.getmtime(s) for s in sources):
             return LIB_PATH
-    cmd = ["nvcc", *NVCC_FLAGS, "-o", LIB_PATH, os.path.join(CSRC, "okin_abi.cu")]
+    cmd = ["nvcc", *NVCC_FLAGS, "-o", LIB_PATH, os.path.join(CSRC, "okin_abi.cu"), "-ldl"]
     if verbose:
         cmd.insert(1, "-Xptxas=-v")
     proc = subprocess.run(cmd, capture_output=True, text=True)
@@ -185,6 +194,33 @@ def build(force: bool = False, verbose: bool = False) -> str:
     if verbose:
         print(proc.stderr)
     return LIB_PATH
+
+
+def nvrtc_available() -> bool:
+    """Whether the toolkit's run-time compiler can be loaded (the specialised lean kernels need it)."""
+    for name in ("libnvrtc.so.12", "libnvrtc.so"):
+        try:
+            ctypes.CDLL(name)
+            return True
+        except OSError:
+            pass
+    return False
+
+
+def spec_compile(program) -> tuple:
+    """``(cubin bytes, log)``: NVRTC compile of ``program``'s specialised lean kernels for sm_100a with
+    ``--ptxas-options=-v`` (registers and spills per register cap in the log).  Needs no device."""
+    log = ctypes.create_string_buffer(1 << 16)
+    n = ctypes.c_int64()
+    src = program.spec_source().encode()
+    from .core.topology import D
+    shim = int(program.hdr[D["OKIN_H_NSHIM"]] > 0)
+    rc = load().okin_spec_compile(src, shim, log, len(log), ctypes.byref(n), None, 0)
+    buf = ctypes.create_string_buffer(max(n.value, 1))
+    if rc == 0:
+        rc = load().okin_spec_compile(src, shim, log, len(log), ctypes.byref(n), buf, len(buf))
+    check(rc, "okin_spec_compile")
+    return buf.raw[:n.value], log.value.decode()
 
 
 def load() -> ctypes.CDLL:
@@ -275,6 +311,7 @@ class DeviceTopology:
         )
         self.handle = ctypes.c_void_p()
         check(load().okin_topology_create(ctypes.byref(desc), ctypes.byref(self.handle)), "okin_topology_create")
+        check(load().okin_topology_set_spec(self.handle, program.spec_source().encode()), "okin_topology_set_spec")
 
     def info(self) -> TopologyInfo:
         out = TopologyInfo()
@@ -289,10 +326,11 @@ class DeviceTopology:
 
     def lean_calibration(self, device: int = 0) -> dict:
         """Lean kernel family chosen for this topology on ``device`` (see ``okin_lean_calibration``)."""
-        regs, wide, narrow = ctypes.c_int32(), ctypes.c_double(), ctypes.c_double()
-        check(load().okin_lean_calibration(self.handle, device, ctypes.byref(regs), ctypes.byref(wide),
-                                           ctypes.byref(narrow)), "okin_lean_calibration")
-        return {"registers": regs.value, "ms_168": wide.value, "ms_128": narrow.value}
+        out = LeanFamily()
+        check(load().okin_lean_calibration(self.handle, device, ctypes.byref(out)), "okin_lean_calibration")
+        return {"registers": out.registers, "specialised": bool(out.specialised), "ms_168": out.ms[0],
+                "ms_128": out.ms[1], "ms_spec_168": out.ms[2], "ms_spec_128": out.ms[3],
+                "spec_compile_s": out.spec_compile_s, "spec_error": out.spec_error.decode()}
 
     def close(self) -> None:
         if self.handle:

@@ -154,6 +154,76 @@ class TopologyProgram:
         off, n = self.hdr[D["OKIN_H_FSEC0"] + 2 * s], self.hdr[D["OKIN_H_FSEC0"] + 2 * s + 1]
         return self.fblob[off: off + n]
 
+    def spec_phases(self) -> list:
+        """Task lists of the lean kernel's hot phases, in the phase order of ``csrc/okin_core.cuh``
+        (OKIN_PH_*): per phase a list of ``(task word, [contribution words])``."""
+        sec = lambda name: [int(w) & 0xFFFFFFFF for w in self.section(name)]   # noqa: E731
+        h = self.hdr
+        nat, nf, nlev = int(h[D["OKIN_H_NAT"]]), int(h[D["OKIN_H_NF"]]), int(h[D["OKIN_H_NLEV"]])
+        aptr, atask, acon = sec("OKIN_S_ASM_PTR"), sec("OKIN_S_ASM_TASK"), sec("OKIN_S_ASM_CON")
+        gptr, gcon = sec("OKIN_S_G_PTR"), sec("OKIN_S_G_CON")
+        phases = [[(atask[t], acon[aptr[t]:aptr[t + 1]]) for t in range(nat)],
+                  [(j, gcon[gptr[j]:gptr[j + 1]]) for j in range(nf)]]
+        lev_upd, upd_mid = sec("OKIN_S_LEV_UPD"), sec("OKIN_S_LEV_UPD_MID")
+        udst, uptr, ucon = sec("OKIN_S_UPD_DST"), sec("OKIN_S_UPD_PTR"), sec("OKIN_S_UPD_CON")
+        lev_scl, scl_mid, scl = sec("OKIN_S_LEV_SCL"), sec("OKIN_S_LEV_SCL_MID"), sec("OKIN_S_SCL")
+        lcp, lcol, doffs = sec("OKIN_S_LEV_COL_PTR"), sec("OKIN_S_LEV_COL"), sec("OKIN_S_DIAG_OFF")
+        for lv in range(nlev):   # the lean kernel never carries tangent right-hand sides: up to the mid pointers
+            phases.append([(udst[t], ucon[uptr[t]:uptr[t + 1]]) for t in range(lev_upd[lv], upd_mid[lv])])
+            phases.append([(doffs[lcol[c]], []) for c in range(lcp[lv], lcp[lv + 1])])
+            phases.append([(scl[t], []) for t in range(lev_scl[lv], scl_mid[lv])])
+        slev, stask, scon = sec("OKIN_S_SOLVE_LEV"), sec("OKIN_S_SOLVE_TASK"), sec("OKIN_S_SOLVE_CON")
+        assert max(doffs, default=0) < 1 << 16
+        for p in list(range(nlev)) + [nlev + 1 + ph for ph in range(nlev)]:
+            # solve task word: FIN | column, with the column's diagonal block offset in the high half
+            phases.append([((stask[k] & 0xFFFF) | doffs[stask[k] & 0x7FFF] << 16,
+                            scon[stask[k] >> 16:stask[k + 1] >> 16]) for k in range(slev[p], slev[p + 1])])
+        return phases
+
+    def spec_source(self) -> str:
+        """C++ header ``okin_spec.h`` of this program for an OKIN_SPEC build of ``csrc/okin_core.cuh``:
+        the header fields as constants, and every hot phase as lane rounds whose task and contribution
+        words are packed lane-major into ``okin_spec_words``.  A round takes up to 32 tasks, longest
+        contribution list first, so the lanes holding slot s are always a prefix of the round."""
+        words, phase_round, rounds, slot_lanes = [], [], [], []
+        for tasks in self.spec_phases():
+            phase_round.append(len(rounds))
+            order = sorted(tasks, key=lambda tc: -len(tc[1]))
+            for r0 in range(0, len(order), 32):
+                chunk = order[r0:r0 + 32]
+                width, slots = len(chunk), len(chunk[0][1])
+                rounds.append((len(words), width, slots, len(slot_lanes)))
+                words += [t for t, _ in chunk]
+                for s in range(slots):
+                    slot_lanes.append(sum(len(c) > s for _, c in chunk))
+                    words += [c[s] if len(c) > s else 0 for _, c in chunk]
+        phase_round.append(len(rounds))
+        as_i32 = lambda w: str(int(np.int32(np.uint32(w))))   # noqa: E731
+        arr = lambda name, vals: (f"constexpr int32_t {name}[] = {{{', '.join(map(str, vals)) or '0'}}};")  # noqa: E731
+        hdr = " ".join(f"case {i}: return {int(v)};" for i, v in enumerate(self.hdr[:D["OKIN_H_SEC0"]]) if v)
+        col = lambda k: [r[k] for r in rounds]   # noqa: E731
+        return "\n".join([
+            "// Generated by core/topology.py (TopologyProgram.spec_source) for one topology.",
+            "#pragma once",
+            f"OKIN_HD constexpr int okin_spec_hdr(int f) {{ switch (f) {{ {hdr} default: return 0; }} }}",
+            "namespace okin_spec {",
+            arr("PHASE_ROUND", phase_round), arr("R_BASE", col(0)), arr("R_WIDTH", col(1)),
+            arr("R_SLOTS", col(2)), arr("R_SLOT0", col(3)), arr("SLOT_LANES", slot_lanes),
+            "OKIN_HD constexpr int phase_round(int p) { return PHASE_ROUND[p]; }",
+            "OKIN_HD constexpr int r_base(int r) { return R_BASE[r]; }",
+            "OKIN_HD constexpr int r_width(int r) { return R_WIDTH[r]; }",
+            "OKIN_HD constexpr int r_slots(int r) { return R_SLOTS[r]; }",
+            "OKIN_HD constexpr int r_slot0(int r) { return R_SLOT0[r]; }",
+            "OKIN_HD constexpr int slot_lanes(int i) { return SLOT_LANES[i]; }",
+            "}  // namespace okin_spec",
+            f"#define OKIN_SPEC_WORDS {max(len(words), 1)}",
+            "#ifdef __CUDACC__",
+            "__device__",
+            "#endif",
+            f"const int32_t okin_spec_words[OKIN_SPEC_WORDS] = {{{', '.join(map(as_i32, words)) or '0'}}};",
+            "",
+        ])
+
 
 # ---------------------------------------------------------------------------
 def _constraint_rows(index: int, c: Constraint, pidx: dict, design_rules: bool) -> list:

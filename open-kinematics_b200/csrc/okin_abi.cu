@@ -7,16 +7,20 @@
 // systems of tens of unknowns (SURVEY.md section 8d; measured: the shared-memory data pipe is the
 // binding unit, profiles/r02_d_*), so tensor cores and TMA have nothing to act on; the only global
 // traffic is the coalesced instance-major hardpoint read and state write.
-// okin_sweep_kernel<FULL, SHIM, MAX_THREADS, SENS> has seven instantiations: full outputs (128 registers)
-// and two lean families (128 / 168 registers), each with / without the camber-shim pre-solve, plus the
-// full outputs with hardpoint sensitivities (no pre-solve); the continuity pass of the diagnostics is a
-// second kernel on the same stream.
+// okin_sweep_kernel<FULL, SHIM, MAX_THREADS, SENS> (okin_kernel.cuh) has seven instantiations here: full
+// outputs (128 registers) and two lean families (128 / 168 registers), each with / without the camber-shim
+// pre-solve, plus the full outputs with hardpoint sensitivities (no pre-solve); the continuity pass of the
+// diagnostics is a second kernel on the same stream.  The two lean families specialised to a topology are
+// compiled at run time (compile_spec, load_spec).
 #include <cuda_runtime.h>
+#include <dlfcn.h>
+#include <nvrtc.h>
 
 #include <pthread.h>
 #include <sched.h>
 
 #include <algorithm>
+#include <chrono>
 #include <condition_variable>
 #include <cstddef>
 #include <cstdio>
@@ -29,7 +33,7 @@
 #include <vector>
 
 #include "../../include/okin.h"
-#include "okin_core.cuh"
+#include "okin_kernel.cuh"
 #include "okin_study.cuh"
 
 // Kernel families.  The register cap follows from the CTA size limit (65536 / threads):
@@ -39,13 +43,12 @@
 //                       gather-loop trip in flight when it is not squeezed for registers; at 128 it sinks
 //                       every LDS to its DFMA, profiles/r02_*)
 // Which lean family is faster depends on the topology (measured: flagship axle 168, corners and the
-// 101-step T-bar axle 128), so the first large launch of a topology on a device times both.
-#define OKIN_MAX_THREADS 512
+// 101-step T-bar axle 128), so the first large launch of a topology on a device times both.  That launch
+// also compiles both lean families specialised to the topology (NVRTC, OKIN_SPEC: the header fields and
+// the hot phases' task lists become constants) and times them too; the fastest of the four is kept.
 #define OKIN_LEAN_WIDE_THREADS 384
-enum { OKIN_FAM_LEAN_WIDE = 0, OKIN_FAM_FULL = 1, OKIN_FAM_LEAN = 2, OKIN_FAM_SENS = 3, OKIN_FAM_COUNT = 4 };
-#ifndef OKIN_DRIFT
-#define OKIN_DRIFT 1             // how many instances a warp may run ahead of the slowest warp of its CTA
-#endif
+enum { OKIN_FAM_LEAN_WIDE = 0, OKIN_FAM_FULL = 1, OKIN_FAM_LEAN = 2, OKIN_FAM_SENS = 3, OKIN_FAM_SPEC_WIDE = 4,
+       OKIN_FAM_SPEC = 5, OKIN_FAM_COUNT = 6 };
 #define OKIN_MAX_DEVICES 16
 #define OKIN_PIPE_SLOTS 3        // streams / workspace slots of the host-buffer pipeline
 #define OKIN_PIPE_CHUNK 32768   // instances per pipelined chunk
@@ -79,9 +82,13 @@ struct DeviceCopy {
   int num_sms = 0;
   // launch shape per kernel family (OKIN_FAM_*)
   struct Shape { int ctas_per_sm = 0, warps_per_cta = 0, smem_bytes = 0; } shape[OKIN_FAM_COUNT];
-  int lean_family = -1;          // OKIN_FAM_LEAN or OKIN_FAM_LEAN_WIDE once timed on this device, -1 before
-  double lean_tune_ms[2] = {0.0, 0.0};   // calibration times {wide, 128-register}
+  int lean_family = -1;          // lean family (OKIN_FAM_LEAN*, OKIN_FAM_SPEC*) once timed on this device, -1 before
+  double lean_tune_ms[4] = {0.0, 0.0, 0.0, 0.0};   // calibration times {wide, 128-register, specialised wide, 128}
   int table_doubles = 0;
+  int spec_table_doubles = 0;    // the specialised kernels also keep the spec's packed words in shared memory
+  bool spec_loaded = false;
+  cudaLibrary_t spec_lib = nullptr;
+  cudaKernel_t spec_kernel[2] = {};   // specialised lean kernels {wide, 128-register}
   int smem_optin = 0;
   // grow-only workspace for the host-buffer entry point
   void* ws = nullptr;
@@ -96,71 +103,13 @@ struct okin_topology {
   std::vector<double> fb;
   DeviceCopy dev[OKIN_MAX_DEVICES];
   std::mutex mu;
+  std::string spec;              // okin_spec.h of this topology (okin_topology_set_spec), empty = none
+  bool spec_compiled = false;    // compiled once per topology, loaded per device
+  std::vector<char> spec_cubin;
+  std::string spec_lowered[2];   // kernel names in the image: {wide, 128-register}
+  std::string spec_error;        // why the specialised kernels are not in use, empty when they are
+  double spec_compile_s = 0.0;
 };
-
-// Shared memory of a CTA = [topology tables (int32 blob)] [one state slice per warp].  The tables are
-// copied once per (persistent) CTA so that every index lookup of the interpreter is a shared-memory
-// load instead of a global one (ncu round 1: long-scoreboard stalls on __ldg were the top stall).
-// SENS: sens_out = [n_instances][n_steps][NSENS][NOUT*3], sens_ws = okin_sens_ws_doubles per resident warp.
-template <bool FULL, bool SHIM, int MAX_THREADS, bool SENS = false>
-__global__ void __launch_bounds__(MAX_THREADS, 1)
-okin_sweep_kernel(const int32_t* __restrict__ hdr, const int32_t* __restrict__ ib, const double* __restrict__ fb,
-                  long long n_instances, int n_steps, OkinSolverCfg cfg, OkinKernelIO io, int n_iblob,
-                  int table_doubles, unsigned long long* __restrict__ counter, double* sens_out, double* sens_ws) {
-  // [section pointers][header][hot tables][one state slice per warp]
-  const int32_t** sec = reinterpret_cast<const int32_t**>(okin_smem);
-  int32_t* shdr = reinterpret_cast<int32_t*>(okin_smem + OKIN_S_COUNT);
-  int32_t* tab = shdr + OKIN_HDR_SIZE;
-  for (int i = threadIdx.x; i < OKIN_HDR_SIZE; i += blockDim.x) shdr[i] = hdr[i];
-  const int n_hot = hdr[OKIN_H_NHOT];
-  for (int i = threadIdx.x; i < n_hot; i += blockDim.x) tab[i] = ib[i];
-  for (int i = threadIdx.x; i < OKIN_S_COUNT; i += blockDim.x) okin_resolve_section(hdr, tab, ib, i, sec);
-  __syncthreads();
-  hdr = shdr;
-  OkinProgram pr{shdr, tab, fb, ib, sec};
-  const int warp = threadIdx.x >> 5;
-  const int warps_per_cta = blockDim.x >> 5;
-  double* sm = okin_smem + table_doubles + (size_t)warp * hdr[FULL ? OKIN_H_SMEM_DOUBLES : OKIN_H_SMEM_DOUBLES_LEAN];
-  const OkinIOShape shape = okin_io_shape(hdr);
-  // Instances are claimed one at a time from a global counter (no static partition: a warp whose
-  // instance is slow -- a failing sweep costs a few normal ones -- simply claims fewer).  The warps of
-  // a CTA are kept loosely in step instead of meeting at a barrier: before claiming, a warp compares its
-  // own count of finished instances with the slowest live warp of the CTA and waits only while it is
-  // more than OKIN_DRIFT - 1 instances ahead.  The slowest warp never waits, so one slow instance delays
-  // nobody until the others are OKIN_DRIFT instances ahead of it; and because the warps stay within a
-  // few instances of each other they run the same code regions at about the same time, which keeps the
-  // (large) interpreter in the instruction cache (round 1 measured -10 % at 1 M instances without any
-  // coupling; a barrier per instance, OKIN_DRIFT == 1, cost 27 % on a batch with 0.8 % failing instances).
-  __shared__ int s_done[OKIN_MAX_THREADS / 32];
-  if ((threadIdx.x & 31) == 0) s_done[warp] = 0;
-  __syncthreads();
-  int mine = 0;
-  for (;;) {
-    // wait while too far ahead of the slowest live warp (finished warps park at INT_MAX)
-    for (;;) {
-      // (progress counters are read and written with shared-memory atomics: a defined cross-warp handshake)
-      int v = (int)(threadIdx.x & 31) < warps_per_cta ? atomicOr(&s_done[threadIdx.x & 31], 0) : 0x7fffffff;
-      for (int o = 16; o > 0; o >>= 1) v = min(v, __shfl_xor_sync(0xffffffffu, v, o));
-      if (mine - v < OKIN_DRIFT) break;
-      __nanosleep(256);
-    }
-    long long i = 0;
-    if ((threadIdx.x & 31) == 0) i = (long long)atomicAdd(counter, 1ull);
-    i = __shfl_sync(0xffffffffu, i, 0);
-    if (i >= n_instances) break;
-    {
-      OkinOutputs out;
-      const double *hp, *par, *tv;
-      if (SENS) out.sens_ws = sens_ws + ((size_t)blockIdx.x * warps_per_cta + warp) * okin_sens_ws_doubles(hdr);
-      okin_instance_io(io, SENS ? sens_out : nullptr, shape, n_steps, i, out, hp, par, tv);
-      okin_sweep<FULL, SHIM, SENS>(pr, sm, hp, par, tv, n_steps, cfg, out);
-      __syncwarp();
-    }
-    ++mine;
-    if ((threadIdx.x & 31) == 0) atomicExch(&s_done[warp], mine);
-  }
-  if ((threadIdx.x & 31) == 0) atomicExch(&s_done[warp], 0x7fffffff);
-}
 
 // Second pass of the sweep diagnostics: one warp per instance walks the instance's position rows
 // (okin_continuity).  Shared memory per warp: 32 displacement histories + thresholds + slots.
@@ -274,8 +223,11 @@ __global__ void okin_study_merge(const OkinMoments* __restrict__ groups, int SQ,
 
 namespace {
 
-const void* kernel_of(int fam, bool shim) {
+const void* kernel_of(const DeviceCopy& d, int fam, bool shim) {
   switch (fam) {
+    case OKIN_FAM_SPEC_WIDE:
+    case OKIN_FAM_SPEC:
+      return (const void*)d.spec_kernel[fam == OKIN_FAM_SPEC];
     case OKIN_FAM_SENS:
       return (const void*)okin_sweep_kernel<true, false, OKIN_MAX_THREADS, true>;
     case OKIN_FAM_FULL:
@@ -288,6 +240,203 @@ const void* kernel_of(int fam, bool shim) {
       return shim ? (const void*)okin_sweep_kernel<false, true, OKIN_LEAN_WIDE_THREADS>
                   : (const void*)okin_sweep_kernel<false, false, OKIN_LEAN_WIDE_THREADS>;
   }
+}
+
+// Launch shape of a kernel family: CTA of W warps sharing one copy of the tables; pick the W that keeps
+// the most warps resident (shared memory, the 64K-register file at the instantiation's register cap, 1 KB
+// per-CTA reservation).  The lean instantiations own a shorter slice than the full ones.
+int family_shape(okin_topology* t, DeviceCopy& d, const cudaDeviceProp& prop, int fam) {
+  const size_t table_bytes = (size_t)(fam >= OKIN_FAM_SPEC_WIDE ? d.spec_table_doubles : d.table_doubles) * 8;
+  const size_t sm_budget = prop.sharedMemPerMultiprocessor;
+  const bool full = fam == OKIN_FAM_FULL || fam == OKIN_FAM_SENS;
+  const size_t slice_bytes =
+      (size_t)t->hdr[full ? OKIN_H_SMEM_DOUBLES : OKIN_H_SMEM_DOUBLES_LEAN] * sizeof(double);
+  const int max_threads = fam == OKIN_FAM_LEAN_WIDE || fam == OKIN_FAM_SPEC_WIDE ? OKIN_LEAN_WIDE_THREADS : OKIN_MAX_THREADS;
+  const int regs_per_thread = (int)(prop.regsPerMultiprocessor / max_threads) & ~7;
+  int best_w = 0, best_ctas = 0;
+  const char* forced = getenv("OKIN_WARPS_PER_CTA");     // kernel experiments
+  for (int w = 1; w <= max_threads / 32; ++w) {
+    if (forced && atoi(forced) > 0 && w != atoi(forced)) continue;
+    const size_t cta_bytes = table_bytes + w * slice_bytes;
+    if (cta_bytes > prop.sharedMemPerBlockOptin) break;
+    int ctas = (int)(sm_budget / (cta_bytes + 1024));
+    ctas = std::min(ctas, (int)(prop.regsPerMultiprocessor / (regs_per_thread * 32 * w)));
+    ctas = std::min(ctas, 32);
+    // most resident warps; on a tie the CTA shape closest to 6-8 warps (measured: 6 x 2 CTAs beats
+    // 3 x 4 -- fewer copies of the tables -- and 12 x 1 -- a barrier group of 12 warps)
+    const bool better_shape = best_w == 0 || (w <= 8 && w > best_w) || (best_w > 8 && w < best_w);
+    if (ctas * w > best_w * best_ctas || (ctas * w == best_w * best_ctas && ctas * w > 0 && better_shape)) {
+      best_w = w;
+      best_ctas = ctas;
+    }
+  }
+  if (best_w == 0 || best_ctas == 0)
+    return fail(OKIN_ERR_USAGE, "topology needs more shared memory per CTA than the device offers");
+  DeviceCopy::Shape& sh = d.shape[fam];
+  sh.warps_per_cta = best_w;
+  sh.smem_bytes = (int)(table_bytes + best_w * slice_bytes);
+  sh.ctas_per_sm = 1 << 30;
+  for (int shim = 0; shim < (fam == OKIN_FAM_SENS ? 1 : 2); ++shim) {
+    if (fam >= OKIN_FAM_SPEC_WIDE && shim != (t->hdr[OKIN_H_NSHIM] > 0)) continue;   // compiled for this topology only
+    const void* kernel = kernel_of(d, fam, shim != 0);
+    OKIN_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, sh.smem_bytes));
+    int ctas = 0;
+    OKIN_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctas, kernel, best_w * 32, sh.smem_bytes));
+    sh.ctas_per_sm = std::min(sh.ctas_per_sm, ctas);
+  }
+  if (sh.ctas_per_sm < 1) return fail(OKIN_ERR_CUDA, "kernel does not fit on an SM");
+  return OKIN_OK;
+}
+
+// ---- topology-specialised lean kernels ------------------------------------------------------
+// NVRTC is loaded at run time: without it (or when a compilation fails) the generic kernels serve, and
+// okin_lean_calibration says why.
+struct Nvrtc {
+  bool ok = false;
+  decltype(&nvrtcCreateProgram) create;
+  decltype(&nvrtcCompileProgram) compile;
+  decltype(&nvrtcAddNameExpression) add_name;
+  decltype(&nvrtcGetLoweredName) lowered;
+  decltype(&nvrtcGetProgramLogSize) log_size;
+  decltype(&nvrtcGetProgramLog) log;
+  decltype(&nvrtcGetCUBINSize) cubin_size;
+  decltype(&nvrtcGetCUBIN) cubin;
+  decltype(&nvrtcDestroyProgram) destroy;
+};
+
+const Nvrtc& nvrtc() {
+  static Nvrtc n = [] {
+    Nvrtc r;
+    void* h = dlopen("libnvrtc.so.12", RTLD_NOW | RTLD_LOCAL);
+    if (!h) h = dlopen("libnvrtc.so", RTLD_NOW | RTLD_LOCAL);
+    if (!h) return r;
+#define OKIN_SYM(f, name) r.f = reinterpret_cast<decltype(r.f)>(dlsym(h, name)); if (!r.f) return r
+    OKIN_SYM(create, "nvrtcCreateProgram"); OKIN_SYM(compile, "nvrtcCompileProgram");
+    OKIN_SYM(add_name, "nvrtcAddNameExpression"); OKIN_SYM(lowered, "nvrtcGetLoweredName");
+    OKIN_SYM(log_size, "nvrtcGetProgramLogSize"); OKIN_SYM(log, "nvrtcGetProgramLog");
+    OKIN_SYM(cubin_size, "nvrtcGetCUBINSize"); OKIN_SYM(cubin, "nvrtcGetCUBIN");
+    OKIN_SYM(destroy, "nvrtcDestroyProgram");
+#undef OKIN_SYM
+    r.ok = true;
+    return r;
+  }();
+  return n;
+}
+
+// The kernel sources sit next to the library (csrc/).
+std::string source_dir() {
+  Dl_info info;
+  if (!dladdr((const void*)&nvrtc, &info) || !info.dli_fname) return ".";
+  std::string p = info.dli_fname;
+  const size_t slash = p.rfind('/');
+  return slash == std::string::npos ? "." : p.substr(0, slash);
+}
+
+// What NVRTC lacks of the C headers the core includes.
+const char* const kRtcPrelude =
+    "typedef signed char int8_t; typedef short int16_t; typedef int int32_t; typedef long long int64_t;\n"
+    "typedef unsigned char uint8_t; typedef unsigned short uint16_t; typedef unsigned int uint32_t;\n"
+    "typedef unsigned long long uint64_t; typedef unsigned long size_t;\n"
+    "#define NAN __longlong_as_double(0x7ff8000000000000LL)\n"
+    "#define INFINITY __longlong_as_double(0x7ff0000000000000LL)\n"
+    "#include \"okin_kernel.cuh\"\n";
+
+const char* lean_kernel_name(bool narrow, bool shim) {
+  static const char* names[2][2] = {{"okin_sweep_kernel<false, false, 384>", "okin_sweep_kernel<false, true, 384>"},
+                                    {"okin_sweep_kernel<false, false, 512>", "okin_sweep_kernel<false, true, 512>"}};
+  return names[narrow][shim];
+}
+
+// Compiles both lean families of one spec for sm_100a (the library's nvcc flags: -O3, -lineinfo,
+// C++17).  On success cubin holds the image and lowered[k] the kernel names of {wide, 128-register}.
+bool compile_spec(const std::string& spec, bool shim, bool verbose, std::vector<char>* cubin,
+                  std::string lowered[2], std::string* log) {
+  const Nvrtc& n = nvrtc();
+  if (!n.ok) {
+    *log = "libnvrtc not found";
+    return false;
+  }
+  nvrtcProgram prog;
+  const char* headers[] = {spec.c_str()};
+  const char* names[] = {"okin_spec.h"};
+  if (n.create(&prog, kRtcPrelude, "okin_spec_kernel.cu", 1, headers, names) != NVRTC_SUCCESS) {
+    *log = "nvrtcCreateProgram failed";
+    return false;
+  }
+  for (int k = 0; k < 2; ++k) n.add_name(prog, lean_kernel_name(k == 1, shim));
+  const std::string inc = "-I" + source_dir();
+  // -default-device: the C ABI declarations of okin.h have no execution space
+  std::vector<const char*> opts = {"-arch=sm_100a", "-std=c++17", "-lineinfo", "-default-device", "-DOKIN_SPEC", inc.c_str()};
+  if (verbose) opts.push_back("--ptxas-options=-v");
+  const nvrtcResult rc = n.compile(prog, (int)opts.size(), opts.data());
+  size_t len = 0;
+  n.log_size(prog, &len);
+  log->assign(len, '\0');
+  if (len) n.log(prog, &(*log)[0]);
+  bool ok = rc == NVRTC_SUCCESS;
+  if (ok) {
+    size_t bytes = 0;
+    ok = n.cubin_size(prog, &bytes) == NVRTC_SUCCESS && bytes > 0;
+    cubin->assign(bytes, 0);
+    ok = ok && n.cubin(prog, cubin->data()) == NVRTC_SUCCESS;
+    for (int k = 0; ok && k < 2; ++k) {
+      const char* name = nullptr;
+      ok = n.lowered(prog, lean_kernel_name(k == 1, shim), &name) == NVRTC_SUCCESS && name;
+      if (ok) lowered[k] = name;
+    }
+  }
+  n.destroy(&prog);
+  return ok;
+}
+
+// Loads the specialised lean kernels of t on device d (compiling them once per topology).  Returns false
+// with t->spec_error set when they are not available; the generic kernels then serve.
+bool load_spec(okin_topology* t, DeviceCopy& d) {
+  std::lock_guard<std::mutex> lock(t->mu);
+  if (d.spec_loaded) return true;
+  if (t->spec.empty()) {
+    t->spec_error = "no topology spec (okin_topology_set_spec)";
+    return false;
+  }
+  if (!t->spec_compiled) {
+    t->spec_compiled = true;
+    const auto t0 = std::chrono::steady_clock::now();
+    std::string log;
+    if (!compile_spec(t->spec, t->hdr[OKIN_H_NSHIM] > 0, false, &t->spec_cubin, t->spec_lowered, &log)) {
+      t->spec_cubin.clear();
+      t->spec_error = "NVRTC: " + log;
+      return false;
+    }
+    t->spec_compile_s = std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
+  }
+  if (t->spec_cubin.empty()) return false;
+  cudaLibrary_t lib = nullptr;
+  cudaError_t err = cudaSetDevice(d.device);
+  if (err == cudaSuccess) err = cudaLibraryLoadData(&lib, t->spec_cubin.data(), nullptr, nullptr, 0, nullptr, nullptr, 0);
+  cudaKernel_t k[2] = {};
+  size_t words_bytes = 0;
+  void* words = nullptr;
+  for (int i = 0; i < 2 && err == cudaSuccess; ++i) {
+    err = cudaLibraryGetKernel(&k[i], lib, t->spec_lowered[i].c_str());
+  }
+  if (err == cudaSuccess) err = cudaLibraryGetGlobal(&words, &words_bytes, lib, "okin_spec_words");
+  if (err != cudaSuccess) {
+    if (lib) cudaLibraryUnload(lib);
+    t->spec_error = std::string("loading the specialised kernels: ") + cudaGetErrorString(err);
+    return false;
+  }
+  d.spec_lib = lib;
+  d.spec_kernel[0] = k[0];
+  d.spec_kernel[1] = k[1];
+  d.spec_table_doubles = d.table_doubles + (int)((words_bytes + 7) / 8);
+  d.spec_loaded = true;
+  return true;
+}
+
+int shape_on(okin_topology* t, DeviceCopy& d, int fam) {
+  cudaDeviceProp prop;
+  OKIN_CUDA(cudaGetDeviceProperties(&prop, d.device));
+  return family_shape(t, d, prop, fam);
 }
 
 int ensure_device(okin_topology* t, int device, DeviceCopy** out) {
@@ -307,53 +456,17 @@ int ensure_device(okin_topology* t, int device, DeviceCopy** out) {
     OKIN_CUDA(cudaGetDeviceProperties(&prop, device));
     d.num_sms = prop.multiProcessorCount;
     d.smem_optin = (int)prop.sharedMemPerBlockOptin;
-    // CTA shape: W warps sharing one copy of the tables; pick the W that keeps the most warps resident
-    // (shared memory, the 64K-register file at the instantiation's register cap, 1 KB per-CTA
-    // reservation).  The lean instantiations own a shorter slice than the full ones.
     d.table_doubles =
         OKIN_S_COUNT + (int)((((size_t)t->hdr[OKIN_H_NHOT] + OKIN_HDR_SIZE) * sizeof(int32_t) + 7) / 8);
-    const size_t table_bytes = (size_t)d.table_doubles * 8;
-    const size_t sm_budget = prop.sharedMemPerMultiprocessor;
-    for (int fam = 0; fam < OKIN_FAM_COUNT; ++fam) {
-      const bool full = fam == OKIN_FAM_FULL || fam == OKIN_FAM_SENS;
-      const size_t slice_bytes =
-          (size_t)t->hdr[full ? OKIN_H_SMEM_DOUBLES : OKIN_H_SMEM_DOUBLES_LEAN] * sizeof(double);
-      const int max_threads = fam == OKIN_FAM_LEAN_WIDE ? OKIN_LEAN_WIDE_THREADS : OKIN_MAX_THREADS;
-      const int regs_per_thread = (int)(prop.regsPerMultiprocessor / max_threads) & ~7;
-      int best_w = 0, best_ctas = 0;
-      const char* forced = getenv("OKIN_WARPS_PER_CTA");     // kernel experiments
-      for (int w = 1; w <= max_threads / 32; ++w) {
-        if (forced && atoi(forced) > 0 && w != atoi(forced)) continue;
-        const size_t cta_bytes = table_bytes + w * slice_bytes;
-        if (cta_bytes > prop.sharedMemPerBlockOptin) break;
-        int ctas = (int)(sm_budget / (cta_bytes + 1024));
-        ctas = std::min(ctas, (int)(prop.regsPerMultiprocessor / (regs_per_thread * 32 * w)));
-        ctas = std::min(ctas, 32);
-        // most resident warps; on a tie the CTA shape closest to 6-8 warps (measured: 6 x 2 CTAs beats
-        // 3 x 4 -- fewer copies of the tables -- and 12 x 1 -- a barrier group of 12 warps)
-        const bool better_shape = best_w == 0 || (w <= 8 && w > best_w) || (best_w > 8 && w < best_w);
-        if (ctas * w > best_w * best_ctas || (ctas * w == best_w * best_ctas && ctas * w > 0 && better_shape)) {
-          best_w = w;
-          best_ctas = ctas;
-        }
-      }
-      if (best_w == 0 || best_ctas == 0)
-        return fail(OKIN_ERR_USAGE, "topology needs more shared memory per CTA than the device offers");
-      DeviceCopy::Shape& sh = d.shape[fam];
-      sh.warps_per_cta = best_w;
-      sh.smem_bytes = (int)(table_bytes + best_w * slice_bytes);
-      sh.ctas_per_sm = 1 << 30;
-      for (int shim = 0; shim < (fam == OKIN_FAM_SENS ? 1 : 2); ++shim) {
-        const void* kernel = kernel_of(fam, shim != 0);
-        OKIN_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, sh.smem_bytes));
-        int ctas = 0;
-        OKIN_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctas, kernel, best_w * 32, sh.smem_bytes));
-        sh.ctas_per_sm = std::min(sh.ctas_per_sm, ctas);
-      }
-      if (sh.ctas_per_sm < 1) return fail(OKIN_ERR_CUDA, "kernel does not fit on an SM");
+    for (int fam = 0; fam < OKIN_FAM_SPEC_WIDE; ++fam) {
+      const int rc = family_shape(t, d, prop, fam);
+      if (rc) return rc;
     }
-    if (const char* fixed = getenv("OKIN_LEAN_REGS"))        // 128 | 168: skip the calibration
-      d.lean_family = atoi(fixed) == 128 ? OKIN_FAM_LEAN : OKIN_FAM_LEAN_WIDE;
+    if (const char* fixed = getenv("OKIN_LEAN_REGS")) {      // 128 | 168 | spec128 | spec168: skip the calibration
+      const bool spec = strncmp(fixed, "spec", 4) == 0;
+      const bool narrow = atoi(spec ? fixed + 4 : fixed) == 128;
+      d.lean_family = spec ? (narrow ? OKIN_FAM_SPEC : OKIN_FAM_SPEC_WIDE) : (narrow ? OKIN_FAM_LEAN : OKIN_FAM_LEAN_WIDE);
+    }
     for (int k = 0; k < OKIN_PIPE_SLOTS; ++k)
       OKIN_CUDA(cudaStreamCreateWithFlags(&d.streams[k], cudaStreamNonBlocking));
     d.ready = true;
@@ -370,7 +483,7 @@ int launch_family(okin_topology* t, DeviceCopy* d, int fam, const OkinSolverCfg&
   const int64_t needed = (n_instances + w - 1) / w;
   const int64_t resident = (int64_t)d->num_sms * sh.ctas_per_sm;
   const int grid = (int)std::min<int64_t>(needed, resident);
-  const void* kernel = kernel_of(fam, t->hdr[OKIN_H_NSHIM] > 0);
+  const void* kernel = kernel_of(*d, fam, t->hdr[OKIN_H_NSHIM] > 0);
   // The attribute belongs to the kernel function of this device context, not to a topology: another
   // live topology may have lowered it since ensure_device ran, so it is set before every launch.
   std::lock_guard<std::mutex> launch_lock(g_launch_mu[d->device]);
@@ -391,7 +504,8 @@ int launch_family(okin_topology* t, DeviceCopy* d, int fam, const OkinSolverCfg&
   if (fam == OKIN_FAM_SENS)
     OKIN_CUDA(cudaMallocAsync(&sens_ws, (size_t)grid * w * okin_sens_ws_doubles(t->hdr.data()) * sizeof(double) + 8,
                               stream));
-  void* args[] = {&d->hdr, &d->ib, &d->fb, &n, &n_steps, &cfg, &kio, &n_iblob, &d->table_doubles, &counter,
+  int table_doubles = fam >= OKIN_FAM_SPEC_WIDE ? d->spec_table_doubles : d->table_doubles;
+  void* args[] = {&d->hdr, &d->ib, &d->fb, &n, &n_steps, &cfg, &kio, &n_iblob, &table_doubles, &counter,
                   &sens_out, &sens_ws};
   const cudaError_t launch_err = cudaLaunchKernel(kernel, dim3(grid), dim3(w * 32), args, sh.smem_bytes, stream);
   OKIN_CUDA(cudaFreeAsync(counter, stream));
@@ -408,16 +522,34 @@ int launch(okin_topology* t, DeviceCopy* d, const okin_solver_cfg* cfg, cudaStre
   int fam = io.hardpoint_sensitivity ? OKIN_FAM_SENS : OKIN_FAM_FULL;
   if (!okin_wants_full(io) && !io.hardpoint_sensitivity) {
     fam = d->lean_family;
+    if (fam >= OKIN_FAM_SPEC_WIDE && !d->spec_loaded) {   // pinned by OKIN_LEAN_REGS
+      if (!load_spec(t, *d)) return fail(OKIN_ERR_USAGE, "specialised lean kernel unavailable: " + t->spec_error);
+      for (int f = OKIN_FAM_SPEC_WIDE; f < OKIN_FAM_COUNT; ++f) {
+        const int rc = shape_on(t, *d, f);
+        if (rc) return rc;
+      }
+    }
     const int64_t sample = 4 * (int64_t)d->num_sms * std::max(d->shape[OKIN_FAM_LEAN].ctas_per_sm * d->shape[OKIN_FAM_LEAN].warps_per_cta,
                                                               d->shape[OKIN_FAM_LEAN_WIDE].ctas_per_sm * d->shape[OKIN_FAM_LEAN_WIDE].warps_per_cta);
     if (fam < 0 && n_instances >= 2 * sample) {
-      // Calibration, once per (topology, device): both lean families solve the same leading instances
-      // of this batch (their results are identical; the batch launch below overwrites them again).
+      // Calibration, once per (topology, device): every lean family solves the same leading instances of
+      // this batch (their results are identical; the batch launch below overwrites them again).  The
+      // specialised families take part when they compile and load (their compile time is not timed).
+      int n_fam = 2;
+      if (load_spec(t, *d)) {
+        n_fam = 4;
+        for (int f = OKIN_FAM_SPEC_WIDE; f < OKIN_FAM_COUNT && n_fam == 4; ++f)
+          if (shape_on(t, *d, f)) {
+            t->spec_error = "specialised lean kernel does not fit: " + g_last_error;
+            n_fam = 2;
+          }
+      }
       cudaEvent_t e[2];
       OKIN_CUDA(cudaEventCreate(&e[0]));
       OKIN_CUDA(cudaEventCreate(&e[1]));
-      const int order[2] = {OKIN_FAM_LEAN_WIDE, OKIN_FAM_LEAN};
-      for (int k = 0; k < 2; ++k) {
+      const int order[4] = {OKIN_FAM_LEAN_WIDE, OKIN_FAM_LEAN, OKIN_FAM_SPEC_WIDE, OKIN_FAM_SPEC};
+      int best = 0;
+      for (int k = 0; k < n_fam; ++k) {
         int rc = launch_family(t, d, order[k], c, stream, sample, n_steps, io);   // warm-up (code, tables)
         if (rc) return rc;
         OKIN_CUDA(cudaEventRecord(e[0], stream));
@@ -428,10 +560,11 @@ int launch(okin_topology* t, DeviceCopy* d, const okin_solver_cfg* cfg, cudaStre
         float ms = 0.f;
         OKIN_CUDA(cudaEventElapsedTime(&ms, e[0], e[1]));
         d->lean_tune_ms[k] = ms;
+        if (ms < d->lean_tune_ms[best]) best = k;
       }
       cudaEventDestroy(e[0]);
       cudaEventDestroy(e[1]);
-      d->lean_family = fam = d->lean_tune_ms[1] < d->lean_tune_ms[0] ? OKIN_FAM_LEAN : OKIN_FAM_LEAN_WIDE;
+      d->lean_family = fam = order[best];
     }
     if (fam < 0) fam = OKIN_FAM_LEAN_WIDE;      // small batch: not worth timing, not recorded
   }
@@ -1037,6 +1170,7 @@ int okin_topology_destroy(okin_topology* t) {
     cudaFree(d.ib);
     cudaFree(d.fb);
     if (d.ws) cudaFree(d.ws);
+    if (d.spec_lib) cudaLibraryUnload(d.spec_lib);
     for (int k = 0; k < OKIN_PIPE_SLOTS; ++k)
       if (d.streams[k]) cudaStreamDestroy(d.streams[k]);
   }
@@ -1077,15 +1211,39 @@ int okin_launch_geometry(okin_topology* t, int32_t device, int64_t n_instances, 
   return OKIN_OK;
 }
 
-int okin_lean_calibration(okin_topology* t, int32_t device, int32_t* registers, double* ms_wide, double* ms_128) {
-  if (!t) return fail(OKIN_ERR_USAGE, "null topology");
+int okin_lean_calibration(okin_topology* t, int32_t device, okin_lean_family* out) {
+  if (!t || !out) return fail(OKIN_ERR_USAGE, "null argument");
   DeviceCopy* d = nullptr;
   int rc = ensure_device(t, device, &d);
   if (rc) return rc;
-  if (registers) *registers = d->lean_family < 0 ? 0 : (d->lean_family == OKIN_FAM_LEAN ? 128 : 168);
-  if (ms_wide) *ms_wide = d->lean_tune_ms[0];
-  if (ms_128) *ms_128 = d->lean_tune_ms[1];
+  std::lock_guard<std::mutex> lock(t->mu);
+  const int f = d->lean_family;
+  out->registers = f < 0 ? 0 : (f == OKIN_FAM_LEAN || f == OKIN_FAM_SPEC ? 128 : 168);
+  out->specialised = f >= OKIN_FAM_SPEC_WIDE;
+  for (int k = 0; k < 4; ++k) out->ms[k] = d->lean_tune_ms[k];
+  out->spec_compile_s = t->spec_compile_s;
+  std::snprintf(out->spec_error, sizeof(out->spec_error), "%s", t->spec_error.c_str());
   return OKIN_OK;
+}
+
+int okin_topology_set_spec(okin_topology* t, const char* source) {
+  if (!t || !source) return fail(OKIN_ERR_USAGE, "null argument");
+  std::lock_guard<std::mutex> lock(t->mu);
+  if (t->spec_compiled) return fail(OKIN_ERR_USAGE, "the topology's specialised kernels are already compiled");
+  t->spec = source;
+  return OKIN_OK;
+}
+
+int okin_spec_compile(const char* source, int32_t shim, char* log, int32_t log_len, int64_t* cubin_bytes,
+                      void* cubin, int64_t cubin_capacity) {
+  if (!source) return fail(OKIN_ERR_USAGE, "null source");
+  std::vector<char> image;
+  std::string lowered[2], text;
+  const bool ok = compile_spec(source, shim != 0, true, &image, lowered, &text);
+  if (log && log_len > 0) std::snprintf(log, (size_t)log_len, "%s", text.c_str());
+  if (cubin_bytes) *cubin_bytes = (int64_t)image.size();
+  if (cubin && (int64_t)image.size() <= cubin_capacity) std::memcpy(cubin, image.data(), image.size());
+  return ok ? OKIN_OK : fail(OKIN_ERR_USAGE, "NVRTC: " + text);
 }
 
 int okin_solve_batch_device(okin_topology* t, const okin_solver_cfg* cfg, int32_t device, void* stream,

@@ -42,12 +42,17 @@
 #ifndef OKIN_COMPACT_LOOPS
 #define OKIN_COMPACT_LOOPS 2
 #endif
+#ifndef __CUDACC_RTC__
 #include <stddef.h>
+#endif
 
 #include "../../include/okin.h"
 #include "okin_defs.h"
 #include "okin_gen_constraints.cuh"
 #include "okin_metrics.cuh"
+#ifdef OKIN_SPEC
+#include "okin_spec.h"
+#endif
 
 // Phase functions are kept out of line on the device: inlining all of them into the sweep loop
 // (each is called from several places) costs registers (255/thread) and instruction cache.  The
@@ -147,6 +152,10 @@ OKIN_HD double okin_red_max(const double* red) {
 }
 #endif
 
+// The hot phases' arithmetic is written as explicit fma: ptxas contracts a separate multiply and add
+// depending on the code around them, and the generic and the topology-specialised builds of these
+// phases must round alike.
+//
 // Gather loops (factor update, triangular solves, assembly): every operand of a contribution is
 // loaded into its own variable before the first FMA.  A warp issues in order, so the shared-memory
 // latency is then paid once per contribution (twelve loads in flight) instead of once per FMA -- but
@@ -155,12 +164,87 @@ OKIN_HD double okin_red_max(const double* red) {
 // kernel runs 12 warps per SM at 168 registers (profiles/r02_*; okin_abi.cu OKIN_LEAN_MAX_THREADS).
 struct OkinProgram {
   const int32_t* hdr;  // [OKIN_HDR_SIZE]
-  const int32_t* ib;   // int32 blob: at least its hot prefix hdr[OKIN_H_NHOT] (shared memory in the kernel)
+  const int32_t* ib;   // int32 blob: at least its hot prefix OKIN_HV(hdr, OKIN_H_NHOT) (shared memory in the kernel)
   const double* fb;    // double blob
   const int32_t* ibc;  // whole int32 blob (global memory); cold sections are read from here
   const int32_t* const* sec;  // [OKIN_S_COUNT] start of every int32 section (hot: in ib, cold: in ibc),
                               // resolved once per CTA by okin_resolve_sections
+  const int32_t* spec = nullptr;  // OKIN_SPEC builds: okin_spec_words (shared memory in the kernel)
 };
+
+// Header fields and the task lists of the hot phases (assembly, factorisation, triangular solves).  The
+// generic build reads the header from shared memory and walks the CSR task lists of the program.  A
+// build that includes a topology's generated spec (OKIN_SPEC: "okin_spec.h", core/topology.py
+// spec_source) gets the header fields and every phase's shape as compile-time constants: a phase is a
+// fixed sequence of lane rounds, and round r reads its task words and contribution words lane-major
+// from okin_spec_words (row 0 the task words, row 1 + s the s-th contribution of each lane's task, row
+// stride = the round's width), so one conflict-free load serves the warp and no table load depends on
+// another.  A lane's contributions keep their order, so both builds do the same arithmetic.
+#ifdef OKIN_SPEC
+#define OKIN_HV(hdr, f) ((void)(hdr), okin_spec_hdr(f))
+#else
+#define OKIN_HV(hdr, f) ((hdr)[f])
+#endif
+
+// Phase numbers of the spec: assembly (block tasks, then gradient tasks), per level the factor update,
+// diagonal and scale phases, then the forward and the backward substitution phases.
+#define OKIN_PH_ASM_BLOCK 0
+#define OKIN_PH_ASM_G 1
+#define OKIN_PH_UPD(lv) (2 + 3 * (lv))
+#define OKIN_PH_DIAG(lv) (3 + 3 * (lv))
+#define OKIN_PH_SCL(lv) (4 + 3 * (lv))
+#define OKIN_PH_FW(nlev, lv) (2 + 3 * (nlev) + (lv))
+#define OKIN_PH_BW(nlev, ph) (2 + 4 * (nlev) + (ph))
+
+template <int I>
+struct OkinConst {
+  static constexpr int value = I;
+};
+
+#ifdef OKIN_SPEC
+// f(OkinConst<I>) for I in [I, N): levels become compile-time constants.
+template <int I, int N, class F>
+OKIN_HD void okin_static_for(F&& f) {
+  if constexpr (I < N) {
+    f(OkinConst<I>{});
+    okin_static_for<I + 1, N>(f);
+  }
+}
+template <int R, int S, class G>
+OKIN_HD void okin_spec_slots(const int32_t* w, int lane, G&& g) {
+  if constexpr (S < okin_spec::r_slots(R)) {
+    constexpr int width = okin_spec::r_width(R), n = okin_spec::slot_lanes(okin_spec::r_slot0(R) + S);
+    if (n == width || lane < n) g((uint32_t)w[(S + 1) * width]);
+    okin_spec_slots<R, S + 1>(w, lane, g);
+  }
+}
+template <int R, int RE, class Body>
+OKIN_HD void okin_spec_rounds(const int32_t* words, int lane, Body&& body) {
+  if constexpr (R < RE) {
+    constexpr int width = okin_spec::r_width(R);
+    if (width == 32 || lane < width) {
+      const int32_t* w = words + okin_spec::r_base(R) + lane;
+      body((uint32_t)w[0], [&](auto&& g) { okin_spec_slots<R, 0>(w, lane, g); });
+    }
+    okin_spec_rounds<R + 1, RE>(words, lane, body);
+  }
+}
+// body(task word, each) for every task of phase P in this lane; each(g) calls g(contribution word) in order.
+template <int P, class Body>
+OKIN_HD void okin_spec_phase(const OkinProgram& pr, int lane, Body&& body) {
+  okin_spec_rounds<okin_spec::phase_round(P), okin_spec::phase_round(P + 1)>(OKIN_SHARED(pr.spec), lane, body);
+}
+#endif
+// f(level) for every elimination level: a constant in a spec build, a loop counter otherwise.
+template <class F>
+OKIN_HD void okin_levels(int nlev, F&& f) {
+#ifdef OKIN_SPEC
+  (void)nlev;
+  okin_static_for<0, okin_spec_hdr(OKIN_H_NLEV)>(f);
+#else
+  for (int lv = 0; lv < nlev; ++lv) f(lv);
+#endif
+}
 
 struct OkinSolverCfg {
   double step_tol;      // converged when the verification (chord) step has max|dx| <= step_tol (mm)
@@ -178,7 +262,7 @@ OKIN_HD const int32_t* okin_sec(const OkinProgram& pr, int s) { return OKIN_SHAR
 OKIN_HD void okin_resolve_section(const int32_t* hdr, const int32_t* ib, const int32_t* ibc, int s,
                                   const int32_t** table) {
   const int off = hdr[OKIN_H_SEC0 + 2 * s];
-  table[s] = (off < hdr[OKIN_H_NHOT] ? ib : ibc) + off;
+  table[s] = (off < OKIN_HV(hdr, OKIN_H_NHOT) ? ib : ibc) + off;
 }
 OKIN_HD int okin_sec_len(const OkinProgram& pr, int s) { return pr.hdr[OKIN_H_SEC0 + 2 * s + 1]; }
 OKIN_HD const double* okin_fsec(const OkinProgram& pr, int s) { return pr.fb + pr.hdr[OKIN_H_FSEC0 + 2 * s]; }
@@ -234,8 +318,8 @@ OKIN_FN void okin_derived_update(const OkinProgram& pr, double* sm, bool active_
   const int32_t* dop = OKIN_SHARED(okin_sec(pr, OKIN_S_DOP));
   const int32_t* lev = OKIN_SHARED(okin_sec(pr, OKIN_S_DOP_LEV));
   const int nlev = okin_sec_len(pr, OKIN_S_DOP_LEV) - 1;
-  double* pos = sm + pr.hdr[OKIN_H_OFF_POS];
-  const double* par = sm + pr.hdr[OKIN_H_OFF_PAR];
+  double* pos = sm + OKIN_HV(pr.hdr, OKIN_H_OFF_POS);
+  const double* par = sm + OKIN_HV(pr.hdr, OKIN_H_OFF_PAR);
   for (int lv = 0; lv < nlev; ++lv) {
     const int b = OKIN_LDG(lev + lv), e = OKIN_LDG(lev + lv + 1);
     OKIN_PHASE_BEGIN
@@ -260,14 +344,14 @@ OKIN_FN void okin_derived_update(const OkinProgram& pr, double* sm, bool active_
 template <typename Dummy = void>
 OKIN_FN void okin_derived_jacobians(const OkinProgram& pr, double* sm) {
   sm = OKIN_SHARED(sm);
-  const int nad = pr.hdr[OKIN_H_NAD];
+  const int nad = OKIN_HV(pr.hdr, OKIN_H_NAD);
   if (nad == 0) return;
   const int32_t* adj = OKIN_SHARED(okin_sec(pr, OKIN_S_ADJ));
   const int32_t* chain = OKIN_SHARED(okin_sec(pr, OKIN_S_ADJ_CHAIN));
   const int32_t* dop = OKIN_SHARED(okin_sec(pr, OKIN_S_DOP));
-  const double* pos = sm + pr.hdr[OKIN_H_OFF_POS];
-  const double* par = sm + pr.hdr[OKIN_H_OFF_PAR];
-  double* dblk = sm + pr.hdr[OKIN_H_OFF_DBLK];
+  const double* pos = sm + OKIN_HV(pr.hdr, OKIN_H_OFF_POS);
+  const double* par = sm + OKIN_HV(pr.hdr, OKIN_H_OFF_PAR);
+  double* dblk = sm + OKIN_HV(pr.hdr, OKIN_H_OFF_DBLK);
   OKIN_PHASE_BEGIN
   OKIN_LANE_LOOP
   for (int t = lane; t < nad; t += 32) {
@@ -318,12 +402,12 @@ template <typename Dummy = void>
 OKIN_FN void okin_shim_presolve(const OkinProgram& pr, double* sm, const double* params, int* invalid) {
   sm = OKIN_SHARED(sm);
   const int32_t* hdr = OKIN_SHARED(pr.hdr);
-  const int nshim = hdr[OKIN_H_NSHIM];
+  const int nshim = OKIN_HV(hdr, OKIN_H_NSHIM);
   if (nshim == 0) return;
   const int32_t* recs = okin_sec(pr, OKIN_S_SHIM);
   const int32_t* lists = okin_sec(pr, OKIN_S_SHIM_PTS);
-  double* pos = sm + hdr[OKIN_H_OFF_POS];
-  double* red = sm + hdr[OKIN_H_OFF_RED];
+  double* pos = sm + OKIN_HV(hdr, OKIN_H_OFF_POS);
+  double* red = sm + OKIN_HV(hdr, OKIN_H_OFF_RED);
   OKIN_PHASE_BEGIN
   red[lane] = 0.0;
   if (lane < nshim) {
@@ -458,10 +542,10 @@ OKIN_FN void okin_setup(const OkinProgram& pr, double* sm, const double* __restr
                         const double* __restrict__ params, int* invalid, bool keep_design) {
   sm = OKIN_SHARED(sm);
   const int32_t* hdr = OKIN_SHARED(pr.hdr);
-  double* pos = sm + hdr[OKIN_H_OFF_POS];
-  double* cst = sm + hdr[OKIN_H_OFF_CST];
-  double* par = sm + hdr[OKIN_H_OFF_PAR];
-  const int nin = hdr[OKIN_H_NIN];
+  double* pos = sm + OKIN_HV(hdr, OKIN_H_OFF_POS);
+  double* cst = sm + OKIN_HV(hdr, OKIN_H_OFF_CST);
+  double* par = sm + OKIN_HV(hdr, OKIN_H_OFF_PAR);
+  const int nin = OKIN_HV(hdr, OKIN_H_NIN);
   const int32_t* in_point = okin_sec(pr, OKIN_S_IN_POINT);
   OKIN_PHASE_BEGIN
   OKIN_LANE_LOOP
@@ -471,7 +555,7 @@ OKIN_FN void okin_setup(const OkinProgram& pr, double* sm, const double* __restr
 
   // Derived-op parameters.  A design projection reads the *authored* position of the derived
   // point (macpherson.py:199-204), which is what pos[] still holds at this moment.
-  const int ndop = hdr[OKIN_H_NDOP];
+  const int ndop = OKIN_HV(hdr, OKIN_H_NDOP);
   const int32_t* dop = OKIN_SHARED(okin_sec(pr, OKIN_S_DOP));
   const int32_t* par_mode = okin_sec(pr, OKIN_S_PAR_MODE);
   const double* par_val = okin_fsec(pr, OKIN_F_PAR_VAL);
@@ -496,9 +580,9 @@ OKIN_FN void okin_setup(const OkinProgram& pr, double* sm, const double* __restr
   okin_derived_update(pr, sm, false);
 
   if (keep_design) {  // design positions kept for the metrics (travel references, rotation datums)
-    const int ndsn = hdr[OKIN_H_NDSN];
+    const int ndsn = OKIN_HV(hdr, OKIN_H_NDSN);
     const int32_t* dpt = okin_sec(pr, OKIN_S_DESIGN_PT);
-    double* dsn = sm + hdr[OKIN_H_OFF_DSN];
+    double* dsn = sm + OKIN_HV(hdr, OKIN_H_OFF_DSN);
     OKIN_PHASE_BEGIN
     OKIN_LANE_LOOP
     for (int t = lane; t < 3 * ndsn; t += 32) dsn[t] = pos[3 * OKIN_LDG(dpt + t / 3) + t % 3];
@@ -507,10 +591,10 @@ OKIN_FN void okin_setup(const OkinProgram& pr, double* sm, const double* __restr
 
   // Per-instance constants: each row's own quantity at the design pose (true norms, no
   // softnorm: vector_utils/geometric.py:17-28, :71-104, :197-214).
-  const int nrows = hdr[OKIN_H_NROW] + hdr[OKIN_H_NREP];
+  const int nrows = OKIN_HV(hdr, OKIN_H_NROW) + OKIN_HV(hdr, OKIN_H_NREP);
   const int32_t* rows = okin_sec(pr, OKIN_S_ROW);
   const double* cst_init = okin_fsec(pr, OKIN_F_CST_INIT);
-  const int ncst = hdr[OKIN_H_NCST];
+  const int ncst = OKIN_HV(hdr, OKIN_H_NCST);
   OKIN_PHASE_BEGIN
   OKIN_LANE_LOOP
   for (int t = lane; t < ncst; t += 32) cst[t] = OKIN_LDG(cst_init + t);
@@ -569,18 +653,18 @@ OKIN_FN void okin_eval_rows(const OkinProgram& pr, double* sm, const double* tva
   const int32_t* hdr = OKIN_SHARED(pr.hdr);
   okin_derived_update(pr, sm, true);
   if (with_grad) okin_derived_jacobians(pr, sm);
-  const int nls = hdr[OKIN_H_NROW];
-  const int nrows = nls + hdr[OKIN_H_NREP];
+  const int nls = OKIN_HV(hdr, OKIN_H_NROW);
+  const int nrows = nls + OKIN_HV(hdr, OKIN_H_NREP);
   const int32_t* rows = OKIN_SHARED(okin_sec(pr, OKIN_S_ROW_HOT));
   const int32_t* der = OKIN_SHARED(okin_sec(pr, OKIN_S_DER));
-  const double* pos = sm + hdr[OKIN_H_OFF_POS];
-  const double* cst = sm + hdr[OKIN_H_OFF_CST];
-  const double* dblk = sm + hdr[OKIN_H_OFF_DBLK];
-  double* r = sm + hdr[OKIN_H_OFF_R];
-  double* rg = sm + hdr[OKIN_H_OFF_RG];
-  double* red = sm + hdr[OKIN_H_OFF_RED];
+  const double* pos = sm + OKIN_HV(hdr, OKIN_H_OFF_POS);
+  const double* cst = sm + OKIN_HV(hdr, OKIN_H_OFF_CST);
+  const double* dblk = sm + OKIN_HV(hdr, OKIN_H_OFF_DBLK);
+  double* r = sm + OKIN_HV(hdr, OKIN_H_OFF_R);
+  double* rg = sm + OKIN_HV(hdr, OKIN_H_OFF_RG);
+  double* red = sm + OKIN_HV(hdr, OKIN_H_OFF_RED);
   const int32_t* drow = OKIN_SHARED(okin_sec(pr, OKIN_S_DROW));
-  const int ndrow = hdr[OKIN_H_NDROW], ngrow = hdr[OKIN_H_NGROW];
+  const int ndrow = OKIN_HV(hdr, OKIN_H_NDROW), ngrow = OKIN_HV(hdr, OKIN_H_NGROW);
   OKIN_PHASE_BEGIN
   double sq = 0.0;
   // Fast path: plain distance rows (most of every shipped topology).  r = sqrt(s + eps^2) - eps - L,
@@ -678,59 +762,72 @@ template <typename Dummy = void>
 OKIN_FN_HOT void okin_assemble(const OkinProgram& pr, double* sm, double mu, bool g_only) {
   sm = OKIN_SHARED(sm);
   const int32_t* hdr = OKIN_SHARED(pr.hdr);
-  const int nat = hdr[OKIN_H_NAT];
-  const int nf = hdr[OKIN_H_NF];
+  const int nat = OKIN_HV(hdr, OKIN_H_NAT);
+  const int nf = OKIN_HV(hdr, OKIN_H_NF);
   const int32_t* aptr = OKIN_SHARED(okin_sec(pr, OKIN_S_ASM_PTR));
   const int32_t* atask = OKIN_SHARED(okin_sec(pr, OKIN_S_ASM_TASK));
   const int32_t* acon = OKIN_SHARED(okin_sec(pr, OKIN_S_ASM_CON));
   const int32_t* gptr = OKIN_SHARED(okin_sec(pr, OKIN_S_G_PTR));
   const int32_t* gcon = OKIN_SHARED(okin_sec(pr, OKIN_S_G_CON));
-  const double* rg = sm + hdr[OKIN_H_OFF_RG];
-  const double* r = sm + hdr[OKIN_H_OFF_R];
-  double* Lb = sm + hdr[OKIN_H_OFF_LB];
-  double* vec = sm + hdr[OKIN_H_OFF_VEC];
+  const double* rg = sm + OKIN_HV(hdr, OKIN_H_OFF_RG);
+  const double* r = sm + OKIN_HV(hdr, OKIN_H_OFF_R);
+  double* Lb = sm + OKIN_HV(hdr, OKIN_H_OFF_LB);
+  double* vec = sm + OKIN_HV(hdr, OKIN_H_OFF_VEC);
   const double damp = 1.0 + mu, lev = mu * 1e-9;
+  // one 3x3 block of A: sum of outer products ga gb^T over the rows coupling the two points
+  auto block = [&](uint32_t task, auto&& each) {
+    double a00 = 0, a01 = 0, a02 = 0, a10 = 0, a11 = 0, a12 = 0, a20 = 0, a21 = 0, a22 = 0;
+    each([&](uint32_t w) {
+      const double* ga = rg + ((w >> 16) & 0x7fffu);
+      const double* gb = rg + (w & 0xffffu);
+      const double sg = (w & OKIN_CON_NEG) ? -1.0 : 1.0;
+      const double p0 = ga[0], p1 = ga[1], p2 = ga[2], y0 = gb[0], y1 = gb[1], y2 = gb[2];
+      const double x0 = sg * p0, x1 = sg * p1, x2 = sg * p2;
+      a00 = fma(x0, y0, a00); a01 = fma(x0, y1, a01); a02 = fma(x0, y2, a02);
+      a10 = fma(x1, y0, a10); a11 = fma(x1, y1, a11); a12 = fma(x1, y2, a12);
+      a20 = fma(x2, y0, a20); a21 = fma(x2, y1, a21); a22 = fma(x2, y2, a22);
+    });
+    // Marquardt scaling plus a small Levenberg shift: a row whose gradient vanishes at the current
+    // point (a spherical joint that is exactly closed) leaves a zero diagonal that scaling alone never
+    // makes positive; MINPACK substitutes 1 for a zero column norm there (lmder, diag(j) = 1).
+    if (task & OKIN_ASM_DIAG) { a00 = fma(a00, damp, lev); a11 = fma(a11, damp, lev); a22 = fma(a22, damp, lev); }
+    double* dst = Lb + 9 * (task & 0xffff);
+    dst[0] = a00; dst[1] = a01; dst[2] = a02; dst[3] = a10; dst[4] = a11; dst[5] = a12;
+    dst[6] = a20; dst[7] = a21; dst[8] = a22;
+  };
+  // one block row of g (task word = elimination column j)
+  auto grad = [&](uint32_t j, auto&& each) {
+    double g0 = 0, g1 = 0, g2 = 0;
+    each([&](uint32_t w) {
+      const double* ga = rg + ((w >> 16) & 0x7fffu);
+      const double res = (w & OKIN_CON_NEG) ? -r[w & 0xffffu] : r[w & 0xffffu];
+      g0 = fma(ga[0], res, g0); g1 = fma(ga[1], res, g1); g2 = fma(ga[2], res, g2);
+    });
+    vec[3 * j] = -g0; vec[3 * j + 1] = -g1; vec[3 * j + 2] = -g2;  // right-hand side of A h = -g
+  };
   OKIN_PHASE_BEGIN
+#ifdef OKIN_SPEC
+  if (!g_only) okin_spec_phase<OKIN_PH_ASM_BLOCK>(pr, lane, block);
+  okin_spec_phase<OKIN_PH_ASM_G>(pr, lane, grad);
+#else
   OKIN_LANE_LOOP
   for (int t = (g_only ? nat : 0) + lane; t < nat + nf; t += 32) {
     if (t < nat) {
-      // one 3x3 block of A: sum of outer products ga gb^T over the rows coupling the two points
       const int b = OKIN_LDG(aptr + t), e = OKIN_LDG(aptr + t + 1);
-      double a00 = 0, a01 = 0, a02 = 0, a10 = 0, a11 = 0, a12 = 0, a20 = 0, a21 = 0, a22 = 0;
-      OKIN_UNROLL_INNER
-      for (int q = b; q < e; ++q) {
-        const uint32_t w = (uint32_t)OKIN_LDG(acon + q);
-        const double* ga = rg + ((w >> 16) & 0x7fffu);
-        const double* gb = rg + (w & 0xffffu);
-        const double sg = (w & OKIN_CON_NEG) ? -1.0 : 1.0;
-        const double p0 = ga[0], p1 = ga[1], p2 = ga[2], y0 = gb[0], y1 = gb[1], y2 = gb[2];
-        const double x0 = sg * p0, x1 = sg * p1, x2 = sg * p2;
-        a00 = fma(x0, y0, a00); a01 = fma(x0, y1, a01); a02 = fma(x0, y2, a02);
-        a10 = fma(x1, y0, a10); a11 = fma(x1, y1, a11); a12 = fma(x1, y2, a12);
-        a20 = fma(x2, y0, a20); a21 = fma(x2, y1, a21); a22 = fma(x2, y2, a22);
-      }
-      const int task = OKIN_LDG(atask + t);
-      // Marquardt scaling plus a small Levenberg shift: a row whose gradient vanishes at the current
-      // point (a spherical joint that is exactly closed) leaves a zero diagonal that scaling alone never
-      // makes positive; MINPACK substitutes 1 for a zero column norm there (lmder, diag(j) = 1).
-      if (task & OKIN_ASM_DIAG) { a00 = a00 * damp + lev; a11 = a11 * damp + lev; a22 = a22 * damp + lev; }
-      double* dst = Lb + 9 * (task & 0xffff);
-      dst[0] = a00; dst[1] = a01; dst[2] = a02; dst[3] = a10; dst[4] = a11; dst[5] = a12;
-      dst[6] = a20; dst[7] = a21; dst[8] = a22;
+      block((uint32_t)OKIN_LDG(atask + t), [&](auto&& g) {
+        OKIN_UNROLL_INNER
+        for (int q = b; q < e; ++q) g((uint32_t)OKIN_LDG(acon + q));
+      });
     } else {
       const int j = t - nat;
       const int b = OKIN_LDG(gptr + j), e = OKIN_LDG(gptr + j + 1);
-      double g0 = 0, g1 = 0, g2 = 0;
-      OKIN_UNROLL_INNER
-      for (int q = b; q < e; ++q) {
-        const uint32_t w = (uint32_t)OKIN_LDG(gcon + q);
-        const double* ga = rg + ((w >> 16) & 0x7fffu);
-        const double res = (w & OKIN_CON_NEG) ? -r[w & 0xffffu] : r[w & 0xffffu];
-        g0 = fma(ga[0], res, g0); g1 = fma(ga[1], res, g1); g2 = fma(ga[2], res, g2);
-      }
-      vec[3 * j] = -g0; vec[3 * j + 1] = -g1; vec[3 * j + 2] = -g2;  // right-hand side of A h = -g
+      grad((uint32_t)j, [&](auto&& g) {
+        OKIN_UNROLL_INNER
+        for (int q = b; q < e; ++q) g((uint32_t)OKIN_LDG(gcon + q));
+      });
     }
   }
+#endif
   OKIN_PHASE_END
 }
 
@@ -743,11 +840,11 @@ OKIN_HD bool okin_chol3(const double* d, double f[9]) {
   const double d00 = d[0], d10 = d[3], d11 = d[4], d20 = d[6], d21 = d[7], d22 = d[8];
   const double i00 = OKIN_RSQRT(d00);
   const double l00 = d00 * i00, l10 = d10 * i00, l20 = d20 * i00;
-  const double t11 = d11 - l10 * l10;
+  const double t11 = fma(-l10, l10, d11);
   const double i11 = OKIN_RSQRT(t11);
   const double l11 = t11 * i11;
-  const double l21 = (d21 - l20 * l10) * i11;
-  const double t22 = d22 - l20 * l20 - l21 * l21;
+  const double l21 = fma(-l20, l10, d21) * i11;
+  const double t22 = fma(-l21, l21, fma(-l20, l20, d22));
   const double i22 = OKIN_RSQRT(t22);
   const double l22 = t22 * i22;
   f[0] = l00; f[1] = l10; f[2] = l11; f[3] = l20; f[4] = l21; f[5] = l22; f[6] = i00; f[7] = i11; f[8] = i22;
@@ -771,7 +868,7 @@ template <typename Dummy = void>
 OKIN_FN_HOT void okin_factor(const OkinProgram& pr, double* sm, OkinState& st, bool carry_tangents) {
   sm = OKIN_SHARED(sm);
   const int32_t* hdr = OKIN_SHARED(pr.hdr);
-  const int nlev = hdr[OKIN_H_NLEV];
+  const int nlev = OKIN_HV(hdr, OKIN_H_NLEV);
   const int32_t* lev_upd = OKIN_SHARED(okin_sec(pr, OKIN_S_LEV_UPD));
   const int32_t* lev_upd_mid = OKIN_SHARED(okin_sec(pr, OKIN_S_LEV_UPD_MID));
   const int32_t* udst = OKIN_SHARED(okin_sec(pr, OKIN_S_UPD_DST));
@@ -783,57 +880,76 @@ OKIN_FN_HOT void okin_factor(const OkinProgram& pr, double* sm, OkinState& st, b
   const int32_t* lcp = OKIN_SHARED(okin_sec(pr, OKIN_S_LEV_COL_PTR));
   const int32_t* lcol = OKIN_SHARED(okin_sec(pr, OKIN_S_LEV_COL));
   const int32_t* doffs = OKIN_SHARED(okin_sec(pr, OKIN_S_DIAG_OFF));
-  double* red = sm + hdr[OKIN_H_OFF_RED];
+  double* red = sm + OKIN_HV(hdr, OKIN_H_OFF_RED);
+  // left-looking update of one block row (or of a carried right-hand side)
+  auto update = [&](uint32_t dst_off, auto&& each) {
+    double* dst = sm + dst_off;
+    double c0 = dst[0], c1 = dst[1], c2 = dst[2];
+    each([&](uint32_t w) {
+      const double* a = sm + (w >> 16);
+      const double* B = sm + (w & 0xffffu);
+      const double a0 = a[0], a1 = a[1], a2 = a[2];
+      const double b0 = B[0], b1 = B[1], b2 = B[2], b3 = B[3], b4 = B[4], b5 = B[5], b6 = B[6], b7 = B[7], b8 = B[8];
+      c0 = fma(-a0, b0, c0); c1 = fma(-a0, b3, c1); c2 = fma(-a0, b6, c2);
+      c0 = fma(-a1, b1, c0); c1 = fma(-a1, b4, c1); c2 = fma(-a1, b7, c2);
+      c0 = fma(-a2, b2, c0); c1 = fma(-a2, b5, c1); c2 = fma(-a2, b8, c2);
+    });
+    dst[0] = c0; dst[1] = c1; dst[2] = c2;
+  };
+  auto scale = [&](uint32_t w, auto&&) {
+    const double* f = sm + (w & 0xffffu);
+    double* b = sm + (w >> 16);
+    const double x0 = b[0] * f[6];
+    const double x1 = fma(-x0, f[1], b[1]) * f[7];
+    const double x2 = fma(-x1, f[4], fma(-x0, f[3], b[2])) * f[8];
+    b[0] = x0; b[1] = x1; b[2] = x2;
+  };
   OKIN_PHASE_BEGIN
   red[lane] = 0.0;
   OKIN_PHASE_END
-  for (int lv = 0; lv < nlev; ++lv) {
+  // per level: update tasks, then the level's diagonal blocks (final now: factored once, in place, one
+  // lane per column, so that the scale tasks and the triangular solves read the factor), then scale tasks
+  auto level = [&](auto lv) {
+#ifdef OKIN_SPEC
+    // the spec is of the lean kernel, which never carries tangent right-hand sides
+    constexpr int L = decltype(lv)::value;
+    OKIN_PHASE_BEGIN
+    okin_spec_phase<OKIN_PH_UPD(L)>(pr, lane, update);
+    OKIN_PHASE_END
+    OKIN_PHASE_BEGIN
+    auto diag = [&](uint32_t doff, auto&&) { okin_write_diag_factor(sm, (int)doff, red, lane); };
+    okin_spec_phase<OKIN_PH_DIAG(L)>(pr, lane, diag);
+    OKIN_PHASE_END
+    OKIN_PHASE_BEGIN
+    okin_spec_phase<OKIN_PH_SCL(L)>(pr, lane, scale);
+    OKIN_PHASE_END
+#else
     const int ub = OKIN_LDG(lev_upd + lv), ue = carry_tangents ? OKIN_LDG(lev_upd + lv + 1) : OKIN_LDG(lev_upd_mid + lv);
     if (ue > ub) {
       OKIN_PHASE_BEGIN
-      // left-looking update of one block row (or of a carried right-hand side), two contributions per trip
       OKIN_LANE_LOOP
       for (int t = ub + lane; t < ue; t += 32) {
         const int b = OKIN_LDG(uptr + t), e = OKIN_LDG(uptr + t + 1);
-        double* dst = sm + OKIN_LDG(udst + t);
-        double c0 = dst[0], c1 = dst[1], c2 = dst[2];
-        OKIN_UNROLL_INNER
-        for (int q = b; q < e; ++q) {
-          const uint32_t w = (uint32_t)OKIN_LDG(ucon + q);
-          const double* a = sm + (w >> 16);
-          const double* B = sm + (w & 0xffffu);
-          const double a0 = a[0], a1 = a[1], a2 = a[2];
-          const double b0 = B[0], b1 = B[1], b2 = B[2], b3 = B[3], b4 = B[4], b5 = B[5], b6 = B[6], b7 = B[7], b8 = B[8];
-          c0 = fma(-a0, b0, c0); c1 = fma(-a0, b3, c1); c2 = fma(-a0, b6, c2);
-          c0 = fma(-a1, b1, c0); c1 = fma(-a1, b4, c1); c2 = fma(-a1, b7, c2);
-          c0 = fma(-a2, b2, c0); c1 = fma(-a2, b5, c1); c2 = fma(-a2, b8, c2);
-        }
-        dst[0] = c0; dst[1] = c1; dst[2] = c2;
+        update((uint32_t)OKIN_LDG(udst + t), [&](auto&& g) {
+          OKIN_UNROLL_INNER
+          for (int q = b; q < e; ++q) g((uint32_t)OKIN_LDG(ucon + q));
+        });
       }
       OKIN_PHASE_END
     }
-    // The level's diagonal blocks are final: factor each once, in place (one lane per column), so that
-    // the scale tasks below and the triangular solves later read the factor instead of recomputing it.
     const int wb = OKIN_LDG(lcp + lv), we = OKIN_LDG(lcp + lv + 1);
     OKIN_PHASE_BEGIN
     OKIN_LANE_LOOP
-    for (int c = wb + lane; c < we; c += 32)
-      okin_write_diag_factor(sm, OKIN_LDG(doffs + OKIN_LDG(lcol + c)), red, lane);
+    for (int c = wb + lane; c < we; c += 32) okin_write_diag_factor(sm, OKIN_LDG(doffs + OKIN_LDG(lcol + c)), red, lane);
     OKIN_PHASE_END
     const int sb = OKIN_LDG(lev_scl + lv), se = carry_tangents ? OKIN_LDG(lev_scl + lv + 1) : OKIN_LDG(lev_scl_mid + lv);
     OKIN_PHASE_BEGIN
     OKIN_LANE_LOOP
-    for (int t = sb + lane; t < se; t += 32) {
-      const uint32_t w = (uint32_t)OKIN_LDG(scl + t);
-      const double* f = sm + (w & 0xffffu);
-      double* b = sm + (w >> 16);
-      const double x0 = b[0] * f[6];
-      const double x1 = (b[1] - x0 * f[1]) * f[7];
-      const double x2 = (b[2] - x0 * f[3] - x1 * f[4]) * f[8];
-      b[0] = x0; b[1] = x1; b[2] = x2;
-    }
+    for (int t = sb + lane; t < se; t += 32) scale((uint32_t)OKIN_LDG(scl + t), 0);
     OKIN_PHASE_END
-  }
+#endif
+  };
+  okin_levels(nlev, level);
   st.notpd = okin_red_sum(red) != 0.0;
 }
 
@@ -845,78 +961,99 @@ template <typename Dummy = void>
 OKIN_FN_HOT void okin_solve(const OkinProgram& pr, double* sm, int first, int nrhs, bool skip_forward) {
   sm = OKIN_SHARED(sm);
   const int32_t* hdr = OKIN_SHARED(pr.hdr);
-  const int nlev = hdr[OKIN_H_NLEV];
-  const int n = 3 * hdr[OKIN_H_NF];
+  const int nlev = OKIN_HV(hdr, OKIN_H_NLEV);
+  const int n = 3 * OKIN_HV(hdr, OKIN_H_NF);
   const int32_t* slev = OKIN_SHARED(okin_sec(pr, OKIN_S_SOLVE_LEV));
   const int32_t* stask = OKIN_SHARED(okin_sec(pr, OKIN_S_SOLVE_TASK));
   const int32_t* scon = OKIN_SHARED(okin_sec(pr, OKIN_S_SOLVE_CON));
   const double* Lb = sm;
   const int32_t* doffs = OKIN_SHARED(okin_sec(pr, OKIN_S_DIAG_OFF));
-  double* vec = sm + hdr[OKIN_H_OFF_VEC] + first * n;
-  for (int lv = 0; lv < (skip_forward ? 0 : nlev); ++lv) {  // L y = b
-    const int tb = OKIN_LDG(slev + lv), te = OKIN_LDG(slev + lv + 1);
+  double* vec = sm + OKIN_HV(hdr, OKIN_H_OFF_VEC) + first * n;
+  // task word: OKIN_SOLVE_FIN | column j, and in the high half the first contribution (generic tables) or
+  // the offset of the column's diagonal factor block (spec words)
+  auto diag_of = [&](uint32_t task) -> const double* {
+#ifdef OKIN_SPEC
+    return sm + (task >> 16);
+#else
+    return sm + OKIN_LDG(doffs + (task & 0x7fffu));
+#endif
+  };
+  auto forward = [&](double* v, uint32_t task, auto&& each) {  // L y = b
+    const int j = task & 0x7fffu;
+    double t0 = v[3 * j], t1 = v[3 * j + 1], t2 = v[3 * j + 2];
+    each([&](uint32_t w) {
+      const double* B = Lb + (w >> 16);
+      const double* y = v + (w & 0xffffu);
+      const double y0 = y[0], y1 = y[1], y2 = y[2];
+      const double b0 = B[0], b1 = B[1], b2 = B[2], b3 = B[3], b4 = B[4], b5 = B[5], b6 = B[6], b7 = B[7], b8 = B[8];
+      t0 = fma(-b0, y0, t0); t1 = fma(-b3, y0, t1); t2 = fma(-b6, y0, t2);
+      t0 = fma(-b1, y1, t0); t1 = fma(-b4, y1, t1); t2 = fma(-b7, y1, t2);
+      t0 = fma(-b2, y2, t0); t1 = fma(-b5, y2, t1); t2 = fma(-b8, y2, t2);
+    });
+    if (task & OKIN_SOLVE_FIN) {
+      const double* f = diag_of(task);
+      t0 = t0 * f[6];
+      t1 = fma(-f[1], t0, t1) * f[7];
+      t2 = fma(-f[4], t1, fma(-f[3], t0, t2)) * f[8];
+    }
+    v[3 * j] = t0; v[3 * j + 1] = t1; v[3 * j + 2] = t2;
+  };
+  auto backward = [&](double* v, uint32_t task, auto&& each) {  // L^T x = y
+    const int j = task & 0x7fffu;
+    double t0 = v[3 * j], t1 = v[3 * j + 1], t2 = v[3 * j + 2];
+    each([&](uint32_t w) {
+      const double* B = Lb + (w >> 16);
+      const double* x = v + (w & 0xffffu);
+      const double x0 = x[0], x1 = x[1], x2 = x[2];
+      const double b0 = B[0], b1 = B[1], b2 = B[2], b3 = B[3], b4 = B[4], b5 = B[5], b6 = B[6], b7 = B[7], b8 = B[8];
+      t0 = fma(-b0, x0, t0); t1 = fma(-b1, x0, t1); t2 = fma(-b2, x0, t2);
+      t0 = fma(-b3, x1, t0); t1 = fma(-b4, x1, t1); t2 = fma(-b5, x1, t2);
+      t0 = fma(-b6, x2, t0); t1 = fma(-b7, x2, t1); t2 = fma(-b8, x2, t2);
+    });
+    if (task & OKIN_SOLVE_FIN) {
+      const double* f = diag_of(task);
+      t2 = t2 * f[8];
+      t1 = fma(-f[4], t2, t1) * f[7];
+      t0 = fma(-f[3], t2, fma(-f[1], t1, t0)) * f[6];
+    }
+    v[3 * j] = t0; v[3 * j + 1] = t1; v[3 * j + 2] = t2;
+  };
+#ifdef OKIN_SPEC
+  // the spec is of the lean kernel: one right-hand side
+  auto fw = [&](uint32_t task, auto&& each) { forward(vec, task, each); };
+  auto bw = [&](uint32_t task, auto&& each) { backward(vec, task, each); };
+  if (!skip_forward) {
+    okin_levels(nlev, [&](auto lv) {
+      OKIN_PHASE_BEGIN
+      okin_spec_phase<OKIN_PH_FW(okin_spec_hdr(OKIN_H_NLEV), decltype(lv)::value)>(pr, lane, fw);
+      OKIN_PHASE_END
+    });
+  }
+  okin_levels(nlev, [&](auto ph) {
+    OKIN_PHASE_BEGIN
+    okin_spec_phase<OKIN_PH_BW(okin_spec_hdr(OKIN_H_NLEV), decltype(ph)::value)>(pr, lane, bw);
+    OKIN_PHASE_END
+  });
+#else
+  // one phase: tasks [slev[p], slev[p + 1]) of the solve lists, nrhs right-hand sides each
+  auto phase = [&](int p, auto&& body) {
+    const int tb = OKIN_LDG(slev + p), te = OKIN_LDG(slev + p + 1);
     OKIN_PHASE_BEGIN
     OKIN_LANE_LOOP
     for (int t = lane; t < (te - tb) * nrhs; t += 32) {
       const int k = tb + t / nrhs;
       const uint32_t task = (uint32_t)OKIN_LDG(stask + k);
-      const int j = task & 0x7fffu;
-      const int qe = (int)((uint32_t)OKIN_LDG(stask + k + 1) >> 16);
-      double* v = vec + (t % nrhs) * n;
-      double t0 = v[3 * j], t1 = v[3 * j + 1], t2 = v[3 * j + 2];
-      OKIN_UNROLL_INNER
-      for (int q = (int)(task >> 16); q < qe; ++q) {
-        const uint32_t w = (uint32_t)OKIN_LDG(scon + q);
-        const double* B = Lb + (w >> 16);
-        const double* y = v + (w & 0xffffu);
-        const double y0 = y[0], y1 = y[1], y2 = y[2];
-        const double b0 = B[0], b1 = B[1], b2 = B[2], b3 = B[3], b4 = B[4], b5 = B[5], b6 = B[6], b7 = B[7], b8 = B[8];
-        t0 = fma(-b0, y0, t0); t1 = fma(-b3, y0, t1); t2 = fma(-b6, y0, t2);
-        t0 = fma(-b1, y1, t0); t1 = fma(-b4, y1, t1); t2 = fma(-b7, y1, t2);
-        t0 = fma(-b2, y2, t0); t1 = fma(-b5, y2, t1); t2 = fma(-b8, y2, t2);
-      }
-      if (task & OKIN_SOLVE_FIN) {
-        const double* f = sm + OKIN_LDG(doffs + j);
-        t0 = t0 * f[6];
-        t1 = (t1 - f[1] * t0) * f[7];
-        t2 = (t2 - f[3] * t0 - f[4] * t1) * f[8];
-      }
-      v[3 * j] = t0; v[3 * j + 1] = t1; v[3 * j + 2] = t2;
+      const int qb = (int)(task >> 16), qe = (int)((uint32_t)OKIN_LDG(stask + k + 1) >> 16);
+      body(vec + (t % nrhs) * n, task, [&](auto&& g) {
+        OKIN_UNROLL_INNER
+        for (int q = qb; q < qe; ++q) g((uint32_t)OKIN_LDG(scon + q));
+      });
     }
     OKIN_PHASE_END
-  }
-  for (int ph = 0; ph < nlev; ++ph) {  // L^T x = y
-    const int tb = OKIN_LDG(slev + nlev + 1 + ph), te = OKIN_LDG(slev + nlev + 2 + ph);
-    OKIN_PHASE_BEGIN
-    OKIN_LANE_LOOP
-    for (int t = lane; t < (te - tb) * nrhs; t += 32) {
-      const int k = tb + t / nrhs;
-      const uint32_t task = (uint32_t)OKIN_LDG(stask + k);
-      const int j = task & 0x7fffu;
-      const int qe = (int)((uint32_t)OKIN_LDG(stask + k + 1) >> 16);
-      double* v = vec + (t % nrhs) * n;
-      double t0 = v[3 * j], t1 = v[3 * j + 1], t2 = v[3 * j + 2];
-      OKIN_UNROLL_INNER
-      for (int q = (int)(task >> 16); q < qe; ++q) {
-        const uint32_t w = (uint32_t)OKIN_LDG(scon + q);
-        const double* B = Lb + (w >> 16);
-        const double* x = v + (w & 0xffffu);
-        const double x0 = x[0], x1 = x[1], x2 = x[2];
-        const double b0 = B[0], b1 = B[1], b2 = B[2], b3 = B[3], b4 = B[4], b5 = B[5], b6 = B[6], b7 = B[7], b8 = B[8];
-        t0 = fma(-b0, x0, t0); t1 = fma(-b1, x0, t1); t2 = fma(-b2, x0, t2);
-        t0 = fma(-b3, x1, t0); t1 = fma(-b4, x1, t1); t2 = fma(-b5, x1, t2);
-        t0 = fma(-b6, x2, t0); t1 = fma(-b7, x2, t1); t2 = fma(-b8, x2, t2);
-      }
-      if (task & OKIN_SOLVE_FIN) {
-        const double* f = sm + OKIN_LDG(doffs + j);
-        t2 = t2 * f[8];
-        t1 = (t1 - f[4] * t2) * f[7];
-        t0 = (t0 - f[1] * t1 - f[3] * t2) * f[6];
-      }
-      v[3 * j] = t0; v[3 * j + 1] = t1; v[3 * j + 2] = t2;
-    }
-    OKIN_PHASE_END
-  }
+  };
+  for (int lv = 0; lv < (skip_forward ? 0 : nlev); ++lv) phase(lv, forward);
+  for (int ph = 0; ph < nlev; ++ph) phase(nlev + 1 + ph, backward);
+#endif
 }
 
 // pos[free] += scale * vec[which]; returns max|vec[which]| (warp-uniform).
@@ -924,11 +1061,11 @@ template <typename Dummy = void>
 OKIN_FN double okin_apply_step(const OkinProgram& pr, double* sm, int which, double scale, bool save) {
   sm = OKIN_SHARED(sm);
   const int32_t* hdr = OKIN_SHARED(pr.hdr);
-  const int n = 3 * hdr[OKIN_H_NF];
+  const int n = 3 * OKIN_HV(hdr, OKIN_H_NF);
   const int32_t* ep = OKIN_SHARED(okin_sec(pr, OKIN_S_ELIM_POINT));
-  double* pos = sm + hdr[OKIN_H_OFF_POS];
-  const double* v = sm + hdr[OKIN_H_OFF_VEC] + which * n;
-  double* red = sm + hdr[OKIN_H_OFF_RED];
+  double* pos = sm + OKIN_HV(hdr, OKIN_H_OFF_POS);
+  const double* v = sm + OKIN_HV(hdr, OKIN_H_OFF_VEC) + which * n;
+  double* red = sm + OKIN_HV(hdr, OKIN_H_OFF_RED);
   OKIN_PHASE_BEGIN
   double mx = 0.0;
   OKIN_LANE_LOOP
@@ -949,10 +1086,10 @@ template <typename Dummy = void>
 OKIN_FN void okin_restore(const OkinProgram& pr, double* sm) {
   sm = OKIN_SHARED(sm);
   const int32_t* hdr = OKIN_SHARED(pr.hdr);
-  const int n = 3 * hdr[OKIN_H_NF];
+  const int n = 3 * OKIN_HV(hdr, OKIN_H_NF);
   const int32_t* ep = OKIN_SHARED(okin_sec(pr, OKIN_S_ELIM_POINT));
-  double* pos = sm + hdr[OKIN_H_OFF_POS];
-  const double* h = sm + hdr[OKIN_H_OFF_VEC];   // the step just applied (vec[0], scale 1)
+  double* pos = sm + OKIN_HV(hdr, OKIN_H_OFF_POS);
+  const double* h = sm + OKIN_HV(hdr, OKIN_H_OFF_VEC);   // the step just applied (vec[0], scale 1)
   OKIN_PHASE_BEGIN
   OKIN_LANE_LOOP
   for (int u = lane; u < n; u += 32) pos[3 * OKIN_LDG(ep + u / 3) + u % 3] -= h[u];
@@ -963,9 +1100,9 @@ OKIN_FN void okin_restore(const OkinProgram& pr, double* sm) {
 template <typename Dummy = void>
 OKIN_FN double okin_vec_max(const OkinProgram& pr, double* sm, int which) {
   sm = OKIN_SHARED(sm);
-  const int n = 3 * pr.hdr[OKIN_H_NF];
-  const double* v = sm + pr.hdr[OKIN_H_OFF_VEC] + which * n;
-  double* red = sm + pr.hdr[OKIN_H_OFF_RED];
+  const int n = 3 * OKIN_HV(pr.hdr, OKIN_H_NF);
+  const double* v = sm + OKIN_HV(pr.hdr, OKIN_H_OFF_VEC) + which * n;
+  double* red = sm + OKIN_HV(pr.hdr, OKIN_H_OFF_RED);
   OKIN_PHASE_BEGIN
   double mx = 0.0;
   OKIN_LANE_LOOP
@@ -989,11 +1126,11 @@ template <typename Dummy = void>
 OKIN_FN void okin_extrapolate(const OkinProgram& pr, double* sm, int order) {
   sm = OKIN_SHARED(sm);
   const int32_t* hdr = OKIN_SHARED(pr.hdr);
-  const int n = 3 * hdr[OKIN_H_NF];
+  const int n = 3 * OKIN_HV(hdr, OKIN_H_NF);
   const int32_t* ep = OKIN_SHARED(okin_sec(pr, OKIN_S_ELIM_POINT));
-  double* pos = sm + hdr[OKIN_H_OFF_POS];
-  double* xprev = sm + hdr[OKIN_H_OFF_XPREV];
-  float* h1 = reinterpret_cast<float*>(sm + hdr[OKIN_H_OFF_DHIST]);
+  double* pos = sm + OKIN_HV(hdr, OKIN_H_OFF_POS);
+  double* xprev = sm + OKIN_HV(hdr, OKIN_H_OFF_XPREV);
+  float* h1 = reinterpret_cast<float*>(sm + OKIN_HV(hdr, OKIN_H_OFF_DHIST));
   float* h2 = h1 + 2 * ((n + 1) / 2);
   float* h3 = h2 + 2 * ((n + 1) / 2);
   OKIN_PHASE_BEGIN
@@ -1024,12 +1161,12 @@ template <typename Dummy = void>
 OKIN_FN void okin_tangent_rhs(const OkinProgram& pr, double* sm) {
   sm = OKIN_SHARED(sm);
   const int32_t* hdr = OKIN_SHARED(pr.hdr);
-  const int nt = hdr[OKIN_H_NT];
-  const int n = 3 * hdr[OKIN_H_NF];
+  const int nt = OKIN_HV(hdr, OKIN_H_NT);
+  const int n = 3 * OKIN_HV(hdr, OKIN_H_NF);
   const int32_t* sptr = OKIN_SHARED(okin_sec(pr, OKIN_S_TGT_SC_PTR));
   const int32_t* sc = OKIN_SHARED(okin_sec(pr, OKIN_S_TGT_SC));
-  const double* rg = sm + hdr[OKIN_H_OFF_RG];
-  double* vec = sm + hdr[OKIN_H_OFF_VEC] + n;
+  const double* rg = sm + OKIN_HV(hdr, OKIN_H_OFF_RG);
+  double* vec = sm + OKIN_HV(hdr, OKIN_H_OFF_VEC) + n;
   OKIN_PHASE_BEGIN
   OKIN_LANE_LOOP
   for (int t = lane; t < nt * n; t += 32) vec[t] = 0.0;
@@ -1052,14 +1189,14 @@ template <typename Dummy = void>
 OKIN_FN void okin_linear_residuals(const OkinProgram& pr, double* sm, OkinState& st) {
   sm = OKIN_SHARED(sm);
   const int32_t* hdr = OKIN_SHARED(pr.hdr);
-  const int nls = hdr[OKIN_H_NROW], nrep = hdr[OKIN_H_NREP];
+  const int nls = OKIN_HV(hdr, OKIN_H_NROW), nrep = OKIN_HV(hdr, OKIN_H_NREP);
   const int32_t* jptr = OKIN_SHARED(okin_sec(pr, OKIN_S_JH_PTR));
   const int32_t* jcon = OKIN_SHARED(okin_sec(pr, OKIN_S_JH_CON));
   const int32_t* rpin = OKIN_SHARED(okin_sec(pr, OKIN_S_REP_PINS));
-  const double* rg = sm + hdr[OKIN_H_OFF_RG];
-  const double* h = sm + hdr[OKIN_H_OFF_VEC];
-  double* r = sm + hdr[OKIN_H_OFF_R];
-  double* red = sm + hdr[OKIN_H_OFF_RED];
+  const double* rg = sm + OKIN_HV(hdr, OKIN_H_OFF_RG);
+  const double* h = sm + OKIN_HV(hdr, OKIN_H_OFF_VEC);
+  double* r = sm + OKIN_HV(hdr, OKIN_H_OFF_R);
+  double* red = sm + OKIN_HV(hdr, OKIN_H_OFF_RED);
   double sq = 0.0, mx = 0.0;
   OKIN_PHASE_BEGIN
   OKIN_LANE_LOOP
@@ -1247,7 +1384,7 @@ OKIN_HD void okin_point_vel_base(const OkinProgram& pr, const double* sm, int p,
   if (p < 0) return;
   const int e = OKIN_LDG(OKIN_SHARED(okin_sec(pr, OKIN_S_POINT_ELIM)) + p);
   if (e < 0) return;
-  const double* V = sm + pr.hdr[OKIN_H_OFF_VEC] + (1 + j) * 3 * pr.hdr[OKIN_H_NF] + 3 * e;
+  const double* V = sm + OKIN_HV(pr.hdr, OKIN_H_OFF_VEC) + (1 + j) * 3 * OKIN_HV(pr.hdr, OKIN_H_NF) + 3 * e;
   v[0] = V[0]; v[1] = V[1]; v[2] = V[2];
 }
 OKIN_HD void okin_point_vel_op(const OkinProgram& pr, const double* sm, int d, const double* da, const double* db,
@@ -1255,8 +1392,8 @@ OKIN_HD void okin_point_vel_op(const OkinProgram& pr, const double* sm, int d, c
   sm = OKIN_SHARED(sm);
   const int32_t* rec = OKIN_SHARED(okin_sec(pr, OKIN_S_DOP)) + d * OKIN_DOP_STRIDE;
   const int ia = OKIN_LDG(rec + 2), ib = OKIN_LDG(rec + 3), ic = OKIN_LDG(rec + 4);
-  const double* pos = sm + pr.hdr[OKIN_H_OFF_POS];
-  const double* par = sm + pr.hdr[OKIN_H_OFF_PAR];
+  const double* pos = sm + OKIN_HV(pr.hdr, OKIN_H_OFF_POS);
+  const double* par = sm + OKIN_HV(pr.hdr, OKIN_H_OFF_PAR);
   double out[3];
   okin_dop_eval(OKIN_LDG(rec + 0), par[OKIN_LDG(rec + 5)], pos + 3 * ia, pos + 3 * (ib < 0 ? ia : ib),
                 pos + 3 * (ic < 0 ? ia : ic), da, db, dc, out, v);
@@ -1289,8 +1426,8 @@ template <typename T>
 OKIN_HD T okin_response(const OkinProgram& pr, const double* sm, const int32_t* rec, int j) {
   sm = OKIN_SHARED(sm);
   const int32_t* hdr = OKIN_SHARED(pr.hdr);
-  const double* pos = sm + hdr[OKIN_H_OFF_POS];
-  const double* dsn = sm + hdr[OKIN_H_OFF_DSN];
+  const double* pos = sm + OKIN_HV(hdr, OKIN_H_OFF_POS);
+  const double* dsn = sm + OKIN_HV(hdr, OKIN_H_OFF_DSN);
   const double* fc = okin_fsec(pr, OKIN_F_MCONST) + OKIN_LDG(rec + 12);
   const int rtype = OKIN_LDG(rec + 1);
   OkinV3<T> P[4];
@@ -1344,8 +1481,8 @@ OKIN_HD T okin_response(const OkinProgram& pr, const double* sm, const int32_t* 
 OKIN_HD void okin_corner_metrics(const OkinProgram& pr, double* sm, const int32_t* rec, double* out, double* ctx) {
   sm = OKIN_SHARED(sm);
   const int32_t* hdr = OKIN_SHARED(pr.hdr);
-  const double* pos = sm + hdr[OKIN_H_OFF_POS];
-  const double* dsn = sm + hdr[OKIN_H_OFF_DSN];
+  const double* pos = sm + OKIN_HV(hdr, OKIN_H_OFF_POS);
+  const double* dsn = sm + OKIN_HV(hdr, OKIN_H_OFF_DSN);
   const double* fc = okin_fsec(pr, OKIN_F_MCONST) + OKIN_LDG(rec + 18);
   const double side = fc[0], cg_z = fc[1], wheelbase = fc[2], bias = fc[3];
   const int flags = OKIN_LDG(rec + 19);
@@ -1471,11 +1608,11 @@ template <typename Dummy = void>
 OKIN_FN void okin_metrics(const OkinProgram& pr, double* sm, double* out) {
   sm = OKIN_SHARED(sm);
   const int32_t* hdr = OKIN_SHARED(pr.hdr);
-  const int nmc = hdr[OKIN_H_NMC], nmop = hdr[OKIN_H_NMOP];
+  const int nmc = OKIN_HV(hdr, OKIN_H_NMC), nmop = OKIN_HV(hdr, OKIN_H_NMOP);
   const int32_t* corners = OKIN_SHARED(okin_sec(pr, OKIN_S_MCORNER));
   const int32_t* mops = OKIN_SHARED(okin_sec(pr, OKIN_S_MOP));
-  double* ctx = sm + hdr[OKIN_H_OFF_MCTX];
-  const int nt = hdr[OKIN_H_NT];
+  double* ctx = sm + OKIN_HV(hdr, OKIN_H_OFF_MCTX);
+  const int nt = OKIN_HV(hdr, OKIN_H_NT);
   OKIN_PHASE_BEGIN
   if (lane < nmc) okin_corner_metrics(pr, sm, corners + lane * OKIN_MCORNER_STRIDE, out, ctx + 4 * lane);
   for (int t = lane - nmc; t < nmop; t += 32 - nmc) {
@@ -1510,11 +1647,11 @@ OKIN_FN void okin_metrics(const OkinProgram& pr, double* sm, double* out) {
     out[OKIN_LDG(rec + 11)] = value;
   }
   OKIN_PHASE_END
-  if (hdr[OKIN_H_NMAXLE]) {
+  if (OKIN_HV(hdr, OKIN_H_NMAXLE)) {
     // axle-level state metrics (axle_metrics.py:18-95)
     const int32_t* rec = OKIN_SHARED(okin_sec(pr, OKIN_S_MAXLE));
-    const double* pos = sm + hdr[OKIN_H_OFF_POS];
-    const double* dsn = sm + hdr[OKIN_H_OFF_DSN];
+    const double* pos = sm + OKIN_HV(hdr, OKIN_H_OFF_POS);
+    const double* dsn = sm + OKIN_HV(hdr, OKIN_H_OFF_DSN);
     OKIN_PHASE_BEGIN
     if (lane == 0) {
       const double* wcL = pos + 3 * OKIN_LDG(rec + 0);
@@ -1570,10 +1707,10 @@ template <typename Dummy = void>
 OKIN_FN void okin_diagnostics(const OkinProgram& pr, double* sm, double* row, bool ok, int status) {
   sm = OKIN_SHARED(sm);
   const int32_t* hdr = OKIN_SHARED(pr.hdr);
-  const int nd = hdr[OKIN_H_NDIAG], nop = hdr[OKIN_H_NDGOP];
-  const double* pos = sm + hdr[OKIN_H_OFF_POS];
-  const double* dsn = sm + hdr[OKIN_H_OFF_DSN];
-  double* red = sm + hdr[OKIN_H_OFF_RED];
+  const int nd = OKIN_HV(hdr, OKIN_H_NDIAG), nop = OKIN_HV(hdr, OKIN_H_NDGOP);
+  const double* pos = sm + OKIN_HV(hdr, OKIN_H_OFF_POS);
+  const double* dsn = sm + OKIN_HV(hdr, OKIN_H_OFF_DSN);
+  double* red = sm + OKIN_HV(hdr, OKIN_H_OFF_RED);
   OKIN_PHASE_BEGIN
   OKIN_LANE_LOOP
   for (int t = lane; t < nd; t += 32) row[t] = t == 3 ? -1.0 : (t < OKIN_DIAG_BASE || ok ? 0.0 : NAN);
@@ -1657,7 +1794,7 @@ template <typename Dummy = void>
 OKIN_HD void okin_continuity(const OkinProgram& pr, double* scratch, int stride, const double* positions,
                              int n_steps, int n_ok, double* diag, double* jumps) {
   const int32_t* hdr = pr.hdr;   // global memory in the continuity kernel
-  const int nf = hdr[OKIN_H_NF], nout3 = 3 * hdr[OKIN_H_NOUT], nd = hdr[OKIN_H_NDIAG];
+  const int nf = OKIN_HV(hdr, OKIN_H_NF), nout3 = 3 * OKIN_HV(hdr, OKIN_H_NOUT), nd = OKIN_HV(hdr, OKIN_H_NDIAG);
   const int32_t* free_out = okin_sec(pr, OKIN_S_FREE_OUT);
   const int ntr = n_ok > 1 ? n_ok - 1 : 0;
   double* thr = scratch + 32 * stride;
@@ -1739,12 +1876,12 @@ template <typename Dummy = void>
 OKIN_FN double okin_factor_multiply(const OkinProgram& pr, double* sm, const double* src, double* dst, bool lt) {
   sm = OKIN_SHARED(sm);
   const int32_t* hdr = OKIN_SHARED(pr.hdr);
-  const int nf = hdr[OKIN_H_NF];
+  const int nf = OKIN_HV(hdr, OKIN_H_NF);
   const int32_t* ptr = okin_sec(pr, lt ? OKIN_S_BW_PTR : OKIN_S_FW_PTR);
   const int32_t* con = okin_sec(pr, lt ? OKIN_S_BW_CON : OKIN_S_FW_CON);
   const int32_t* doffs = OKIN_SHARED(okin_sec(pr, OKIN_S_DIAG_OFF));
   const double* Lb = sm;
-  double* red = sm + hdr[OKIN_H_OFF_RED];
+  double* red = sm + OKIN_HV(hdr, OKIN_H_OFF_RED);
   OKIN_PHASE_BEGIN
   double acc = 0.0;
   OKIN_LANE_LOOP
@@ -1780,8 +1917,8 @@ OKIN_FN double okin_factor_multiply(const OkinProgram& pr, double* sm, const dou
 template <typename Dummy = void>
 OKIN_FN double okin_scale_norm2(const OkinProgram& pr, double* sm, double* v, double s) {
   sm = OKIN_SHARED(sm);
-  const int n = 3 * pr.hdr[OKIN_H_NF];
-  double* red = sm + pr.hdr[OKIN_H_OFF_RED];
+  const int n = 3 * OKIN_HV(pr.hdr, OKIN_H_NF);
+  double* red = sm + OKIN_HV(pr.hdr, OKIN_H_OFF_RED);
   OKIN_PHASE_BEGIN
   double acc = 0.0;
   OKIN_LANE_LOOP
@@ -1799,8 +1936,8 @@ OKIN_FN double okin_scale_norm2(const OkinProgram& pr, double* sm, double* v, do
 template <typename Dummy = void>
 OKIN_FN double okin_dot(const OkinProgram& pr, double* sm, const double* a, const double* b) {
   sm = OKIN_SHARED(sm);
-  const int n = 3 * pr.hdr[OKIN_H_NF];
-  double* red = sm + pr.hdr[OKIN_H_OFF_RED];
+  const int n = 3 * OKIN_HV(pr.hdr, OKIN_H_NF);
+  double* red = sm + OKIN_HV(pr.hdr, OKIN_H_OFF_RED);
   OKIN_PHASE_BEGIN
   double acc = 0.0;
   OKIN_LANE_LOOP
@@ -1812,7 +1949,7 @@ OKIN_FN double okin_dot(const OkinProgram& pr, double* sm, const double* a, cons
 
 template <typename Dummy = void>
 OKIN_FN void okin_copy(const OkinProgram& pr, double* dst, const double* src) {
-  const int n = 3 * pr.hdr[OKIN_H_NF];
+  const int n = 3 * OKIN_HV(pr.hdr, OKIN_H_NF);
   OKIN_PHASE_BEGIN
   OKIN_LANE_LOOP
   for (int u = lane; u < n; u += 32) dst[u] = src[u];
@@ -1825,8 +1962,8 @@ struct OkinGram2 { double aa, ab, bb; };
 template <typename Dummy = void>
 OKIN_FN OkinGram2 okin_orthonormalise2(const OkinProgram& pr, double* sm, double* a, double* b) {
   sm = OKIN_SHARED(sm);
-  const int n = 3 * pr.hdr[OKIN_H_NF];
-  double* red = sm + pr.hdr[OKIN_H_OFF_RED];
+  const int n = 3 * OKIN_HV(pr.hdr, OKIN_H_NF);
+  double* red = sm + OKIN_HV(pr.hdr, OKIN_H_OFF_RED);
   OkinGram2 g;
   g.aa = okin_dot(pr, sm, a, a);
   g.ab = okin_dot(pr, sm, a, b);
@@ -1878,10 +2015,10 @@ template <typename Dummy = void>
 OKIN_FN void okin_tangent_health(const OkinProgram& pr, double* sm, bool notpd, double* out2) {
   sm = OKIN_SHARED(sm);
   const int32_t* hdr = OKIN_SHARED(pr.hdr);
-  const int n = 3 * hdr[OKIN_H_NF];
-  double* x1 = sm + hdr[OKIN_H_OFF_RG];
+  const int n = 3 * OKIN_HV(hdr, OKIN_H_NF);
+  double* x1 = sm + OKIN_HV(hdr, OKIN_H_OFF_RG);
   double* x2 = x1 + n;
-  double* v0 = sm + hdr[OKIN_H_OFF_VEC];
+  double* v0 = sm + OKIN_HV(hdr, OKIN_H_OFF_VEC);
   const double tol2 = OKIN_HEALTH_TOL * OKIN_HEALTH_TOL;
   double theta[2] = {0.0, 0.0};     // top Ritz values of A and of A^{-1}
   for (int inverse = 0; inverse < 2 && !notpd; ++inverse) {
@@ -1951,8 +2088,8 @@ OKIN_FN void okin_tangent_health(const OkinProgram& pr, double* sm, bool notpd, 
 // ---------------------------------------------------------------------------------------
 OKIN_HD const int32_t* okin_sec_cold(const OkinProgram& pr, int s) { return pr.ibc + pr.hdr[OKIN_H_SEC0 + 2 * s]; }
 OKIN_HD size_t okin_sens_ws_doubles(const int32_t* hdr) {
-  return (size_t)hdr[OKIN_H_NSENS] * (hdr[OKIN_H_NCST] + hdr[OKIN_H_NPAR]) + 13 * (size_t)hdr[OKIN_H_NROW] +
-         3 * (size_t)hdr[OKIN_H_P];
+  return (size_t)OKIN_HV(hdr, OKIN_H_NSENS) * (OKIN_HV(hdr, OKIN_H_NCST) + OKIN_HV(hdr, OKIN_H_NPAR)) + 13 * (size_t)OKIN_HV(hdr, OKIN_H_NROW) +
+         3 * (size_t)OKIN_HV(hdr, OKIN_H_P);
 }
 
 // d out / d par of a derived op: the unit direction its parameter scales (okin_dop_eval).
@@ -1983,7 +2120,7 @@ OKIN_FN void okin_sens_points(const OkinProgram& pr, double* sm, int coord, cons
                               bool design, double* tan) {
   sm = OKIN_SHARED(sm);
   const int32_t* hdr = OKIN_SHARED(pr.hdr);
-  const int np = hdr[OKIN_H_P];
+  const int np = OKIN_HV(hdr, OKIN_H_P);
   const int32_t* kind = okin_sec(pr, OKIN_S_POINT_KIND);
   const int32_t* pelim = OKIN_SHARED(okin_sec(pr, OKIN_S_POINT_ELIM));
   const int moved = OKIN_LDG(okin_sec(pr, OKIN_S_IN_POINT) + coord / 3), axis = coord % 3;
@@ -2000,8 +2137,8 @@ OKIN_FN void okin_sens_points(const OkinProgram& pr, double* sm, int coord, cons
   const int32_t* dop = OKIN_SHARED(okin_sec(pr, OKIN_S_DOP));
   const int32_t* lev = OKIN_SHARED(okin_sec(pr, OKIN_S_DOP_LEV));
   const int nlev = okin_sec_len(pr, OKIN_S_DOP_LEV) - 1;
-  const double* pos = sm + hdr[OKIN_H_OFF_POS];
-  const double* par = sm + hdr[OKIN_H_OFF_PAR];
+  const double* pos = sm + OKIN_HV(hdr, OKIN_H_OFF_POS);
+  const double* par = sm + OKIN_HV(hdr, OKIN_H_OFF_PAR);
   for (int lv = 0; lv < nlev; ++lv) {
     const int b = OKIN_LDG(lev + lv), e = OKIN_LDG(lev + lv + 1);
     OKIN_PHASE_BEGIN
@@ -2029,15 +2166,15 @@ template <typename Dummy = void>
 OKIN_FN void okin_sens_setup(const OkinProgram& pr, double* sm, const double* __restrict__ hardpoints, double* ws) {
   sm = OKIN_SHARED(sm);
   const int32_t* hdr = OKIN_SHARED(pr.hdr);
-  const int nsens = hdr[OKIN_H_NSENS], ncst = hdr[OKIN_H_NCST], npar = hdr[OKIN_H_NPAR];
-  const int ndop = hdr[OKIN_H_NDOP], nls = hdr[OKIN_H_NROW];
+  const int nsens = OKIN_HV(hdr, OKIN_H_NSENS), ncst = OKIN_HV(hdr, OKIN_H_NCST), npar = OKIN_HV(hdr, OKIN_H_NPAR);
+  const int ndop = OKIN_HV(hdr, OKIN_H_NDOP), nls = OKIN_HV(hdr, OKIN_H_NROW);
   const int32_t* sens_in = okin_sec_cold(pr, OKIN_S_SENS_IN);
   const int32_t* in_point = okin_sec(pr, OKIN_S_IN_POINT);
   const int32_t* dop = OKIN_SHARED(okin_sec(pr, OKIN_S_DOP));
   const int32_t* par_mode = okin_sec(pr, OKIN_S_PAR_MODE);
   const int32_t* rows = okin_sec(pr, OKIN_S_ROW);
-  const double* pos = sm + hdr[OKIN_H_OFF_POS];
-  const double* cst = sm + hdr[OKIN_H_OFF_CST];
+  const double* pos = sm + OKIN_HV(hdr, OKIN_H_OFF_POS);
+  const double* cst = sm + OKIN_HV(hdr, OKIN_H_OFF_CST);
   double* tan = ws + (size_t)nsens * (ncst + npar) + 13 * (size_t)nls;
   for (int k = 0; k < nsens; ++k) {
     const int coord = OKIN_LDG(sens_in + k), moved = OKIN_LDG(in_point + coord / 3), axis = coord % 3;
@@ -2119,16 +2256,16 @@ template <typename Dummy = void>
 OKIN_FN void okin_sens_state(const OkinProgram& pr, double* sm, const double* tval, double* ws, double* dst) {
   sm = OKIN_SHARED(sm);
   const int32_t* hdr = OKIN_SHARED(pr.hdr);
-  const int nsens = hdr[OKIN_H_NSENS], ncst = hdr[OKIN_H_NCST], npar = hdr[OKIN_H_NPAR];
-  const int nls = hdr[OKIN_H_NROW], nout = hdr[OKIN_H_NOUT], n = 3 * hdr[OKIN_H_NF];
-  const int group = 1 + hdr[OKIN_H_NT];
+  const int nsens = OKIN_HV(hdr, OKIN_H_NSENS), ncst = OKIN_HV(hdr, OKIN_H_NCST), npar = OKIN_HV(hdr, OKIN_H_NPAR);
+  const int nls = OKIN_HV(hdr, OKIN_H_NROW), nout = OKIN_HV(hdr, OKIN_H_NOUT), n = 3 * OKIN_HV(hdr, OKIN_H_NF);
+  const int group = 1 + OKIN_HV(hdr, OKIN_H_NT);
   const int32_t* sens_in = okin_sec_cold(pr, OKIN_S_SENS_IN);
   const int32_t* rows = okin_sec(pr, OKIN_S_ROW);
   const int32_t* out_point = OKIN_SHARED(okin_sec(pr, OKIN_S_OUT_POINT));
-  const double* pos = sm + hdr[OKIN_H_OFF_POS];
-  const double* cst = sm + hdr[OKIN_H_OFF_CST];
-  double* r = sm + hdr[OKIN_H_OFF_R];
-  double* vec = sm + hdr[OKIN_H_OFF_VEC];
+  const double* pos = sm + OKIN_HV(hdr, OKIN_H_OFF_POS);
+  const double* cst = sm + OKIN_HV(hdr, OKIN_H_OFF_CST);
+  double* r = sm + OKIN_HV(hdr, OKIN_H_OFF_R);
+  double* vec = sm + OKIN_HV(hdr, OKIN_H_OFF_VEC);
   double* grad = ws + (size_t)nsens * (ncst + npar);
   double* tan = grad + 13 * (size_t)nls;
   // Row gradients J_x at the state (the tangent health uses their storage as scratch), and the
@@ -2226,9 +2363,9 @@ template <typename Dummy = void>
 OKIN_FN int okin_worst_row(const OkinProgram& pr, double* sm) {
   sm = OKIN_SHARED(sm);
   const int32_t* hdr = OKIN_SHARED(pr.hdr);
-  const int nrows = hdr[OKIN_H_NROW] + hdr[OKIN_H_NREP];
-  const double* r = sm + hdr[OKIN_H_OFF_R];
-  double* red = sm + hdr[OKIN_H_OFF_RED];
+  const int nrows = OKIN_HV(hdr, OKIN_H_NROW) + OKIN_HV(hdr, OKIN_H_NREP);
+  const double* r = sm + OKIN_HV(hdr, OKIN_H_OFF_R);
+  double* red = sm + OKIN_HV(hdr, OKIN_H_OFF_RED);
   OKIN_PHASE_BEGIN
   double mx = -1.0;
   OKIN_LANE_LOOP
@@ -2270,17 +2407,20 @@ template <bool FULL, bool SHIM, bool SENS = false>
 OKIN_HD void okin_sweep(const OkinProgram& pr, double* sm, const double* __restrict__ hardpoints,
                         const double* __restrict__ params, const double* __restrict__ tvals, int n_steps,
                         const OkinSolverCfg& cfg, const OkinOutputs& out) {
+#ifdef OKIN_SPEC
+  static_assert(!FULL && !SENS, "a topology spec describes the lean kernel's phases only");
+#endif
   sm = OKIN_SHARED(sm);
   const int32_t* hdr = OKIN_SHARED(pr.hdr);
-  const int nt = hdr[OKIN_H_NT];
-  const int n = 3 * hdr[OKIN_H_NF];
-  const int nout = hdr[OKIN_H_NOUT];
+  const int nt = OKIN_HV(hdr, OKIN_H_NT);
+  const int n = 3 * OKIN_HV(hdr, OKIN_H_NF);
+  const int nout = OKIN_HV(hdr, OKIN_H_NOUT);
   const int32_t* out_point = OKIN_SHARED(okin_sec(pr, OKIN_S_OUT_POINT));
   const int32_t* ecol = okin_sec(pr, OKIN_S_ELIM_COL);
   const int32_t* elim_point = OKIN_SHARED(okin_sec(pr, OKIN_S_ELIM_POINT));
-  double* pos = sm + hdr[OKIN_H_OFF_POS];
-  double* vec = sm + hdr[OKIN_H_OFF_VEC];
-  const double* xprev = sm + hdr[OKIN_H_OFF_XPREV];
+  double* pos = sm + OKIN_HV(hdr, OKIN_H_OFF_POS);
+  double* vec = sm + OKIN_HV(hdr, OKIN_H_OFF_VEC);
+  const double* xprev = sm + OKIN_HV(hdr, OKIN_H_OFF_XPREV);
   // outputs only the full instantiation knows about
   double* const o_tangents = FULL ? out.tangents : nullptr;
   double* const o_velocities = FULL ? out.velocities : nullptr;
@@ -2303,14 +2443,14 @@ OKIN_HD void okin_sweep(const OkinProgram& pr, double* sm, const double* __restr
   int status = invalid ? OKIN_STATUS_INVALID_GEOMETRY : OKIN_STATUS_OK, failed = invalid ? 0 : -1;
   // Target values of the current step, their increments and the previous increments live in shared
   // memory (runtime-indexed per-thread arrays would be local memory).
-  double* tcur = sm + hdr[OKIN_H_OFF_TGT];
+  double* tcur = sm + OKIN_HV(hdr, OKIN_H_OFF_TGT);
   double* dt = tcur + OKIN_MAX_TARGETS;
-  double* red = sm + hdr[OKIN_H_OFF_RED];
+  double* red = sm + OKIN_HV(hdr, OKIN_H_OFF_RED);
   OKIN_PHASE_BEGIN
   OKIN_LANE_LOOP
   for (int j = lane; j < 2 * OKIN_MAX_TARGETS; j += 32) tcur[j] = 0.0;
   {   // increment history of the extrapolation predictor
-    float* h = reinterpret_cast<float*>(sm + hdr[OKIN_H_OFF_DHIST]);
+    float* h = reinterpret_cast<float*>(sm + OKIN_HV(hdr, OKIN_H_OFF_DHIST));
     OKIN_LANE_LOOP
     for (int u = lane; u < 6 * ((n + 1) / 2); u += 32) h[u] = 0.0f;
   }
@@ -2407,7 +2547,7 @@ OKIN_HD void okin_sweep(const OkinProgram& pr, double* sm, const double* __restr
       OKIN_PHASE_END
     }
     if (FULL && o_metrics) {
-      const int nm = hdr[OKIN_H_NM];
+      const int nm = OKIN_HV(hdr, OKIN_H_NM);
       double* dst = o_metrics + (size_t)s * nm;
       if (ok) {
         okin_metrics(pr, sm, dst);
@@ -2439,8 +2579,8 @@ OKIN_HD void okin_sweep(const OkinProgram& pr, double* sm, const double* __restr
       }
       OKIN_PHASE_END
     }
-    if (FULL && o_diagnostics && hdr[OKIN_H_NDIAG])
-      okin_diagnostics(pr, sm, o_diagnostics + (size_t)s * hdr[OKIN_H_NDIAG], ok,
+    if (FULL && o_diagnostics && OKIN_HV(hdr, OKIN_H_NDIAG))
+      okin_diagnostics(pr, sm, o_diagnostics + (size_t)s * OKIN_HV(hdr, OKIN_H_NDIAG), ok,
                        failed == s ? status : OKIN_STATUS_OK);
     if (FULL && o_health) {
       if (ok) {
@@ -2452,7 +2592,7 @@ OKIN_HD void okin_sweep(const OkinProgram& pr, double* sm, const double* __restr
       }
     }
     if (SENS && o_sens) {
-      const int nsens = hdr[OKIN_H_NSENS];
+      const int nsens = OKIN_HV(hdr, OKIN_H_NSENS);
       double* dst = o_sens + (size_t)s * nsens * 3 * nout;
       if (ok) {
         okin_sens_state(pr, sm, tcur, out.sens_ws, dst);
@@ -2496,7 +2636,9 @@ struct OkinKernelIO {
   const double* instance_targets;
   int32_t* worst_row;
 };
+#ifndef __CUDACC_RTC__   // checked by the library build; NVRTC has no offsetof
 static_assert(sizeof(OkinKernelIO) == offsetof(okin_batch_io, hardpoint_sensitivity), "OkinKernelIO layout");
+#endif
 
 // The fields of okin_batch_io in struct order.
 enum okin_io_field {
@@ -2514,7 +2656,7 @@ struct OkinIOShape {
   const int32_t* hdr;
 };
 OKIN_HD OkinIOShape okin_io_shape(const int32_t* hdr) {
-  return {hdr[OKIN_H_NIN], hdr[OKIN_H_NOUT], hdr[OKIN_H_NT], 3 * hdr[OKIN_H_NF], hdr};
+  return {OKIN_HV(hdr, OKIN_H_NIN), OKIN_HV(hdr, OKIN_H_NOUT), OKIN_HV(hdr, OKIN_H_NT), 3 * OKIN_HV(hdr, OKIN_H_NF), hdr};
 }
 
 // Elements of field f that belong to one instance (int32 for status, failed_step, iters and
@@ -2523,19 +2665,19 @@ OKIN_HD size_t okin_io_count(int f, const OkinIOShape& h, int n_steps) {
   const size_t S = (size_t)n_steps;
   switch (f) {
     case OKIN_IO_HARDPOINTS: return 3 * (size_t)h.nin;
-    case OKIN_IO_PARAMS: return (size_t)h.hdr[OKIN_H_NPARAM];
+    case OKIN_IO_PARAMS: return (size_t)OKIN_HV(h.hdr, OKIN_H_NPARAM);
     case OKIN_IO_POSITIONS: return S * 3 * h.nout;
     case OKIN_IO_ITERS:
     case OKIN_IO_MAX_RESIDUAL: return S;
     case OKIN_IO_TANGENTS: return S * h.nt * h.n;
     case OKIN_IO_VELOCITIES: return S * h.nt * 3 * h.nout;
     case OKIN_IO_TANGENT_HEALTH: return S * 2;
-    case OKIN_IO_METRICS: return S * h.hdr[OKIN_H_NM];
+    case OKIN_IO_METRICS: return S * OKIN_HV(h.hdr, OKIN_H_NM);
     case OKIN_IO_DESIGN: return 3 * (size_t)h.nout;
-    case OKIN_IO_DIAGNOSTICS: return S * h.hdr[OKIN_H_NDIAG];
+    case OKIN_IO_DIAGNOSTICS: return S * OKIN_HV(h.hdr, OKIN_H_NDIAG);
     case OKIN_IO_JUMPS: return S * (h.n / 3);
     case OKIN_IO_INSTANCE_TARGETS: return (size_t)h.nt * S;
-    case OKIN_IO_HARDPOINT_SENSITIVITY: return S * h.hdr[OKIN_H_NSENS] * 3 * h.nout;
+    case OKIN_IO_HARDPOINT_SENSITIVITY: return S * OKIN_HV(h.hdr, OKIN_H_NSENS) * 3 * h.nout;
     case OKIN_IO_TARGET_VALUES: return 0;
     default: return 1;   // status, failed_step, worst_row
   }

@@ -3,8 +3,10 @@
 // include it too.
 #pragma once
 
+#ifndef __CUDACC_RTC__
 #include <math.h>
 #include <stdint.h>
+#endif
 
 #if defined(__CUDACC__)
 #define OKIN_HD __host__ __device__ __forceinline__
