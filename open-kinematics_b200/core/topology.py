@@ -178,13 +178,37 @@ class TopologyProgram:
             # solve task word: FIN | column, with the column's diagonal block offset in the high half
             phases.append([((stask[k] & 0xFFFF) | doffs[stask[k] & 0x7FFF] << 16,
                             scon[stask[k] >> 16:stask[k + 1] >> 16]) for k in range(slev[p], slev[p + 1])])
+        # distance rows: one slot per task, in slot order (every task has two contributions, so the packing
+        # keeps slot s in lane s % 32 of round s // 32, as the generic loop runs it)
+        drow, ndrow = sec("OKIN_S_DROW"), int(h[D["OKIN_H_NDROW"]])
+        phases.append([(drow[s], [drow[ndrow + s], drow[2 * ndrow + s]]) for s in range(ndrow)])
+        # linear-model residuals: task = least-squares row, contributions = its JH_CON words in order
+        jptr, jcon = sec("OKIN_S_JH_PTR"), sec("OKIN_S_JH_CON")
+        phases.append([(t, jcon[jptr[t]:jptr[t + 1]]) for t in range(int(h[D["OKIN_H_NROW"]]))])
+        # derived points, per dependency level: all ops, then the active ones only (okin_derived_update).
+        # task = output point | op << 16, contributions = {a | b << 16, c | param << 16}, missing inputs = a
+        dop = [self.section("OKIN_S_DOP")[k:k + D["OKIN_DOP_STRIDE"]]
+               for k in range(0, len(self.section("OKIN_S_DOP")), D["OKIN_DOP_STRIDE"])]
+        dlev = sec("OKIN_S_DOP_LEV")
+        for active_only in (False, True):
+            for lv in range(len(dlev) - 1):
+                tasks = []
+                for d in range(dlev[lv], dlev[lv + 1]):
+                    op, o, ia, ib, ic, p = (int(v) for v in dop[d][:6])
+                    if active_only and not dop[d][7]:
+                        continue
+                    ib, ic = ia if ib < 0 else ib, ia if ic < 0 else ic
+                    assert max(o, ia, ib, ic, p) < 1 << 16
+                    tasks.append((o | op << 16, [ia | ib << 16, ic | p << 16]))
+                phases.append(tasks)
         return phases
 
     def spec_source(self) -> str:
         """C++ header ``okin_spec.h`` of this program for an OKIN_SPEC build of ``csrc/okin_core.cuh``:
         the header fields as constants, and every hot phase as lane rounds whose task and contribution
         words are packed lane-major into ``okin_spec_words``.  A round takes up to 32 tasks, longest
-        contribution list first, so the lanes holding slot s are always a prefix of the round."""
+        contribution list first (a stable sort: tasks with equal-length lists keep their order), so the
+        lanes holding slot s are always a prefix of the round."""
         words, phase_round, rounds, slot_lanes = [], [], [], []
         for tasks in self.spec_phases():
             phase_round.append(len(rounds))
@@ -215,6 +239,7 @@ class TopologyProgram:
             "OKIN_HD constexpr int r_slots(int r) { return R_SLOTS[r]; }",
             "OKIN_HD constexpr int r_slot0(int r) { return R_SLOT0[r]; }",
             "OKIN_HD constexpr int slot_lanes(int i) { return SLOT_LANES[i]; }",
+            f"constexpr int DOP_NLEV = {len(self.section('OKIN_S_DOP_LEV')) - 1};",
             "}  // namespace okin_spec",
             f"#define OKIN_SPEC_WORDS {max(len(words), 1)}",
             "#ifdef __CUDACC__",

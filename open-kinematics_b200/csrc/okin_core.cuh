@@ -187,7 +187,9 @@ struct OkinProgram {
 #endif
 
 // Phase numbers of the spec: assembly (block tasks, then gradient tasks), per level the factor update,
-// diagonal and scale phases, then the forward and the backward substitution phases.
+// diagonal and scale phases, then the forward and the backward substitution phases; then the distance
+// rows, the linear-model residuals, and per derived-point level the update of all ops and of the active
+// ops (dl < okin_spec::DOP_NLEV).
 #define OKIN_PH_ASM_BLOCK 0
 #define OKIN_PH_ASM_G 1
 #define OKIN_PH_UPD(lv) (2 + 3 * (lv))
@@ -195,6 +197,9 @@ struct OkinProgram {
 #define OKIN_PH_SCL(lv) (4 + 3 * (lv))
 #define OKIN_PH_FW(nlev, lv) (2 + 3 * (nlev) + (lv))
 #define OKIN_PH_BW(nlev, ph) (2 + 4 * (nlev) + (ph))
+#define OKIN_PH_DROW(nlev) (2 + 5 * (nlev))
+#define OKIN_PH_JH(nlev) (3 + 5 * (nlev))
+#define OKIN_PH_DOP(nlev, ndl, active, dl) (4 + 5 * (nlev) + ((active) ? (ndl) : 0) + (dl))
 
 template <int I>
 struct OkinConst {
@@ -315,11 +320,37 @@ OKIN_HD void okin_dop_eval(int op, double par, const double* a, const double* b,
 template <typename Dummy = void>
 OKIN_FN void okin_derived_update(const OkinProgram& pr, double* sm, bool active_only) {
   sm = OKIN_SHARED(sm);
+  double* pos = sm + OKIN_HV(pr.hdr, OKIN_H_OFF_POS);
+  const double* par = sm + OKIN_HV(pr.hdr, OKIN_H_OFF_PAR);
+  // one op: point o from the inputs a, b, c (a missing input is a) and parameter p
+  auto op_eval = [&](int op, int o, int ia, int ib, int ic, int p) {
+    const double z[3] = {0.0, 0.0, 0.0};
+    double out[3], dout[3];
+    okin_dop_eval(op, par[p], pos + 3 * ia, pos + 3 * ib, pos + 3 * ic, z, z, z, out, dout);
+    pos[3 * o] = out[0]; pos[3 * o + 1] = out[1]; pos[3 * o + 2] = out[2];
+  };
+#ifdef OKIN_SPEC
+  // task word = o | op << 16, contributions = {a | b << 16, c | p << 16}
+  auto level = [&](auto dl, auto active) {
+    OKIN_PHASE_BEGIN
+    okin_spec_phase<OKIN_PH_DOP(okin_spec_hdr(OKIN_H_NLEV), okin_spec::DOP_NLEV, decltype(active)::value,
+                                decltype(dl)::value)>(pr, lane, [&](uint32_t t, auto&& each) {
+      uint32_t w[2];
+      int k = 0;
+      each([&](uint32_t c) { w[k++] = c; });
+      op_eval((int)(t >> 16), (int)(t & 0xffffu), (int)(w[0] & 0xffffu), (int)(w[0] >> 16), (int)(w[1] & 0xffffu),
+              (int)(w[1] >> 16));
+    });
+    OKIN_PHASE_END
+  };
+  if (active_only)
+    okin_static_for<0, okin_spec::DOP_NLEV>([&](auto dl) { level(dl, OkinConst<1>{}); });
+  else
+    okin_static_for<0, okin_spec::DOP_NLEV>([&](auto dl) { level(dl, OkinConst<0>{}); });
+#else
   const int32_t* dop = OKIN_SHARED(okin_sec(pr, OKIN_S_DOP));
   const int32_t* lev = OKIN_SHARED(okin_sec(pr, OKIN_S_DOP_LEV));
   const int nlev = okin_sec_len(pr, OKIN_S_DOP_LEV) - 1;
-  double* pos = sm + OKIN_HV(pr.hdr, OKIN_H_OFF_POS);
-  const double* par = sm + OKIN_HV(pr.hdr, OKIN_H_OFF_PAR);
   for (int lv = 0; lv < nlev; ++lv) {
     const int b = OKIN_LDG(lev + lv), e = OKIN_LDG(lev + lv + 1);
     OKIN_PHASE_BEGIN
@@ -327,16 +358,12 @@ OKIN_FN void okin_derived_update(const OkinProgram& pr, double* sm, bool active_
     for (int d = b + lane; d < e; d += 32) {
       const int32_t* rec = dop + d * OKIN_DOP_STRIDE;
       if (active_only && !OKIN_LDG(rec + 7)) continue;
-      const double z[3] = {0.0, 0.0, 0.0};
       const int ia = OKIN_LDG(rec + 2), ib = OKIN_LDG(rec + 3), ic = OKIN_LDG(rec + 4);
-      double out[3], dout[3];
-      okin_dop_eval(OKIN_LDG(rec + 0), par[OKIN_LDG(rec + 5)], pos + 3 * ia, pos + 3 * (ib < 0 ? ia : ib),
-                    pos + 3 * (ic < 0 ? ia : ic), z, z, z, out, dout);
-      const int o = OKIN_LDG(rec + 1);
-      pos[3 * o] = out[0]; pos[3 * o + 1] = out[1]; pos[3 * o + 2] = out[2];
+      op_eval(OKIN_LDG(rec + 0), OKIN_LDG(rec + 1), ia, ib < 0 ? ia : ib, ic < 0 ? ia : ic, OKIN_LDG(rec + 5));
     }
     OKIN_PHASE_END
   }
+#endif
 }
 
 // Jacobian blocks d(derived)/d(free base point) by seeding one coordinate per task and
@@ -668,23 +695,36 @@ OKIN_FN void okin_eval_rows(const OkinProgram& pr, double* sm, const double* tva
   OKIN_PHASE_BEGIN
   double sq = 0.0;
   // Fast path: plain distance rows (most of every shipped topology).  r = sqrt(s + eps^2) - eps - L,
-  // u = (p2 - p1)/sqrt(s + eps^2) is the whole gradient (dR/dp2 = u, dR/dp1 = -u).
-  OKIN_LANE_LOOP
-  for (int slot = lane; slot < ndrow; slot += 32) {
-    const uint32_t pp = (uint32_t)OKIN_LDG(drow + slot), oo = (uint32_t)OKIN_LDG(drow + ndrow + slot);
+  // u = (p2 - p1)/sqrt(s + eps^2) is the whole gradient (dR/dp2 = u, dR/dp1 = -u).  Slot s runs in lane
+  // s % 32 in both builds, so the per-lane sum of squares adds the same rows in the same order.
+  auto dist = [&](uint32_t pp, uint32_t oo, int row) {
     const double* a = pos + 3 * (pp & 0xffffu);
     const double* b = pos + 3 * (pp >> 16);
     const double dx = b[0] - a[0], dy = b[1] - a[1], dz = b[2] - a[2];
-    const double s2 = dx * dx + dy * dy + dz * dz + OKIN_EPS_SQ;
+    // explicit fma, in the order ptxas contracted the generic build's dx*dx+dy*dy+dz*dz, s2*inv-eps, sq+res*res
+    const double s2 = fma(dz, dz, fma(dx, dx, dy * dy)) + OKIN_EPS_SQ;
     const double inv = OKIN_RSQRT(s2);
-    const double res = s2 * inv - OKIN_EPS - cst[oo & 0xffffu];
-    r[OKIN_LDG(drow + 2 * ndrow + slot)] = res;
-    sq += res * res;
+    const double res = fma(s2, inv, -OKIN_EPS) - cst[oo & 0xffffu];
+    r[row] = res;
+    sq = fma(res, res, sq);
     if (with_grad) {
       double* u = rg + (oo >> 16);
       u[0] = dx * inv; u[1] = dy * inv; u[2] = dz * inv;
     }
-  }
+  };
+#ifdef OKIN_SPEC
+  // task word = {p0 | p1 << 16}, contributions = {cst_off | rg_off << 16}, {row}
+  okin_spec_phase<OKIN_PH_DROW(okin_spec_hdr(OKIN_H_NLEV))>(pr, lane, [&](uint32_t pp, auto&& each) {
+    uint32_t w[2];
+    int k = 0;
+    each([&](uint32_t c) { w[k++] = c; });
+    dist(pp, w[0], (int)w[1]);
+  });
+#else
+  OKIN_LANE_LOOP
+  for (int slot = lane; slot < ndrow; slot += 32)
+    dist((uint32_t)OKIN_LDG(drow + slot), (uint32_t)OKIN_LDG(drow + ndrow + slot), OKIN_LDG(drow + 2 * ndrow + slot));
+#endif
   OKIN_LANE_LOOP
   for (int slot = lane; slot < ngrow; slot += 32) {
     const int32_t* rec = rows + slot * OKIN_ROW_STRIDE;
@@ -1198,20 +1238,30 @@ OKIN_FN void okin_linear_residuals(const OkinProgram& pr, double* sm, OkinState&
   double* r = sm + OKIN_HV(hdr, OKIN_H_OFF_R);
   double* red = sm + OKIN_HV(hdr, OKIN_H_OFF_RED);
   double sq = 0.0, mx = 0.0;
-  OKIN_PHASE_BEGIN
-  OKIN_LANE_LOOP
-  for (int t = lane; t < nls; t += 32) {
+  // one least-squares row (task word = row t): its (gradient, step) contributions in order
+  auto row = [&](uint32_t t, auto&& each) {
     double acc = r[t];
-    for (int q = OKIN_LDG(jptr + t), e = OKIN_LDG(jptr + t + 1); q < e; ++q) {
-      const uint32_t w = (uint32_t)OKIN_LDG(jcon + q);
+    each([&](uint32_t w) {
       const double* g = rg + ((w >> 16) & 0x7fffu);
       const double* x = h + (w & 0xffffu);
       const double g0 = g[0], g1 = g[1], g2 = g[2], x0 = x[0], x1 = x[1], x2 = x[2];
       const double dot = fma(g0, x0, fma(g1, x1, g2 * x2));
       acc += (w & OKIN_CON_NEG) ? -dot : dot;
-    }
+    });
     r[t] = acc;
+  };
+  OKIN_PHASE_BEGIN
+#ifdef OKIN_SPEC
+  okin_spec_phase<OKIN_PH_JH(okin_spec_hdr(OKIN_H_NLEV))>(pr, lane, row);
+#else
+  OKIN_LANE_LOOP
+  for (int t = lane; t < nls; t += 32) {
+    const int b = OKIN_LDG(jptr + t), e = OKIN_LDG(jptr + t + 1);
+    row((uint32_t)t, [&](auto&& g) {
+      for (int q = b; q < e; ++q) g((uint32_t)OKIN_LDG(jcon + q));
+    });
   }
+#endif
   OKIN_PHASE_END
   OKIN_PHASE_BEGIN
   double lsq = 0.0, lmx = 0.0;
