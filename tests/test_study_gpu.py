@@ -47,16 +47,31 @@ def check_study(solver, smp, n, seed, want_metrics, **kw):
     return res
 
 
-def test_study_c1_lean():
+def c1_lean_study(solver) -> tuple:
+    """``(sampling, n_instances, seed, study keywords)`` of the lean C1 study: every output coordinate and
+    the function evaluations, histogrammed, over two full chunks and a partial one."""
     from open_kinematics_b200.core.study import Sampling
+    smp = Sampling(solver).normal("all", 0.5)
+    names = [f"{k.name.lower()}_{a}" for k in solver.program.out_keys for a in "xyz"] + ["solver_nfev"]
+    hist = {n: (-1e3, 1e3) for n in names}
+    hist["solver_nfev"] = (0.0, 12.0)
+    return smp, 2 * CHUNK + 4321, 11, dict(points="all", solver_quantities=("solver_nfev",), histograms=hist, bins=24)
+
+
+def tbar_shim_study(solver) -> tuple:
+    """The same for the C4 shimmed T-bar study: uniform setup thicknesses, one full chunk and a partial one."""
+    from open_kinematics_b200.core.study import Sampling
+    prog = solver.program
+    smp = Sampling(solver, mirror_right=True).normal("all", 0.25)
+    smp.uniform([n for n in prog.param_names if n.endswith("setup_thickness")], 0.5)
+    return smp, CHUNK + 999, 5, dict(points=prog.out_keys[:6], solver_quantities=("solver_nfev",))
+
+
+def test_study_c1_lean():
     solver = solver_of("c1_dw_corner_bump")
     try:
-        smp = Sampling(solver).normal("all", 0.5)
-        names = [f"{k.name.lower()}_{a}" for k in solver.program.out_keys for a in "xyz"] + ["solver_nfev"]
-        hist = {n: (-1e3, 1e3) for n in names}
-        hist["solver_nfev"] = (0.0, 12.0)
-        res = check_study(solver, smp, 2 * CHUNK + 4321, 11, False, points="all", solver_quantities=("solver_nfev",),
-                          histograms=hist, bins=24)
+        smp, n, seed, kw = c1_lean_study(solver)
+        res = check_study(solver, smp, n, seed, False, **kw)
         assert res.status_counts.sum() == 2 * CHUNK + 4321
     finally:
         solver.close()
@@ -75,13 +90,10 @@ def test_study_flagship_full():
 
 
 def test_study_tbar_uniform_shims():
-    from open_kinematics_b200.core.study import Sampling
     solver = solver_of("c4_tbar_heave_shim_bump")
     try:
-        prog = solver.program
-        smp = Sampling(solver, mirror_right=True).normal("all", 0.25)
-        smp.uniform([n for n in prog.param_names if n.endswith("setup_thickness")], 0.5)
-        check_study(solver, smp, CHUNK + 999, 5, False, points=prog.out_keys[:6], solver_quantities=("solver_nfev",))
+        smp, n, seed, kw = tbar_shim_study(solver)
+        check_study(solver, smp, n, seed, False, **kw)
     finally:
         solver.close()
 
