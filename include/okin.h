@@ -233,6 +233,25 @@ int okin_fp64_peak(int32_t device, double* tflops_out);
  *     normal: z = sqrt(-2 log(1 - u)) * cospi(2 u');  uniform: z = 2u - 1 in [-1, 1)
  *   grid (full factorial): node = i mod prod(L_g) over the grid variates, the first grid variate
  *     varying fastest; d_g = mixed-radix digit g of node; z = d_g / (L_g - 1) * 2.0 - 1.0
+ *   sobol uniform / sobol normal: scrambled Sobol' sequence, 52-bit integers X, bit 51 = the 2^-1
+ *     digit.  The Sobol' variates take dimensions d = 0, 1, ... in variate order (counting Sobol'
+ *     variates only).  Point index j = i / prod(L_g) over the grid variates (j = i without grid
+ *     variates), so every grid node sees the same Sobol' sample (a crossed design).
+ *     Unscrambled: direction numbers V[d][0..52) of Joe-Kuo new-joe-kuo-6.21201 (SciPy's table):
+ *     poly_d of degree m (bit length - 1), m_k = vinit[d][k] for k < m and, for k >= m,
+ *     m_k = m_{k-m} ^ XOR_{l=1..m, bit (m-l) of poly_d set} 2^l m_{k-l};  m_k = 1 for all k when d = 0;
+ *     V[d][k] = m_k << (51 - k).  Point j: X = XOR of V[d][k] over the set bits k of j ^ (j >> 1)
+ *     (SciPy's order: qmc.Sobol(D, scramble=False, bits=52) gives X * 2^-52).
+ *     Scramble (linear matrix scramble + digital shift, per Sobol' variate v, always on): with
+ *     W(a) = ((x1 << 32 | x0) >> 12) of Philox4x32-10 under the key above at counter (a, 0, v, 1),
+ *     row k < 52 of a lower-triangular GF(2) matrix M_v with unit diagonal is
+ *     R_k = (W(k) & ~(2^(51-k) - 1)) | 2^(51-k) (digit k, bit 51 - k, of M x is the parity of
+ *     R_k & x), and the shift is S_v = W(52).  Scrambled X = S_v ^ XOR over the same bits k of
+ *     M_v V[d][k].  Instance draws use counter word 3 = 0, so the two counter spaces never meet.
+ *     sobol uniform: z = X * 2^-51 - 1 (exact, in [-1, 1));
+ *     sobol normal: z = PPND16((2X + 1) * 2^-53), Wichura's AS241 inverse normal CDF in fp64.
+ *     Limits (usage errors): at most OKIN_SOBOL_MAX_VARIATES Sobol' variates, no saturated grid
+ *     period (prod(L_g) >= 2^63), j < 2^52.  Estimates are best at N = 2^m instances (per grid node).
  * Coordinate c (3 * input slot + axis, then the params, n_coords = 3 * n_in_points + n_params) takes
  *   value_c = nominal_c + scale_c * z_{source_c}   (nominal_c when source_c = -1).
  * Reduction: a quantity's value at (instance, step) counts iff the step was accepted (status OK or
@@ -248,6 +267,10 @@ int okin_fp64_peak(int32_t device, double* tflops_out);
 #define OKIN_VARIATE_NORMAL 0
 #define OKIN_VARIATE_UNIFORM 1
 #define OKIN_VARIATE_GRID 2
+#define OKIN_VARIATE_SOBOL_UNIFORM 3
+#define OKIN_VARIATE_SOBOL_NORMAL 4
+#define OKIN_SOBOL_MAX_VARIATES 1024
+#define OKIN_SOBOL_BITS 52
 
 #define OKIN_QUANTITY_POSITION 0      /* index = 3 * output slot + axis (positions_out column) */
 #define OKIN_QUANTITY_METRIC 1        /* index = metric column */

@@ -16,7 +16,8 @@ import numpy as np
 
 from .primitives.point_ref import PointRef, Side
 
-VARIATE_NORMAL, VARIATE_UNIFORM, VARIATE_GRID = 0, 1, 2
+VARIATE_NORMAL, VARIATE_UNIFORM, VARIATE_GRID, VARIATE_SOBOL_UNIFORM, VARIATE_SOBOL_NORMAL = 0, 1, 2, 3, 4
+SEQUENCES = ("philox", "sobol")
 QUANTITY_POSITION, QUANTITY_METRIC, QUANTITY_MAX_RESIDUAL, QUANTITY_NFEV = 0, 1, 2, 3
 SOLVER_QUANTITIES = ("solver_max_residual", "solver_nfev")
 AXES = "xyz"
@@ -37,7 +38,14 @@ class Sampling:
     param name, ``"all"``, or a list of these.  ``"all"`` is every hardpoint coordinate except
     centre-line y coordinates whose nominal is 0 (the T-bar pivot build validation needs them there).
     With ``mirror_right`` every right-side point with a left twin follows that twin: it shares the
-    twin's variate with the y scale negated, and cannot be assigned itself."""
+    twin's variate with the y scale negated, and cannot be assigned itself.
+
+    ``normal`` and ``uniform`` draw Philox pseudo-random variates by default; ``sequence="sobol"``
+    draws them from a scrambled Sobol' sequence instead (one Sobol' dimension per variate, in the
+    order assigned), whose mean and std estimates converge close to ``N^-1`` for smooth responses
+    rather than ``N^-1/2``.  They are best at ``N = 2^m`` instances.  The kinds mix freely; with grid
+    factors every grid node sees the same Sobol' sample (instance ``i`` takes Sobol' point
+    ``i // prod(levels)``), a crossed design."""
 
     def __init__(self, solver, mirror_right: bool = False):
         prog = solver.program
@@ -112,13 +120,21 @@ class Sampling:
                 self.source[r], self.scale[r] = v, -float(w) if c % 3 == 1 else float(w)
         return self
 
-    def normal(self, coords, sigma) -> "Sampling":
-        """Independent normal variation with standard deviation ``sigma`` (scalar or one per coordinate)."""
-        return self._assign(coords, VARIATE_NORMAL, sigma)
+    @staticmethod
+    def _kind(sequence: str, philox: int, sobol: int) -> int:
+        if sequence not in SEQUENCES:
+            raise ValueError(f"Unknown sequence {sequence!r}; expected one of {SEQUENCES}")
+        return sobol if sequence == "sobol" else philox
 
-    def uniform(self, coords, half_width) -> "Sampling":
-        """Independent uniform variation on ``[nominal - half_width, nominal + half_width)``."""
-        return self._assign(coords, VARIATE_UNIFORM, half_width)
+    def normal(self, coords, sigma, sequence: str = "philox") -> "Sampling":
+        """Independent normal variation with standard deviation ``sigma`` (scalar or one per coordinate),
+        drawn from ``sequence`` (``"philox"`` or ``"sobol"``)."""
+        return self._assign(coords, self._kind(sequence, VARIATE_NORMAL, VARIATE_SOBOL_NORMAL), sigma)
+
+    def uniform(self, coords, half_width, sequence: str = "philox") -> "Sampling":
+        """Independent uniform variation on ``[nominal - half_width, nominal + half_width)``, drawn
+        from ``sequence`` (``"philox"`` or ``"sobol"``)."""
+        return self._assign(coords, self._kind(sequence, VARIATE_UNIFORM, VARIATE_SOBOL_UNIFORM), half_width)
 
     def grid(self, coords, half_range, levels: int) -> "Sampling":
         """Full-factorial factors: ``levels`` equally spaced values on ``nominal +- half_range``.

@@ -798,9 +798,8 @@ void run_shard(okin_topology* t, const okin_solver_cfg* cfg, const HostBatch& hb
 }
 
 // ---- tolerance studies ------------------------------------------------------------------------
-// Generator part of a study descriptor; fills the mixed-radix place values of the grid variates.
-int study_check_generator(const okin_topology* t, const okin_study_desc* desc, std::vector<uint64_t>* stride,
-                          uint64_t* period) {
+// Generator part of a study descriptor, checked and turned into the host generator tables.
+int study_check_generator(const okin_topology* t, const okin_study_desc* desc, OkinStudyHostTables* g) {
   if (!t || !desc) return fail(OKIN_ERR_USAGE, "null topology or study descriptor");
   const int32_t* h = t->hdr.data();
   const int nc = 3 * h[OKIN_H_NIN] + h[OKIN_H_NPARAM], nv = desc->n_variates;
@@ -810,17 +809,28 @@ int study_check_generator(const okin_topology* t, const okin_study_desc* desc, s
     return fail(OKIN_ERR_USAGE, "null study generator table");
   for (int v = 0; v < nv; ++v) {
     const int kind = desc->variate_kind[v];
-    if (kind < OKIN_VARIATE_NORMAL || kind > OKIN_VARIATE_GRID) return fail(OKIN_ERR_USAGE, "unknown variate kind");
+    if (kind < OKIN_VARIATE_NORMAL || kind > OKIN_VARIATE_SOBOL_NORMAL) return fail(OKIN_ERR_USAGE, "unknown variate kind");
     if (kind == OKIN_VARIATE_GRID && desc->grid_levels[v] < 2)
       return fail(OKIN_ERR_USAGE, "a grid variate needs at least 2 levels");
   }
-  stride->assign(nv + 1, 0);
-  okin_study_grid_places(nv, desc->variate_kind, desc->grid_levels, stride->data(), period);
+  g->index(nv, desc->variate_kind, desc->grid_levels);
+  if (g->n_sobol > OKIN_SOBOL_MAX_VARIATES)
+    return fail(OKIN_ERR_USAGE, "a study takes at most 1024 Sobol' variates");
+  if (g->n_sobol > 0 && g->period == 0)
+    return fail(OKIN_ERR_USAGE, "Sobol' variates need a grid period below 2^63 (the product of the grid levels)");
   for (int c = 0; c < nc; ++c) {
     if (desc->source[c] < -1 || desc->source[c] >= nv) return fail(OKIN_ERR_USAGE, "study source out of range");
     if (!std::isfinite(desc->nominal[c]) || !std::isfinite(desc->scale[c]))
       return fail(OKIN_ERR_USAGE, "non-finite study nominal or scale");
   }
+  g->scramble(desc->seed, nv);
+  return OKIN_OK;
+}
+
+// Sobol' point indices (instance id / grid period) must stay below 2^52.
+int study_check_point_index(const OkinStudyHostTables& g, uint64_t max_id) {
+  if (g.n_sobol > 0 && max_id / g.period >= (UINT64_C(1) << OKIN_SOBOL_BITS))
+    return fail(OKIN_ERR_USAGE, "Sobol' point index (instance id / grid period) must be below 2^52");
   return OKIN_OK;
 }
 
@@ -879,27 +889,34 @@ struct DeviceAllocs {
 };
 
 // The generator tables of `desc` on the current device.
-int upload_study_tables(const okin_study_desc* desc, const std::vector<uint64_t>& stride, uint64_t period,
-                        DeviceAllocs& a, OkinStudyTables* t) {
+int upload_study_tables(const okin_study_desc* desc, const OkinStudyHostTables& g, DeviceAllocs& a, OkinStudyTables* t) {
   const int nc = desc->n_coords, nv = desc->n_variates;
   double *nominal, *scale;
-  int32_t *source, *kind, *levels;
-  uint64_t* st;
+  int32_t *source, *kind, *levels, *rank;
+  uint64_t *st, *dirs, *shift;
   OKIN_CUDA(a.alloc(&nominal, nc));
   OKIN_CUDA(a.alloc(&scale, nc));
   OKIN_CUDA(a.alloc(&source, nc));
   OKIN_CUDA(a.alloc(&kind, nv));
   OKIN_CUDA(a.alloc(&levels, nv));
   OKIN_CUDA(a.alloc(&st, nv));
+  OKIN_CUDA(a.alloc(&rank, nv));
+  OKIN_CUDA(a.alloc(&dirs, g.sobol_dirs.size()));
+  OKIN_CUDA(a.alloc(&shift, g.sobol_shift.size()));
   OKIN_CUDA(cudaMemcpy(nominal, desc->nominal, nc * sizeof(double), cudaMemcpyHostToDevice));
   OKIN_CUDA(cudaMemcpy(scale, desc->scale, nc * sizeof(double), cudaMemcpyHostToDevice));
   OKIN_CUDA(cudaMemcpy(source, desc->source, nc * sizeof(int32_t), cudaMemcpyHostToDevice));
   if (nv > 0) {
     OKIN_CUDA(cudaMemcpy(kind, desc->variate_kind, nv * sizeof(int32_t), cudaMemcpyHostToDevice));
     OKIN_CUDA(cudaMemcpy(levels, desc->grid_levels, nv * sizeof(int32_t), cudaMemcpyHostToDevice));
-    OKIN_CUDA(cudaMemcpy(st, stride.data(), nv * sizeof(uint64_t), cudaMemcpyHostToDevice));
+    OKIN_CUDA(cudaMemcpy(st, g.stride.data(), nv * sizeof(uint64_t), cudaMemcpyHostToDevice));
+    OKIN_CUDA(cudaMemcpy(rank, g.sobol_rank.data(), nv * sizeof(int32_t), cudaMemcpyHostToDevice));
   }
-  *t = OkinStudyTables{desc->seed, period, nc, nominal, scale, source, kind, levels, st};
+  if (g.n_sobol > 0) {
+    OKIN_CUDA(cudaMemcpy(dirs, g.sobol_dirs.data(), g.sobol_dirs.size() * sizeof(uint64_t), cudaMemcpyHostToDevice));
+    OKIN_CUDA(cudaMemcpy(shift, g.sobol_shift.data(), g.sobol_shift.size() * sizeof(uint64_t), cudaMemcpyHostToDevice));
+  }
+  *t = OkinStudyTables{desc->seed, g.period, nc, nominal, scale, source, kind, levels, st, rank, dirs, shift};
   return OKIN_OK;
 }
 
@@ -923,8 +940,7 @@ struct StudyRun {
   int32_t S;
   const double* target_values;
   const okin_study_desc* desc;
-  std::vector<uint64_t> stride;
-  uint64_t period = 0;
+  OkinStudyHostTables gen;
   int Q = 0, SQ = 0, nb = 0, n_devices = 0, slots = 0;
   bool want_pos = false, want_met = false;
   int64_t n_chunks = 0, window = 0;
@@ -981,7 +997,7 @@ int run_study_shard_body(StudyRun& run, StudyShard& sh, DeviceAllocs& a) {
   const int64_t n_mine = run.n_chunks > sh.index ? (run.n_chunks - sh.index + G - 1) / G : 0;
   const int slots = (int)std::min<int64_t>(run.slots, n_mine);
   OkinStudyTables tab;
-  int rc = upload_study_tables(run.desc, run.stride, run.period, a, &tab);
+  int rc = upload_study_tables(run.desc, run.gen, a, &tab);
   if (rc) return rc;
   int32_t *qkind, *qindex;
   double *lo = nullptr, *hi = nullptr, *tv = nullptr;
@@ -1298,10 +1314,11 @@ int okin_study(okin_topology* t, const okin_solver_cfg* cfg, int64_t n_instances
                const double* target_values, const okin_study_desc* desc, okin_study_out* out,
                const int32_t* device_ids, int32_t n_devices) {
   StudyRun run;
-  int rc = study_check_generator(t, desc, &run.stride, &run.period);
+  int rc = study_check_generator(t, desc, &run.gen);
   if (rc) return rc;
   if (!cfg) return fail(OKIN_ERR_USAGE, "null solver config");
   if (n_instances < 0 || n_steps < 0) return fail(OKIN_ERR_USAGE, "negative size");
+  if (n_instances > 0 && (rc = study_check_point_index(run.gen, (uint64_t)(n_instances - 1)))) return rc;
   if (n_steps == 0) return fail(OKIN_ERR_USAGE, "a study needs at least one sweep step");
   if (t->hdr[OKIN_H_NT] > 0 && !target_values) return fail(OKIN_ERR_USAGE, "null target_values");
   if ((rc = check_cfg(cfg))) return rc;
@@ -1349,23 +1366,24 @@ int okin_study(okin_topology* t, const okin_solver_cfg* cfg, int64_t n_instances
 
 int okin_study_sample(okin_topology* t, const okin_study_desc* desc, int64_t n_ids, const int64_t* instance_ids,
                       double* hardpoints_out, double* params_out, int32_t device) {
-  std::vector<uint64_t> stride;
-  uint64_t period = 0;
-  int rc = study_check_generator(t, desc, &stride, &period);
+  OkinStudyHostTables gen;
+  int rc = study_check_generator(t, desc, &gen);
   if (rc) return rc;
   const int nin3 = 3 * t->hdr[OKIN_H_NIN], npar = t->hdr[OKIN_H_NPARAM];
   if (n_ids < 0) return fail(OKIN_ERR_USAGE, "negative n_ids");
   if (n_ids > 0 && (!instance_ids || !hardpoints_out || (npar > 0 && !params_out)))
     return fail(OKIN_ERR_USAGE, "null study sample buffer");
-  for (int64_t r = 0; r < n_ids; ++r)
+  for (int64_t r = 0; r < n_ids; ++r) {
     if (instance_ids[r] < 0) return fail(OKIN_ERR_USAGE, "negative instance id");
+    if ((rc = study_check_point_index(gen, (uint64_t)instance_ids[r]))) return rc;
+  }
   if (n_ids == 0) return OKIN_OK;
   DeviceCopy* d = nullptr;
   if ((rc = ensure_device(t, device, &d))) return rc;
   OKIN_CUDA(cudaSetDevice(device));
   DeviceAllocs a;
   OkinStudyTables tab;
-  if ((rc = upload_study_tables(desc, stride, period, a, &tab))) return rc;
+  if ((rc = upload_study_tables(desc, gen, a, &tab))) return rc;
   long long* ids;
   double *hp, *par = nullptr;
   OKIN_CUDA(a.alloc(&ids, n_ids));

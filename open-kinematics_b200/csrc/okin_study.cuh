@@ -6,7 +6,10 @@
 #include <math.h>
 #include <stdint.h>
 
+#include <vector>
+
 #include "../../include/okin.h"
+#include "okin_sobol.h"
 
 #if defined(__CUDACC__)
 #define OKIN_STUDY_HD __host__ __device__
@@ -65,6 +68,9 @@ OKIN_STUDY_HD inline double okin_study_axpy(double scale, double z, double nomin
 
 // Generator tables (device or host addresses).  stride[v] / period: mixed-radix place value of grid
 // variate v and the product of all grid levels; 0 = beyond 2^63 (that digit is 0, no wrap).
+// sobol_rank[v]: Sobol' dimension of variate v (-1 for the other kinds); sobol_dirs[d][k] and
+// sobol_shift[d]: the scrambled direction numbers and the digital shift of dimension d.  The device
+// reads these three; the host (the lane emulation) derives the same integers from the seed.
 struct OkinStudyTables {
   uint64_t seed, period;
   int32_t n_coords;
@@ -74,7 +80,116 @@ struct OkinStudyTables {
   const int32_t* kind;
   const int32_t* levels;
   const uint64_t* stride;
+  const int32_t* sobol_rank;
+  const uint64_t* sobol_dirs;
+  const uint64_t* sobol_shift;
 };
+
+// Host: V[d][0..52) of the unscrambled Sobol' sequence (include/okin.h), d < OKIN_SOBOL_DIMS.
+inline void okin_sobol_directions(int d, uint64_t V[OKIN_SOBOL_BITS]) {
+  uint64_t m[OKIN_SOBOL_BITS];
+  const uint32_t poly = okin_sobol_poly[d];
+  int deg = 0;
+  while (poly >> (deg + 1)) ++deg;
+  for (int k = 0; k < OKIN_SOBOL_BITS; ++k) {
+    if (d == 0) {
+      m[k] = 1;
+    } else if (k < deg) {
+      m[k] = okin_sobol_vinit[d][k];
+    } else {
+      uint64_t x = m[k - deg];
+      for (int l = 1; l <= deg; ++l)
+        if ((poly >> (deg - l)) & 1u) x ^= m[k - l] << l;
+      m[k] = x;
+    }
+  }
+  for (int k = 0; k < OKIN_SOBOL_BITS; ++k) V[k] = m[k] << (OKIN_SOBOL_BITS - 1 - k);
+}
+
+// Host: 52-bit word W(a) of Sobol' variate v's scramble stream (counter (a, 0, v, 1)).
+inline uint64_t okin_sobol_scramble_word(uint64_t seed, int v, uint32_t a) {
+  uint32_t c[4] = {a, 0u, (uint32_t)v, 1u};
+  okin_philox4x32_10(c, (uint32_t)seed, (uint32_t)(seed >> 32));
+  return (((uint64_t)c[1] << 32) | c[0]) >> (64 - OKIN_SOBOL_BITS);
+}
+
+// Host: rows R_k of the scramble matrix M_v of Sobol' variate v, lower triangular in digit order
+// (digit k = bit 51 - k) with unit diagonal.
+inline void okin_sobol_matrix(uint64_t seed, int v, uint64_t row[OKIN_SOBOL_BITS]) {
+  for (int k = 0; k < OKIN_SOBOL_BITS; ++k) {
+    const uint64_t diag = UINT64_C(1) << (OKIN_SOBOL_BITS - 1 - k);
+    row[k] = (okin_sobol_scramble_word(seed, v, (uint32_t)k) & ~(diag - 1)) | diag;
+  }
+}
+
+// Host: M x; digit k of the result is the parity of R_k & x.
+inline uint64_t okin_sobol_apply(const uint64_t row[OKIN_SOBOL_BITS], uint64_t x) {
+  uint64_t y = 0;
+  for (int k = 0; k < OKIN_SOBOL_BITS; ++k)
+    y |= (uint64_t)(__builtin_popcountll(row[k] & x) & 1) << (OKIN_SOBOL_BITS - 1 - k);
+  return y;
+}
+
+// x XOR dir[k] over the set bits k of g.
+OKIN_STUDY_HD inline uint64_t okin_sobol_gray_xor(const uint64_t* dir, uint64_t g, uint64_t x) {
+  for (; g; g &= g - 1) {
+#if defined(__CUDA_ARCH__)
+    x ^= dir[__ffsll((long long)g) - 1];
+#else
+    x ^= dir[__builtin_ctzll(g)];
+#endif
+  }
+  return x;
+}
+
+// Wichura, Algorithm AS 241 (PPND16): the standard normal quantile of p in (0, 1), relative error
+// about 1e-16.  The polynomials are evaluated with explicit fma so host and device round alike.
+OKIN_STUDY_HD inline double okin_ppnd16(double p) {
+  const double q = p - 0.5;
+  if (fabs(q) <= 0.425) {
+    const double r = fma(-q, q, 0.180625);
+    const double num =
+        fma(fma(fma(fma(fma(fma(fma(2.5090809287301226727e+3, r, 3.3430575583588128105e+4), r,
+                                    6.7265770927008700853e+4), r, 4.5921953931549871457e+4), r,
+                        1.3731693765509461125e+4), r, 1.9715909503065514427e+3), r, 1.3314166789178437745e+2), r,
+            3.3871328727963666080e+0);
+    const double den =
+        fma(fma(fma(fma(fma(fma(fma(5.2264952788528545610e+3, r, 2.8729085735721942674e+4), r,
+                                    3.9307895800092710610e+4), r, 2.1213794301586595867e+4), r,
+                        5.3941960214247511077e+3), r, 6.8718700749205790830e+2), r, 4.2313330701600911252e+1), r,
+            1.0);
+    return q * num / den;
+  }
+  double r = sqrt(-log(q < 0.0 ? p : 1.0 - p)), z;
+  if (r <= 5.0) {
+    r -= 1.6;
+    const double num =
+        fma(fma(fma(fma(fma(fma(fma(7.74545014278341407640e-4, r, 2.27238449892691845833e-2), r,
+                                    2.41780725177450611770e-1), r, 1.27045825245236838258e+0), r,
+                        3.64784832476320460504e+0), r, 5.76949722146069140550e+0), r, 4.63033784615654529590e+0), r,
+            1.42343711074968357734e+0);
+    const double den =
+        fma(fma(fma(fma(fma(fma(fma(1.05075007164441684324e-9, r, 5.47593808499534494600e-4), r,
+                                    1.51986665636164571966e-2), r, 1.48103976427480074590e-1), r,
+                        6.89767334985100004550e-1), r, 1.67638483018380384940e+0), r, 2.05319162663775882187e+0), r,
+            1.0);
+    z = num / den;
+  } else {
+    r -= 5.0;
+    const double num =
+        fma(fma(fma(fma(fma(fma(fma(2.01033439929228813265e-7, r, 2.71155556874348757815e-5), r,
+                                    1.24266094738807843860e-3), r, 2.65321895265761230930e-2), r,
+                        2.96560571828504891230e-1), r, 1.78482653991729133580e+0), r, 5.46378491116411436990e+0), r,
+            6.65790464350110377720e+0);
+    const double den =
+        fma(fma(fma(fma(fma(fma(fma(2.04426310338993978564e-15, r, 1.42151175831644588870e-7), r,
+                                    1.84631831751005468180e-5), r, 7.86869131145613259100e-4), r,
+                        1.48753612908506148525e-2), r, 1.36929880922735805310e-1), r, 5.99832206555887937690e-1), r,
+            1.0);
+    z = num / den;
+  }
+  return q < 0.0 ? -z : z;
+}
 
 // Host: the place values and period above for validated variates (grid levels >= 2).
 inline void okin_study_grid_places(int n_variates, const int32_t* kind, const int32_t* levels, uint64_t* stride,
@@ -91,12 +206,68 @@ inline void okin_study_grid_places(int n_variates, const int32_t* kind, const in
   *period = saturated ? 0 : place;
 }
 
+// Host: the generator tables of validated variates that okin_study builds once per call and uploads:
+// grid place values and period, Sobol' ranks, and the scrambled direction numbers
+// dirs[rank][0..52) = M_v V[rank][k] and shifts shift[rank] = S_v of every Sobol' variate v.
+struct OkinStudyHostTables {
+  std::vector<uint64_t> stride, sobol_dirs, sobol_shift;
+  std::vector<int32_t> sobol_rank;
+  uint64_t period = 0;
+  int n_sobol = 0;
+
+  // Place values, period and ranks (cheap; the caller checks n_sobol before scramble()).
+  void index(int n_variates, const int32_t* kind, const int32_t* levels) {
+    stride.assign(n_variates + 1, 0);
+    okin_study_grid_places(n_variates, kind, levels, stride.data(), &period);
+    sobol_rank.assign(n_variates + 1, -1);
+    n_sobol = 0;
+    for (int v = 0; v < n_variates; ++v)
+      if (kind[v] == OKIN_VARIATE_SOBOL_UNIFORM || kind[v] == OKIN_VARIATE_SOBOL_NORMAL) sobol_rank[v] = n_sobol++;
+  }
+
+  // The scramble of every Sobol' variate under `seed` (n_sobol <= OKIN_SOBOL_DIMS).
+  void scramble(uint64_t seed, int n_variates) {
+    sobol_dirs.assign((size_t)n_sobol * OKIN_SOBOL_BITS + 1, 0);
+    sobol_shift.assign(n_sobol + 1, 0);
+    for (int v = 0; v < n_variates; ++v) {
+      const int d = sobol_rank[v];
+      if (d < 0) continue;
+      uint64_t row[OKIN_SOBOL_BITS], V[OKIN_SOBOL_BITS];
+      okin_sobol_matrix(seed, v, row);
+      okin_sobol_directions(d, V);
+      for (int k = 0; k < OKIN_SOBOL_BITS; ++k)
+        sobol_dirs[(size_t)d * OKIN_SOBOL_BITS + k] = okin_sobol_apply(row, V[k]);
+      sobol_shift[d] = okin_sobol_scramble_word(seed, v, OKIN_SOBOL_BITS);
+    }
+  }
+};
+
 OKIN_STUDY_HD inline double okin_study_variate(const OkinStudyTables& t, uint64_t i, int v) {
   if (t.kind[v] == OKIN_VARIATE_GRID) {
     const uint64_t node = t.period ? i % t.period : i;
     const int64_t L = t.levels[v];
     const uint64_t d = t.stride[v] ? (node / t.stride[v]) % (uint64_t)L : 0;
     return (double)d / (double)(L - 1) * 2.0 - 1.0;
+  }
+  if (t.kind[v] == OKIN_VARIATE_SOBOL_UNIFORM || t.kind[v] == OKIN_VARIATE_SOBOL_NORMAL) {
+    const uint64_t j = i / t.period, g = j ^ (j >> 1);
+#if defined(__CUDA_ARCH__)
+    const int d = t.sobol_rank[v];
+    const uint64_t x = okin_sobol_gray_xor(t.sobol_dirs + (size_t)d * OKIN_SOBOL_BITS, g, t.sobol_shift[d]);
+#else
+    // M_v (XOR of V[d][k]) ^ S_v from the definition: by linearity over GF(2) the same integer as the
+    // device's XOR of the scrambled direction numbers.
+    int d = 0;
+    for (int w = 0; w < v; ++w)
+      d += t.kind[w] == OKIN_VARIATE_SOBOL_UNIFORM || t.kind[w] == OKIN_VARIATE_SOBOL_NORMAL;
+    uint64_t V[OKIN_SOBOL_BITS], row[OKIN_SOBOL_BITS];
+    okin_sobol_directions(d, V);
+    okin_sobol_matrix(t.seed, v, row);
+    const uint64_t x =
+        okin_sobol_apply(row, okin_sobol_gray_xor(V, g, 0)) ^ okin_sobol_scramble_word(t.seed, v, OKIN_SOBOL_BITS);
+#endif
+    if (t.kind[v] == OKIN_VARIATE_SOBOL_UNIFORM) return (double)x * 0x1p-51 - 1.0;
+    return okin_ppnd16((double)(2 * x + 1) * 0x1p-53);
   }
   uint32_t c[4] = {(uint32_t)i, (uint32_t)(i >> 32), (uint32_t)v, 0u};
   okin_philox4x32_10(c, (uint32_t)t.seed, (uint32_t)(t.seed >> 32));

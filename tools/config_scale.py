@@ -12,6 +12,8 @@ c4: double-wishbone axle with torsion bars, T-bar ARB, rocker-to-rocker heave li
 c5: DoE sensitivity sweep over a hardpoint grid: 1e8 instance-steps (4 761 905 instances x 21 steps of
     the flagship axle, each instance one node of a 13-level, 6-factor full factorial on +-2 mm) with
     every metric column evaluated on the device.
+``--sequence sobol`` draws c4's variates from the scrambled Sobol' sequence instead of Philox, and
+replaces c5's grid by Sobol' uniforms on the same +-2 mm box; the default ``philox`` is the above.
 
 Arms, run alternately in one call (``--arm both``):
   study   ``BatchSolver.study`` end to end (generation, sweep kernel, reduction, host fold), timed on
@@ -51,19 +53,25 @@ C5_RANGE_COLUMNS = ("roll_center_z", "camber_left", "deriv_damper_length_wrt_hub
                     "deriv_arb_twist_wrt_hub_z_left")
 
 
-def c4_sampling(solver) -> Sampling:
-    smp = Sampling(solver, mirror_right=True).normal("all", 0.25)
-    return smp.uniform([n for n in solver.program.param_names if n.endswith("setup_thickness")], 0.5)
+def c4_sampling(solver, sequence: str = "philox") -> Sampling:
+    smp = Sampling(solver, mirror_right=True).normal("all", 0.25, sequence=sequence)
+    return smp.uniform([n for n in solver.program.param_names if n.endswith("setup_thickness")], 0.5,
+                       sequence=sequence)
 
 
-def c5_sampling(solver) -> tuple:
+def c5_sampling(solver, sequence: str = "philox") -> tuple:
     """(sampling, factor coordinates): six left / centre hardpoint coordinates on a 13-level grid of
-    +-2 mm, the first factor varying fastest; right points mirror their left twins."""
+    +-2 mm, the first factor varying fastest; right points mirror their left twins.  With
+    ``sequence="sobol"`` the factors are Sobol' uniforms on the same +-2 mm box instead of the grid."""
     own, _ = bench.perturbation_mask(solver.program)
     coords = [3 * int(own[k % own.size]) + k % 3 for k in range(0, 6 * 5, 5)]
     smp = Sampling(solver, mirror_right=True)
     for c in coords:
-        smp.grid((solver.program.in_keys[c // 3], c % 3), 2.0, 13)
+        key = (solver.program.in_keys[c // 3], c % 3)
+        if sequence == "sobol":
+            smp.uniform(key, 2.0, sequence="sobol")
+        else:
+            smp.grid(key, 2.0, 13)
     return smp, coords
 
 
@@ -77,14 +85,14 @@ def case(args):
         steps = args.steps or 101
         sweep = build_sweep(axle_sweep(steps, 50.0, args.mode == "roll"), sus)
         solver = BatchSolver(sus, sweep, tune_layout=True)
-        return (solver, c4_sampling(solver), args.instances or 10_000_000,
+        return (solver, c4_sampling(solver, args.sequence), args.instances or 10_000_000,
                 f"c4_tbar_heave_shim_{args.mode}{steps}_montecarlo", dict(points="all", solver_quantities=(
                     "solver_nfev",)))
     meta, _ = load_golden("c3_rocker_ubar_coilover_roll")
     sus, sweep = build_case(meta)
     solver = BatchSolver(sus, sweep, tune_layout=True)
     total = args.instances or -(-100_000_000 // sweep.n_steps)      # 1e8 instance-steps
-    return (solver, c5_sampling(solver)[0], total, "c5_doe_grid_c3_axle_roll21_all_metrics",
+    return (solver, c5_sampling(solver, args.sequence)[0], total, "c5_doe_grid_c3_axle_roll21_all_metrics",
             dict(metrics="all", solver_quantities=("solver_nfev",)))
 
 
@@ -195,6 +203,9 @@ def main() -> None:
     ap.add_argument("--repeats", type=int, default=1)
     ap.add_argument("--devices", default="0", help="comma-separated device ids of the study arm")
     ap.add_argument("--seed", type=int, default=1234)
+    ap.add_argument("--sequence", default="philox", choices=["philox", "sobol"],
+                    help="c4: the sequence of its normal / uniform variates; c5: sobol replaces the 13-level "
+                         "grid by Sobol' uniforms on the same box")
     ap.add_argument("--memory", action="store_true", help="sample device memory during the study arm")
     ap.add_argument("--profile", action="store_true", help="kernel-time split of one study run")
     args = ap.parse_args()
@@ -209,7 +220,7 @@ def main() -> None:
     base = {"config": label, "instances_total": total, "sweep_steps": int(solver.values.shape[1]),
             "instance_steps_total": total * int(solver.values.shape[1]), "devices": devices,
             "n_metric_columns": len(solver.program.metric_names) if kw.get("metrics") else 0,
-            "n_unknowns": solver.program.n_unknowns}
+            "n_unknowns": solver.program.n_unknowns, "sequence": args.sequence}
     for rep in range(args.repeats):
         for arm in arms:
             if arm == "study":
